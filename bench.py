@@ -2,7 +2,7 @@
 """bench.py -- particle-updates/s of one EKS (ALDI) step on B200, the headline metric of BASELINE.json.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload target|cfg3|cfg1|cfg2|cfg4|small]
-                    [--impl reference] [--no-configs] [--no-parity] [--no-cpu-baseline]
+                    [--impl reference] [--no-configs] [--no-parity] [--no-cpu-baseline] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one ensemble Kalman update (sampling.eks_update_aldi,
 ces/calibrate.py:451-490) of the synthetic linear-Gaussian ensemble of SURVEY.md section 8(d).
@@ -28,6 +28,9 @@ ces/calibrate.py:451-490) of the synthetic linear-Gaussian ensemble of SURVEY.md
              the numpy port (oracle/, kind "port") only if the staged files are absent.
   --impl reference  times only that CPU arm: K steps of the real sampling.eks_update_aldi at J_sample (named in
              config), all host threads (torchrun's OMP_NUM_THREADS=1 is overridden), rank 0 only.
+  --dump-outputs DIR  after the timed steps of the selected workload, what its last step returned to the caller as
+             DIR/<name>.npy (float64, at most 64 MB in all; see dump_outputs), rank 0's column shard when N > 1.  The
+             inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import os
 import sys
@@ -80,7 +83,14 @@ def parse():
     ap.add_argument("--formulation", default="interaction", choices=["interaction", "factored"],
                     help="'interaction' forms the J x J matrix D like the reference (the graded formulation, default); "
                          "'factored' is the opt-in algorithmically reduced path (same update to rounding, D never formed)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (GPU arm only)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm; --impl reference has none")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------ flop models
@@ -424,6 +434,37 @@ def emit(line):
         sys.stdout.flush()
 
 
+DUMP_BYTES = 64 * 10 ** 6       # --dump-outputs: array data written in all
+
+
+def dump_outputs(path, arrays):
+    """Write ``arrays`` (name -> CUDA tensor, numpy array or number) as ``path/<name>.npy`` in float64, numbers as
+    one-element arrays.  When they would exceed DUMP_BYTES, every (rows, particles) array keeps the same sorted sample of
+    particle columns, drawn with a fixed seed, so that two runs are compared column for column."""
+    import torch
+
+    def host(a):
+        return np.atleast_1d(a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)).astype(np.float64)
+
+    wide = [n for n, a in arrays.items() if getattr(a, "ndim", 0) == 2]
+    rest = {n: host(a) for n, a in arrays.items() if n not in wide}
+    cols = {arrays[n].shape[1] for n in wide}
+    assert len(cols) <= 1, "the (rows, particles) outputs must share one particle axis"
+    rows = sum(arrays[n].shape[0] for n in wide)
+    room = DUMP_BYTES - sum(a.nbytes for a in rest.values()) - 128 * len(arrays)     # 128: .npy header
+    idx = None
+    if wide and 8 * rows * max(cols) > room:
+        idx = np.sort(np.random.default_rng(0).choice(max(cols), size=room // (8 * rows), replace=False))
+    os.makedirs(path, exist_ok=True)
+    for n in wide:
+        a = arrays[n]
+        if idx is not None:
+            a = a[:, torch.as_tensor(idx, device=a.device)] if torch.is_tensor(a) else np.asarray(a)[:, idx]
+        np.save(os.path.join(path, n + ".npy"), host(a))
+    for n, a in rest.items():
+        np.save(os.path.join(path, n + ".npy"), a)
+
+
 class Ctx(object):
     """Device, ranks and the timing protocol shared by every workload of the GPU arm."""
 
@@ -564,8 +605,10 @@ def parity_probe(ctx, d, k, J, y, ustar_h, U, G, xi, out, hk, ncols=128):
     return res
 
 
-def update_workload(ctx, name, steps, warmup, formulation="interaction", with_cpu=True, with_parity=True, publish=False):
-    """The headline measurement on one linear-Gaussian shape; returns the JSON record on rank 0 (None elsewhere)."""
+def update_workload(ctx, name, steps, warmup, formulation="interaction", with_cpu=True, with_parity=True, publish=False,
+                    dump=None):
+    """The headline measurement on one linear-Gaussian shape; returns the JSON record on rank 0 (None elsewhere).
+    ``dump``: directory for dump_outputs of the last timed step."""
     torch, dist, world, rank, dev = ctx.torch, ctx.dist, ctx.world, ctx.rank, ctx.dev
     from ces_b200 import calibrate
     from ces_b200.engine import Engine, shard_range
@@ -596,10 +639,10 @@ def update_workload(ctx, name, steps, warmup, formulation="interaction", with_cp
         s.group = ctx.group
     eng = s._get_engine(J, ctx.group)
     s._sync_problem(eng, y_h, Gamma)
-    hk_box = [0.0]
+    last = [None]       # (U_next, hk, metrics) of the latest step
 
     def step_dev():
-        hk_box[0] = eng.step("aldi", U, G, xi, out=out, formulation=formulation)[1]
+        last[0] = eng.step("aldi", U, G, xi, out=out, formulation=formulation)
 
     warmup = max(warmup, 3)
     for _ in range(warmup):
@@ -620,10 +663,13 @@ def update_workload(ctx, name, steps, warmup, formulation="interaction", with_cp
     clocks = sampler.stop(t0, t1) if rank == 0 else None
     ms_per_step = ms / steps
     value = J / (ms_per_step * 1e-3)
+    hk = last[0][1]
+    if dump is not None and rank == 0:
+        dump_outputs(dump, dict(last[0][2], U_next=last[0][0], hk=hk))
 
     parity = None
     if with_parity and formulation == "interaction":
-        parity = parity_probe(ctx, d, k, J, y, ustar_h, U, G, xi, out, hk_box[0])
+        parity = parity_probe(ctx, d, k, J, y, ustar_h, U, G, xi, out, hk)
 
     if publish and rank == 0:
         PARTIAL["line"] = {"metric": METRIC, "value": value, "unit": "particle-updates/s", "n_gpus": world, "steps": steps,
@@ -689,8 +735,9 @@ def update_workload(ctx, name, steps, warmup, formulation="interaction", with_cp
     return line
 
 
-def darcy_workload(ctx, name, steps, warmup, with_cpu=True):
-    """cfg2 | cfg4: one ensemble Kalman iteration = batched Darcy forward solve of every member + update."""
+def darcy_workload(ctx, name, steps, warmup, with_cpu=True, dump=None):
+    """cfg2 | cfg4: one ensemble Kalman iteration = batched Darcy forward solve of every member + update.
+    ``dump``: directory for dump_outputs of the last timed step."""
     torch, dist, world, rank, dev = ctx.torch, ctx.dist, ctx.world, ctx.rank, ctx.dev
     from ces_b200 import calibrate
     from ces_b200 import darcy as cdarcy
@@ -714,6 +761,7 @@ def darcy_workload(ctx, name, steps, warmup, with_cpu=True):
     G = torch.empty(n_obs, hi - lo, dtype=torch.float64, device=dev)
     out = torch.empty_like(U)
     stats = {"iters": 0, "members": 0, "ms": 0.0}
+    last = [None]       # (U_next, hk, metrics) of the latest step
 
     def step_dev():
         model.evaluate_ensemble(eng, U, G)
@@ -721,7 +769,7 @@ def darcy_workload(ctx, name, steps, warmup, with_cpu=True):
         stats["iters"] += it_
         stats["members"] += m_
         stats["ms"] += ms_
-        eng.step(rule, U, G, None if rule == "eki" else xi, out=out)
+        last[0] = eng.step(rule, U, G, None if rule == "eki" else xi, out=out)
 
     warmup = max(warmup, 3)
     for _ in range(warmup):
@@ -738,6 +786,8 @@ def darcy_workload(ctx, name, steps, warmup, with_cpu=True):
     launches = eng.launch_count() - n0
     clocks = sampler.stop(t0, t1) if rank == 0 else None
     ms_per_step = ms / steps
+    if dump is not None and rank == 0:
+        dump_outputs(dump, dict(last[0][2], G=G, U_next=last[0][0], hk=last[0][1]))
     eng.close()
 
     # ---- end to end: sampling.run for ONE iteration from host arrays (H2D of U0, forward, update, the final forward
@@ -804,11 +854,12 @@ def darcy_workload(ctx, name, steps, warmup, with_cpu=True):
     return line
 
 
-def cfg1_workload(ctx, repeats=3, with_cpu=True):
+def cfg1_workload(ctx, repeats=3, with_cpu=True, dump=None):
     """BASELINE.json configs[0] through the reference-facing loop: sampling.run(T=1000) on the linear.ipynb problem
     (lineal, d=2, k=10, J=100), host arrays in, Uall / Gall / Ustar / metrics out -- exactly what ces/calibrate.py:270-416
     does in 1.1-1.3 s (BASELINE.md section 2).  Single GPU (J = 100 does not shard); value == e2e: the whole run is the
-    public call, timed by CUDA events around it and by the wall clock."""
+    public call, timed by CUDA events around it and by the wall clock.  ``dump``: directory for dump_outputs of the
+    last run."""
     torch = ctx.torch
     from ces_b200 import calibrate, utils
 
@@ -833,6 +884,8 @@ def cfg1_workload(ctx, repeats=3, with_cpu=True):
             launches = s._engine.launch_count() - n0
         steps = len(s.metrics["t"])
         post_mean = s.Ustar.mean(axis=1).tolist()
+        if dump is not None and i == repeats:
+            dump_outputs(dump, dict(s.metrics, Uall=s.Uall, Gall=s.Gall, Ustar=s.Ustar, Gstar=s.Gstar))
         s._engine.close()
         s._engine = None
     value = pr["J"] * steps / (best_ms * 1e-3)
@@ -881,11 +934,11 @@ def main():
     ctx = Ctx()
     cpu = not args.no_cpu_baseline
     if args.workload in DARCY_WORKLOADS:
-        line = darcy_workload(ctx, args.workload, args.steps, args.warmup, with_cpu=cpu)
+        line = darcy_workload(ctx, args.workload, args.steps, args.warmup, with_cpu=cpu, dump=args.dump_outputs)
     elif args.workload == "cfg1":
         line = None
         if ctx.rank == 0:
-            rec = cfg1_workload(ctx, with_cpu=cpu)
+            rec = cfg1_workload(ctx, with_cpu=cpu, dump=args.dump_outputs)
             line = {"metric": rec["metric"], "value": rec["value"], "unit": rec["unit"], "n_gpus": ctx.world, "steps": rec["steps"],
                     "warmup": 1, "ms_per_step": rec["ms_per_step"], "higher_is_better": True, "scaling": "strong",
                     "vs_baseline": None, "dtype": "f64", "data": "synthetic"}
@@ -894,7 +947,7 @@ def main():
         ctx.barrier()
     else:
         line = update_workload(ctx, args.workload, args.steps, args.warmup, args.formulation, with_cpu=cpu,
-                               with_parity=not args.no_parity, publish=True)
+                               with_parity=not args.no_parity, publish=True, dump=args.dump_outputs)
         if args.workload == "target" and args.formulation == "interaction" and not args.no_configs:
             # the other BASELINE.json configs, short runs in the same process (cfg1 / cfg2 are single-GPU shapes)
             configs = []

@@ -44,6 +44,24 @@ def test_gpu_arm_line():
     assert p["ok"] is True and p["hk_rel"] <= 1e-10 and p["probe_rel"] <= 1e-10 and p["tol"] == 1e-10
 
 
+def test_dump_outputs_are_the_timed_step_and_repeat(tmp_path):
+    """--dump-outputs writes what the last timed step returned (U_next, hk, the four metrics) in float64; the seeded
+    inputs make a second run with the same arguments write the same outputs."""
+    import numpy as np
+
+    runs = []
+    for name in ("a", "b"):
+        d = _run("--steps", "2", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / name))
+        assert d["steps"] == 2
+        runs.append({f[:-4]: np.load(str(tmp_path / name / f)) for f in os.listdir(str(tmp_path / name))})
+    a, b = runs
+    assert sorted(a) == ["U_next", "bias", "bias-data", "hk", "self-bias", "self-bias-data"]
+    assert a["U_next"].shape == (64, 1024) and a["hk"].shape == (1,) and all(v.dtype == np.float64 for v in a.values())
+    assert np.isfinite(a["U_next"]).all() and a["hk"][0] > 0
+    for key in a:
+        assert np.abs(a[key] - b[key]).max() <= 1e-12 * np.abs(a[key]).max(), key
+
+
 def test_reference_arm_line():
     d = _run("--impl", "reference")
     for key in REQUIRED + ("impl", "cpu_baseline"):

@@ -178,6 +178,43 @@ def test_reference_arm_of_bench_runs_on_the_host(tmp_path):
     assert d["steps"] == 2 and d["warmup"] == 0 and d["gpu_launches"] == 0
 
 
+def test_bench_dump_outputs_keeps_one_seeded_column_sample_within_the_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 files, numbers as one-element arrays, and when the outputs exceed the budget the
+    same seeded particle columns of every (rows, particles) array, identical from call to call."""
+    import importlib.util
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_module", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 200000)
+    rng = np.random.default_rng(3)
+    U, G = rng.standard_normal((24, 1000)), rng.standard_normal((7, 1000)).astype(np.float32)
+    for name in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / name), {"U_next": U, "G": G, "hk": 0.25, "t": [0.5, 0.75]})
+    files = sorted(os.listdir(str(tmp_path / "a")))
+    assert files == ["G.npy", "U_next.npy", "hk.npy", "t.npy"]
+    assert sum(os.path.getsize(str(tmp_path / "a" / f)) for f in files) <= 200000
+    a = {f[:-4]: np.load(str(tmp_path / "a" / f)) for f in files}
+    assert all(v.dtype == np.float64 for v in a.values()) and a["hk"].tolist() == [0.25] and a["t"].tolist() == [0.5, 0.75]
+    ncols = a["U_next"].shape[1]
+    assert 0 < ncols < 1000 and a["G"].shape == (7, ncols)
+    cols = [int(np.flatnonzero((U == a["U_next"][:, j][:, None]).all(axis=0))[0]) for j in range(ncols)]
+    assert cols == sorted(set(cols)) and np.array_equal(a["G"], G[:, cols].astype(np.float64))
+    for f in files:
+        assert np.array_equal(a[f[:-4]], np.load(str(tmp_path / "b" / f)))
+
+
+def test_bench_rejects_a_step_count_below_one():
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                         timeout=120, cwd=root)
+    assert out.returncode == 2 and "--steps" in out.stderr and out.stdout == ""
+
+
 def test_bench_flop_models_agree_with_the_oracle():
     """bench.py carries its own copies of the flop models (the GPU arm must not import oracle/ for them): W_step of SURVEY.md
     section 8(d) and the reference-as-written model of BASELINE.md section 3 stay identical to the oracle's."""
