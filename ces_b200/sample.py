@@ -13,6 +13,11 @@ The forward model must be one of the device maps of ``ces_b200.utils`` (``lineal
 ``banana``) with p <= 32, k <= 64.  ``gp_mh`` (Metropolis-Hastings on a GPflow emulator, ces/sample.py:17-119) is not
 provided: it needs trained GPflow models (``emulate.predict_gps``, ces/emulate.py:17-79), a third-party library that is
 absent here and whose predictions could not be pinned; that half of SURVEY.md section 8f-4 stays out of scope.
+
+``emulator_mh`` (new) is the same sampler on an emulator of the forward model: a ``ces_b200.emulate.GPEmulator`` (exact
+GPs on the device, trained on the calibrated ensemble) replaces the model, and the misfit becomes the emulated one in
+whitened coordinates (see ces_b200/emulate.py).  Proposals, prior term, accept test, resume behaviour and the random
+numbers are ``model_mh``'s.
 """
 from __future__ import print_function
 
@@ -107,6 +112,62 @@ class MCMC(object):
         self.accept = accepted[0] / float(n_mcmc)            # :196
         if n_chains > 1:
             self.samples_chains = samples.transpose(0, 2, 1)     # (n_chains, p, n + 1)
+            self.accept_chains = accepted / float(n_mcmc)
+
+    def emulator_mh(self, emulator, n_mcmc, prior, enka, delta=1., enka_scaling=True, update=None, beta=0.5, n_chains=1,
+                    seed=0, use_variance=True):
+        """``model_mh`` through a ``GPEmulator``: Phi(u) = 1/2 sum_i (ytil_i - mean_i(u))^2 / (1 + var_i(u))
+        + 1/2 sum_i log(1 + var_i(u)) (without the variance terms when ``use_variance`` is False), ytil = T y_obs,
+        plus -prior.logpdf(u) unless pCN.  Chains run on the device (csrc/emulate.cu); results as ``model_mh``."""
+        p, k = int(emulator.p), int(emulator.k)
+        if update not in (None, 'pCN'):
+            raise ValueError("unknown update %r" % (update,))
+        pcn = update == 'pCN'
+        if enka_scaling:
+            scales = delta * np.linalg.cholesky(np.cov(enka.Ustar).reshape(p, p))
+        else:
+            scales = delta * np.eye(p)
+        if pcn:
+            scales = np.linalg.cholesky(np.asarray(prior.cov, dtype=np.float64).reshape(p, p))
+        mean = np.asarray(enka.Ustar, dtype=np.float64).mean(axis=1)
+        ytil = np.ascontiguousarray(emulator.transform @ np.asarray(self.y_obs, dtype=np.float64).reshape(k))
+        mu = Pinv = None
+        if not pcn:
+            mu = np.ascontiguousarray(np.asarray(prior.mean, dtype=np.float64).reshape(p))
+            Pinv = np.ascontiguousarray(np.linalg.inv(np.asarray(prior.cov, dtype=np.float64).reshape(p, p)))
+        previous = None
+        if hasattr(self, 'samples'):
+            previous = np.asarray(self.samples, dtype=np.float64)
+            first = previous[:, -1].copy()
+        else:
+            first = mean.copy()
+        n_chains = int(n_chains)
+        start = np.tile(first, (n_chains, 1))
+        if n_chains > 1:
+            J = enka.Ustar.shape[1]
+            start[1:] = np.asarray(enka.Ustar, dtype=np.float64).T[np.arange(1, n_chains) % J]
+        phi_point = np.tile(mean, (n_chains, 1))
+        phi_point[1:] = start[1:]
+        st = np.random.get_state()
+        mt = np.empty(626, dtype=np.uint32)
+        mt[:624], mt[624], mt[625] = st[1], st[2], st[3]
+        gauss = np.array([st[4]], dtype=np.float64)
+        samples = np.empty((n_chains, int(n_mcmc) + 1, p))
+        accepted = np.zeros(n_chains, dtype=np.int32)
+        emulator.condition()
+        _lib.check(_lib.load().ces_gp_mh(
+            emulator._h, _lib.host_ptr(ytil), 1 if use_variance else 0, _lib.host_ptr(mu) if mu is not None else None,
+            _lib.host_ptr(Pinv) if Pinv is not None else None, _lib.host_ptr(np.ascontiguousarray(scales, dtype=np.float64)),
+            1 if pcn else 0, float(beta), int(n_mcmc), n_chains, _lib.host_ptr(start), _lib.host_ptr(phi_point),
+            mt.ctypes.data, _lib.host_ptr(gauss), int(seed), _lib.host_ptr(samples), accepted.ctypes.data))
+        np.random.set_state(('MT19937', mt[:624].copy(), int(mt[624]), int(mt[625]), float(gauss[0])))
+        chain0 = samples[0]
+        if previous is not None:
+            chain0 = np.vstack([previous.T, samples[0][1:]])
+        self.samples = np.array(chain0).T
+        self.accept = accepted[0] / float(n_mcmc)
+        if n_chains > 1:
+            self.samples_chains = samples.transpose(0, 2, 1)
             self.accept_chains = accepted / float(n_mcmc)
 
     def random_walk(self, current, scales, n_dim):

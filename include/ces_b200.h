@@ -309,6 +309,37 @@ int ces_mcmc_model_mh(void* stream, int map_kind, int64_t p, int64_t k, const do
                       uint32_t* mt_state_host, double* mt_gauss_host, uint64_t seed, double* samples_host,
                       int32_t* accepted_host);
 
+/* ---- Emulate: exact GP emulators of the whitened forward map and MH chains through them (csrc/emulate.cu) ----------
+ * One GP per whitened output i < k on the training inputs X (p x n, row-major, one point per column) and outputs
+ * Y = T G - ybar (k x n; T = diag(lam^-1/2) Q^T from Gamma = Q diag(lam) Q^T, ybar the row means), all fixed by the caller.
+ * theta_i = [log sf2, log l_1..l_p, log sn2];  k(x, z) = sf2 exp(-1/2 sum_d (x_d - z_d)^2 / l_d^2);
+ * K = k(X, X) + (sn2 + jitter) I;  L = chol(K);  alpha = K^-1 y_i.  Limits: 1 <= p <= 32, 1 <= k <= 64, n >= 2 (n is
+ * otherwise bounded by device memory: CES_ERR_NOMEM).  A K that is not positive definite returns CES_ERR_NOT_SPD.
+ * ces_gp_create copies X, Y, ybar to the device on `stream`; every later call runs on that stream. */
+int ces_gp_create(void* stream, int64_t p, int64_t k, int64_t n, const double* X_host, const double* Y_host,
+                  const double* ybar_host, void** out);
+int ces_gp_destroy(void* model);
+/* LML_i = -1/2 y_i^T alpha - sum_j log L_jj - n/2 log 2 pi for outputs i0 <= i < i1 (theta_host: (i1 - i0) x (p + 2)) and,
+ * with grad_host != NULL, dLML_i/dtheta_i = 1/2 sum_ab (alpha alpha^T - K^-1)_ab dK_ab/dtheta ((i1 - i0) x (p + 2)).
+ * Fixed-order reductions: repeated calls return bit-identical results.  Synchronises. */
+int ces_gp_lml(void* model, int64_t i0, int64_t i1, const double* theta_host, double jitter, double* lml_host,
+               double* grad_host);
+/* Conditions every output on theta_host (k x (p + 2)): keeps L_i^-1 and alpha_i for ces_gp_predict / ces_gp_mh. */
+int ces_gp_condition(void* model, const double* theta_host, double jitter);
+/* Latent-f prediction at the m points U (p x m on the device, ld ldu):  mean_i(u) = ybar_i + k_i(u)^T alpha_i,
+ * var_i(u) = max(sf2_i - ||L_i^-1 k_i(u)||^2, 0), into mean / var (k x m on the device).  Asynchronous on the stream. */
+int ces_gp_predict(void* model, const double* U_dev, int64_t ldu, int64_t m, double* mean_dev, int64_t ldm,
+                   double* var_dev, int64_t ldv);
+/* MCMC.emulator_mh: ces_mcmc_model_mh's chains (proposal, prior term, accept test, random numbers, outputs; arguments from
+ * mu_host onwards as there) with the forward misfit replaced by the emulated one at the whitened data ytil_host (k):
+ *   Phi(u) = 1/2 sum_i (ytil_i - mean_i(u))^2 / (1 + var_i(u)) + 1/2 sum_i log(1 + var_i(u))   (use_variance != 0)
+ *   Phi(u) = 1/2 sum_i (ytil_i - mean_i(u))^2                                                  (use_variance == 0)
+ * Needs ces_gp_condition.  Synchronises. */
+int ces_gp_mh(void* model, const double* ytil_host, int use_variance, const double* mu_host, const double* Pinv_host,
+              const double* scales_host, int pcn, double beta, int64_t n_mcmc, int64_t n_chains, const double* start_host,
+              const double* phi_point_host, uint32_t* mt_state_host, double* mt_gauss_host, uint64_t seed,
+              double* samples_host, int32_t* accepted_host);
+
 #ifdef __cplusplus
 }
 #endif
