@@ -30,7 +30,7 @@ EXPORTS = (
     "ces_timeline_mark", "ces_timeline_read", "ces_host_begin", "ces_host_sums_g", "ces_host_centre_g", "ces_host_sums_u",
     "ces_host_centre_u", "ces_host_interact_own", "ces_host_update", "ces_ipc_export", "ces_ipc_import", "ces_peer_gather",
     "ces_peer_gather_wait", "ces_host_interact_chunk", "ces_small_run", "ces_mcmc_model_mh", "ces_host_chunk_schedule",
-    "ces_gp_create", "ces_gp_destroy", "ces_gp_lml", "ces_gp_condition", "ces_gp_predict", "ces_gp_mh",
+    "ces_gp_create", "ces_gp_destroy", "ces_gp_lml", "ces_gp_condition", "ces_gp_predict", "ces_gp_mh", "ces_darcy_mh",
 )
 
 _i64, _int, _dbl, _vp = ctypes.c_int64, ctypes.c_int, ctypes.c_double, ctypes.c_void_p
@@ -106,6 +106,8 @@ def load():
     lib.ces_gp_predict.argtypes = [_vp, _dp, _i64, _i64, _dp, _i64, _dp, _i64]
     lib.ces_gp_mh.argtypes = [_vp, _dp, _int, _dp, _dp, _dp, _int, _dbl, _i64, _i64, _dp, _dp, _dp, _dp, ctypes.c_uint64,
                               _dp, _dp]
+    lib.ces_darcy_mh.argtypes = [_vp, _dbl, _int, _dp, _dp, _dp, _dp, _dp, _int, _dbl, _i64, _i64, _dp, _dp, _dp, _dp,
+                                 ctypes.c_uint64, _dp, _dp]
     lib.ces_host_chunk_schedule.argtypes = [_i64, _i64, _i64, _int, _dbl, ctypes.POINTER(_i64)]
     lib.ces_forward_map.argtypes = [_vp, _int, _dp, _i64, _dp, _dp, _dp, _i64, _dp, _i64]
     lib.ces_buffer.argtypes = [_vp, ctypes.c_char_p, ctypes.POINTER(_vp), ctypes.POINTER(_i64),

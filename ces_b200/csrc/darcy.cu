@@ -851,17 +851,23 @@ int ces_darcy_destroy(void* handle) {
     return CES_OK;
 }
 
-int ces_darcy_forward(void* handle, const double* U, int64_t ldu, int64_t cols, double* G, int64_t ldg, int full_solution,
-                      double tol, int max_iter, int* iters_host) {
-    DarcyModel* m = static_cast<DarcyModel*>(handle);
-    if (!m || !U || !G || cols < 0 || ldu < cols || ldg < cols) return fail(CES_ERR_INVALID, "ces_darcy_forward: bad argument%s", "");
-    if (!full_solution && m->n_obs == 0) return fail(CES_ERR_STATE, "ces_darcy_forward: no obs_index was given%s", "");
+}  // extern "C"
+
+namespace ces {
+
+int darcy_max_iter(const DarcyModel* m, int max_iter) { return max_iter > 0 ? max_iter : 40 * m->N; }
+
+DarcyShape darcy_shape(const DarcyModel* m) { return DarcyShape{m->N, m->p, m->n_obs, m->st, m->iters}; }
+
+// The pipeline of ces_darcy_forward without its final synchronisation; the chains of darcy_mh.cu call it once per step.
+int darcy_forward_async(DarcyModel* m, const double* U, int64_t ldu, int64_t cols, double* G, int64_t ldg, int full_solution,
+                        double tol, int max_iter) {
     if (cols == 0) return CES_OK;
     const int N = m->N, p = m->p, ldn = m->ldn;
     const int64_t cells = (int64_t)N * ldn;        // doubles per stored field
     cudaStream_t st = m->st;
     if (tol <= 0.0) tol = 1e-13;
-    if (max_iter <= 0) max_iter = 40 * N;
+    max_iter = darcy_max_iter(m, max_iter);
     const int64_t chunk = cols < m->chunk ? cols : m->chunk;
     if (!m->B0) {
         const size_t bytes = (size_t)m->chunk * cells * sizeof(double);
@@ -935,6 +941,22 @@ int ces_darcy_forward(void* handle, const double* U, int64_t ldu, int64_t cols, 
         darcy_gather_kernel<<<grid, 256, 0, st>>>(m->B2, cells, (int)mc, full_solution ? nullptr : m->obs, rows, G + c0, ldg, N, ldn);
         CES_LAUNCHED(1);
     }
+    return CES_OK;
+}
+
+}  // namespace ces
+
+extern "C" {
+
+int ces_darcy_forward(void* handle, const double* U, int64_t ldu, int64_t cols, double* G, int64_t ldg, int full_solution,
+                      double tol, int max_iter, int* iters_host) {
+    DarcyModel* m = static_cast<DarcyModel*>(handle);
+    if (!m || !U || !G || cols < 0 || ldu < cols || ldg < cols) return fail(CES_ERR_INVALID, "ces_darcy_forward: bad argument%s", "");
+    if (!full_solution && m->n_obs == 0) return fail(CES_ERR_STATE, "ces_darcy_forward: no obs_index was given%s", "");
+    if (cols == 0) return CES_OK;
+    CES_TRY(darcy_forward_async(m, U, ldu, cols, G, ldg, full_solution, tol, max_iter));
+    max_iter = darcy_max_iter(m, max_iter);
+    cudaStream_t st = m->st;
     int iters = 0;
     CES_CUDA(cudaMemcpyAsync(&iters, m->iters, sizeof(int), cudaMemcpyDeviceToHost, st));
     CES_CUDA(cudaStreamSynchronize(st));

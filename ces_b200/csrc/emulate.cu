@@ -264,30 +264,8 @@ __global__ void __launch_bounds__(GP_PROPOSE_THREADS) gp_propose_kernel(const Gp
     __syncthreads();
     const int c = blockIdx.x * blockDim.x + threadIdx.x, tid = threadIdx.x;
     if (c >= a.n_chains) return;
-    double u;
-    if (a.use_mt && c == 0) {
-        Mt rng;
-        rng.key = a.mt; rng.pos = (int)a.mt[624]; rng.has_gauss = (int)a.mt[625]; rng.gauss = a.mt_gauss[0];
-        for (int q = 0; q < p; ++q) zs[q][tid] = mt_gauss(rng);
-        u = mt_double(rng);
-        a.mt[624] = (uint32_t)rng.pos; a.mt[625] = (uint32_t)rng.has_gauss; a.mt_gauss[0] = rng.gauss;
-    } else {
-        const uint32_t k0 = (uint32_t)a.seed, k1 = (uint32_t)(a.seed >> 32);
-        for (int q2 = 0; 2 * q2 < p; ++q2) {                         // Box-Muller pairs (2 q2, 2 q2 + 1)
-            uint32_t ctr[4] = {(uint32_t)it, (uint32_t)c, (uint32_t)q2, 0x4750u};
-            philox4(ctr, k0, k1);
-            const double u1 = u53(ctr[0], ctr[1]), u2 = u53(ctr[2], ctr[3]);
-            const double rad = sqrt(-2.0 * log(u1));
-            double sn, cs;
-            sincospi(2.0 * u2, &sn, &cs);
-            zs[2 * q2][tid] = rad * cs;
-            if (2 * q2 + 1 < p) zs[2 * q2 + 1][tid] = rad * sn;
-        }
-        uint32_t ctr[4] = {(uint32_t)it, (uint32_t)c, 0xffffffffu, 0x4750u};
-        philox4(ctr, k0, k1);
-        u = u53(ctr[0], ctr[1]);
-    }
-    a.u[c] = u;
+    a.u[c] = mh_chain_draw(p, it, c, (a.use_mt && c == 0) ? a.mt : nullptr, a.mt_gauss, a.seed, 0x4750u, &zs[0][tid],
+                           GP_PROPOSE_THREADS);
     const double a_cur = a.pcn ? sqrt(1.0 - a.beta * a.beta) : 1.0, a_z = a.pcn ? sqrt(a.beta) : 1.0;
     for (int q = 0; q < p; ++q) {
         double s = 0.0;

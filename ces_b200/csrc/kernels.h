@@ -133,6 +133,20 @@ struct SmallRunCall {
 };
 int small_run(cudaStream_t st, const SmallStepCall& c, const SmallRunCall& rc);
 
+// darcy.cu -- the body of ces_darcy_forward without its final synchronisation (valid arguments assumed): enqueues the
+// pipeline for U (p x cols) -> G on the model's stream and leaves the largest / summed CG iteration count of the call in
+// the device ints `iters` of darcy_shape.  darcy_max_iter resolves the iteration limit (<= 0: the default, 40 N).
+struct DarcyModel;
+struct DarcyShape {
+    int N, p, n_obs;
+    cudaStream_t st;
+    const int* iters;
+};
+int darcy_forward_async(DarcyModel* m, const double* U, int64_t ldu, int64_t cols, double* G, int64_t ldg, int full_solution,
+                        double tol, int max_iter);
+int darcy_max_iter(const DarcyModel* m, int max_iter);
+DarcyShape darcy_shape(const DarcyModel* m);
+
 // forward.cu
 int exp_map(cudaStream_t st, const double* X, int64_t ldx, int64_t rows, int64_t cols, double* out, int64_t ldo);
 int elliptic_map(cudaStream_t st, const double* U, int64_t ldu, int64_t cols, double x1, double x2, double* G, int64_t ldg);

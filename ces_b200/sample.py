@@ -10,7 +10,10 @@ by ``np.random.uniform()`` would, and leaves the generator where the reference's
 ``accept_chains``.
 
 The forward model must be one of the device maps of ``ces_b200.utils`` (``lineal``, ``lineal_log``, ``elliptic``,
-``banana``) with p <= 32, k <= 64.  ``gp_mh`` (Metropolis-Hastings on a GPflow emulator, ces/sample.py:17-119) is not
+``banana``) with p <= 32, k <= 64, or a Darcy model of ``ces_b200.darcy`` (``model``, ``model_trunc``) with an
+``obs_index``: then all chains step in lockstep (``ces_darcy_mh``, csrc/darcy_mh.cu), every step solving each chain's
+proposal in one batched Darcy call with the model's ``tol`` / ``max_iter``, and a solve that does not converge makes the
+call fail (numpy's generator and ``samples`` untouched) instead of a chain continuing on it.  ``gp_mh`` (Metropolis-Hastings on a GPflow emulator, ces/sample.py:17-119) is not
 provided: it needs trained GPflow models (``emulate.predict_gps``, ces/emulate.py:17-79), a third-party library that is
 absent here and whose predictions could not be pinned; that half of SURVEY.md section 8f-4 stays out of scope.
 
@@ -46,10 +49,18 @@ class MCMC(object):
         if not torch.cuda.is_available():
             raise RuntimeError("ces_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         kind = getattr(model, 'device_kind', None)
-        if getattr(model, 'type', None) != 'map' or kind not in _lib.MAPS or getattr(model, 'flag_noise', False):
+        darcy = kind == 'darcy'
+        if getattr(model, 'type', None) != 'map' or (kind not in _lib.MAPS and not darcy) or getattr(model, 'flag_noise', False):
             raise NotImplementedError("model_mh on the device covers the ces_b200.utils maps (lineal, lineal_log, elliptic, "
-                                      "banana) without in-model noise; got %r" % (model,))
+                                      "banana) and the ces_b200.darcy models without in-model noise; got %r" % (model,))
         p, k = int(enka.p), int(enka.n_obs)
+        if darcy:
+            obs = getattr(model, 'obs_index', None)
+            if obs is None or np.size(obs) == 0:
+                raise ValueError("model_mh on a Darcy model needs model.obs_index: the cells whose pressure is observed")
+            if int(model.p) != p or np.size(obs) != k:
+                raise ValueError("model_mh: the Darcy model has p = %d and %d observed cells, the ensemble p = %d and n_obs = %d"
+                                 % (int(model.p), np.size(obs), p, k))
         pcn = kwargs.get('update', None) == 'pCN'
         if kwargs.get('update', None) not in (None, 'pCN'):
             raise ValueError("unknown update %r" % (kwargs.get('update'),))     # the reference would fail on `proposal`
@@ -91,18 +102,24 @@ class MCMC(object):
         gauss = np.array([st[4]], dtype=np.float64)
         samples = np.empty((n_chains, int(n_mcmc) + 1, p))
         accepted = np.zeros(n_chains, dtype=np.int32)
-        A_dev, lda, b_dev, params = model._device_args(torch)
-        par = np.ascontiguousarray(params, dtype=np.float64) if params is not None else None
-        stream = torch.cuda.current_stream().cuda_stream
-        _lib.check(_lib.load().ces_mcmc_model_mh(
-            ctypes.c_void_p(stream), _lib.MAPS[kind], p, k,
-            ctypes.c_void_p(A_dev.data_ptr()) if A_dev is not None else None, int(lda),
-            ctypes.c_void_p(b_dev.data_ptr()) if b_dev is not None else None,
-            _lib.host_ptr(par) if par is not None else None, _lib.host_ptr(y), _lib.host_ptr(Ginv2),
-            _lib.host_ptr(mu) if mu is not None else None, _lib.host_ptr(Pinv) if Pinv is not None else None,
-            _lib.host_ptr(np.ascontiguousarray(scales, dtype=np.float64)), 1 if pcn else 0, float(kwargs.get('beta', 0.5)),
-            int(n_mcmc), n_chains, _lib.host_ptr(start), _lib.host_ptr(phi_point), mt.ctypes.data, _lib.host_ptr(gauss), seed,
-            _lib.host_ptr(samples), accepted.ctypes.data))
+        # arguments shared by both device samplers, from y onwards (include/ces_b200.h)
+        common = (_lib.host_ptr(y), _lib.host_ptr(Ginv2), _lib.host_ptr(mu) if mu is not None else None,
+                  _lib.host_ptr(Pinv) if Pinv is not None else None, _lib.host_ptr(np.ascontiguousarray(scales, dtype=np.float64)),
+                  1 if pcn else 0, float(kwargs.get('beta', 0.5)), int(n_mcmc), n_chains, _lib.host_ptr(start),
+                  _lib.host_ptr(phi_point), mt.ctypes.data, _lib.host_ptr(gauss), seed, _lib.host_ptr(samples),
+                  accepted.ctypes.data)
+        if darcy:
+            # chains stepped in lockstep through the batched Darcy solver (csrc/darcy_mh.cu), with the model's tol / max_iter
+            _lib.check(_lib.load().ces_darcy_mh(model._handle(True), float(model.tol), int(model.max_iter), *common))
+        else:
+            A_dev, lda, b_dev, params = model._device_args(torch)
+            par = np.ascontiguousarray(params, dtype=np.float64) if params is not None else None
+            stream = torch.cuda.current_stream().cuda_stream
+            _lib.check(_lib.load().ces_mcmc_model_mh(
+                ctypes.c_void_p(stream), _lib.MAPS[kind], p, k,
+                ctypes.c_void_p(A_dev.data_ptr()) if A_dev is not None else None, int(lda),
+                ctypes.c_void_p(b_dev.data_ptr()) if b_dev is not None else None,
+                _lib.host_ptr(par) if par is not None else None, *common))
         np.random.set_state(('MT19937', mt[:624].copy(), int(mt[624]), int(mt[625]), float(gauss[0])))
         chain0 = samples[0]
         if previous is not None:

@@ -309,6 +309,24 @@ int ces_mcmc_model_mh(void* stream, int map_kind, int64_t p, int64_t k, const do
                       uint32_t* mt_state_host, double* mt_gauss_host, uint64_t seed, double* samples_host,
                       int32_t* accepted_host);
 
+/* MCMC.model_mh on the Darcy models (csrc/darcy_mh.cu): n_chains chains of n_mcmc proposals stepped in lockstep on a
+ * Darcy model created with an obs_index (ces_darcy_create), on that model's stream, with no host synchronisation inside
+ * the step loop.  One step draws every chain's noise (random numbers exactly as ces_mcmc_model_mh: chain 0 from numpy's
+ * stream when mt_state_host != NULL, the others from Philox keyed by (seed, step, chain)), forms the proposals
+ * b cur + a scales z as one DMMA GEMM (random walk a = b = 1; pCN a = sqrt(beta), b = sqrt(1 - beta^2)), evaluates them in
+ * one batched ces_darcy_forward pipeline (CG to `tol`, at most max_iter iterations; <= 0: the defaults of
+ * ces_darcy_forward), and accepts with Phi = (G - y)^T Ginv2 (G - y) (+ 1/2 (u - mu)^T Pinv (u - mu) unless pCN) as
+ * GEMMs, so p and n_obs are limited only by the model.  Arguments from y_host onwards as ces_mcmc_model_mh (p and
+ * k = n_obs are the model's).  If any solve -- the initial one at phi_point or a proposal's -- reaches max_iter, returns
+ * CES_ERR_STATE naming the first such step and leaves samples, acceptances and the generator state untouched.
+ * A model without obs_index, NULL pointers, n_mcmc < 1 or n_chains < 1 return CES_ERR_INVALID before any device work.
+ * Synchronises. */
+int ces_darcy_mh(void* model, double tol, int max_iter, const double* y_host, const double* Ginv2_host,
+                 const double* mu_host, const double* Pinv_host, const double* scales_host, int pcn, double beta,
+                 int64_t n_mcmc, int64_t n_chains, const double* start_host, const double* phi_point_host,
+                 uint32_t* mt_state_host, double* mt_gauss_host, uint64_t seed, double* samples_host,
+                 int32_t* accepted_host);
+
 /* ---- Emulate: exact GP emulators of the whitened forward map and MH chains through them (csrc/emulate.cu) ----------
  * One GP per whitened output i < k on the training inputs X (p x n, row-major, one point per column) and outputs
  * Y = T G - ybar (k x n; T = diag(lam^-1/2) Q^T from Gamma = Q diag(lam) Q^T, ybar the row means), all fixed by the caller.
