@@ -17,6 +17,7 @@ RULES = {"eks": 0, "aldi": 1, "aldi_constant": 2, "eki": 3}
 TS_FROBENIUS, TS_FIXED, TS_KEEP = 0, 1, 2
 FORMULATIONS = {"interaction": 0, "factored": 1}
 MAPS = {"lineal": 0, "lineal_log": 1, "elliptic": 2, "banana": 3}
+GP_KERNELS = {"SquaredExponential": 0, "Matern12": 1, "Matern32": 2, "Matern52": 3}   # CES_GP_* (GPflow's class names)
 
 # every symbol include/ces_b200.h declares (tests/test_abi.py checks the .so exports them all)
 EXPORTS = (
@@ -31,6 +32,7 @@ EXPORTS = (
     "ces_host_centre_u", "ces_host_interact_own", "ces_host_update", "ces_ipc_export", "ces_ipc_import", "ces_peer_gather",
     "ces_peer_gather_wait", "ces_host_interact_chunk", "ces_small_run", "ces_mcmc_model_mh", "ces_host_chunk_schedule",
     "ces_gp_create", "ces_gp_destroy", "ces_gp_lml", "ces_gp_condition", "ces_gp_predict", "ces_gp_mh", "ces_darcy_mh",
+    "ces_gp_set_kernel",
 )
 
 _i64, _int, _dbl, _vp = ctypes.c_int64, ctypes.c_int, ctypes.c_double, ctypes.c_void_p
@@ -101,6 +103,7 @@ def load():
                                       _dp, _dp, _dp, _dp, ctypes.c_uint64, _dp, _dp]
     lib.ces_gp_create.argtypes = [_vp, _i64, _i64, _i64, _dp, _dp, _dp, ctypes.POINTER(_vp)]
     lib.ces_gp_destroy.argtypes = [_vp]
+    lib.ces_gp_set_kernel.argtypes = [_vp, _int]
     lib.ces_gp_lml.argtypes = [_vp, _i64, _i64, _dp, _dbl, _dp, _dp]
     lib.ces_gp_condition.argtypes = [_vp, _dp, _dbl]
     lib.ces_gp_predict.argtypes = [_vp, _dp, _i64, _i64, _dp, _i64, _dp, _i64]

@@ -2,17 +2,24 @@
 // Metropolis-Hastings chains through them (MCMC.emulator_mh).
 //
 // Model (one independent GP per whitened output i < k; training inputs X (p x n), outputs Y = T G - ybar (k x n)):
-//   theta_i = [log sf2, log l_1..l_p, log sn2]                (sklearn's theta of C*RBF(ARD)+White)
-//   k(x, z) = sf2 exp(-1/2 sum_d (x_d - z_d)^2 / l_d^2),  K = k(X, X) + (sn2 + jitter) I,  L = chol(K),  alpha = K^-1 y_i
+//   theta_i = [log sf2, log l_1..l_p, log sn2]                (sklearn's theta of C*RBF(ARD)+White, or C*Matern(ARD)+White)
+//   D_d = (x_d - z_d)^2 / l_d^2,  r^2 = sum_d D_d,  k(x, z) = K_f(r) with the family fixed per model (ces_gp_set_kernel):
+//             SE  sf2 exp(-r^2/2)          Matern12  sf2 exp(-r)
+//             Matern32  sf2 (1 + sqrt3 r) exp(-sqrt3 r)          Matern52  sf2 (1 + sqrt5 r + 5 r^2 / 3) exp(-sqrt5 r)
+//   K = k(X, X) + (sn2 + jitter) I,  L = chol(K),  alpha = K^-1 y_i
 //   LML     = -1/2 y_i^T alpha - sum log L_jj - n/2 log 2 pi
 //   dLML/dtheta_j = 1/2 sum_ab W_ab dK_ab/dtheta_j,  W = alpha alpha^T - K^-1
-//             dK/dlog sf2 = K_f,  dK/dlog l_d = K_f (x_d - z_d)^2 / l_d^2,  dK/dlog sn2 = sn2 I   (K_f: no noise, no jitter)
+//             dK/dlog sf2 = K_f,  dK/dlog l_d = sf2 g(r) D_d,  dK/dlog sn2 = sn2 I   (K_f: no noise, no jitter)
+//             g(r): SE exp(-r^2/2) (so sf2 g = K_f),  Matern12 exp(-r) / r and 0 at r = 0 (sklearn's convention),
+//                   Matern32 3 exp(-sqrt3 r),  Matern52 5/3 (1 + sqrt5 r) exp(-sqrt5 r)
 //   mean_i(u) = ybar_i + k_i(u)^T alpha_i,   var_i(u) = max(sf2 - ||L_i^-1 k_i(u)||^2, 0)   (latent f, no sn2)
 //   Phi(u)  = 1/2 sum_i (ytil_i - mean_i)^2 / (1 + var_i) + 1/2 sum_i log(1 + var_i)   [use_variance]
 //             1/2 sum_i (ytil_i - mean_i)^2                                            [otherwise]
 //
 // Device layout.  Covariance blocks are assembled by one tile kernel batched over outputs on blockIdx.z, from the
-// coordinates divided by the lengthscales and staged in shared memory (p <= 32).  The factorisations are the DMMA
+// coordinates divided by the lengthscales and staged in shared memory (p <= 32).  The family is a template parameter
+// of the covariance and gradient kernels, dispatched once per launch; r^2 always comes from direct differences (no
+// |a|^2 + |b|^2 - 2 a.b expansion, which cancels near r = 0).  The factorisations are the DMMA
 // Cholesky / triangular solves of chol.cu.  The gradient is one pass over the lower triangle of K that recomputes K_f
 // on the fly and contracts it with W into p + 2 per-CTA partial sums, finished in fixed order by one more kernel: no
 // atomics, so repeated calls are bit-identical (the L-BFGS fit relies on it).  Conditioning keeps L_i^-1 explicitly,
@@ -48,9 +55,38 @@ __device__ __forceinline__ double scaled_dist2(const double (*sa)[GP_TB + 1], co
     return s;
 }
 
+// The covariance family (CES_GP_*) as a function of the scaled squared distance r2 = r^2: gp_kf = K_f / sf2 and
+// gp_g = g(r), the weight of D_d in dK/dlog l_d = sf2 g(r) D_d.  gp_g is not used for SE, where g = K_f / sf2.
+constexpr double GP_SQRT3 = 1.7320508075688772935, GP_SQRT5 = 2.2360679774997896964;
+
+template <int KIND> __device__ __forceinline__ double gp_kf(double r2);
+template <> __device__ __forceinline__ double gp_kf<CES_GP_SE>(double r2) { return exp(-0.5 * r2); }
+template <> __device__ __forceinline__ double gp_kf<CES_GP_MATERN12>(double r2) { return exp(-sqrt(r2)); }
+template <> __device__ __forceinline__ double gp_kf<CES_GP_MATERN32>(double r2) {
+    const double t = GP_SQRT3 * sqrt(r2);
+    return (1.0 + t) * exp(-t);
+}
+template <> __device__ __forceinline__ double gp_kf<CES_GP_MATERN52>(double r2) {
+    const double t = GP_SQRT5 * sqrt(r2);
+    return (1.0 + t + t * t / 3.0) * exp(-t);
+}
+
+template <int KIND> __device__ __forceinline__ double gp_g(double r2);
+template <> __device__ __forceinline__ double gp_g<CES_GP_MATERN12>(double r2) {
+    if (r2 == 0.0) return 0.0;                      // sklearn's value at r = 0: D_d = 0 there, so dK/dlog l_d = 0
+    const double r = sqrt(r2);
+    return exp(-r) / r;
+}
+template <> __device__ __forceinline__ double gp_g<CES_GP_MATERN32>(double r2) { return 3.0 * exp(-GP_SQRT3 * sqrt(r2)); }
+template <> __device__ __forceinline__ double gp_g<CES_GP_MATERN52>(double r2) {
+    const double t = GP_SQRT5 * sqrt(r2);
+    return (5.0 / 3.0) * (1.0 + t) * exp(-t);
+}
+
 // out_z[r][c] = k_z(A[:, r], B[:, c]) for r < nr, c < nc (+ sn2 + jitter where `train` and r == c); rows nr <= r < nr_pad
 // are written as zeros.  train: only tiles on or below the diagonal (the Cholesky reads the lower triangle).
 // Output z uses theta row z0 + z.
+template <int KIND>
 __global__ void __launch_bounds__(256) gp_cov_kernel(const double* __restrict__ A, long long lda, int nr, int nr_pad,
                                                      const double* __restrict__ B, long long ldb, int nc, int p,
                                                      const double* __restrict__ theta, int z0, double jitter, int train,
@@ -71,16 +107,18 @@ __global__ void __launch_bounds__(256) gp_cov_kernel(const double* __restrict__ 
         if (gr >= nr_pad || gc >= nc) continue;
         double v = 0.0;
         if (gr < nr) {
-            v = sf2 * exp(-0.5 * scaled_dist2(sa, sb, r, c, p));
+            v = sf2 * gp_kf<KIND>(scaled_dist2(sa, sb, r, c, p));
             if (train && gr == gc) v += diag;
         }
         o[(size_t)gr * ldo + gc] = v;
     }
 }
 
-// One CTA per 32 x 32 tile on or below the diagonal of K (linear index blockIdx.x): M_ab = w_ab W_ab K_f,ab with
-// W = alpha alpha^T - K^-1 and w_ab the multiplicity of the pair in the full matrix (2 off the diagonal, 1 on it), then
-// part[tile] = { sum M, sum M (s_ad - s_bd)^2 for d < p, sum_a W_aa }.
+// One CTA per 32 x 32 tile on or below the diagonal of K (linear index blockIdx.x): M_ab = w_ab W_ab K_f,ab and
+// M'_ab = w_ab W_ab sf2 g(r_ab) with W = alpha alpha^T - K^-1 and w_ab the multiplicity of the pair in the full matrix
+// (2 off the diagonal, 1 on it), then part[tile] = { sum M, sum M' (s_ad - s_bd)^2 for d < p, sum_a W_aa }.
+// For SE, M' = M: the same value, kept in the same register.
+template <int KIND>
 __global__ void __launch_bounds__(256) gp_grad_kernel(const double* __restrict__ X, long long ldx, int n, int p,
                                                       const double* __restrict__ th, const double* __restrict__ Kinv,
                                                       long long ldk, const double* __restrict__ alpha, long long lda,
@@ -101,13 +139,17 @@ __global__ void __launch_bounds__(256) gp_grad_kernel(const double* __restrict__
     double s_f = 0.0, s_tr = 0.0;
     for (int r = w; r < GP_TB; r += 8) {
         const int gr = r0 + r, gc = c0 + c;
-        double m = 0.0;
+        double m = 0.0, mg = 0.0;
         if (gr < n && gc < n && (tr != tc || c <= r)) {
             const double W = alpha[(size_t)gr * lda] * alpha[(size_t)gc * lda] - Kinv[(size_t)gr * ldk + gc];
-            m = (gr == gc ? 1.0 : 2.0) * W * (sf2 * exp(-0.5 * scaled_dist2(sa, sb, r, c, p)));
+            const double r2 = scaled_dist2(sa, sb, r, c, p);
+            const double wW = (gr == gc ? 1.0 : 2.0) * W;
+            m = wW * (sf2 * gp_kf<KIND>(r2));
+            if constexpr (KIND == CES_GP_SE) mg = m;
+            else mg = wW * (sf2 * gp_g<KIND>(r2));
             if (gr == gc) s_tr += W;
         }
-        sm[r][c] = m;
+        sm[r][c] = mg;
         s_f += m;
     }
     __syncthreads();
@@ -295,12 +337,20 @@ __global__ void __launch_bounds__(128) gp_accept_kernel(const GpMhArgs a, int it
     }
 }
 
+// the instantiations per family, indexed by CES_GP_*: the one dispatch of every covariance / gradient launch
+constexpr int GP_KINDS = 4;
+decltype(&gp_cov_kernel<CES_GP_SE>) const GP_COV_KERNEL[GP_KINDS] = {
+    gp_cov_kernel<CES_GP_SE>, gp_cov_kernel<CES_GP_MATERN12>, gp_cov_kernel<CES_GP_MATERN32>, gp_cov_kernel<CES_GP_MATERN52>};
+decltype(&gp_grad_kernel<CES_GP_SE>) const GP_GRAD_KERNEL[GP_KINDS] = {
+    gp_grad_kernel<CES_GP_SE>, gp_grad_kernel<CES_GP_MATERN12>, gp_grad_kernel<CES_GP_MATERN32>, gp_grad_kernel<CES_GP_MATERN52>};
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------ host side
 struct GpModel {
     cudaStream_t st = nullptr;
     int p = 0, k = 0, n = 0;
+    int kind = CES_GP_SE;       // covariance family (ces_gp_set_kernel)
     int64_t ldn = 0, npad = 0;
     double* X = nullptr;        // p x n (ldn)
     double* Y = nullptr;        // k x n (ldn), whitened and centred
@@ -354,8 +404,8 @@ int gp_ntiles(int n) {
 // K_z (lower triangle, + (sn2 + jitter) I) of output z, with theta row z of `theta`
 int gp_assemble_train(GpModel* g, const double* theta, int z, double jitter) {
     const unsigned t = (unsigned)ceil_div(g->n, GP_TB);
-    gp_cov_kernel<<<dim3(t, t, 1), 256, 0, g->st>>>(g->X, g->ldn, g->n, g->n, g->X, g->ldn, g->n, g->p, theta, z, jitter, 1,
-                                                    g->K, g->ldn, 0);
+    GP_COV_KERNEL[g->kind]<<<dim3(t, t, 1), 256, 0, g->st>>>(g->X, g->ldn, g->n, g->n, g->X, g->ldn, g->n, g->p, theta, z,
+                                                             jitter, 1, g->K, g->ldn, 0);
     CES_LAUNCHED(1);
     return CES_OK;
 }
@@ -395,7 +445,7 @@ int gp_predict(GpModel* g, const double* U, int64_t ldu, int64_t m, double* mean
         g->m_cap = m;
     }
     const int64_t ld = padded_ld(g->m_cap), batch = g->npad * ld;
-    gp_cov_kernel<<<dim3((unsigned)ceil_div(m, GP_TB), (unsigned)(g->npad / GP_TB), (unsigned)g->k), 256, 0, g->st>>>(
+    GP_COV_KERNEL[g->kind]<<<dim3((unsigned)ceil_div(m, GP_TB), (unsigned)(g->npad / GP_TB), (unsigned)g->k), 256, 0, g->st>>>(
         g->X, g->ldn, g->n, (int)g->npad, U, ldu, (int)m, g->p, g->ctheta, 0, 0.0, 0, g->KS, ld, batch);
     CES_LAUNCHED(1);
     GemmCall c;                                     // V_i = L_i^-1 K*_i for every output at once
@@ -477,6 +527,16 @@ extern "C" int ces_gp_destroy(void* h) {
     return CES_OK;
 }
 
+extern "C" int ces_gp_set_kernel(void* h, int kind) {
+    GpModel* g = static_cast<GpModel*>(h);
+    if (!g || kind < 0 || kind >= GP_KINDS)
+        return fail(CES_ERR_INVALID, "ces_gp_set_kernel: needs a model and a kind CES_GP_SE .. CES_GP_MATERN52, got %s%lld", "",
+                    (long long)kind);
+    g->kind = kind;
+    g->conditioned = false;
+    return CES_OK;
+}
+
 extern "C" int ces_gp_lml(void* h, int64_t i0, int64_t i1, const double* theta_host, double jitter, double* lml_host,
                           double* grad_host) {
     GpModel* g = static_cast<GpModel*>(h);
@@ -493,8 +553,9 @@ extern "C" int ces_gp_lml(void* h, int64_t i0, int64_t i1, const double* theta_h
         CES_LAUNCHED(1);
         if (grad_host) {
             CES_TRY(spd_inverse_from_factor(g->st, g->K, g->ldn, g->n, g->Lblk, CHOL_NB, g->Kinv, g->ldn));
-            gp_grad_kernel<<<(unsigned)g->ntiles, 256, 0, g->st>>>(g->X, g->ldn, g->n, g->p, thz, g->Kinv, g->ldn, g->rhs,
-                                                                  GP_RHS_LD, g->part + (size_t)z * g->ntiles * np2);
+            GP_GRAD_KERNEL[g->kind]<<<(unsigned)g->ntiles, 256, 0, g->st>>>(g->X, g->ldn, g->n, g->p, thz, g->Kinv, g->ldn,
+                                                                           g->rhs, GP_RHS_LD,
+                                                                           g->part + (size_t)z * g->ntiles * np2);
             CES_LAUNCHED(1);
         }
     }

@@ -2,7 +2,9 @@
 
 The Calibrate -> Emulate -> Sample pipeline trains one GP per output on the calibrated ensemble ``(Ustar, Gstar)`` and then
 runs Metropolis-Hastings on the emulator (``MCMC.emulator_mh``) instead of the expensive model.  The model is GPflow's
-``GPR`` + ``SquaredExponential`` (ARD) + ``Gaussian`` likelihood -- scikit-learn's ``C * RBF + WhiteKernel`` --:
+``GPR`` + ``SquaredExponential`` (ARD) + ``Gaussian`` likelihood -- scikit-learn's ``C * RBF + WhiteKernel`` -- or, with
+``kernel="Matern12"`` / ``"Matern32"`` / ``"Matern52"``, GPflow's Matern kernel of that order (sklearn's
+``C * Matern(nu=0.5 / 1.5 / 2.5) + WhiteKernel``), with the same hyperparameters:
 
 Whitening (host, once): ``Gamma = Q diag(lam) Q^T`` (``numpy.linalg.eigh``), ``T = diag(lam^-1/2) Q^T``; the training
 outputs are ``Y = T G``, each row centred by its mean ``ybar_i`` (a constant mean function).  ``transform`` (T) and
@@ -11,7 +13,11 @@ coordinates the noise covariance is I, so the outputs get independent GPs.
 
 Per output i: ``theta_i = [log sf2, log l_1..l_p, log sn2]`` (sklearn's order; GPflow's ``kernel.variance``,
 ``kernel.lengthscales``, ``likelihood.variance``),
-    k(x, z) = sf2 exp(-1/2 sum_d (x_d - z_d)^2 / l_d^2),   K = k(X, X) + (sn2 + jitter) I,   L = chol(K),   alpha = K^-1 y_i
+    r = |(x - z) / l|,   k(x, z) = sf2 exp(-r^2/2)                            (SquaredExponential)
+                                   sf2 exp(-r)                               (Matern12)
+                                   sf2 (1 + sqrt3 r) exp(-sqrt3 r)           (Matern32)
+                                   sf2 (1 + sqrt5 r + 5 r^2 / 3) exp(-sqrt5 r)   (Matern52)
+    K = k(X, X) + (sn2 + jitter) I,   L = chol(K),   alpha = K^-1 y_i
     LML = -1/2 y_i^T alpha - sum log L_jj - n/2 log 2 pi,   dLML/dtheta = 1/2 tr((alpha alpha^T - K^-1) dK/dtheta)
     mean_i(u) = ybar_i + k_i(u)^T alpha,   var_i(u) = max(sf2 - |L^-1 k_i(u)|^2, 0)       (latent f: GPflow's predict_f)
 The emulated misfit of ``MCMC.emulator_mh`` at the whitened data ``ytil = T y_obs`` is
@@ -30,9 +36,11 @@ from . import _lib
 class GPEmulator(object):
     """One exact GP per whitened output, trained on ``enka.Ustar`` / ``enka.Gstar`` (or ``U`` (p x n) / ``G`` (k x n))."""
 
-    def __init__(self, enka=None, Gamma=None, U=None, G=None, jitter=1e-10):
+    def __init__(self, enka=None, Gamma=None, U=None, G=None, jitter=1e-10, kernel="SquaredExponential"):
         import torch
 
+        if kernel not in _lib.GP_KERNELS:
+            raise ValueError("GPEmulator: kernel must be one of %s, got %r" % (", ".join(_lib.GP_KERNELS), kernel))
         if not torch.cuda.is_available():
             raise RuntimeError("ces_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         if Gamma is None:
@@ -57,6 +65,8 @@ class GPEmulator(object):
                                            _lib.host_ptr(self.X), _lib.host_ptr(self.Y),
                                            _lib.host_ptr(np.ascontiguousarray(self.offset)), ctypes.byref(h)))
         self._h = h
+        self._kernel = kernel
+        _lib.check(self._lib.ces_gp_set_kernel(h, _lib.GP_KERNELS[kernel]))
         self._conditioned = None
         self.theta = self.default_init()
 
@@ -65,6 +75,11 @@ class GPEmulator(object):
         if h is not None and h.value:
             self._lib.ces_gp_destroy(h)
             self._h = None
+
+    @property
+    def kernel(self):
+        """The covariance family, by GPflow's class name (fixed at construction)."""
+        return self._kernel
 
     # ---- hyperparameters
     def default_init(self):
@@ -89,7 +104,8 @@ class GPEmulator(object):
         return np.exp(self.theta[:, -1])
 
     def set_hyperparameters(self, variance, lengthscales, noise_variance):
-        """Set theta from GPflow-named values (per output, or one value for every output); e.g. reuse a GPflow training."""
+        """Set theta from GPflow-named values (per output, or one value for every output); e.g. reuse a GPflow training
+        whose kernel is this emulator's family: ``kernel.variance``, ``kernel.lengthscales``, ``likelihood.variance``."""
         var = np.broadcast_to(np.asarray(variance, dtype=np.float64), (self.k,))
         ls = np.broadcast_to(np.asarray(lengthscales, dtype=np.float64).reshape(-1, self.p) if np.ndim(lengthscales) else
                              np.full((1, self.p), float(lengthscales)), (self.k, self.p))

@@ -18,7 +18,7 @@ provided: it needs trained GPflow models (``emulate.predict_gps``, ces/emulate.p
 absent here and whose predictions could not be pinned; that half of SURVEY.md section 8f-4 stays out of scope.
 
 ``emulator_mh`` (new) is the same sampler on an emulator of the forward model: a ``ces_b200.emulate.GPEmulator`` (exact
-GPs on the device, trained on the calibrated ensemble) replaces the model, and the misfit becomes the emulated one in
+GPs on the device, trained on the calibrated ensemble, with any of its kernel families) replaces the model, and the misfit becomes the emulated one in
 whitened coordinates (see ces_b200/emulate.py).  Proposals, prior term, accept test, resume behaviour and the random
 numbers are ``model_mh``'s.
 """
@@ -135,7 +135,8 @@ class MCMC(object):
                     seed=0, use_variance=True):
         """``model_mh`` through a ``GPEmulator``: Phi(u) = 1/2 sum_i (ytil_i - mean_i(u))^2 / (1 + var_i(u))
         + 1/2 sum_i log(1 + var_i(u)) (without the variance terms when ``use_variance`` is False), ytil = T y_obs,
-        plus -prior.logpdf(u) unless pCN.  Chains run on the device (csrc/emulate.cu); results as ``model_mh``."""
+        plus -prior.logpdf(u) unless pCN, with mean / var the emulator's latent prediction under its kernel family
+        (``emulator.kernel``).  Chains run on the device (csrc/emulate.cu); results as ``model_mh``."""
         p, k = int(emulator.p), int(emulator.k)
         if update not in (None, 'pCN'):
             raise ValueError("unknown update %r" % (update,))

@@ -5,14 +5,17 @@ observed cells drawn proportionally to the true pressure, noise sd 0.005, and on
 All four stages run on the B200:
 
   Calibrate   sampling.run (the ensemble Kalman sampler) from prior draws
-  Emulate     GPEmulator(eks, Gamma).fit(): one exact GP per whitened observation, trained on (eks.Ustar, eks.Gstar)
+  Emulate     GPEmulator(eks, Gamma, kernel=...).fit(): one exact GP per whitened observation, trained on
+              (eks.Ustar, eks.Gstar), with the squared-exponential kernel or a Matern one (--kernel)
   Sample      MCMC.emulator_mh through the emulator, 64 chains, proposals scaled by eks.Ustar
   Gold        MCMC.model_mh on the Darcy model itself, 64 chains stepped in lockstep through the batched solver
 
 It prints the mean and standard deviation of every mode for the EKS ensemble, the emulator chains and the true-model chains,
-and the wall time of each stage; main() returns them.
+the gap between the emulator's and the true model's posterior means in true-posterior standard deviations, the ratio of
+their standard deviations, and the wall time of each stage; main() returns them.
 
     python examples/darcy_ces.py [--nmesh 16] [--p 10] [--J 100] [--T 200] [--n-mcmc 20000] [--chains 64]
+                                 [--kernel SquaredExponential|Matern12|Matern32|Matern52]
 """
 import argparse
 import os
@@ -45,6 +48,8 @@ def main(argv=None):
     ap.add_argument("--n-mcmc", type=int, default=20000)
     ap.add_argument("--chains", type=int, default=64)
     ap.add_argument("--delta", type=float, default=0.7)
+    ap.add_argument("--kernel", default="SquaredExponential", choices=["SquaredExponential", "Matern12", "Matern32", "Matern52"],
+                    help="the emulator's covariance family (GPflow's class names)")
     args = ap.parse_args(argv)
 
     # ---- the problem (examples/darcy_flow.py on model_trunc)
@@ -72,7 +77,7 @@ def main(argv=None):
 
     # ---- Emulate
     t0 = time.perf_counter()
-    emulator = GPEmulator(eks, Gamma).fit()
+    emulator = GPEmulator(eks, Gamma, kernel=args.kernel).fit()
     times["emulate"] = time.perf_counter() - t0
 
     # ---- Sample through the emulator, and the gold standard on the true model
@@ -94,14 +99,17 @@ def main(argv=None):
            "model_mean": model_x.mean(axis=1), "model_sd": model_x.std(axis=1, ddof=1),
            "emulator_accept": float(np.mean(getattr(emu_mcmc, "accept_chains", emu_mcmc.accept))),
            "model_accept": float(np.mean(getattr(model_mcmc, "accept_chains", model_mcmc.accept))),
-           "times": times, "burn": burn, "eks": eks, "emulator": emulator, "emulator_mcmc": emu_mcmc, "model_mcmc": model_mcmc}
-    print("Darcy %d^2, %d KL modes, %d observations; EKS J = %d (%d iterations), %d chains x %d steps (burn-in %d)"
-          % (args.nmesh, p, n_obs, args.J, len(eks.metrics["t"]), args.chains, args.n_mcmc, burn))
-    print("mode   truth      EKS mean / sd         emulator mean / sd    true-model mean / sd   (emu - model) / sd")
+           "kernel": args.kernel, "times": times, "burn": burn, "eks": eks, "emulator": emulator, "emulator_mcmc": emu_mcmc, "model_mcmc": model_mcmc}
+    print("Darcy %d^2, %d KL modes, %d observations; EKS J = %d (%d iterations), %d chains x %d steps (burn-in %d); "
+          "emulator kernel %s" % (args.nmesh, p, n_obs, args.J, len(eks.metrics["t"]), args.chains, args.n_mcmc, burn, args.kernel))
+    print("mode   truth      EKS mean / sd         emulator mean / sd    true-model mean / sd   (emu - model) / sd   emu sd / model sd")
     for i in range(p):
-        print("%4d  %8.4f   %8.4f / %-8.4f   %8.4f / %-8.4f   %8.4f / %-8.4f    %+.3f"
+        print("%4d  %8.4f   %8.4f / %-8.4f   %8.4f / %-8.4f   %8.4f / %-8.4f    %+.3f               %.3f"
               % (i, out["truth"][i], out["eks_mean"][i], out["eks_sd"][i], out["emulator_mean"][i], out["emulator_sd"][i],
-                 out["model_mean"][i], out["model_sd"][i], (out["emulator_mean"][i] - out["model_mean"][i]) / out["model_sd"][i]))
+                 out["model_mean"][i], out["model_sd"][i], (out["emulator_mean"][i] - out["model_mean"][i]) / out["model_sd"][i],
+                 out["emulator_sd"][i] / out["model_sd"][i]))
+    gap, ratio = np.abs(out["emulator_mean"] - out["model_mean"]) / out["model_sd"], out["emulator_sd"] / out["model_sd"]
+    print("emulator vs true model: max |mean gap| %.3f sd, sd ratio %.3f .. %.3f" % (gap.max(), ratio.min(), ratio.max()))
     print("acceptance: emulator %.3f, true model %.3f" % (out["emulator_accept"], out["model_accept"]))
     print("wall time [s]: " + ", ".join("%s %.2f" % kv for kv in times.items()))
     return out

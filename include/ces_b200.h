@@ -60,6 +60,12 @@ extern "C" {
 #define CES_MAP_ELLIPTIC 2        /* :72-89  (p = 2, k = 2; params = {x1, x2})                       */
 #define CES_MAP_BANANA 3          /* :116-122 (p = 2, k = 2; params = {a, b})                        */
 
+/* covariance families of the GP emulator (ces_gp_set_kernel; GPflow's class names) */
+#define CES_GP_SE 0               /* SquaredExponential (the default)                                 */
+#define CES_GP_MATERN12 1         /* Matern12 = sklearn's Matern(nu=0.5)                              */
+#define CES_GP_MATERN32 2         /* Matern32 = sklearn's Matern(nu=1.5)                              */
+#define CES_GP_MATERN52 3         /* Matern52 = sklearn's Matern(nu=2.5)                              */
+
 typedef struct ces_handle_s* ces_handle_t;
 
 /* Library / build identification ("ces_b200 <version> sm_100a"). */
@@ -330,13 +336,19 @@ int ces_darcy_mh(void* model, double tol, int max_iter, const double* y_host, co
 /* ---- Emulate: exact GP emulators of the whitened forward map and MH chains through them (csrc/emulate.cu) ----------
  * One GP per whitened output i < k on the training inputs X (p x n, row-major, one point per column) and outputs
  * Y = T G - ybar (k x n; T = diag(lam^-1/2) Q^T from Gamma = Q diag(lam) Q^T, ybar the row means), all fixed by the caller.
- * theta_i = [log sf2, log l_1..l_p, log sn2];  k(x, z) = sf2 exp(-1/2 sum_d (x_d - z_d)^2 / l_d^2);
+ * theta_i = [log sf2, log l_1..l_p, log sn2];  r^2 = sum_d (x_d - z_d)^2 / l_d^2;  k(x, z) by the model's family:
+ *   CES_GP_SE sf2 exp(-r^2/2) (the default),  CES_GP_MATERN12 sf2 exp(-r),  CES_GP_MATERN32 sf2 (1 + sqrt3 r) exp(-sqrt3 r),
+ *   CES_GP_MATERN52 sf2 (1 + sqrt5 r + 5 r^2 / 3) exp(-sqrt5 r);
  * K = k(X, X) + (sn2 + jitter) I;  L = chol(K);  alpha = K^-1 y_i.  Limits: 1 <= p <= 32, 1 <= k <= 64, n >= 2 (n is
  * otherwise bounded by device memory: CES_ERR_NOMEM).  A K that is not positive definite returns CES_ERR_NOT_SPD.
  * ces_gp_create copies X, Y, ybar to the device on `stream`; every later call runs on that stream. */
 int ces_gp_create(void* stream, int64_t p, int64_t k, int64_t n, const double* X_host, const double* Y_host,
                   const double* ybar_host, void** out);
 int ces_gp_destroy(void* model);
+/* Selects the covariance family (CES_GP_*) of every output.  Clears the conditioned state: ces_gp_predict and ces_gp_mh
+ * return CES_ERR_STATE until ces_gp_condition runs again.  A NULL model or an unknown kind returns CES_ERR_INVALID.
+ * No device work. */
+int ces_gp_set_kernel(void* model, int kind);
 /* LML_i = -1/2 y_i^T alpha - sum_j log L_jj - n/2 log 2 pi for outputs i0 <= i < i1 (theta_host: (i1 - i0) x (p + 2)) and,
  * with grad_host != NULL, dLML_i/dtheta_i = 1/2 sum_ab (alpha alpha^T - K^-1)_ab dK_ab/dtheta ((i1 - i0) x (p + 2)).
  * Fixed-order reductions: repeated calls return bit-identical results.  Synchronises. */

@@ -1,9 +1,10 @@
 """Benchmark of the Emulate stage on the device: GP fit, prediction and MH through the emulator (JSON lines).
 
-    python tools/bench_emulate.py [--out FILE] [--quick]
+    python tools/bench_emulate.py [--out FILE] [--quick] [--kernel SquaredExponential|Matern12|Matern32|Matern52 ...]
 
 Workloads: the notebook scale of linear.ipynb (p = 2, k = 10, n = 100; 1 and 1024 chains) and a large emulator (p = 32,
-k = 64, n = 4096; 4096 chains).  Every line carries the GPU name and power limit read in the same run.  Times are CUDA
+k = 64, n = 4096; 4096 chains), for each covariance family named by --kernel (default: the squared exponential), the
+families alternating within each workload.  Every line carries the GPU name and power limit read in the same run.  Times are CUDA
 events around work that ends in a device synchronise, every shape warmed up first.  FLOP model of one prediction of m
 points: k n^2 m (the lower-triangular GEMM V = L^-1 K*) + k n m (3 p + 2) (assembly of K*: p scaled differences, squares
 and sums plus the scale and exp per entry, counted as 3 p + 2) + 4 k n m (mean and sum of squares).  The notebook quotes
@@ -62,7 +63,7 @@ def timed(fn, reps):
     return a.elapsed_time(b) / 1e3 / reps
 
 
-def run(p, k, n, chains, n_mcmc, predict_m, reps, do_fit, info):
+def run(p, k, n, chains, n_mcmc, predict_m, reps, do_fit, info, kernel="SquaredExponential"):
     import torch
     from scipy.stats import multivariate_normal
 
@@ -71,8 +72,8 @@ def run(p, k, n, chains, n_mcmc, predict_m, reps, do_fit, info):
     from ces_b200.sample import MCMC
 
     X, G = problem(p, k, n)
-    emu = GPEmulator(U=X, G=G, Gamma=0.01 * np.eye(k))
-    base = dict(info, p=p, k=k, n=n)
+    emu = GPEmulator(U=X, G=G, Gamma=0.01 * np.eye(k), kernel=kernel)
+    base = dict(info, kernel=kernel, p=p, k=k, n=n)
     lines = []
     if do_fit:
         torch.cuda.synchronize()
@@ -115,6 +116,8 @@ def main(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=None)
     ap.add_argument("--quick", action="store_true", help="small sizes only (a functional run)")
+    ap.add_argument("--kernel", nargs="+", default=["SquaredExponential"],
+                    choices=["SquaredExponential", "Matern12", "Matern32", "Matern52"], help="covariance families to run")
     args = ap.parse_args(argv)
     import torch
 
@@ -122,10 +125,12 @@ def main(argv=None):
         raise SystemExit("bench_emulate needs a CUDA device")
     info = gpu_info()
     lines = []
-    lines += run(2, 10, 100, 1, 2000, 1024, 200, True, info)
-    lines += run(2, 10, 100, 1024, 2000, 1024, 200, False, info)
+    workloads = [(2, 10, 100, 1, 2000, 1024, 200, True), (2, 10, 100, 1024, 2000, 1024, 200, False)]
     if not args.quick:
-        lines += run(32, 64, 4096, 4096, 20, 4096, 5, False, info)
+        workloads.append((32, 64, 4096, 4096, 20, 4096, 5, False))
+    for w in workloads:
+        for kernel in args.kernel:
+            lines += run(*w, info, kernel=kernel)
     out = open(args.out, "w") if args.out else None
     for ln in lines:
         s = json.dumps(ln)
