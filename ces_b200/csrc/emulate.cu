@@ -29,6 +29,7 @@
 // to a device samples buffer that is copied back once at the end.
 #include <vector>
 #include "kernels.h"
+#include "chains.cuh"
 #include "rng.cuh"
 
 namespace ces {
@@ -237,103 +238,59 @@ __global__ void __launch_bounds__(128) gp_column_kernel(const double* __restrict
     var[(size_t)z * ldv + j] = fmax(exp(theta[(size_t)z * (p + 2)]) - (q0 + q1), 0.0);
 }
 
-struct GpMhArgs {
-    int p, k, n_mcmc, n_chains, pcn, use_mt, use_variance;
-    double beta;
-    long long ld;               // pitch of the p x n_chains / k x n_chains state arrays
+// Phi of chain c at its evaluated point (column c of prop) from its predicted mean / var: emulated misfit, plus the prior
+// term 1/2 (x - mu)^T Pinv (x - mu) unless pCN.  One thread, fixed order.
+struct GpPhi {
+    int k, use_variance, pcn;
     const double* ytil;         // k
+    const double* mean;         // k x ld
+    const double* var;          // k x ld
     const double* mu;           // p
     const double* Pinv;         // p x p
-    const double* scales;       // p x p
-    double* cur;                // p x n_chains
-    double* prop;               // p x n_chains
-    const double* mean;         // k x n_chains
-    const double* var;          // k x n_chains
-    double* u;                  // n_chains: the accept test's uniform of this step
-    double* phi_cur;            // n_chains
-    double* samples;            // n_chains x (n_mcmc + 1) x p
-    int* accepted;              // n_chains
-    uint32_t* mt;               // 624 key words, pos, has_gauss
-    double* mt_gauss;
-    unsigned long long seed;
+    __device__ double operator()(const ChainState& a, int c) const {
+        const double* x = a.prop;
+        double phi = 0.0;
+        for (int i = 0; i < k; ++i) {
+            const double r = ytil[i] - mean[(size_t)i * a.ld + c];
+            if (use_variance) {
+                const double s = 1.0 + var[(size_t)i * a.ld + c];
+                phi += r * r / s + log(s);
+            } else {
+                phi = fma(r, r, phi);
+            }
+        }
+        phi *= 0.5;
+        if (!pcn) {
+            double pp = 0.0;
+            for (int q = 0; q < a.p; ++q) {
+                double t = 0.0;
+                for (int m = 0; m < a.p; ++m) t = fma(Pinv[(size_t)q * a.p + m], x[(size_t)m * a.ld + c] - mu[m], t);
+                pp = fma(0.5 * (x[(size_t)q * a.ld + c] - mu[q]), t, pp);
+            }
+            phi += pp;
+        }
+        return phi;
+    }
 };
 
-// Phi of chain c at the point x (column c of a p x n_chains array) from its predicted mean / var: emulated misfit, plus the
-// prior term 1/2 (x - mu)^T Pinv (x - mu) unless pCN.  One thread, fixed order.
-__device__ double gp_phi(const GpMhArgs& a, const double* x, int c) {
-    double phi = 0.0;
-    for (int i = 0; i < a.k; ++i) {
-        const double r = a.ytil[i] - a.mean[(size_t)i * a.ld + c];
-        if (a.use_variance) {
-            const double s = 1.0 + a.var[(size_t)i * a.ld + c];
-            phi += r * r / s + log(s);
-        } else {
-            phi = fma(r, r, phi);
-        }
-    }
-    phi *= 0.5;
-    if (!a.pcn) {
-        double pp = 0.0;
-        for (int q = 0; q < a.p; ++q) {
-            double t = 0.0;
-            for (int m = 0; m < a.p; ++m) t = fma(a.Pinv[(size_t)q * a.p + m], x[(size_t)m * a.ld + c] - a.mu[m], t);
-            pp = fma(0.5 * (x[(size_t)q * a.ld + c] - a.mu[q]), t, pp);
-        }
-        phi += pp;
-    }
-    return phi;
-}
-
-// stage 0: the initial Phi_current at the evaluated points (in cur); stage 1: then cur <- start, state 0 of every chain
-__global__ void __launch_bounds__(128) gp_mh_init_kernel(const GpMhArgs a, const double* __restrict__ start) {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= a.n_chains) return;
-    a.phi_cur[c] = gp_phi(a, a.cur, c);
-    double* out = a.samples + (size_t)c * (a.n_mcmc + 1) * a.p;
-    for (int q = 0; q < a.p; ++q) {
-        const double v = start[(size_t)c * a.p + q];
-        a.cur[(size_t)q * a.ld + c] = v;
-        out[q] = v;
-    }
-}
-
 // z ~ N(0, I_p) and u ~ U(0, 1) per chain (chain 0 from numpy's stream when use_mt), proposal = random walk / pCN.
-__global__ void __launch_bounds__(GP_PROPOSE_THREADS) gp_propose_kernel(const GpMhArgs a, int it) {
+__global__ void __launch_bounds__(GP_PROPOSE_THREADS) gp_propose_kernel(const ChainState a, const double* scales, int pcn,
+                                                                       double beta, int it) {
     __shared__ double zs[GP_P_MAX][GP_PROPOSE_THREADS];
     __shared__ double sc[GP_P_MAX * GP_P_MAX];
     const int p = a.p;
-    for (int e = threadIdx.x; e < p * p; e += blockDim.x) sc[e] = a.scales[e];
+    for (int e = threadIdx.x; e < p * p; e += blockDim.x) sc[e] = scales[e];
     __syncthreads();
     const int c = blockIdx.x * blockDim.x + threadIdx.x, tid = threadIdx.x;
     if (c >= a.n_chains) return;
     a.u[c] = mh_chain_draw(p, it, c, (a.use_mt && c == 0) ? a.mt : nullptr, a.mt_gauss, a.seed, 0x4750u, &zs[0][tid],
                            GP_PROPOSE_THREADS);
-    const double a_cur = a.pcn ? sqrt(1.0 - a.beta * a.beta) : 1.0, a_z = a.pcn ? sqrt(a.beta) : 1.0;
+    const double a_cur = pcn ? sqrt(1.0 - beta * beta) : 1.0, a_z = pcn ? sqrt(beta) : 1.0;
     for (int q = 0; q < p; ++q) {
         double s = 0.0;
         for (int m = 0; m < p; ++m) s = fma(sc[q * p + m], zs[m][tid], s);       // np.matmul(scales, z)
         const double x = a.cur[(size_t)q * a.ld + c];
-        a.prop[(size_t)q * a.ld + c] = a.pcn ? a_cur * x + a_z * s : x + s;
-    }
-}
-
-__global__ void __launch_bounds__(128) gp_accept_kernel(const GpMhArgs a, int it) {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= a.n_chains) return;
-    const double phi_prop = gp_phi(a, a.prop, c);
-    const bool take = log(a.u[c]) < a.phi_cur[c] - phi_prop;          // NaN compares false: the proposal is rejected
-    double* out = a.samples + ((size_t)c * (a.n_mcmc + 1) + it + 1) * a.p;
-    for (int q = 0; q < a.p; ++q) {
-        double x = a.cur[(size_t)q * a.ld + c];
-        if (take) {
-            x = a.prop[(size_t)q * a.ld + c];
-            a.cur[(size_t)q * a.ld + c] = x;
-        }
-        out[q] = x;
-    }
-    if (take) {
-        a.phi_cur[c] = phi_prop;
-        a.accepted[c] += 1;
+        a.prop[(size_t)q * a.ld + c] = pcn ? a_cur * x + a_z * s : x + s;
     }
 }
 
@@ -613,81 +570,40 @@ extern "C" int ces_gp_mh(void* h, const double* ytil_host, int use_variance, con
                          const double* scales_host, int pcn, double beta, int64_t n_mcmc, int64_t n_chains,
                          const double* start_host, const double* phi_point_host, uint32_t* mt_state_host,
                          double* mt_gauss_host, uint64_t seed, double* samples_host, int32_t* accepted_host) {
+    const ChainHost ch{"ces_gp_mh", n_mcmc, n_chains, pcn, ytil_host, scales_host, mu_host, Pinv_host, start_host,
+                       phi_point_host, mt_state_host, mt_gauss_host, seed, samples_host, accepted_host};
+    CES_TRY(chain_check(ch));
     GpModel* g = static_cast<GpModel*>(h);
-    if (!g || !ytil_host || !scales_host || n_mcmc < 1 || n_chains < 1 || n_chains > (1 << 24) || !start_host ||
-        !phi_point_host || !samples_host || !accepted_host || (!pcn && (!mu_host || !Pinv_host)) ||
-        (mt_state_host && !mt_gauss_host))
-        return fail(CES_ERR_INVALID, "ces_gp_mh: needs a model, n_mcmc >= 1, n_chains >= 1 and non-null arguments%s", "");
+    if (!g) return fail(CES_ERR_INVALID, "ces_gp_mh: null model%s", "");
     if (!g->conditioned) return fail(CES_ERR_STATE, "ces_gp_mh: call ces_gp_condition first%s", "");
     const int p = g->p, k = g->k;
     const int64_t ld = padded_ld(n_chains);
-    const size_t nsamp = (size_t)n_chains * (n_mcmc + 1) * p;
-    const size_t nd = (size_t)k + p + 2 * (size_t)p * p + 2 * (size_t)p * ld + 2 * (size_t)k * ld + 2 * (size_t)ld + 1 +
-                      (size_t)n_chains * p + nsamp;
-    double* dbuf = nullptr;
-    uint32_t* ibuf = nullptr;
-    if (cudaMalloc(&dbuf, nd * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return fail(CES_ERR_NOMEM, "ces_gp_mh: allocation failed%s", ""); }
-    if (cudaMalloc(&ibuf, (626 + (size_t)n_chains) * sizeof(uint32_t)) != cudaSuccess) { cudaFree(dbuf); cudaGetLastError(); return fail(CES_ERR_NOMEM, "ces_gp_mh: allocation failed%s", ""); }
-    int s = CES_OK;
-    do {
-        double* q = dbuf;
-        auto put = [&](const double* src, size_t cnt) -> double* {
-            double* dst = q;
-            q += cnt;
-            if (src && cudaMemcpyAsync(dst, src, cnt * sizeof(double), cudaMemcpyHostToDevice, g->st) != cudaSuccess) s = CES_ERR_CUDA;
-            return dst;
-        };
-        // the p x n_chains state arrays hold one chain per column: transpose the row-per-chain host inputs
-        std::vector<double> phiT((size_t)p * ld, 0.0);
-        for (int64_t c = 0; c < n_chains; ++c)
-            for (int d = 0; d < p; ++d) phiT[(size_t)d * ld + c] = phi_point_host[(size_t)c * p + d];
-        GpMhArgs a;
-        a.p = p; a.k = k; a.n_mcmc = (int)n_mcmc; a.n_chains = (int)n_chains; a.pcn = pcn ? 1 : 0;
-        a.use_mt = mt_state_host != nullptr; a.use_variance = use_variance ? 1 : 0;
-        a.beta = beta; a.ld = ld;
-        a.ytil = put(ytil_host, k);
-        a.mu = put(pcn ? nullptr : mu_host, p);
-        a.Pinv = put(pcn ? nullptr : Pinv_host, (size_t)p * p);
-        a.scales = put(scales_host, (size_t)p * p);
-        a.cur = put(phiT.data(), (size_t)p * ld);
-        a.prop = put(nullptr, (size_t)p * ld);
-        double* mean = put(nullptr, (size_t)k * ld);
-        double* var = put(nullptr, (size_t)k * ld);
-        a.mean = mean; a.var = var;
-        a.u = put(nullptr, ld);
-        a.phi_cur = put(nullptr, ld);
-        a.mt_gauss = put(mt_state_host ? mt_gauss_host : nullptr, 1);
-        const double* start = put(start_host, (size_t)n_chains * p);
-        a.samples = put(nullptr, nsamp);
-        a.mt = ibuf;
-        a.accepted = reinterpret_cast<int*>(ibuf + 626);
-        a.seed = seed;
-        if (s != CES_OK) { s = fail(CES_ERR_CUDA, "ces_gp_mh: upload failed%s", ""); break; }
-        if (mt_state_host && cudaMemcpyAsync(ibuf, mt_state_host, 626 * sizeof(uint32_t), cudaMemcpyHostToDevice, g->st) != cudaSuccess) { s = fail(CES_ERR_CUDA, "ces_gp_mh: upload failed%s", ""); break; }
-        if (cudaMemsetAsync(a.accepted, 0, (size_t)n_chains * sizeof(int), g->st) != cudaSuccess) { s = fail(CES_ERR_CUDA, "ces_gp_mh: upload failed%s", ""); break; }
-        const unsigned blocks = (unsigned)ceil_div(n_chains, 128);
-        if ((s = gp_predict(g, a.cur, ld, n_chains, mean, ld, var, ld)) != CES_OK) break;
-        gp_mh_init_kernel<<<blocks, 128, 0, g->st>>>(a, start);
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        for (int it = 0; it < (int)n_mcmc && s == CES_OK; ++it) {
-            gp_propose_kernel<<<(unsigned)ceil_div(n_chains, GP_PROPOSE_THREADS), GP_PROPOSE_THREADS, 0, g->st>>>(a, it);
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-            if ((s = gp_predict(g, a.prop, ld, n_chains, mean, ld, var, ld)) != CES_OK) break;
-            gp_accept_kernel<<<blocks, 128, 0, g->st>>>(a, it);
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-        }
-        if (s != CES_OK) break;
-        if (cudaGetLastError() != cudaSuccess) { s = fail(CES_ERR_CUDA, "ces_gp_mh: launch failed%s", ""); break; }
-        cudaMemcpyAsync(samples_host, a.samples, nsamp * sizeof(double), cudaMemcpyDeviceToHost, g->st);
-        cudaMemcpyAsync(accepted_host, a.accepted, (size_t)n_chains * sizeof(int), cudaMemcpyDeviceToHost, g->st);
-        if (mt_state_host) {
-            cudaMemcpyAsync(mt_state_host, ibuf, 626 * sizeof(uint32_t), cudaMemcpyDeviceToHost, g->st);
-            cudaMemcpyAsync(mt_gauss_host, a.mt_gauss, sizeof(double), cudaMemcpyDeviceToHost, g->st);
-        }
-        if (cudaStreamSynchronize(g->st) != cudaSuccess) { s = fail(CES_ERR_CUDA, "ces_gp_mh: kernel failure%s", ""); break; }
-    } while (0);
-    cudaStreamSynchronize(g->st);
-    cudaFree(dbuf);
-    cudaFree(ibuf);
-    return s;
+    ChainRun run(ch, p, g->st);
+    ChainState a;
+    GpPhi phi;
+    phi.k = k; phi.use_variance = use_variance ? 1 : 0; phi.pcn = pcn ? 1 : 0;
+    const double* scales = nullptr;
+    double *mean = nullptr, *var = nullptr;
+    CES_TRY(run.build([&] {
+        a = chain_state(run, ld);
+        phi.ytil = run.put(ytil_host, k);
+        phi.mu = run.put(pcn ? nullptr : mu_host, p);
+        phi.Pinv = run.put(pcn ? nullptr : Pinv_host, (size_t)p * p);
+        scales = run.put(scales_host, (size_t)p * p);
+        phi.mean = mean = run.take((size_t)k * ld);
+        phi.var = var = run.take((size_t)k * ld);
+    }));
+    CES_TRY(gp_predict(g, a.prop, ld, n_chains, mean, ld, var, ld));
+    const unsigned blocks = (unsigned)ceil_div(n_chains, CHAIN_THREADS);
+    chain_init_kernel<<<blocks, CHAIN_THREADS, 0, g->st>>>(a, phi);
+    CES_LAUNCHED(1);
+    for (int it = 0; it < a.n_mcmc; ++it) {
+        gp_propose_kernel<<<(unsigned)ceil_div(n_chains, GP_PROPOSE_THREADS), GP_PROPOSE_THREADS, 0, g->st>>>(a, scales, pcn,
+                                                                                                          beta, it);
+        CES_LAUNCHED(1);
+        CES_TRY(gp_predict(g, a.prop, ld, n_chains, mean, ld, var, ld));
+        chain_accept_kernel<<<blocks, CHAIN_THREADS, 0, g->st>>>(a, phi, it);
+        CES_LAUNCHED(1);
+    }
+    return run.copy_back();
 }

@@ -18,6 +18,7 @@
 // products; the variates themselves can differ from glibc's in the last bit of log).  The other chains use Philox
 // keyed by (seed, chain, iteration).
 #include "kernels.h"
+#include "chains.cuh"
 #include "rng.cuh"
 
 namespace ces {
@@ -25,6 +26,7 @@ namespace ces {
 namespace {
 
 constexpr int MH_P_MAX = 32, MH_K_MAX = 64, MH_WARPS = 4;
+constexpr uint32_t MH_TAG = 0x4d48u;        // Philox counter word of this sampler ("MH")
 
 struct MhArgs {
     int p, k, n_mcmc, n_chains, map_kind, pcn, use_mt;
@@ -45,12 +47,6 @@ struct MhArgs {
     double* mt_gauss;
     unsigned long long seed;
 };
-
-__device__ __forceinline__ double warp_sum_fixed(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
 
 // Phi(x) for the point in xs[0..p) (shared memory of this warp): misfit (+ prior term unless pCN).  gs / ygs: scratch.
 __device__ double mh_phi(const MhArgs& a, const double* xs, double* gs, double* ygs, double* ds, int lane) {
@@ -82,7 +78,7 @@ __device__ double mh_phi(const MhArgs& a, const double* xs, double* gs, double* 
         for (int n = 0; n < k; ++n) t = fma(a.Ginv2[(size_t)m * k + n], ygs[n], t);
         part = fma(ygs[m], t, part);            // yg . solve(2 Gamma, yg)   (:170, :174)
     }
-    double phi = warp_sum_fixed(part);
+    double phi = warp_sum(part);
     if (!a.pcn) {                               // - prior.logpdf(x) up to its constant (cancels in the ratio; :171-176)
         for (int q = lane; q < p; q += 32) ds[q] = xs[q] - a.mu[q];
         __syncwarp();
@@ -92,7 +88,7 @@ __device__ double mh_phi(const MhArgs& a, const double* xs, double* gs, double* 
             for (int n = 0; n < p; ++n) t = fma(a.Pinv[(size_t)q * p + n], ds[n], t);
             pp = fma(0.5 * ds[q], t, pp);
         }
-        phi += warp_sum_fixed(pp);
+        phi += warp_sum(pp);
     }
     __syncwarp();
     return phi;
@@ -144,20 +140,9 @@ __global__ void __launch_bounds__(32 * MH_WARPS) mh_chain_kernel(const MhArgs a)
             }
         } else {
             for (int q2 = lane; 2 * q2 < p; q2 += 32) {             // Box-Muller pairs (2 q2, 2 q2 + 1)
-                uint32_t c[4] = {(uint32_t)it, (uint32_t)chain, (uint32_t)q2, 0x4d48u};
-                philox4(c, (uint32_t)a.seed, (uint32_t)(a.seed >> 32));
-                const double u1 = u53(c[0], c[1]), u2 = u53(c[2], c[3]);
-                const double rad = sqrt(-2.0 * log(u1));
-                double sn, cs;
-                sincospi(2.0 * u2, &sn, &cs);
-                zs[2 * q2] = rad * cs;
-                if (2 * q2 + 1 < p) zs[2 * q2 + 1] = rad * sn;
+                philox_normal_pair(a.seed, it, chain, q2, MH_TAG, &zs[2 * q2], 2 * q2 + 1 < p ? &zs[2 * q2 + 1] : nullptr);
             }
-            if (lane == 31) {                                       // the uniform of the accept test: its own counter
-                uint32_t c[4] = {(uint32_t)it, (uint32_t)chain, 0xffffffffu, 0x4d48u};
-                philox4(c, (uint32_t)a.seed, (uint32_t)(a.seed >> 32));
-                zs[p] = u53(c[0], c[1]);
-            }
+            if (lane == 31) zs[p] = philox_accept_uniform(a.seed, it, chain, MH_TAG);
         }
         __syncwarp();
         for (int q = lane; q < p; q += 32) {
@@ -196,60 +181,36 @@ extern "C" int ces_mcmc_model_mh(void* stream, int map_kind, int64_t p, int64_t 
                                  const double* scales_host, int pcn, double beta, int64_t n_mcmc, int64_t n_chains,
                                  const double* start_host, const double* phi_point_host, uint32_t* mt_state_host,
                                  double* mt_gauss_host, uint64_t seed, double* samples_host, int32_t* accepted_host) {
-    if (p < 1 || p > MH_P_MAX || k < 1 || k > MH_K_MAX || n_mcmc < 1 || n_chains < 1 || !y_host || !Ginv2_host || !scales_host ||
-        !start_host || !phi_point_host || !samples_host || !accepted_host || (!pcn && (!mu_host || !Pinv_host)))
+    const ChainHost h{"ces_mcmc_model_mh", n_mcmc, n_chains, pcn, y_host, scales_host, mu_host, Pinv_host, start_host,
+                      phi_point_host, mt_state_host, mt_gauss_host, seed, samples_host, accepted_host};
+    CES_TRY(chain_check(h));
+    if (p < 1 || p > MH_P_MAX || k < 1 || k > MH_K_MAX || !Ginv2_host)
         return fail(CES_ERR_INVALID, "ces_mcmc_model_mh: needs 1 <= p <= 32, 1 <= k <= 64 and non-null arguments%s", "");
     if (map_kind < CES_MAP_LINEAL || map_kind > CES_MAP_BANANA) return fail(CES_ERR_INVALID, "ces_mcmc_model_mh: unknown map kind%s", "");
     if ((map_kind == CES_MAP_LINEAL || map_kind == CES_MAP_LINEAL_LOG) ? !A_dev : (!params_host || p != 2 || k != 2))
         return fail(CES_ERR_INVALID, "ces_mcmc_model_mh: the map needs A (lineal) or two parameters with p = k = 2%s", "");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const size_t nd = (size_t)k + (size_t)k * k + (size_t)p + 2 * (size_t)p * p + 2 * (size_t)n_chains * p +
-                      (size_t)n_chains * (n_mcmc + 1) * p + 1;
-    double* dbuf = nullptr;
-    uint32_t* ibuf = nullptr;
-    if (cudaMalloc(&dbuf, nd * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return fail(CES_ERR_NOMEM, "ces_mcmc_model_mh: allocation failed%s", ""); }
-    if (cudaMalloc(&ibuf, (626 + (size_t)n_chains) * sizeof(uint32_t)) != cudaSuccess) { cudaFree(dbuf); cudaGetLastError(); return fail(CES_ERR_NOMEM, "ces_mcmc_model_mh: allocation failed%s", ""); }
-    int s = CES_OK;
-    do {
-        double* q = dbuf;
-        auto put = [&](const double* src, size_t n) -> double* {
-            double* dst = q;
-            q += n;
-            if (src && cudaMemcpyAsync(dst, src, n * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess) s = CES_ERR_CUDA;
-            return dst;
-        };
-        MhArgs a;
-        a.p = (int)p; a.k = (int)k; a.n_mcmc = (int)n_mcmc; a.n_chains = (int)n_chains; a.map_kind = map_kind; a.pcn = pcn ? 1 : 0;
-        a.use_mt = mt_state_host != nullptr;
-        a.beta = beta;
-        a.A = A_dev; a.lda = lda; a.b = b_dev;
-        a.par0 = params_host ? params_host[0] : 0.0; a.par1 = params_host ? params_host[1] : 0.0;
-        a.y = put(y_host, k);
-        a.Ginv2 = put(Ginv2_host, (size_t)k * k);
-        a.mu = put(mu_host, p);
-        a.Pinv = put(Pinv_host, (size_t)p * p);
-        a.scales = put(scales_host, (size_t)p * p);
-        a.start = put(start_host, (size_t)n_chains * p);
-        a.phi_point = put(phi_point_host, (size_t)n_chains * p);
-        a.samples = put(nullptr, (size_t)n_chains * (n_mcmc + 1) * p);
-        a.mt_gauss = put(mt_gauss_host && mt_state_host ? mt_gauss_host : nullptr, 1);
-        a.mt = ibuf;
-        a.accepted = reinterpret_cast<int*>(ibuf + 626);
-        a.seed = seed;
-        if (s != CES_OK) { s = fail(CES_ERR_CUDA, "ces_mcmc_model_mh: upload failed%s", ""); break; }
-        if (mt_state_host && cudaMemcpyAsync(ibuf, mt_state_host, 626 * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess) { s = fail(CES_ERR_CUDA, "ces_mcmc_model_mh: upload failed%s", ""); break; }
-        mh_chain_kernel<<<(unsigned)ceil_div(n_chains, MH_WARPS), 32 * MH_WARPS, 0, st>>>(a);
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        if (cudaGetLastError() != cudaSuccess) { s = fail(CES_ERR_CUDA, "ces_mcmc_model_mh: launch failed%s", ""); break; }
-        cudaMemcpyAsync(samples_host, a.samples, (size_t)n_chains * (n_mcmc + 1) * p * sizeof(double), cudaMemcpyDeviceToHost, st);
-        cudaMemcpyAsync(accepted_host, a.accepted, (size_t)n_chains * sizeof(int), cudaMemcpyDeviceToHost, st);
-        if (mt_state_host) {
-            cudaMemcpyAsync(mt_state_host, ibuf, 626 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
-            if (mt_gauss_host) cudaMemcpyAsync(mt_gauss_host, a.mt_gauss, sizeof(double), cudaMemcpyDeviceToHost, st);
-        }
-        if (cudaStreamSynchronize(st) != cudaSuccess) { s = fail(CES_ERR_CUDA, "ces_mcmc_model_mh: kernel failure%s", ""); break; }
-    } while (0);
-    cudaFree(dbuf);
-    cudaFree(ibuf);
-    return s;
+    ChainRun run(h, (int)p, static_cast<cudaStream_t>(stream));
+    MhArgs a;
+    a.p = (int)p; a.k = (int)k; a.n_mcmc = (int)n_mcmc; a.n_chains = (int)n_chains; a.map_kind = map_kind; a.pcn = pcn ? 1 : 0;
+    a.use_mt = mt_state_host != nullptr;
+    a.beta = beta;
+    a.A = A_dev; a.lda = lda; a.b = b_dev;
+    a.par0 = params_host ? params_host[0] : 0.0; a.par1 = params_host ? params_host[1] : 0.0;
+    a.seed = seed;
+    CES_TRY(run.build([&] {
+        a.y = run.put(y_host, k);
+        a.Ginv2 = run.put(Ginv2_host, (size_t)k * k);
+        a.mu = run.put(mu_host, p);
+        a.Pinv = run.put(Pinv_host, (size_t)p * p);
+        a.scales = run.put(scales_host, (size_t)p * p);
+        a.start = run.put(start_host, (size_t)n_chains * p);
+        a.phi_point = run.put(phi_point_host, (size_t)n_chains * p);
+        a.samples = run.samples;
+        a.accepted = run.accepted;
+        a.mt = run.mt;
+        a.mt_gauss = run.mt_gauss;
+    }));
+    mh_chain_kernel<<<(unsigned)ceil_div(n_chains, MH_WARPS), 32 * MH_WARPS, 0, run.st>>>(a);
+    CES_LAUNCHED(1);
+    return run.copy_back();
 }

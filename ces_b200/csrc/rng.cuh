@@ -80,12 +80,31 @@ __device__ __forceinline__ double u53(uint32_t hi, uint32_t lo) {
     return ((double)((((unsigned long long)hi << 32) | lo) >> 11) + 0.5) * (1.0 / 9007199254740992.0);
 }
 
+// Philox4x32-10 keyed by `seed` at the counter (it, c, j, tag): the Box-Muller pair, normals 2 j and 2 j + 1 of chain c at
+// step it, into *z0 and (unless z1 is NULL, when p is odd) *z1.  `tag` keeps the streams of different samplers apart.
+__device__ __forceinline__ void philox_normal_pair(unsigned long long seed, int it, int c, int j, uint32_t tag, double* z0,
+                                                   double* z1) {
+    uint32_t ctr[4] = {(uint32_t)it, (uint32_t)c, (uint32_t)j, tag};
+    philox4(ctr, (uint32_t)seed, (uint32_t)(seed >> 32));
+    const double u1 = u53(ctr[0], ctr[1]), u2 = u53(ctr[2], ctr[3]);
+    const double rad = sqrt(-2.0 * log(u1));
+    double sn, cs;
+    sincospi(2.0 * u2, &sn, &cs);
+    *z0 = rad * cs;
+    if (z1) *z1 = rad * sn;
+}
+// the accept test's uniform of chain c at step it: its own counter (it, c, 0xffffffff, tag)
+__device__ __forceinline__ double philox_accept_uniform(unsigned long long seed, int it, int c, uint32_t tag) {
+    uint32_t ctr[4] = {(uint32_t)it, (uint32_t)c, 0xffffffffu, tag};
+    philox4(ctr, (uint32_t)seed, (uint32_t)(seed >> 32));
+    return u53(ctr[0], ctr[1]);
+}
+
 // The random numbers of one proposal of chain c at step it, for the samplers that step all chains in lockstep
 // (emulate.cu, darcy_mh.cu): z[q * zstride] ~ N(0, 1) for q < p, and the accept test's uniform as the return value.
 // With mt != nullptr the chain consumes numpy's stream (mt: 624 key words, position, has_gauss; *cached: the cached
 // variate) in the order np.random.normal(0, 1, p) then np.random.uniform() draw, and the advanced state is written back.
-// Otherwise Box-Muller pairs (2 j, 2 j + 1) come from Philox4x32-10 keyed by `seed` with the counter (it, c, j, tag), and
-// the uniform from the counter (it, c, 0xffffffff, tag); `tag` keeps the streams of different samplers apart.
+// Otherwise the normals and the uniform come from philox_normal_pair and philox_accept_uniform.
 __device__ inline double mh_chain_draw(int p, int it, int c, uint32_t* mt, double* cached, unsigned long long seed,
                                        uint32_t tag, double* z, int zstride) {
     if (mt) {
@@ -96,20 +115,11 @@ __device__ inline double mh_chain_draw(int p, int it, int c, uint32_t* mt, doubl
         mt[624] = (uint32_t)rng.pos; mt[625] = (uint32_t)rng.has_gauss; cached[0] = rng.gauss;
         return u;
     }
-    const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
     for (int q2 = 0; 2 * q2 < p; ++q2) {
-        uint32_t ctr[4] = {(uint32_t)it, (uint32_t)c, (uint32_t)q2, tag};
-        philox4(ctr, k0, k1);
-        const double u1 = u53(ctr[0], ctr[1]), u2 = u53(ctr[2], ctr[3]);
-        const double rad = sqrt(-2.0 * log(u1));
-        double sn, cs;
-        sincospi(2.0 * u2, &sn, &cs);
-        z[(size_t)(2 * q2) * zstride] = rad * cs;
-        if (2 * q2 + 1 < p) z[(size_t)(2 * q2 + 1) * zstride] = rad * sn;
+        philox_normal_pair(seed, it, c, q2, tag, &z[(size_t)(2 * q2) * zstride],
+                           2 * q2 + 1 < p ? &z[(size_t)(2 * q2 + 1) * zstride] : nullptr);
     }
-    uint32_t ctr[4] = {(uint32_t)it, (uint32_t)c, 0xffffffffu, tag};
-    philox4(ctr, k0, k1);
-    return u53(ctr[0], ctr[1]);
+    return philox_accept_uniform(seed, it, c, tag);
 }
 
 }  // namespace ces

@@ -25,6 +25,7 @@ numbers are ``model_mh``'s.
 from __future__ import print_function
 
 import ctypes
+import types
 
 import numpy as np
 
@@ -61,56 +62,18 @@ class MCMC(object):
             if int(model.p) != p or np.size(obs) != k:
                 raise ValueError("model_mh: the Darcy model has p = %d and %d observed cells, the ensemble p = %d and n_obs = %d"
                                  % (int(model.p), np.size(obs), p, k))
-        pcn = kwargs.get('update', None) == 'pCN'
         if kwargs.get('update', None) not in (None, 'pCN'):
             raise ValueError("unknown update %r" % (kwargs.get('update'),))     # the reference would fail on `proposal`
-        # RW needs the proposal distribution (:123-129); pCN proposes according to the prior
-        if enka_scaling:
-            scales = delta * np.linalg.cholesky(np.cov(enka.Ustar).reshape(p, p))
-        else:
-            scales = delta * np.eye(p)
-        if pcn:
-            scales = np.linalg.cholesky(np.asarray(prior.cov, dtype=np.float64).reshape(p, p))
-        mean = np.asarray(enka.Ustar, dtype=np.float64).mean(axis=1)            # :131
+        pcn = kwargs.get('update', None) == 'pCN'
+        c = self._chains(p, n_mcmc, prior, enka, delta, enka_scaling, pcn, float(kwargs.get('beta', 0.5)),
+                         int(kwargs.get('n_chains', 1)), int(kwargs.get('seed', 0)))
         y = np.ascontiguousarray(np.asarray(self.y_obs, dtype=np.float64).reshape(k))
         Gam = np.asarray(Gamma, dtype=np.float64).reshape(k, k)
         Ginv2 = np.ascontiguousarray(np.linalg.inv(2.0 * Gam))
-        mu = Pinv = None
-        if not pcn:
-            mu = np.ascontiguousarray(np.asarray(prior.mean, dtype=np.float64).reshape(p))
-            Pinv = np.ascontiguousarray(np.linalg.inv(np.asarray(prior.cov, dtype=np.float64).reshape(p, p)))
-        # resume (:156-164): continue from the last sample; Phi_current stays the ensemble mean's, like the reference
-        previous = None
-        if hasattr(self, 'samples'):
-            previous = np.asarray(self.samples, dtype=np.float64)
-            first = previous[:, -1].copy()
-        else:
-            first = mean.copy()
-        n_chains = int(kwargs.get('n_chains', 1))
-        seed = int(kwargs.get('seed', 0))
-        start = np.tile(first, (n_chains, 1))
-        if n_chains > 1:
-            # the extra chains start from ensemble members (over-dispersed starts), deterministically chosen
-            J = enka.Ustar.shape[1]
-            start[1:] = np.asarray(enka.Ustar, dtype=np.float64).T[np.arange(1, n_chains) % J]
-        phi_point = np.tile(mean, (n_chains, 1))
-        phi_point[1:] = start[1:]
-        # numpy's global generator: ('MT19937', key[624], pos, has_gauss, cached_gaussian)
-        st = np.random.get_state()
-        mt = np.empty(626, dtype=np.uint32)
-        mt[:624], mt[624], mt[625] = st[1], st[2], st[3]
-        gauss = np.array([st[4]], dtype=np.float64)
-        samples = np.empty((n_chains, int(n_mcmc) + 1, p))
-        accepted = np.zeros(n_chains, dtype=np.int32)
-        # arguments shared by both device samplers, from y onwards (include/ces_b200.h)
-        common = (_lib.host_ptr(y), _lib.host_ptr(Ginv2), _lib.host_ptr(mu) if mu is not None else None,
-                  _lib.host_ptr(Pinv) if Pinv is not None else None, _lib.host_ptr(np.ascontiguousarray(scales, dtype=np.float64)),
-                  1 if pcn else 0, float(kwargs.get('beta', 0.5)), int(n_mcmc), n_chains, _lib.host_ptr(start),
-                  _lib.host_ptr(phi_point), mt.ctypes.data, _lib.host_ptr(gauss), seed, _lib.host_ptr(samples),
-                  accepted.ctypes.data)
         if darcy:
             # chains stepped in lockstep through the batched Darcy solver (csrc/darcy_mh.cu), with the model's tol / max_iter
-            _lib.check(_lib.load().ces_darcy_mh(model._handle(True), float(model.tol), int(model.max_iter), *common))
+            _lib.check(_lib.load().ces_darcy_mh(model._handle(True), float(model.tol), int(model.max_iter),
+                                                _lib.host_ptr(y), _lib.host_ptr(Ginv2), *c.args))
         else:
             A_dev, lda, b_dev, params = model._device_args(torch)
             par = np.ascontiguousarray(params, dtype=np.float64) if params is not None else None
@@ -119,17 +82,8 @@ class MCMC(object):
                 ctypes.c_void_p(stream), _lib.MAPS[kind], p, k,
                 ctypes.c_void_p(A_dev.data_ptr()) if A_dev is not None else None, int(lda),
                 ctypes.c_void_p(b_dev.data_ptr()) if b_dev is not None else None,
-                _lib.host_ptr(par) if par is not None else None, *common))
-        np.random.set_state(('MT19937', mt[:624].copy(), int(mt[624]), int(mt[625]), float(gauss[0])))
-        chain0 = samples[0]
-        if previous is not None:
-            # the reference appends to list(self.samples.T) WITHOUT repeating the state it resumes from (:158-160)
-            chain0 = np.vstack([previous.T, samples[0][1:]])
-        self.samples = np.array(chain0).T                    # (p, n + 1), :195
-        self.accept = accepted[0] / float(n_mcmc)            # :196
-        if n_chains > 1:
-            self.samples_chains = samples.transpose(0, 2, 1)     # (n_chains, p, n + 1)
-            self.accept_chains = accepted / float(n_mcmc)
+                _lib.host_ptr(par) if par is not None else None, _lib.host_ptr(y), _lib.host_ptr(Ginv2), *c.args))
+        self._publish(c, n_mcmc)
 
     def emulator_mh(self, emulator, n_mcmc, prior, enka, delta=1., enka_scaling=True, update=None, beta=0.5, n_chains=1,
                     seed=0, use_variance=True):
@@ -140,53 +94,68 @@ class MCMC(object):
         p, k = int(emulator.p), int(emulator.k)
         if update not in (None, 'pCN'):
             raise ValueError("unknown update %r" % (update,))
-        pcn = update == 'pCN'
+        c = self._chains(p, n_mcmc, prior, enka, delta, enka_scaling, update == 'pCN', float(beta), int(n_chains), int(seed))
+        ytil = np.ascontiguousarray(emulator.transform @ np.asarray(self.y_obs, dtype=np.float64).reshape(k))
+        emulator.condition()
+        _lib.check(_lib.load().ces_gp_mh(emulator._h, _lib.host_ptr(ytil), 1 if use_variance else 0, *c.args))
+        self._publish(c, n_mcmc)
+
+    def _chains(self, p, n_mcmc, prior, enka, delta, enka_scaling, pcn, beta, n_chains, seed):
+        """The host set-up every device sampler shares (ces/sample.py:123-166): proposal scales, prior mean / precision
+        unless pCN, resume, every chain's start and phi_point, numpy's generator state and the output buffers.  ``args``
+        are the C arguments from mu_host onwards (include/ces_b200.h)."""
+        # RW needs the proposal distribution (:123-129); pCN proposes according to the prior
         if enka_scaling:
             scales = delta * np.linalg.cholesky(np.cov(enka.Ustar).reshape(p, p))
         else:
             scales = delta * np.eye(p)
         if pcn:
             scales = np.linalg.cholesky(np.asarray(prior.cov, dtype=np.float64).reshape(p, p))
-        mean = np.asarray(enka.Ustar, dtype=np.float64).mean(axis=1)
-        ytil = np.ascontiguousarray(emulator.transform @ np.asarray(self.y_obs, dtype=np.float64).reshape(k))
+        mean = np.asarray(enka.Ustar, dtype=np.float64).mean(axis=1)            # :131
         mu = Pinv = None
         if not pcn:
             mu = np.ascontiguousarray(np.asarray(prior.mean, dtype=np.float64).reshape(p))
             Pinv = np.ascontiguousarray(np.linalg.inv(np.asarray(prior.cov, dtype=np.float64).reshape(p, p)))
-        previous = None
+        # resume (:156-164): continue from the last sample; Phi_current stays the ensemble mean's, like the reference
+        c = types.SimpleNamespace(previous=None)
         if hasattr(self, 'samples'):
-            previous = np.asarray(self.samples, dtype=np.float64)
-            first = previous[:, -1].copy()
+            c.previous = np.asarray(self.samples, dtype=np.float64)
+            first = c.previous[:, -1].copy()
         else:
             first = mean.copy()
-        n_chains = int(n_chains)
         start = np.tile(first, (n_chains, 1))
         if n_chains > 1:
+            # the extra chains start from ensemble members (over-dispersed starts), deterministically chosen
             J = enka.Ustar.shape[1]
             start[1:] = np.asarray(enka.Ustar, dtype=np.float64).T[np.arange(1, n_chains) % J]
         phi_point = np.tile(mean, (n_chains, 1))
         phi_point[1:] = start[1:]
+        # numpy's global generator: ('MT19937', key[624], pos, has_gauss, cached_gaussian)
         st = np.random.get_state()
-        mt = np.empty(626, dtype=np.uint32)
-        mt[:624], mt[624], mt[625] = st[1], st[2], st[3]
-        gauss = np.array([st[4]], dtype=np.float64)
-        samples = np.empty((n_chains, int(n_mcmc) + 1, p))
-        accepted = np.zeros(n_chains, dtype=np.int32)
-        emulator.condition()
-        _lib.check(_lib.load().ces_gp_mh(
-            emulator._h, _lib.host_ptr(ytil), 1 if use_variance else 0, _lib.host_ptr(mu) if mu is not None else None,
-            _lib.host_ptr(Pinv) if Pinv is not None else None, _lib.host_ptr(np.ascontiguousarray(scales, dtype=np.float64)),
-            1 if pcn else 0, float(beta), int(n_mcmc), n_chains, _lib.host_ptr(start), _lib.host_ptr(phi_point),
-            mt.ctypes.data, _lib.host_ptr(gauss), int(seed), _lib.host_ptr(samples), accepted.ctypes.data))
-        np.random.set_state(('MT19937', mt[:624].copy(), int(mt[624]), int(mt[625]), float(gauss[0])))
-        chain0 = samples[0]
-        if previous is not None:
-            chain0 = np.vstack([previous.T, samples[0][1:]])
-        self.samples = np.array(chain0).T
-        self.accept = accepted[0] / float(n_mcmc)
-        if n_chains > 1:
-            self.samples_chains = samples.transpose(0, 2, 1)
-            self.accept_chains = accepted / float(n_mcmc)
+        c.mt = np.empty(626, dtype=np.uint32)
+        c.mt[:624], c.mt[624], c.mt[625] = st[1], st[2], st[3]
+        c.gauss = np.array([st[4]], dtype=np.float64)
+        c.samples = np.empty((n_chains, int(n_mcmc) + 1, p))
+        c.accepted = np.zeros(n_chains, dtype=np.int32)
+        # the C arguments point into these arrays: they live as long as c
+        c.inputs = (mu, Pinv, np.ascontiguousarray(scales, dtype=np.float64), start, phi_point)
+        mu_p, Pinv_p, scales_p, start_p, phi_p = (_lib.host_ptr(a) if a is not None else None for a in c.inputs)
+        c.args = (mu_p, Pinv_p, scales_p, 1 if pcn else 0, beta, int(n_mcmc), n_chains, start_p, phi_p, c.mt.ctypes.data,
+                  _lib.host_ptr(c.gauss), seed, _lib.host_ptr(c.samples), c.accepted.ctypes.data)
+        return c
+
+    def _publish(self, c, n_mcmc):
+        """After a successful device run: numpy's advanced generator state and the results attributes of model_mh."""
+        np.random.set_state(('MT19937', c.mt[:624].copy(), int(c.mt[624]), int(c.mt[625]), float(c.gauss[0])))
+        chain0 = c.samples[0]
+        if c.previous is not None:
+            # the reference appends to list(self.samples.T) WITHOUT repeating the state it resumes from (:158-160)
+            chain0 = np.vstack([c.previous.T, c.samples[0][1:]])
+        self.samples = np.array(chain0).T                    # (p, n + 1), :195
+        self.accept = c.accepted[0] / float(n_mcmc)          # :196
+        if len(c.accepted) > 1:
+            self.samples_chains = c.samples.transpose(0, 2, 1)     # (n_chains, p, n + 1)
+            self.accept_chains = c.accepted / float(n_mcmc)
 
     def random_walk(self, current, scales, n_dim):
         """ces/sample.py:198-199 (host helper, kept for API parity; the device chains draw their own)."""

@@ -307,7 +307,10 @@ int ces_posv(void* stream, double* A_dev, int64_t lda, int64_t n, double* B_dev,
  * global MT19937 stream exactly as np.random.normal(0, 1, p) followed by np.random.uniform() would -- mt_state_host =
  * 624 key words, position, has_gauss flag (626 uint32), *mt_gauss_host = the cached Gaussian; both are updated to the
  * state after the run --; every other chain (all of them with NULL) draws from Philox keyed by (seed, chain, iteration).
- * Outputs: samples (n_chains x (n_mcmc + 1) x p, state 0 = start) and the number of accepted proposals per chain. */
+ * Outputs: samples (n_chains x (n_mcmc + 1) x p, state 0 = start) and the number of accepted proposals per chain.
+ * Limits shared by every sampler (ces_darcy_mh, ces_gp_mh too): 1 <= n_mcmc < 2^31 - 1, 1 <= n_chains <= 2^24, mt_gauss_host
+ * non-NULL whenever mt_state_host is, mu_host / Pinv_host non-NULL unless pcn; otherwise CES_ERR_INVALID before any
+ * device work.  A samples buffer beyond 4e18 bytes returns CES_ERR_NOMEM.  Synchronises. */
 int ces_mcmc_model_mh(void* stream, int map_kind, int64_t p, int64_t k, const double* A_dev, int64_t lda,
                       const double* b_dev, const double* params_host, const double* y_host, const double* Ginv2_host,
                       const double* mu_host, const double* Pinv_host, const double* scales_host, int pcn, double beta,
@@ -325,8 +328,8 @@ int ces_mcmc_model_mh(void* stream, int map_kind, int64_t p, int64_t k, const do
  * GEMMs, so p and n_obs are limited only by the model.  Arguments from y_host onwards as ces_mcmc_model_mh (p and
  * k = n_obs are the model's).  If any solve -- the initial one at phi_point or a proposal's -- reaches max_iter, returns
  * CES_ERR_STATE naming the first such step and leaves samples, acceptances and the generator state untouched.
- * A model without obs_index, NULL pointers, n_mcmc < 1 or n_chains < 1 return CES_ERR_INVALID before any device work.
- * Synchronises. */
+ * The limits of ces_mcmc_model_mh apply (checked before the model); a model without obs_index also returns
+ * CES_ERR_INVALID before any device work.  Synchronises. */
 int ces_darcy_mh(void* model, double tol, int max_iter, const double* y_host, const double* Ginv2_host,
                  const double* mu_host, const double* Pinv_host, const double* scales_host, int pcn, double beta,
                  int64_t n_mcmc, int64_t n_chains, const double* start_host, const double* phi_point_host,
@@ -364,7 +367,7 @@ int ces_gp_predict(void* model, const double* U_dev, int64_t ldu, int64_t m, dou
  * mu_host onwards as there) with the forward misfit replaced by the emulated one at the whitened data ytil_host (k):
  *   Phi(u) = 1/2 sum_i (ytil_i - mean_i(u))^2 / (1 + var_i(u)) + 1/2 sum_i log(1 + var_i(u))   (use_variance != 0)
  *   Phi(u) = 1/2 sum_i (ytil_i - mean_i(u))^2                                                  (use_variance == 0)
- * Needs ces_gp_condition.  Synchronises. */
+ * The limits of ces_mcmc_model_mh apply (checked before the model).  Needs ces_gp_condition.  Synchronises. */
 int ces_gp_mh(void* model, const double* ytil_host, int use_variance, const double* mu_host, const double* Pinv_host,
               const double* scales_host, int pcn, double beta, int64_t n_mcmc, int64_t n_chains, const double* start_host,
               const double* phi_point_host, uint32_t* mt_state_host, double* mt_gauss_host, uint64_t seed,
