@@ -441,9 +441,9 @@ __global__ void __launch_bounds__(256) fill_normal_kernel(double* __restrict__ X
         k0 += 0x9E3779B9u;
         k1 += 0xBB67AE85u;
     }
-    const double two53 = 1.0 / 9007199254740992.0;
-    const double u1 = ((double)((((unsigned long long)c[0] << 32) | c[1]) >> 11) + 0.5) * two53;   // (0, 1)
-    const double u2 = ((double)((((unsigned long long)c[2] << 32) | c[3]) >> 11) + 0.5) * two53;
+    const double two53 = 1.0 / 9007199254740992.0;      // (0, 1): the top 53-bit value would round to 1.0 without the fmin
+    const double u1 = fmin(((double)((((unsigned long long)c[0] << 32) | c[1]) >> 11) + 0.5) * two53, 1.0 - two53);
+    const double u2 = fmin(((double)((((unsigned long long)c[2] << 32) | c[3]) >> 11) + 0.5) * two53, 1.0 - two53);
     const double rad = sqrt(-2.0 * log(u1));
     double sn, cs;
     sincospi(2.0 * u2, &sn, &cs);

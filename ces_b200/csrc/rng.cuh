@@ -75,9 +75,11 @@ __device__ __forceinline__ void philox4(uint32_t (&c)[4], uint32_t k0, uint32_t 
         k1 += 0xBB67AE85u;
     }
 }
-// uniform in (0, 1) from 53 bits of a Philox output pair
+// uniform in (0, 1) from 53 bits of a Philox output pair.  The top value 2^53 - 1 + 1/2 rounds to 2^53 in double: the fmin
+// keeps it below 1, and every other value is (n + 1/2) / 2^53 as rounded.
 __device__ __forceinline__ double u53(uint32_t hi, uint32_t lo) {
-    return ((double)((((unsigned long long)hi << 32) | lo) >> 11) + 0.5) * (1.0 / 9007199254740992.0);
+    return fmin(((double)((((unsigned long long)hi << 32) | lo) >> 11) + 0.5) * (1.0 / 9007199254740992.0),
+                1.0 - 1.0 / 9007199254740992.0);
 }
 
 // Philox4x32-10 keyed by `seed` at the counter (it, c, j, tag): the Box-Muller pair, normals 2 j and 2 j + 1 of chain c at

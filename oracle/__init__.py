@@ -22,6 +22,10 @@ mcmc_oracle      numpy restatement of ``MCMC.model_mh`` (ces/sample.py:121-196).
                  (tests/golden/mcmc_cases.npz; tests/test_oracle_mcmc.py).
 darcy_pcg_oracle / lorenz_oracle   restatements of the device's own solver / RK4 scheme (see
                  their headers).
+philox_oracle    numpy restatement of the device's Philox4x32-10 streams
+                 (``ces_fill_normal`` and the MH chains beside chain 0).  Parity
+                 PINNED to the Random123 known-answer vectors
+                 (tests/test_philox_oracle.py).
 reference_loader loads the real reference from /root/reference when present
                  (never at run time on the GPU box).
 """

@@ -117,9 +117,10 @@ def phi(mean, var, ytil, use_variance=True):
 
 
 def emulator_mh(predict_one, n_mcmc, prior, Ustar, ytil, delta=1.0, enka_scaling=True, update=None, beta=0.5,
-                samples=None, use_variance=True):
+                samples=None, use_variance=True, start=None, noise=None):
     """One chain of ``MCMC.emulator_mh``: ``model_mh``'s loop (oracle/mcmc_oracle.py) with Phi the emulated misfit at the
-    whitened data ``ytil``; ``predict_one(u) -> (mean (k), var (k))``.  Returns ``(samples, accept_rate)``."""
+    whitened data ``ytil``; ``predict_one(u) -> (mean (k), var (k))``.  ``start`` and ``noise`` as in
+    ``mcmc_oracle.model_mh``.  Returns ``(samples, accept_rate)``."""
     Ustar = np.asarray(Ustar, dtype=float)
     p = Ustar.shape[0]
     if enka_scaling:
@@ -135,7 +136,7 @@ def emulator_mh(predict_one, n_mcmc, prior, Ustar, ytil, delta=1.0, enka_scaling
             v -= prior.logpdf(theta)
         return v
 
-    current = Ustar.mean(axis=1)
+    current = Ustar.mean(axis=1) if start is None else np.asarray(start, dtype=float)
     phi_current = Phi(current)
     if samples is not None:
         chain = list(np.asarray(samples).T)
@@ -143,14 +144,16 @@ def emulator_mh(predict_one, n_mcmc, prior, Ustar, ytil, delta=1.0, enka_scaling
     else:
         chain = [current.flatten()]
     accept = 0.0
-    for _ in range(int(n_mcmc)):
-        z = np.random.normal(0, 1, p)
+    for it in range(int(n_mcmc)):
+        z, u = noise(it) if noise is not None else (np.random.normal(0, 1, p), None)
         if update is None:
             proposal = current + np.matmul(scales, z)
         else:
             proposal = np.sqrt(1 - beta ** 2) * current + np.sqrt(beta) * np.matmul(scales, z)
         phi_proposal = Phi(proposal)
-        if np.log(np.random.uniform()) < phi_current - phi_proposal:
+        if u is None:
+            u = np.random.uniform()
+        if np.log(u) < phi_current - phi_proposal:
             current = np.copy(proposal)
             phi_current = phi_proposal
             accept += 1.0

@@ -12,14 +12,18 @@ The restatement is functional where the reference is a method with state on ``se
 resume state (``self.samples``) is passed in and returned.  Random numbers come from numpy's global generator in the
 reference's order: ``normal(0, 1, p)`` for the proposal (:198-202), whatever the model draws in its evaluation (the
 reference's ``banana`` draws ``normal(0, 1, [2])`` even without noise, ces/utils.py:122 -- pass ``forward_draws=2``), then
-``uniform()`` for the accept test (:182).
+``uniform()`` for the accept test (:182).  The device chains beside the reference's one are restated with ``start``, their
+first state (also the point of the initial Phi), and ``noise``, their Philox draws (oracle/philox_oracle.py).
 """
 import numpy as np
 
 
 def model_mh(forward, n_mcmc, prior, Ustar, y_obs, Gamma, delta=1.0, enka_scaling=True, update=None, beta=0.5,
-             samples=None, forward_draws=0):
-    """Returns ``(samples (p, n + 1 [+ previous]), accept_rate)``.  ``prior``: object with ``logpdf`` and ``cov``."""
+             samples=None, forward_draws=0, start=None, noise=None):
+    """Returns ``(samples (p, n + 1 [+ previous]), accept_rate)``.  ``prior``: object with ``logpdf`` and ``cov``.
+    ``start``: the first state and the point of the initial Phi (default: the ensemble mean).  ``noise``: a callable
+    ``it -> (z (p), u)`` giving step it's normals and accept uniform (default: numpy's global generator, in the
+    reference's order)."""
     Ustar = np.asarray(Ustar, dtype=float)
     p = Ustar.shape[0]
     if enka_scaling:                                                      # :123-126
@@ -34,7 +38,7 @@ def model_mh(forward, n_mcmc, prior, Ustar, y_obs, Gamma, delta=1.0, enka_scalin
             np.random.normal(0, 1, [forward_draws])                       # drawn inside the reference's model call
         return np.asarray(forward(theta), dtype=float)
 
-    current = Ustar.mean(axis=1)                                          # :131
+    current = Ustar.mean(axis=1) if start is None else np.asarray(start, dtype=float)   # :131
     yg = G(current.flatten()) - y_obs                                     # :137-139
     phi_current = (yg * np.linalg.solve(2 * Gamma, yg)).sum()             # :140
     if update != "pCN":
@@ -45,8 +49,8 @@ def model_mh(forward, n_mcmc, prior, Ustar, y_obs, Gamma, delta=1.0, enka_scalin
     else:
         chain = [current.flatten()]
     accept = 0.0
-    for _ in range(int(n_mcmc)):
-        z = np.random.normal(0, 1, p)
+    for it in range(int(n_mcmc)):
+        z, u = noise(it) if noise is not None else (np.random.normal(0, 1, p), None)
         if update is None:                                                # :167-168, :198-199
             proposal = current + np.matmul(scales, z)
         else:                                                             # :169-170, :201-202
@@ -55,7 +59,9 @@ def model_mh(forward, n_mcmc, prior, Ustar, y_obs, Gamma, delta=1.0, enka_scalin
         phi_proposal = (yg * np.linalg.solve(2 * Gamma, yg)).sum()
         if update != "pCN":
             phi_proposal -= prior.logpdf(proposal.flatten())              # :179-182
-        if np.log(np.random.uniform()) < phi_current - phi_proposal:      # :188-191
+        if u is None:
+            u = np.random.uniform()
+        if np.log(u) < phi_current - phi_proposal:                        # :188-191
             current = np.copy(proposal)
             phi_current = np.copy(phi_proposal)
             accept += 1.0
