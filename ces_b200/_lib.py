@@ -16,6 +16,7 @@ CES_ERR_INVALID, CES_ERR_STATE, CES_ERR_ALIGN, CES_ERR_NOT_SPD, CES_ERR_CUDA, CE
 RULES = {"eks": 0, "aldi": 1, "aldi_constant": 2, "eki": 3}
 TS_FROBENIUS, TS_FIXED, TS_KEEP = 0, 1, 2
 FORMULATIONS = {"interaction": 0, "factored": 1}
+NOISES = {"cholesky": 0, "ensemble": 1}            # CES_NOISE_*
 MAPS = {"lineal": 0, "lineal_log": 1, "elliptic": 2, "banana": 3}
 GP_KERNELS = {"SquaredExponential": 0, "Matern12": 1, "Matern32": 2, "Matern52": 3}   # CES_GP_* (GPflow's class names)
 
@@ -32,7 +33,7 @@ EXPORTS = (
     "ces_host_centre_u", "ces_host_interact_own", "ces_host_update", "ces_ipc_export", "ces_ipc_import", "ces_peer_gather",
     "ces_peer_gather_wait", "ces_host_interact_chunk", "ces_small_run", "ces_mcmc_model_mh", "ces_host_chunk_schedule",
     "ces_gp_create", "ces_gp_destroy", "ces_gp_lml", "ces_gp_condition", "ces_gp_predict", "ces_gp_mh", "ces_darcy_mh",
-    "ces_gp_set_kernel",
+    "ces_gp_set_kernel", "ces_set_noise", "ces_fill_ensemble_noise",
 )
 
 _i64, _int, _dbl, _vp = ctypes.c_int64, ctypes.c_int, ctypes.c_double, ctypes.c_void_p
@@ -126,6 +127,8 @@ def load():
     lib.ces_darcy_last_stats.argtypes = [_vp, ctypes.POINTER(_i64), ctypes.POINTER(_i64), ctypes.POINTER(_dbl)]
     lib.ces_frobenius.argtypes = [_vp, _dp, _i64, _i64, _i64, ctypes.POINTER(_dbl)]
     lib.ces_fill_normal.argtypes = [_vp, ctypes.c_uint64, ctypes.c_uint64, _dp, _i64, _i64, _i64, _i64]
+    lib.ces_set_noise.argtypes = [_vp, _int, ctypes.c_uint64, ctypes.c_uint64, _dp, _i64]
+    lib.ces_fill_ensemble_noise.argtypes = [_vp, ctypes.c_uint64, ctypes.c_uint64, _dp, _i64, _i64, _i64, _i64, _i64]
     lib.ces_gemm.argtypes = [_vp, _int, _int, _i64, _i64, _i64, _dbl, _dp, _i64, _dp, _i64, _dbl, _dp, _i64]
     lib.ces_potrf.argtypes = [_vp, _dp, _i64, _i64]
     lib.ces_posv.argtypes = [_vp, _dp, _i64, _i64, _dp, _i64, _i64]

@@ -29,6 +29,12 @@ ces/calibrate.py:404-416).  What differs is where the arithmetic runs:
   two k x k Gram matrices -- identical to rounding (~1e-15), ``O(d k J + k^2 J)`` instead of ``O((k + d) J^2)``.
 * ``rng='device'`` (kwarg of ``run`` or attribute, with ``seed``) generates the noise on the GPU (Philox + Box-Muller,
   ``ces_fill_normal``) instead of drawing it with numpy on the host: a different but equally distributed stream.
+* ``noise='ensemble'`` (kwarg of ``run`` / ``eks_update*`` or attribute; default ``'cholesky'``, the reference's
+  ``sqrt(2h) chol(C^uu) xi``) forms the noise of eks / aldi / aldi_constant from the ensemble itself:
+  ``sqrt(2h / n_C) (U - ubar) xi`` with a J x J ``xi`` (n_C = J for eks, J - 1 for the aldi rules; DESIGN.md section 4g).
+  Same covariance as the Cholesky form minus its 1e-8 regularisation, but inside span(U - ubar) and without a
+  factorisation.  ``xi`` is drawn on the device from ``seed`` at step ``len(self.metrics['t'])`` unless passed as
+  ``xi=``; numpy's global generator is not advanced by the update and ``rng`` does not apply.
 * Multi-GPU: if ``self.group`` is a ``torch.distributed`` process group, every rank
   calls ``run`` with the same arguments and the ensemble is sharded by particle
   columns (SURVEY.md section 8e).
@@ -454,6 +460,26 @@ class sampling(enka):
                 "time_step='adaptive' calls a method the reference does not define (ces/calibrate.py:255)")
         raise ValueError("unknown time_step %r" % (kind,))
 
+    def _noise_options(self, rule, kwargs, J, cols=None):
+        """(ensemble?, explicit J x J xi or None) from the ``noise`` kwarg / attribute, checked before any device work.
+        ``cols``: this rank's column count when the caller may pass only its own columns of xi (``local_shard``)."""
+        mode = kwargs.get('noise', getattr(self, 'noise', 'cholesky'))
+        if mode not in ('cholesky', 'ensemble'):
+            raise ValueError("noise must be 'cholesky' or 'ensemble', got %r" % (mode,))
+        if mode == 'cholesky' or rule == 'eki':                  # eki has no noise term
+            return False, None
+        if kwargs.get('formulation', getattr(self, 'formulation', 'interaction')) == 'factored':
+            raise ValueError("noise='ensemble' needs formulation='interaction': the factored formulation never gathers "
+                             "U - ubar")
+        xi = kwargs.get('xi', None)
+        if xi is None:
+            return True, None
+        xi = np.asarray(xi, dtype=np.float64)
+        shapes = [(J, J)] + ([(J, cols)] if cols is not None else [])
+        if xi.ndim != 2 or xi.shape not in shapes:
+            raise ValueError("noise='ensemble' takes xi of shape %s, got %s" % (" or ".join(map(str, shapes)), xi.shape))
+        return True, xi
+
     # ------------------------------------------------------------------ single updates on numpy arrays
     def _update_host(self, rule, y_obs, U0, Geval, Gamma, kwargs):
         self._ensure_metrics()
@@ -461,11 +487,27 @@ class sampling(enka):
         U0 = np.asarray(U0, dtype=np.float64)
         group = getattr(self, 'group', None)
         local = bool(kwargs.get('local_shard', False)) and group is not None
-        eng = self._get_engine(self.J if local else U0.shape[1], group)
+        Jg = self.J if local else U0.shape[1]
+        cols = None
+        if local:
+            import torch.distributed as dist
+
+            from .engine import shard_range
+
+            lo, hi = shard_range(Jg, dist.get_rank(group), dist.get_world_size(group))
+            cols = hi - lo
+        ensemble, xi_ens = self._noise_options(rule, kwargs, Jg, cols)
+        eng = self._get_engine(Jg, group)
         stale = self._sync_problem(eng, y_obs, Gamma, defer_large=True)
         Gk = np.asarray(Geval, dtype=np.float64)[:self.n_obs]
         xi = None
-        if rule != 'eki':
+        noise = None
+        if ensemble:
+            # the J x J xi: this rank's columns of the caller's array, or the device's Philox stream keyed by the step
+            if xi_ens is not None and xi_ens.shape[1] == eng.J and eng.cols != eng.J:
+                xi_ens = xi_ens[:, eng.col_lo:eng.col_hi]
+            noise = ('ensemble', int(kwargs.get('seed', getattr(self, 'seed', 0))), len(self.metrics['t']), xi_ens)
+        elif rule != 'eki':
             # the full (p, J) draw on every rank -- the same global stream as the reference -- unless the caller
             # passes its own (possibly sharded) noise
             xi = self._draw_noise((U0.shape[0], eng.J), kwargs)
@@ -479,7 +521,7 @@ class sampling(enka):
         elif local and xi is not None and xi.shape[1] == eng.J and eng.J != eng.cols:
             xi = xi[:, eng.col_lo:eng.col_hi]
         opts = dict(fixed_h=fixed, switch=kwargs.get('switch', 1.), resolve=resolve,
-                    formulation=kwargs.get('formulation', getattr(self, 'formulation', 'interaction')))
+                    formulation=kwargs.get('formulation', getattr(self, 'formulation', 'interaction')), noise=noise)
         Uk, hk, met = eng.step_host(rule, U0, Gk, xi, **opts)
         if stale is not None and stale():
             # a large problem array was edited in place since the previous call: the device copy has just been
@@ -504,7 +546,13 @@ class sampling(enka):
         self._advance_time(hk)
 
     def eks_update(self, y_obs, U0, Geval, Gamma, iter, **kwargs):
-        """Semi-implicit EKS step (ces/calibrate.py:418-449)."""
+        """Semi-implicit EKS step (ces/calibrate.py:418-449).
+
+        ``noise='ensemble'`` (here and in the aldi updates) replaces the reference's ``sqrt(2h) chol(C^uu) xi`` by
+        ``sqrt(2h / n_C) (U - ubar) xi`` with a J x J ``xi``: ``xi=`` an explicit (J, J) array ((J, cols) with
+        ``local_shard=True``), or by default the device's Philox stream keyed by ``seed`` and the step count
+        ``len(self.metrics['t'])``.  The update then draws nothing from numpy's global generator (``rng`` does not apply);
+        a forward model's own draws, such as ``banana``'s, are unaffected."""
         self.update_rule = 'eks_update'
         return self._update_host('eks', y_obs, U0, Geval, Gamma, kwargs)
 
@@ -541,7 +589,8 @@ class sampling(enka):
         if not (device_map and eng.nranks == 1 and kind in _lib.MAPS and self.p <= 8 and self.n_obs <= 16
                 and 2 <= eng.J <= 512 and self.T >= 1 and self._step_options(rule, kwargs) == (None, None)
                 and kwargs.get('formulation', getattr(self, 'formulation', 'interaction')) == 'interaction'
-                and getattr(self, 'fused_run', True) and kwargs.get('xi', None) is None):
+                and getattr(self, 'fused_run', True) and kwargs.get('xi', None) is None
+                and not self._noise_options(rule, kwargs, eng.J)[0]):
             return False
         p, k, J, T = self.p, self.n_obs, eng.J, int(self.T)
         if (T + 1) * (2 * p + k) * J * 8 > (1 << 28):
@@ -616,7 +665,10 @@ class sampling(enka):
     def run(self, y_obs, U0, model, Gamma, Jnoise, save_online=False, trace=True, **kwargs):
         """Ensemble Kalman sampler loop (ces/calibrate.py:270-416): forward -> trace -> update -> (save) ->
         stop when the cumulative pseudo-time exceeds ``t_tol`` (default 2.0) or after ``self.T`` iterations.
-        ``Jnoise`` is accepted and ignored like in the reference (it recomputes cholesky(Gamma), :437)."""
+        ``Jnoise`` is accepted and ignored like in the reference (it recomputes cholesky(Gamma), :437).
+        ``noise='ensemble'``: the ensemble form of the noise (see ``eks_update``), drawn on the device from ``seed`` at
+        step ``len(self.metrics['t'])`` -- a resumed run continues the stream -- or ``xi=`` one (J, J) array used at every
+        iteration; numpy's global generator is then advanced only by the forward model's own draws."""
         import torch
 
         mtype = model.type          # AttributeError if absent, like :294-297
@@ -633,6 +685,7 @@ class sampling(enka):
 
         U0 = np.ascontiguousarray(U0, dtype=np.float64)
         J = U0.shape[1]
+        ensemble, xi_ens = self._noise_options(rule, kwargs, J)     # validates noise / xi before any work
         eng = self._get_engine(J, group)
         self._sync_problem(eng, y_obs, Gamma)
         lo, hi = eng.col_lo, eng.col_hi
@@ -648,6 +701,8 @@ class sampling(enka):
         if self._fused_small_run(eng, y_obs, U0, model, rule, kwargs, save_online, trace, known and device_model):
             return
         U_dev = torch.from_numpy(U0[:, lo:hi].copy()).to(dev)
+        if xi_ens is not None:
+            xi_ens = torch.from_numpy(np.ascontiguousarray(xi_ens[:, lo:hi])).to(dev)     # the same xi every iteration
         if is_pde:
             # initial conditions of the integrator, one per particle (ces/calibrate.py:317-327)
             t_ode, ws_pool = kwargs.get('t', None), kwargs.get('ws', None)
@@ -770,8 +825,10 @@ class sampling(enka):
             if known:
                 setattr(self, 'update_rule', {'eks': 'eks_update', 'aldi': 'eks_update_linear',
                                               'aldi_constant': 'eks_update_aldi', 'eki': 'eki_update'}[rule])
-                xi_dev = None
-                if rule != 'eki':
+                xi_dev, noise = None, None
+                if ensemble:
+                    noise = ('ensemble', int(kwargs.get('seed', getattr(self, 'seed', 0))), len(self.metrics['t']), xi_ens)
+                elif rule != 'eki':
                     if kwargs.get('rng', getattr(self, 'rng', 'numpy')) == 'device':
                         # production mode: Philox noise generated on the device, nothing crosses PCIe
                         xi_dev = eng.normal_noise(self.p, kwargs.get('seed', getattr(self, 'seed', 0)),
@@ -781,7 +838,7 @@ class sampling(enka):
                         xi_dev = torch.from_numpy(np.ascontiguousarray(xi[:, lo:hi])).to(dev)
                 fixed, resolve = self._step_options(rule, kwargs)     # 'mix' depends on the time reached so far
                 U_dev, hk, met = eng.step(rule, U_dev, G_cur, xi_dev, fixed_h=fixed, switch=kwargs.get('switch', 1.),
-                                          resolve=resolve,
+                                          resolve=resolve, noise=noise,
                                           formulation=kwargs.get('formulation', getattr(self, 'formulation', 'interaction')))
                 self._record(met, hk)
                 if resolve == 'spectral':

@@ -18,6 +18,12 @@ struct ces_handle_s {
     bool forward_only = false;          // created for ces_forward_map only: no update workspace
     bool use_small = true;              // single-kernel path for small problems (CES_NO_SMALL_PATH=1 disables it)
     int last_rule = -1;
+    // noise term of the noisy rules (ces_set_noise): the reference's sqrt(2h) chol(C^uu) xi, or sqrt(2h / n_C) (U - ubar) xi
+    // with xi (J x J) from the Philox stream at (noise_seed, noise_step) or the caller's device matrix noise_xi
+    int noise_kind = CES_NOISE_CHOLESKY;
+    uint64_t noise_seed = 0, noise_step = 0;
+    const double* noise_xi = nullptr;
+    int64_t noise_ldxi = 0;
     // problem data (device)
     double *y = nullptr, *ginv_diag = nullptr, *Ginv = nullptr, *mu = nullptr, *ustar = nullptr;
     double *sinv_diag = nullptr, *sig_diag = nullptr, *Sinv = nullptr, *Sigma0 = nullptr, *bprior = nullptr;
@@ -152,6 +158,14 @@ int device_spd_inverse(ces_handle_t h, const double* host, int64_t n, double* ds
     cudaFree(F);
     cudaFree(Fi);
     return s;
+}
+
+bool ensemble_noise(ces_handle_t h) { return h->noise_kind == CES_NOISE_ENSEMBLE; }
+
+// 1 / n_C of the rule's own C^uu (api.cu centre_u_all: J for eks, J - 1 otherwise) in ensemble-noise mode; 0 otherwise
+double ens_inv_nc(ces_handle_t h, int rule) {
+    if (!ensemble_noise(h) || rule == CES_RULE_EKI) return 0.0;
+    return rule == CES_RULE_EKS ? 1.0 / (double)h->Jg : 1.0 / (double)(h->Jg - 1);
 }
 
 int valid(ces_handle_t h, bool need_problem) {
@@ -554,8 +568,8 @@ static int start_cholesky(ces_handle_t h, int rule) {
     cudaStream_t st = h->st;
     // chol(C^uu)  (K7); EKI has no noise term and skips it.  Only the noise GEMM of phase 4 needs the factor, so it
     // is computed on a high-priority side stream while the main stream runs the D and V GEMMs (its ~50 small
-    // launches would otherwise sit on the critical path: 3 % of a cfg3 step).
-    if (rule != CES_RULE_EKI) {
+    // launches would otherwise sit on the critical path: 3 % of a cfg3 step).  The ensemble noise needs no factor.
+    if (rule != CES_RULE_EKI && !ensemble_noise(h)) {
         if (!h->aux_st) {
             int lo = 0, hi = 0;
             CES_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
@@ -578,7 +592,7 @@ int ces_peek_step_size(ces_handle_t h, int ts_kind, double fixed_h, double* hk_h
     CES_TRY(valid(h, true));
     if (ts_kind != CES_TS_FROBENIUS && ts_kind != CES_TS_FIXED) return fail(CES_ERR_INVALID, "unknown step-size rule%s", "");
     const double alphaJ = (double)(h->p + 1) / (double)h->Jg;
-    CES_TRY(step_scalars(h->st, h->S, ts_kind == CES_TS_FIXED ? 1 : 0, fixed_h, alphaJ));
+    CES_TRY(step_scalars(h->st, h->S, ts_kind == CES_TS_FIXED ? 1 : 0, fixed_h, alphaJ, ens_inv_nc(h, h->last_rule)));
     CES_CUDA(cudaMemcpyAsync(h->hS, h->S, S_COUNT * sizeof(double), cudaMemcpyDeviceToHost, h->st));
     CES_CUDA(cudaStreamSynchronize(h->st));
     if (hk_host) *hk_host = h->hS[S_H];
@@ -672,6 +686,8 @@ __global__ void __launch_bounds__(256) gram_dot_kernel(const double* __restrict_
 int ces_phase3f_products(ces_handle_t h, int rule) {
     CES_TRY(valid(h, true));
     if (rule != h->last_rule) return fail(CES_ERR_STATE, "phase3f: rule differs from phase2%s", "");
+    if (ensemble_noise(h) && rule != CES_RULE_EKI)
+        return fail(CES_ERR_INVALID, "ensemble noise needs the interaction formulation (the factored one never gathers U~)%s", "");
     const int64_t p = h->p, k = h->k, ld = h->ldJ;
     cudaStream_t st = h->st;
     if (!h->P1) {
@@ -758,11 +774,46 @@ int ces_phase4a_drift(ces_handle_t h, double switch_) {
     return CES_OK;
 }
 
+// Ensemble noise (CES_NOISE_ENSEMBLE) for the local columns [c0, c0 + nc) of U_next, added into C (= Uout + c0):
+//   C += sqrt(2h / n_C) sum_s U~_s xi[s's particles, the columns' global particles]
+// over the source blocks s of every rank (all of U~ is on this rank after the gathers), column panel by column panel.
+// Philox mode materialises each xi block in the D-panel workspace, which phase 4 no longer needs; it is not generated in
+// the GEMM's producer, where every row tile of U~ would regenerate it on the FP64 pipe the DMMAs use.
+static int add_ensemble_noise(ces_handle_t h, int64_t c0, int64_t nc, double* C, int64_t ldc) {
+    cudaStream_t st = h->st;
+    const int64_t col0 = (int64_t)h->rank * h->Jl;         // global particle of local column 0
+    mark(h, "noise:begin");
+    for (int64_t q0 = c0; q0 < c0 + nc; q0 += h->panel) {
+        const int64_t nq = (c0 + nc - q0) < h->panel ? (c0 + nc - q0) : h->panel;
+        for (int s = 0; s < h->nranks; ++s) {
+            const int64_t lo = (int64_t)s * h->Jl < h->Jg ? (int64_t)s * h->Jl : h->Jg;
+            const int64_t ks = (lo + h->Jl < h->Jg ? lo + h->Jl : h->Jg) - lo;     // particles of block s
+            if (ks < 1) continue;
+            GemmCall g;
+            g.a_mode = A_MK; g.b_mode = B_KN;
+            g.M = (int)h->p; g.N = (int)nq; g.K = (int)ks;
+            g.A = ut_block(h, s); g.lda = h->ldJ;
+            if (h->noise_xi) {
+                g.B = h->noise_xi + lo * h->noise_ldxi + q0; g.ldb = h->noise_ldxi;
+            } else {
+                CES_TRY(fill_ensemble_noise(st, h->D, h->ldD, ks, nq, lo, col0 + q0, h->noise_seed, h->noise_step));
+                g.B = h->D; g.ldb = h->ldD;
+            }
+            g.C = C + (q0 - c0); g.ldc = ldc;
+            g.alpha_dev = h->S + S_ENS_ALPHA; g.beta = 1.0;
+            CES_TRY(gemm(st, g));
+        }
+    }
+    mark(h, "noise:end");
+    return CES_OK;
+}
+
 int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, const double* U, int64_t ldu,
                       const double* xi, int64_t ldxi, double* Uout, int64_t ldo, double* hk_host, double* metrics_host) {
     CES_TRY(valid(h, true));
     if (rule != h->last_rule) return fail(CES_ERR_STATE, "phase4: rule differs from phase2%s", "");
-    if (!U || !Uout || (rule != CES_RULE_EKI && !xi)) return fail(CES_ERR_INVALID, "phase4: null pointer%s", "");
+    const bool ens = ensemble_noise(h);
+    if (!U || !Uout || (rule != CES_RULE_EKI && !ens && !xi)) return fail(CES_ERR_INVALID, "phase4: null pointer%s", "");
     if (ts_kind != CES_TS_FROBENIUS && ts_kind != CES_TS_FIXED && ts_kind != CES_TS_KEEP)
         return fail(CES_ERR_INVALID, "unknown step-size rule%s", "");
     const int64_t p = h->p, ld = h->ldJ;
@@ -772,9 +823,9 @@ int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, con
     double* Ut = ut_block(h, h->rank);
 
     // noise operand: TMA needs a 16-byte aligned base and an even leading dimension
-    const double* xi_use = xi;
+    const double* xi_use = ens ? nullptr : xi;         // ensemble mode ignores xi
     int64_t ldxi_use = ldxi;
-    if (xi && (((reinterpret_cast<uintptr_t>(xi) & 15) != 0) || (ldxi & 1))) {
+    if (xi_use && (((reinterpret_cast<uintptr_t>(xi) & 15) != 0) || (ldxi & 1))) {
         if (!h->xi_pad) { CES_TRY(dalloc(h, &h->xi_pad, p * ld)); }
         CES_TRY(pad_copy(st, xi, ldxi, p, h->cols, h->xi_pad, ld));
         xi_use = h->xi_pad; ldxi_use = ld;
@@ -787,7 +838,7 @@ int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, con
     }
     mark(h, "phase4:chol_ready");
     const int kind = (rule == CES_RULE_ALDI_CONSTANT) ? 2 : (ts_kind == CES_TS_FIXED ? 1 : 0);
-    if (ts_kind != CES_TS_KEEP || rule == CES_RULE_ALDI_CONSTANT) CES_TRY(step_scalars(st, S, kind, fixed_h, alphaJ));
+    if (ts_kind != CES_TS_KEEP || rule == CES_RULE_ALDI_CONSTANT) CES_TRY(step_scalars(st, S, kind, fixed_h, alphaJ, ens_inv_nc(h, rule)));
 
     GemmCall noise;   // += sqrt(2h) chol(C) xi     (K8; L lower triangular -> skip the zero blocks)
     noise.a_mode = A_MK; noise.b_mode = B_KN;
@@ -841,11 +892,11 @@ int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, con
             g.A = h->Cuu; g.lda = h->ldp; g.B = h->Z + c0; g.ldb = ld; g.C = Uout + c0; g.ldc = ldo;
             g.alpha_dev = S + S_NEG_H; g.beta = 1.0;
             CES_TRY(gemm(st, g));
-            CES_TRY(gemm(st, nz));
+            CES_TRY(ens ? add_ensemble_noise(h, c0, nc, Uout + c0, ldo) : gemm(st, nz));
         } else if (rule == CES_RULE_ALDI_CONSTANT) {
             // U + h drift + sqrt(2h) L xi                         (:525-527)
             CES_TRY(axpbypcz(st, p, nc, 1.0, U + c0, ldu, 1.0, S + S_H, h->T + c0, ld, 0.0, nullptr, nullptr, 0, Uout + c0, ldo));
-            CES_TRY(gemm(st, nz));
+            CES_TRY(ens ? add_ensemble_noise(h, c0, nc, Uout + c0, ldo) : gemm(st, nz));
         } else {                                                   // EKI
             CES_TRY(axpbypcz(st, p, nc, 1.0, U + c0, ldu, 1.0, S + S_NEG_H, h->V + c0, ld, 0.0, nullptr, nullptr, 0, Uout + c0, ldo));
         }
@@ -880,7 +931,7 @@ int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, con
                 g.A = h->Sigma0; g.lda = h->ldp; g.B = h->T; g.ldb = ld; g.C = Uout; g.ldc = ldo;
                 CES_TRY(gemm(st, g));
             }
-            CES_TRY(gemm(st, noise));
+            CES_TRY(ens ? add_ensemble_noise(h, 0, h->cols, Uout, ldo) : gemm(st, noise));
         }
     }
     CES_CUDA(cudaMemcpyAsync(h->hS, S, S_COUNT * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -918,7 +969,10 @@ int ces_step(ces_handle_t h, int rule, int ts_kind, double fixed_h, double switc
              double* hk_host, double* metrics_host) {
     CES_TRY(valid(h, true));
     if (h->nranks != 1) return fail(CES_ERR_STATE, "ces_step is single-GPU; use the phases with nranks > 1%s", "");
-    if (h->use_small && formulation == CES_FORM_INTERACTION && small_step_eligible(h->p, h->k, h->Jl)) {
+    if (formulation == CES_FORM_FACTORED && ensemble_noise(h) && rule != CES_RULE_EKI)
+        return fail(CES_ERR_INVALID, "ensemble noise needs the interaction formulation (the factored one never gathers U~)%s", "");
+    // the single-kernel path draws the reference's Cholesky noise only
+    if (h->use_small && !ensemble_noise(h) && formulation == CES_FORM_INTERACTION && small_step_eligible(h->p, h->k, h->Jl)) {
         // small problems: the whole update in one single-CTA kernel (launch latency dominates otherwise)
         if (rule < CES_RULE_EKS || rule > CES_RULE_EKI) return fail(CES_ERR_INVALID, "unknown update rule %s%lld", "", rule);
         if (ts_kind != CES_TS_FROBENIUS && ts_kind != CES_TS_FIXED) return fail(CES_ERR_INVALID, "unknown step-size rule%s", "");
@@ -1042,6 +1096,8 @@ int ces_host_begin(ces_handle_t h, int rule, int formulation, const double* U, c
     CES_TRY(valid(h, true));
     if (rule < CES_RULE_EKS || rule > CES_RULE_EKI) return fail(CES_ERR_INVALID, "unknown update rule %s%lld", "", rule);
     if (formulation != CES_FORM_INTERACTION && formulation != CES_FORM_FACTORED) return fail(CES_ERR_INVALID, "unknown formulation%s", "");
+    if (formulation == CES_FORM_FACTORED && ensemble_noise(h) && rule != CES_RULE_EKI)
+        return fail(CES_ERR_INVALID, "ensemble noise needs the interaction formulation (the factored one never gathers U~)%s", "");
     if ((!U || !G) && h->cols > 0) return fail(CES_ERR_INVALID, "ces_host_begin: null pointer%s", "");
     CES_TRY(host_staging(h));
     const int64_t p = h->p, k = h->k, ld = h->ldJ, w = h->cols;
@@ -1197,7 +1253,8 @@ int ces_step_host(ces_handle_t h, int rule, int ts_kind, double fixed_h, double 
     if (h->nranks != 1) return fail(CES_ERR_STATE, "ces_step_host is single-GPU; use the ces_host_* pieces with nranks > 1%s", "");
     if (!U || !G || !Uout) return fail(CES_ERR_INVALID, "ces_step_host: null pointer%s", "");
     const int64_t p = h->p, k = h->k, ld = h->ldJ;
-    const bool small = h->use_small && formulation == CES_FORM_INTERACTION && small_step_eligible(h->p, h->k, h->Jl);
+    const bool small = h->use_small && !ensemble_noise(h) && formulation == CES_FORM_INTERACTION &&
+                       small_step_eligible(h->p, h->k, h->Jl);
     if (small) {
         // tiny problems keep everything on one stream -- extra streams and events would cost more than the copies
         CES_TRY(host_staging(h));
@@ -1486,6 +1543,30 @@ int ces_buffer(ces_handle_t h, const char* name, double** ptr, int64_t* rows, in
     if (cols) *cols = c;
     if (ld) *ld = l;
     return CES_OK;
+}
+
+int ces_set_noise(ces_handle_t h, int kind, uint64_t seed, uint64_t step, const double* xi_dev, int64_t ldxi) {
+    // arguments that need no handle first
+    if (kind != CES_NOISE_CHOLESKY && kind != CES_NOISE_ENSEMBLE) return fail(CES_ERR_INVALID, "ces_set_noise: unknown noise kind %s%lld", "", kind);
+    if (kind == CES_NOISE_ENSEMBLE && xi_dev && (((reinterpret_cast<uintptr_t>(xi_dev) & 15) != 0) || (ldxi & 1) || ldxi < 1))
+        return fail(CES_ERR_ALIGN, "ces_set_noise: xi needs a 16-byte aligned base and an even leading dimension%s", "");
+    CES_TRY(valid(h, false));
+    if (kind == CES_NOISE_ENSEMBLE && h->Jg < 2) return fail(CES_ERR_INVALID, "ces_set_noise: ensemble noise needs J >= 2%s", "");
+    if (kind == CES_NOISE_ENSEMBLE && xi_dev && ldxi < h->cols)
+        return fail(CES_ERR_ALIGN, "ces_set_noise: leading dimension of xi below the local column count%s", "");
+    h->noise_kind = kind;
+    h->noise_seed = seed;
+    h->noise_step = step;
+    h->noise_xi = kind == CES_NOISE_ENSEMBLE ? xi_dev : nullptr;
+    h->noise_ldxi = kind == CES_NOISE_ENSEMBLE && xi_dev ? ldxi : 0;
+    return CES_OK;
+}
+
+int ces_fill_ensemble_noise(void* stream, uint64_t seed, uint64_t step, double* X, int64_t ld, int64_t rows, int64_t cols,
+                            int64_t row_offset, int64_t col_offset) {
+    if (!X || rows < 0 || cols < 0 || ld < cols || row_offset < 0 || col_offset < 0)
+        return fail(CES_ERR_INVALID, "ces_fill_ensemble_noise: bad argument%s", "");
+    return fill_ensemble_noise(static_cast<cudaStream_t>(stream), X, ld, rows, cols, row_offset, col_offset, seed, step);
 }
 
 int ces_fill_normal(void* stream, uint64_t seed, uint64_t step, double* X, int64_t ld, int64_t rows, int64_t cols,

@@ -2,6 +2,7 @@
 // forms for the diagnostics, step-size scalars and the final assembly of U_{n+1}.
 // Reference arithmetic: ces/calibrate.py:423-435, 459-467, 475-488 (see DESIGN.md kernel table).
 #include "kernels.h"
+#include "rng.cuh"
 
 namespace ces {
 
@@ -301,7 +302,8 @@ int scale_vector(cudaStream_t st, const double* d, const double* x, double* y, i
 //   kind 0: hk = 1 / (sqrt(ssq) + 1e-8)          (default, :248)
 //   kind 1: hk = fixed                           ('constant', :253; 'mix' after spin-up, :260)
 //   kind 2: hk = 0.1 / max|drift|                ('aldi_constant', :519)
-__global__ void step_scalars_kernel(double* __restrict__ S, int kind, double fixed_h, double alpha_J) {
+//   inv_nc > 0 (ensemble noise): S_ENS_ALPHA = sqrt(2 h / n_C), the scale of (U - ubar) xi; left untouched otherwise
+__global__ void step_scalars_kernel(double* __restrict__ S, int kind, double fixed_h, double alpha_J, double inv_nc) {
     double h;
     if (kind == 0) h = 1.0 / (sqrt(S[S_SSQ]) + 1e-8);
     else if (kind == 1) h = fixed_h;
@@ -310,9 +312,10 @@ __global__ void step_scalars_kernel(double* __restrict__ S, int kind, double fix
     S[S_SQRT2H] = sqrt(2.0 * h);
     S[S_NEG_H] = -h;
     S[S_H_ALPHA] = h * alpha_J;
+    if (inv_nc > 0.0) S[S_ENS_ALPHA] = sqrt(2.0 * h * inv_nc);
 }
-int step_scalars(cudaStream_t st, double* S, int kind, double fixed_h, double alpha_J) {
-    step_scalars_kernel<<<1, 1, 0, st>>>(S, kind, fixed_h, alpha_J);
+int step_scalars(cudaStream_t st, double* S, int kind, double fixed_h, double alpha_J, double inv_nc) {
+    step_scalars_kernel<<<1, 1, 0, st>>>(S, kind, fixed_h, alpha_J, inv_nc);
     CES_LAUNCHED(1);
     return CES_OK;
 }
@@ -457,6 +460,41 @@ int fill_normal(cudaStream_t st, double* X, int64_t ld, int64_t rows, int64_t co
     const int64_t pairs = ((col_offset + cols - 1) >> 1) - (col_offset >> 1) + 1;
     dim3 grid((unsigned)ceil_div(pairs, 256), (unsigned)rows);
     fill_normal_kernel<<<grid, 256, 0, st>>>(X, ld, (int)rows, cols, col_offset, seed, step);
+    CES_LAUNCHED(1);
+    return CES_OK;
+}
+
+// xi (J x J) of the ensemble noise sqrt(2h / n_C) (U - ubar) xi: element (s, j) -- source particle s, target particle j --
+// from Philox4x32-10 keyed by the seed at the counter (j >> 1, TAG_ENS, s, step), the cosine of the Box-Muller pair for
+// even j and the sine for odd j.  Word 1 carries the tag where fill_normal has the high half of its pair index, so the two
+// streams never share a counter at the same (seed, step).  An element depends only on (seed, step, global s, global j):
+// any block of rows and columns, odd offsets included, reproduces what one GPU draws.  Rows go on blockIdx.y with a
+// grid-stride loop (gridDim.y <= 65535 < J).
+constexpr uint32_t TAG_ENS = 0x454E;
+__global__ void __launch_bounds__(256) fill_ensemble_noise_kernel(double* __restrict__ X, long long ld, long long rows,
+                                                                  long long cols, long long row_offset, long long col_offset,
+                                                                  unsigned long long seed, unsigned long long step) {
+    const unsigned long long gpair = ((unsigned long long)col_offset >> 1) + (unsigned long long)blockIdx.x * 256 + threadIdx.x;
+    const long long j = (long long)(2 * gpair) - col_offset;               // local index of the pair's first column (may be -1)
+    if (j >= cols) return;
+    for (long long r = blockIdx.y; r < rows; r += gridDim.y) {
+        uint32_t c[4] = {(uint32_t)gpair, TAG_ENS, (uint32_t)(row_offset + r), (uint32_t)step};
+        philox4(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+        const double rad = sqrt(-2.0 * log(u53(c[0], c[1])));
+        double sn, cs;
+        sincospi(2.0 * u53(c[2], c[3]), &sn, &cs);
+        double* row = X + (size_t)r * ld;
+        if (j >= 0) row[j] = rad * cs;
+        if (j + 1 < cols) row[j + 1] = rad * sn;
+    }
+}
+int fill_ensemble_noise(cudaStream_t st, double* X, int64_t ld, int64_t rows, int64_t cols, int64_t row_offset,
+                        int64_t col_offset, uint64_t seed, uint64_t step) {
+    if (rows < 1 || cols < 1) return CES_OK;
+    if (row_offset < 0 || col_offset < 0) return fail(CES_ERR_INVALID, "fill_ensemble_noise: negative offset%s", "");
+    const int64_t pairs = ((col_offset + cols - 1) >> 1) - (col_offset >> 1) + 1;
+    dim3 grid((unsigned)ceil_div(pairs, 256), (unsigned)(rows < 65535 ? rows : 65535));
+    fill_ensemble_noise_kernel<<<grid, 256, 0, st>>>(X, ld, rows, cols, row_offset, col_offset, seed, step);
     CES_LAUNCHED(1);
     return CES_OK;
 }

@@ -49,6 +49,7 @@ enum StepScalars : int {
     S_BIAS_DATA = 4,  // sum_j (r_j^T Gamma^-1 r_j)^2
     S_MAXDRIFT = 5,   // max |drift| (aldi_constant)
     S_H = 6, S_SQRT2H = 7, S_NEG_H = 8, S_H_ALPHA = 9,
+    S_ENS_ALPHA = 10, // sqrt(2h / n_C): scale of the ensemble noise (U - ubar) xi (CES_NOISE_ENSEMBLE)
     S_INFO = 15,      // small path: 1 + index of the first non-positive Cholesky pivot (0 = ok)
     S_COUNT = 16,
 };
@@ -70,7 +71,7 @@ int sum_vector(cudaStream_t st, const double* v, int64_t n, double* out);
 int row_sumsq(cudaStream_t st, const double* X, int64_t ld, int64_t rows, int64_t cols, double* out);
 int matvec(cudaStream_t st, const double* M, int64_t ld, int64_t n, const double* x, double* y);
 int scale_vector(cudaStream_t st, const double* d, const double* x, double* y, int64_t n);
-int step_scalars(cudaStream_t st, double* S, int kind, double fixed_h, double alpha_J);
+int step_scalars(cudaStream_t st, double* S, int kind, double fixed_h, double alpha_J, double inv_nc);
 int axpbypcz(cudaStream_t st, int64_t rows, int64_t cols, double a, const double* X, int64_t ldx, double b,
              const double* b_dev, const double* Y, int64_t ldy, double c, const double* c_dev, const double* Z,
              int64_t ldz, double* out, int64_t ldo);
@@ -81,6 +82,8 @@ int add_col_vector(cudaStream_t st, double* X, int64_t ld, int64_t rows, int64_t
                    const double* s_dev);
 int fill_normal(cudaStream_t st, double* X, int64_t ld, int64_t rows, int64_t cols, int64_t col_offset, uint64_t seed,
                 uint64_t step);
+int fill_ensemble_noise(cudaStream_t st, double* X, int64_t ld, int64_t rows, int64_t cols, int64_t row_offset,
+                        int64_t col_offset, uint64_t seed, uint64_t step);
 int form_implicit(cudaStream_t st, const double* C, int64_t ldc, const double* Sigma0, int64_t lds,
                   const double* sig_diag, const double* h_dev, int64_t p, double* M, int64_t ldm);
 

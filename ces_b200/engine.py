@@ -378,6 +378,36 @@ class Engine(object):
                                                 int(self.cols), int(self.col_lo)))
         return out
 
+    def set_noise(self, kind, seed=0, step=0, xi=None):
+        """Noise term of the following steps (ces_set_noise): "cholesky" (the reference's sqrt(2h) chol(C^uu) xi with the
+        (p, cols) xi given to each step) or "ensemble" (sqrt(2h / n_C) (U - ubar) xi with a J x J xi: from the device's
+        Philox stream at (seed, step) when ``xi`` is None, else ``xi``, a (J, cols) float64 CUDA tensor holding this rank's
+        columns, kept alive here until the next call)."""
+        if kind not in _lib.NOISES:
+            raise ValueError("noise must be 'cholesky' or 'ensemble'")
+        if kind == "ensemble" and xi is not None:
+            if tuple(xi.shape) != (self.J, self.cols):
+                raise ValueError("ensemble noise xi must be (J, cols) = (%d, %d), got %s" % (self.J, self.cols, tuple(xi.shape)))
+            if xi.stride(1) != 1 or xi.stride(0) % 2 or xi.stride(0) < 1 or xi.data_ptr() % 16:
+                # the GEMM reads xi through TMA: 16-byte aligned base, even leading dimension (odd J, narrow shards)
+                padded = self.torch.zeros(self.J, -(-max(self.cols, 1) // 16) * 16, dtype=self.torch.float64, device="cuda")
+                padded[:, :self.cols] = xi
+                xi = padded[:, :self.cols]
+            Xp, ldx = self._dev(xi)
+        else:
+            xi, Xp, ldx = None, None, 0
+        _lib.check(self.lib.ces_set_noise(self.h, _lib.NOISES[kind], int(seed), int(step), Xp, ldx))
+        self._noise_xi = xi
+
+    def _apply_noise(self, noise):
+        """``noise``: None (the reference's Cholesky form) or ("ensemble", seed, step, xi or None); a host xi is uploaded."""
+        if noise is None:
+            return self.set_noise("cholesky")
+        kind, seed, step, xi = noise
+        if xi is not None and not hasattr(xi, "is_cuda"):
+            xi = self.torch.from_numpy(np.ascontiguousarray(xi, dtype=np.float64)).cuda()
+        self.set_noise(kind, seed, step, xi)
+
     def launch_count(self):
         return int(self.lib.ces_launch_count(self.h))
 
@@ -388,15 +418,18 @@ class Engine(object):
         return ctypes.c_void_p(t.data_ptr()), int(t.stride(0))
 
     # ------------------------------------------------------------------ one update
-    def step(self, rule, U, G, xi, out=None, fixed_h=None, switch=1.0, resolve=None, formulation="interaction"):
+    def step(self, rule, U, G, xi, out=None, fixed_h=None, switch=1.0, resolve=None, formulation="interaction", noise=None):
         with self.on_stream():
-            return self._step(rule, U, G, xi, out, fixed_h, switch, resolve, formulation)
+            return self._step(rule, U, G, xi, out, fixed_h, switch, resolve, formulation, noise)
 
-    def _step(self, rule, U, G, xi, out, fixed_h, switch, resolve, formulation):
+    def _step(self, rule, U, G, xi, out, fixed_h, switch, resolve, formulation, noise=None):
         """One update on this rank's columns.  U (p, cols), G (k, cols), xi (p, cols) are float64 CUDA
         tensors; returns (U_next, hk, metrics dict).  ``fixed_h`` gives the step size ('constant', 'mix' after
-        spin-up); ``resolve`` asks for the hk C^pp + Gamma re-solve of D (see ``run_phases``)."""
+        spin-up); ``resolve`` asks for the hk C^pp + Gamma re-solve of D (see ``run_phases``).  ``noise``: None for
+        the reference's Cholesky noise, or ("ensemble", seed, step, xi_ens or None) (``set_noise``; xi is then
+        ignored and may be None)."""
         torch = self.torch
+        self._apply_noise(noise)
         r = _lib.RULES[rule]
         ts = _lib.TS_FIXED if fixed_h is not None else _lib.TS_FROBENIUS
         fh = float(fixed_h) if fixed_h is not None else 0.0
@@ -468,22 +501,24 @@ class Engine(object):
         met = {key: float(self._met[i]) for i, key in enumerate(_METRIC_KEYS)}
         return out, float(self._hk.value), met
 
-    def step_host(self, rule, U, G, xi, fixed_h=None, switch=1.0, resolve=None, formulation="interaction"):
+    def step_host(self, rule, U, G, xi, fixed_h=None, switch=1.0, resolve=None, formulation="interaction", noise=None):
         """The same update on host numpy arrays: the copies to and from the device are part of the call.  This is what
         ``sampling.eks_update*`` invoke.  Single GPU: (p, J) / (k, J) arrays through ``ces_step_host``.  Column-sharded
         (``nranks > 1``): this rank's (p, cols) / (k, cols) shards in, its (p, cols) shard of U_next out, the phases
-        with their collectives in between (``_step_host_sharded``)."""
+        with their collectives in between (``_step_host_sharded``).  ``noise`` as in ``step`` (a host xi_ens is
+        uploaded)."""
         if formulation not in _lib.FORMULATIONS:
             raise ValueError("formulation must be 'interaction' or 'factored'")
         if self.nranks != 1:
-            return self._step_host_sharded(rule, U, G, xi, fixed_h, switch, resolve, formulation)
+            return self._step_host_sharded(rule, U, G, xi, fixed_h, switch, resolve, formulation, noise)
         if resolve is not None:
             # non-default time_step: the phase-by-phase device path, with explicit copies around it
             torch = self.torch
             dev = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).cuda()
             out, hk, met = self.step(rule, dev(U), dev(G), dev(xi) if xi is not None else None, fixed_h=fixed_h,
-                                     switch=switch, resolve=resolve, formulation=formulation)
+                                     switch=switch, resolve=resolve, formulation=formulation, noise=noise)
             return out.cpu().numpy(), hk, met
+        self._apply_noise(noise)
         r = _lib.RULES[rule]
         ts = _lib.TS_FIXED if fixed_h is not None else _lib.TS_FROBENIUS
         fh = float(fixed_h) if fixed_h is not None else 0.0
@@ -496,7 +531,7 @@ class Engine(object):
             out = self.torch.empty((self.p, self.J), dtype=self.torch.float64, pin_memory=True).numpy()
         else:
             out = np.empty_like(U)
-        if xi is not None:
+        if xi is not None and noise is None:
             xi = np.ascontiguousarray(xi, dtype=np.float64)
             assert xi.shape == U.shape
             xp = _lib.host_ptr(xi)
@@ -515,7 +550,7 @@ class Engine(object):
             self._views[key] = self.torch.empty(tuple(shape), dtype=self.torch.float64, pin_memory=True)
         return self._views[key]
 
-    def _step_host_sharded(self, rule, U, G, xi, fixed_h, switch, resolve, formulation):
+    def _step_host_sharded(self, rule, U, G, xi, fixed_h, switch, resolve, formulation, noise=None):
         """Column shard on host arrays.  Default rule set (no re-solve of D, interaction formulation): the pipelined
         pieces of the library's host step (include/ces_b200.h) with this rank's collectives in between -- G uploads in
         row chunks while the chunks already on the device are summed (all-reduce of that slice of the means), centred and
@@ -525,6 +560,8 @@ class Engine(object):
         U = np.ascontiguousarray(U, dtype=np.float64)
         G = np.ascontiguousarray(G, dtype=np.float64)
         assert U.shape == (self.p, self.cols) and G.shape == (self.k, self.cols), (U.shape, G.shape, self.cols)
+        if noise is not None:
+            xi = None                               # ensemble noise: the J x J xi replaces the (p, cols) one
         if xi is not None:
             xi = np.ascontiguousarray(xi, dtype=np.float64)
             assert xi.shape == U.shape
@@ -532,6 +569,7 @@ class Engine(object):
         ptr = lambda a: (_lib.host_ptr(a) if a is not None and a.size else None)
         with self.on_stream():
             if resolve is None and formulation == "interaction":
+                self._apply_noise(noise)
                 r = _lib.RULES[rule]
                 ts = _lib.TS_FIXED if fixed_h is not None else _lib.TS_FROBENIUS
                 nch, bounds = ctypes.c_int(), (ctypes.c_int64 * 9)()
@@ -578,7 +616,8 @@ class Engine(object):
             # the last phase downloads U_next itself, in column chunks overlapped with their assembly
             _lib.check(lib.ces_set_pending_output(h, host.data_ptr() if self.cols else None))
             try:
-                out, hk, met = self._step(rule, Ud, Gd, Xd if xi is not None else None, Od, fixed_h, switch, resolve, formulation)
+                out, hk, met = self._step(rule, Ud, Gd, Xd if xi is not None else None, Od, fixed_h, switch, resolve, formulation,
+                                          noise)
             finally:
                 lib.ces_set_pending_output(h, None)
             main.synchronize()

@@ -54,6 +54,10 @@ extern "C" {
 #define CES_FORM_INTERACTION 0    /* D = (1/J) E^T W formed in panels, V = U~ D (the reference's formulation) */
 #define CES_FORM_FACTORED 1       /* V = (1/J)(U~ E^T) W, ||D||_F from Gram matrices; same update to rounding */
 
+/* noise term of the noisy rules eks, aldi, aldi_constant (ces_set_noise); n_C = J for eks, J - 1 for aldi / aldi_constant */
+#define CES_NOISE_CHOLESKY 0      /* sqrt(2h) chol(C^uu) xi, xi p x J: the reference's (default)     */
+#define CES_NOISE_ENSEMBLE 1      /* sqrt(2h / n_C) (U - ubar) xi, xi J x J                           */
+
 /* forward maps (ces/utils.py) */
 #define CES_MAP_LINEAL 0          /* A theta + b           :25-31  */
 #define CES_MAP_LINEAL_LOG 1      /* A exp(phi) + b        :39-42  */
@@ -97,10 +101,10 @@ int ces_set_problem(ces_handle_t h, const double* y_host, const double* Gamma_ho
  * phase 2  centring E, R, W = Gamma^-1 R, U~, Z = Sigma0^-1 (U - mu); local partial sums of the four
  *          diagnostics; local partial covariance U~ U~^T
  *          [host: all-reduce(sum) of "cuu"; all-gather of "e_all" and "ut_all" (rank-major blocks)]
- * phase 3  chol(C^uu); D = (1/J) E^T W by source block and column panel with sum of squares; V = U~ D
+ * phase 3  chol(C^uu) (Cholesky noise only); D = (1/J) E^T W by source block and column panel with sum of squares; V = U~ D
  *          [host: all-reduce(sum) of the first 5 doubles of "scalars"]
  * phase 4a (aldi_constant only) drift and its local max-abs  [host: all-reduce(max) of scalars[5]]
- * phase 4  step size, prior term, noise term, assembly of U_{n+1}; returns hk and the four diagnostics
+ * phase 4  step size, prior term, noise term (ces_set_noise), assembly of U_{n+1}; returns hk and the four diagnostics
  *          (self-bias, bias, self-bias-data, bias-data: ces/calibrate.py:432-435) on the host.
  * U, G, xi, U_out are device pointers to this rank's columns with leading dimensions ld*.  */
 int ces_phase1_sums(ces_handle_t h, const double* U_dev, int64_t ldu, const double* G_dev, int64_t ldg);
@@ -138,6 +142,21 @@ int ces_phase4a_drift(ces_handle_t h, double switch_);
 int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, const double* U_dev, int64_t ldu,
                       const double* xi_dev, int64_t ldxi, double* Uout_dev, int64_t ldo, double* hk_host,
                       double* metrics_host /* [4] */);
+
+/* Noise term of the noisy rules for the following steps (the setting stays on the handle until the next call; set
+ * (seed, step) before each step).  CES_NOISE_CHOLESKY: the reference's sqrt(2h) chol(C^uu + 1e-8 I) xi with the p x J
+ * xi passed to phase 4 / ces_step / ces_step_host.  CES_NOISE_ENSEMBLE:
+ *     sqrt(2h / n_C) (U - ubar) xi,   xi in R^{J x J} i.i.d. N(0, 1),  xi[s, j]: source particle s, target particle j,
+ * with n_C the normalisation of the rule's own C^uu (J for eks, J - 1 for aldi and aldi_constant).  Given U every column
+ * is N(0, 2h (C^uu - 1e-8 I)) and lies in span(U - ubar); it costs 2 p J^2 flop and no factorisation (chol(C^uu) is not
+ * computed in this mode).  The rest of the step is unchanged; eki has no noise term.  xi_dev == NULL: xi from Philox at
+ * (seed, step), exactly as ces_fill_ensemble_noise draws it; otherwise a J_global x cols_local device matrix of this
+ * rank's columns (row s = global particle s) with a 16-byte aligned base and an even ldxi >= cols_local (else
+ * CES_ERR_ALIGN), which must stay valid until the step's phase 4 has run.  In ensemble mode the xi argument of phase 4,
+ * ces_step and ces_step_host is ignored and may be NULL, and the single-kernel path of small problems is not taken.
+ * CES_ERR_INVALID for an unknown kind or a NULL handle; ensemble mode with CES_FORM_FACTORED (which never gathers
+ * U - ubar) is refused by ces_step, ces_host_begin and ces_phase3f_products.  No device work. */
+int ces_set_noise(ces_handle_t h, int kind, uint64_t seed, uint64_t step, const double* xi_dev, int64_t ldxi);
 
 /* One whole single-GPU step on device buffers (nranks must be 1). */
 int ces_step(ces_handle_t h, int rule, int ts_kind, double fixed_h, double switch_, int formulation,
@@ -285,6 +304,14 @@ int ces_frobenius(void* stream, const double* X_dev, int64_t ld, int64_t rows, i
  * (seed, step, row, global column), so a column-sharded ensemble draws exactly what one GPU would (col_offset even). */
 int ces_fill_normal(void* stream, uint64_t seed, uint64_t step, double* X_dev, int64_t ld, int64_t rows, int64_t cols,
                     int64_t col_offset);
+
+/* The xi of CES_NOISE_ENSEMBLE on the device: rows [row_offset, row_offset + rows) (source particles) and columns
+ * [col_offset, col_offset + cols) (target particles) into X_dev (ld >= cols).  Philox4x32-10 keyed by (seed low, seed high)
+ * at the counter (j >> 1, 0x454E, s, step mod 2^32); even j takes the Box-Muller cosine, odd j the sine (the uniforms and
+ * Box-Muller of ces_fill_normal).  Element (s, j) depends only on (seed, step, s, j), so any sharding of rows or columns
+ * reproduces a single draw; counter word 1 keeps the stream apart from ces_fill_normal's. */
+int ces_fill_ensemble_noise(void* stream, uint64_t seed, uint64_t step, double* X_dev, int64_t ld, int64_t rows,
+                            int64_t cols, int64_t row_offset, int64_t col_offset);
 
 /* ---- building blocks exported for tests and for callers that own their orchestration ---------------
  * C[M,N] = alpha * op(A) op(B) + beta * C on the FP64 tensor cores.  a_mode: 0 = A is M x K row-major,
