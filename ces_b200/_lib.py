@@ -33,11 +33,28 @@ EXPORTS = (
     "ces_host_centre_u", "ces_host_interact_own", "ces_host_update", "ces_ipc_export", "ces_ipc_import", "ces_peer_gather",
     "ces_peer_gather_wait", "ces_host_interact_chunk", "ces_small_run", "ces_mcmc_model_mh", "ces_host_chunk_schedule",
     "ces_gp_create", "ces_gp_destroy", "ces_gp_lml", "ces_gp_condition", "ces_gp_predict", "ces_gp_mh", "ces_darcy_mh",
-    "ces_gp_set_kernel", "ces_set_noise", "ces_fill_ensemble_noise",
+    "ces_gp_set_kernel", "ces_set_noise", "ces_fill_ensemble_noise", "ces_potri", "ces_gemm_ex",
 )
 
 _i64, _int, _dbl, _vp = ctypes.c_int64, ctypes.c_int, ctypes.c_double, ctypes.c_void_p
 _dp = ctypes.c_void_p  # double* (host or device) passed as an address
+
+
+class GemmDesc(ctypes.Structure):
+    """ces_gemm_desc (test support: the whole DMMA GEMM family, see include/ces_b200.h)."""
+    _fields_ = [("struct_size", _i64), ("a_mode", ctypes.c_int32), ("b_mode", ctypes.c_int32),
+                ("M", _i64), ("N", _i64), ("K", _i64), ("A", _dp), ("lda", _i64), ("B", _dp), ("ldb", _i64),
+                ("C", _dp), ("ldc", _i64), ("alpha", _dbl), ("beta", _dbl), ("alpha_dev", _dp),
+                ("flags", ctypes.c_int32), ("group_m", ctypes.c_int32), ("splits", ctypes.c_int32),
+                ("wave_ctas", ctypes.c_int32), ("serpentine", ctypes.c_int32), ("reserved", ctypes.c_int32),
+                ("splitk_ws", _dp), ("splitk_ws_elems", _i64), ("diag_add", _dbl), ("ssq_partials", _dp),
+                ("ssq_partials_elems", _i64), ("batch", _i64), ("a_batch_rows", _i64), ("b_batch_rows", _i64),
+                ("c_batch_elems", _i64)]
+
+    def __init__(self, **kw):
+        base = dict(struct_size=ctypes.sizeof(GemmDesc), alpha=1.0, serpentine=-1, batch=1)
+        base.update(kw)
+        super().__init__(**base)
 
 
 class CesError(RuntimeError):
@@ -132,6 +149,8 @@ def load():
     lib.ces_gemm.argtypes = [_vp, _int, _int, _i64, _i64, _i64, _dbl, _dp, _i64, _dp, _i64, _dbl, _dp, _i64]
     lib.ces_potrf.argtypes = [_vp, _dp, _i64, _i64]
     lib.ces_posv.argtypes = [_vp, _dp, _i64, _i64, _dp, _i64, _i64]
+    lib.ces_potri.argtypes = [_vp, _dp, _i64, _i64, _dp, _i64]
+    lib.ces_gemm_ex.argtypes = [_vp, ctypes.POINTER(GemmDesc)]
     for name in EXPORTS:
         fn = getattr(lib, name)
         if fn.restype is ctypes.c_int and name not in ("ces_version", "ces_last_error", "ces_launch_count"):

@@ -1590,15 +1590,53 @@ int ces_frobenius(void* stream, const double* X, int64_t ld, int64_t rows, int64
     return s;
 }
 
+// A leading dimension below the stored row width would make consecutive rows overlap.
+static bool gemm_ld_ok(int a_mode, int b_mode, int64_t M, int64_t N, int64_t K, int64_t lda, int64_t ldb, int64_t ldc) {
+    return lda >= (a_mode == A_MK ? K : M) && ldb >= (b_mode == B_KN ? N : K) && ldc >= N;
+}
+
 int ces_gemm(void* stream, int a_mode, int b_mode, int64_t M, int64_t N, int64_t K, double alpha, const double* A, int64_t lda,
              const double* B, int64_t ldb, double beta, double* C, int64_t ldc) {
     if (a_mode < 0 || a_mode > 1 || b_mode < 0 || b_mode > 1 || M > (1ll << 30) || N > (1ll << 30) || K > (1ll << 30))
         return fail(CES_ERR_INVALID, "ces_gemm: bad mode or size%s", "");
+    if (!gemm_ld_ok(a_mode, b_mode, M, N, K, lda, ldb, ldc))
+        return fail(CES_ERR_INVALID, "ces_gemm: leading dimension smaller than the operand's stored row%s", "");
     GemmCall g;
     g.a_mode = a_mode; g.b_mode = b_mode;
     g.M = (int)M; g.N = (int)N; g.K = (int)K;
     g.A = A; g.lda = lda; g.B = B; g.ldb = ldb; g.C = C; g.ldc = ldc;
     g.alpha = alpha; g.beta = beta;
+    return gemm(static_cast<cudaStream_t>(stream), g);
+}
+
+int ces_gemm_ex(void* stream, const ces_gemm_desc* d) {
+    if (!d || d->struct_size != (int64_t)sizeof(ces_gemm_desc))
+        return fail(CES_ERR_INVALID, "ces_gemm_ex: null descriptor or struct_size != sizeof(ces_gemm_desc)%s", "");
+    const int64_t lim = 1ll << 30;
+    if (d->a_mode < 0 || d->a_mode > 1 || d->b_mode < 0 || d->b_mode > 1 || d->M < 1 || d->N < 1 || d->K < 1 || d->M > lim ||
+        d->N > lim || d->K > lim || d->batch < 1 || d->batch > 65535 || d->a_batch_rows < 0 || d->b_batch_rows < 0 ||
+        d->a_batch_rows > lim || d->b_batch_rows > lim || d->c_batch_elems < 0 || d->splits < 0 || d->splits > 65535 || d->group_m < 0 ||
+        (d->flags & ~(GEMM_A_LOWER_TRI | GEMM_C_LOWER_ONLY | GEMM_B_UPPER_TRI)) != 0)
+        return fail(CES_ERR_INVALID, "ces_gemm_ex: bad mode, size, batch or flags%s", "");
+    if (!gemm_ld_ok(d->a_mode, d->b_mode, d->M, d->N, d->K, d->lda, d->ldb, d->ldc))
+        return fail(CES_ERR_INVALID, "ces_gemm_ex: leading dimension smaller than the operand's stored row%s", "");
+    // capacities: the planes the kernel writes into the workspace and the partial slots of every tile of every problem
+    const int64_t kb = ceil_div(d->K, GEMM_BK);
+    const int64_t planes = d->batch > 1 ? d->batch : (d->splits > 1 ? (d->splits < kb ? d->splits : kb) : 1);
+    if (d->splitk_ws && planes * d->M * d->N > d->splitk_ws_elems)
+        return fail(CES_ERR_INVALID, "ces_gemm_ex: workspace smaller than (splits or batch) * M * N%s", "");
+    if (d->ssq_partials && (int64_t)gemm_tiles((int)d->M, (int)d->N) * d->batch > d->ssq_partials_elems)
+        return fail(CES_ERR_INVALID, "ces_gemm_ex: partials buffer smaller than gemm_tiles(M, N) * batch%s", "");
+    GemmCall g;
+    g.a_mode = d->a_mode; g.b_mode = d->b_mode;
+    g.M = (int)d->M; g.N = (int)d->N; g.K = (int)d->K;
+    g.A = d->A; g.lda = d->lda; g.B = d->B; g.ldb = d->ldb; g.C = d->C; g.ldc = d->ldc;
+    g.alpha = d->alpha; g.beta = d->beta; g.alpha_dev = d->alpha_dev;
+    g.flags = d->flags; g.group_m = d->group_m;
+    g.ssq_partials = d->ssq_partials;
+    g.splits = d->splits; g.splitk_ws = d->splitk_ws; g.diag_add = d->diag_add;
+    g.batch = d->batch; g.a_batch_rows = d->a_batch_rows; g.b_batch_rows = d->b_batch_rows; g.c_batch_elems = d->c_batch_elems;
+    g.wave_ctas = d->wave_ctas; g.serpentine = d->serpentine;
     return gemm(static_cast<cudaStream_t>(stream), g);
 }
 
@@ -1636,6 +1674,26 @@ int ces_posv(void* stream, double* A, int64_t lda, int64_t n, double* B, int64_t
     if (s == CES_OK) s = trsm_lower(st, A, lda, n, Linv, kLinvLd, B, ldb, nrhs, false);
     if (s == CES_OK) s = trsm_lower(st, A, lda, n, Linv, kLinvLd, B, ldb, nrhs, true);
     if (cudaStreamSynchronize(st) != cudaSuccess && s == CES_OK) s = fail(CES_ERR_CUDA, "ces_posv: kernel failure%s", "");
+    cudaFree(Linv);
+    cudaFree(info);
+    return s;
+}
+
+int ces_potri(void* stream, double* A, int64_t ld, int64_t n, double* Ainv, int64_t ldo) {
+    if (!A || !Ainv || n < 1 || ld < n || ldo < n) return fail(CES_ERR_INVALID, "ces_potri: bad argument%s", "");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    double* Linv = nullptr;
+    int* info = nullptr;
+    CES_CUDA(cudaMalloc(&Linv, (size_t)round_up(n, CHOL_NB) * kLinvLd * sizeof(double)));
+    if (cudaMalloc(&info, sizeof(int)) != cudaSuccess) { cudaFree(Linv); return fail(CES_ERR_NOMEM, "cudaMalloc failed%s", ""); }
+    cudaMemsetAsync(info, 0, sizeof(int), st);
+    int s = potrf_lower(st, A, ld, n, Linv, kLinvLd, info);
+    int hinfo = 0;
+    if (s == CES_OK && cudaMemcpyAsync(&hinfo, info, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess) s = CES_ERR_CUDA;
+    if (s == CES_OK && cudaStreamSynchronize(st) != cudaSuccess) s = fail(CES_ERR_CUDA, "ces_potri: kernel failure%s", "");
+    if (s == CES_OK && hinfo != 0) s = fail(CES_ERR_NOT_SPD, "ces_potri: matrix is not positive definite (pivot %s%lld)", "", hinfo);
+    if (s == CES_OK) s = spd_inverse_from_factor(st, A, ld, n, Linv, kLinvLd, Ainv, ldo);
+    if (cudaStreamSynchronize(st) != cudaSuccess && s == CES_OK) s = fail(CES_ERR_CUDA, "ces_potri: kernel failure%s", "");
     cudaFree(Linv);
     cudaFree(info);
     return s;

@@ -42,15 +42,37 @@ int gemm_sm_count() {
 }
 
 int gemm(cudaStream_t st, const GemmCall& c) {
+    // every argument check runs before the tensor maps are built (those need the driver), so a rejected call does no
+    // device work at all
     if (c.M < 1 || c.N < 1 || c.K < 1 || !c.A || !c.B || !c.C) return fail(CES_ERR_INVALID, "gemm: bad shape or null operand%s", "");
-    CUtensorMap ma, mb;
-    // tensor-map row extents cover every batch of a batched operand
     const int64_t nb = c.batch > 1 ? c.batch : 1;
-    const int64_t a_rows = (c.a_mode == A_MK ? c.M : c.K) + (nb - 1) * c.a_batch_rows;
-    const int64_t b_rows = (c.b_mode == B_NK ? c.N : c.K) + (nb - 1) * c.b_batch_rows;
     // a batch either writes one C per problem (c_batch_elems) or, with a workspace, is summed into a single C
     // (one plane per batch, reduced like split-K); it cannot be combined with split-K itself
     if (nb > 1 && c.splits > 1) return fail(CES_ERR_INVALID, "gemm: batching excludes split-K%s", "");
+    const int kb_total = (int)ceil_div(c.K, GEMM_BK);
+    int splits = c.splits > 1 ? c.splits : 1;
+    if (splits > kb_total) splits = kb_total;
+    // With a workspace the kernel writes raw partial products and the reduce kernel applies
+    // alpha / beta / diag_add and mirrors symmetric results (also used with a single split).
+    const bool via_ws = c.splitk_ws != nullptr;
+    if (splits > 1 && !via_ws) return fail(CES_ERR_INVALID, "gemm: split-K needs a workspace%s", "");
+    if (via_ws && c.ssq_partials) return fail(CES_ERR_INVALID, "gemm: workspace path cannot produce sum-of-squares partials%s", "");
+    if (!via_ws && c.diag_add != 0.0) return fail(CES_ERR_INVALID, "gemm: diag_add needs the workspace path%s", "");
+    if (c.flags & GEMM_C_LOWER_ONLY) {
+        if (c.M != c.N) return fail(CES_ERR_INVALID, "gemm: GEMM_C_LOWER_ONLY needs a square C%s", "");
+        // the skipped tiles would leave their partial slots unwritten
+        if (c.ssq_partials) return fail(CES_ERR_INVALID, "gemm: GEMM_C_LOWER_ONLY cannot produce sum-of-squares partials%s", "");
+    }
+    // The last contraction box of batch z reads rows K .. round_up(K, 16) of a row-batched operand, which are batch z+1's.
+    // That is harmless only where the other operand is zero-filled there (A_MK / B_NK, or a shared operand).
+    if (nb > 1 && c.a_mode == A_KM && c.b_mode == B_KN && c.a_batch_rows != 0 && c.b_batch_rows != 0 && c.K % GEMM_BK != 0)
+        return fail(CES_ERR_INVALID, "gemm: A_KM x B_KN with both operands batched needs K %% 16 == 0%s", "");
+    if (c.wave_ctas < 0 || c.serpentine < -1 || c.serpentine > 1) return fail(CES_ERR_INVALID, "gemm: bad wave_ctas or serpentine%s", "");
+
+    CUtensorMap ma, mb;
+    // tensor-map row extents cover every batch of a batched operand
+    const int64_t a_rows = (c.a_mode == A_MK ? c.M : c.K) + (nb - 1) * c.a_batch_rows;
+    const int64_t b_rows = (c.b_mode == B_NK ? c.N : c.K) + (nb - 1) * c.b_batch_rows;
     // problems with at most 64 rows run the 64-row tile variant (half the A tile, no DMMA wasted on zero rows)
     const int bm = (c.M <= 64 && nb == 1) ? 64 : GEMM_BM;
     if (c.a_mode == A_MK) CES_TRY(make_map_2d(&ma, c.A, c.K, a_rows, c.lda, 16, bm));
@@ -68,24 +90,15 @@ int gemm(cudaStream_t st, const GemmCall& c) {
     static const int env_group = []() { const char* e = std::getenv("CES_GEMM_GROUP_M"); return e ? atoi(e) : 0; }();
     a.group_m = c.group_m > 0 ? c.group_m : (env_group > 0 ? env_group : 16);
     a.flags = c.flags;
-    a.splits = 1;
-    a.kblocks_per_split = 0;
-    a.splitk_ws = nullptr;
     {
-        a.wave_ctas = gemm_sm_count();
+        a.wave_ctas = c.wave_ctas > 0 ? c.wave_ctas : gemm_sm_count();
         static const int env_serp = []() { const char* e = std::getenv("CES_GEMM_SERPENTINE"); return e ? atoi(e) : -1; }();
         // default on: -23 % DRAM reads on the D GEMM (profiles/r01_gemm_raster_sweep.csv); CES_GEMM_SERPENTINE=0 disables
-        if (env_serp != 0) a.flags |= GEMM_SERPENTINE_K;
+        const bool serp = c.serpentine >= 0 ? c.serpentine == 1 : env_serp != 0;
+        if (serp) a.flags |= GEMM_SERPENTINE_K;
+        else      a.flags &= ~GEMM_SERPENTINE_K;
     }
     a.a_batch_rows = (int)c.a_batch_rows; a.b_batch_rows = (int)c.b_batch_rows; a.c_batch_elems = c.c_batch_elems;
-    const int kb_total = (int)ceil_div(c.K, GEMM_BK);
-    int splits = c.splits > 1 ? c.splits : 1;
-    if (splits > kb_total) splits = kb_total;
-    // With a workspace the kernel writes raw partial products and the reduce kernel applies
-    // alpha / beta / diag_add and mirrors symmetric results (also used with a single split).
-    const bool via_ws = c.splitk_ws != nullptr;
-    if (splits > 1 && !via_ws) return fail(CES_ERR_INVALID, "gemm: split-K needs a workspace%s", "");
-    if (via_ws && c.ssq_partials) return fail(CES_ERR_INVALID, "gemm: workspace path cannot produce sum-of-squares partials%s", "");
     a.kblocks_per_split = (int)ceil_div(kb_total, splits);
     a.splits = (int)ceil_div(kb_total, a.kblocks_per_split);
     a.splitk_ws = c.splitk_ws;

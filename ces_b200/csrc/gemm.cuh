@@ -47,7 +47,9 @@ struct GemmArgs {
     int kblocks_per_split, splits;
     int flags;
     // batching over blockIdx.y: batch z uses operand rows shifted by z*{a,b}_batch_rows (0 = shared operand)
-    // and writes C + z*c_batch_elems.  A batched operand must fill whole TMA boxes along its row axis.
+    // and writes C + z*c_batch_elems.  When K % 16 != 0 the last k-box of problem z also reads stored rows K .. round_up(K, 16)
+    // of a batched A_KM / B_KN operand, which belong to problem z+1 (or to the padding between problems): those rows must be
+    // finite and meet a zero-filled operand (A_MK / B_NK, or a shared operand).  gemm() refuses A_KM x B_KN with both batched.
     int a_batch_rows, b_batch_rows;
     long long c_batch_elems;
     int wave_ctas;             // CTAs resident at once (SM count); used by GEMM_SERPENTINE_K

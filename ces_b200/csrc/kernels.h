@@ -34,6 +34,9 @@ struct GemmCall {
     double diag_add = 0.0;            // reduce epilogue only
     // batched form: `batch` problems, operand rows shifted by z*{a,b}_batch_rows (0 = shared), C by z*c_batch_elems
     int64_t batch = 1, a_batch_rows = 0, b_batch_rows = 0, c_batch_elems = 0;
+    // walk of the contraction axis (ces_gemm_ex): CTAs per wave (0 = SM count), serpentine -1 = CES_GEMM_SERPENTINE / on,
+    // 0 = off, 1 = on
+    int wave_ctas = 0, serpentine = -1;
 };
 
 int gemm(cudaStream_t st, const GemmCall& c);

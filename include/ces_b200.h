@@ -316,13 +316,52 @@ int ces_fill_ensemble_noise(void* stream, uint64_t seed, uint64_t step, double* 
 /* ---- building blocks exported for tests and for callers that own their orchestration ---------------
  * C[M,N] = alpha * op(A) op(B) + beta * C on the FP64 tensor cores.  a_mode: 0 = A is M x K row-major,
  * 1 = A is stored K x M (i.e. A^T given); b_mode: 0 = B is K x N row-major, 1 = B stored N x K.
- * Operands need 16-byte aligned bases and even leading dimensions. */
+ * Operands need 16-byte aligned bases and even leading dimensions no smaller than their stored rows (lda >= K or M,
+ * ldb >= N or K, ldc >= N; CES_ERR_INVALID otherwise). */
 int ces_gemm(void* stream, int a_mode, int b_mode, int64_t M, int64_t N, int64_t K, double alpha, const double* A_dev,
              int64_t lda, const double* B_dev, int64_t ldb, double beta, double* C_dev, int64_t ldc);
 /* In-place lower Cholesky of an n x n SPD matrix on the device (strict upper triangle zeroed). */
 int ces_potrf(void* stream, double* A_dev, int64_t ld, int64_t n);
 /* X = A^-1 B for SPD A (n x n) and B (n x nrhs), both on the device; A is overwritten by its factor. */
 int ces_posv(void* stream, double* A_dev, int64_t lda, int64_t n, double* B_dev, int64_t ldb, int64_t nrhs);
+/* Ainv = A^-1 (n x n, ld ldo) for SPD A on the device, through the blocked Cholesky and two triangular solves of the
+ * identity (the inverse the GP gradient uses); A is overwritten by its factor.  CES_ERR_NOT_SPD names the failing pivot. */
+int ces_potri(void* stream, double* A_dev, int64_t ld, int64_t n, double* Ainv_dev, int64_t ldo);
+
+/* ---- test support: not part of the stable interface --------------------------------------------------------------
+ * The whole DMMA GEMM family behind ces_gemm, for tests that pin each of its features:
+ *   C[M,N] = alpha (* *alpha_dev) * sum_kk op(A)(m,kk) op(B)(kk,n) + beta * C  (+ diag_add on the diagonal)
+ * flags: 1 = op(A) lower triangular (row tile tm reads kk < 128 (tm + 1) only, entries above the diagonal inside that
+ * range must be zero), 2 = only tiles on or below the diagonal (square C; mirrored when a workspace is given),
+ * 4 = op(B) upper triangular (column tile tn reads kk < 128 (tn + 1) only).  splits > 1 splits the contraction into
+ * planes of splitk_ws (splits*M*N doubles) that a reduce kernel sums; with a workspace alpha / beta / diag_add are
+ * applied there.  ssq_partials (no workspace, flag 2 excluded) receives one sum of squares of the stored values per
+ * 128 x 128 tile and problem.  batch > 1: problem z shifts A's and B's stored rows by z*a_batch_rows / z*b_batch_rows
+ * (0 = shared) and writes C + z*c_batch_elems, or, with a workspace, all problems are summed into C.  group_m (0 = 16):
+ * row tiles per rasterisation group.  wave_ctas (0 = SM count) and serpentine (-1 = environment default, 0 = off,
+ * 1 = on): odd waves of wave_ctas CTAs walk the contraction backwards.  struct_size must be sizeof(ces_gemm_desc), the
+ * capacities (in doubles) must cover what the call writes; otherwise CES_ERR_INVALID before any device work. */
+typedef struct ces_gemm_desc {
+    int64_t struct_size;
+    int32_t a_mode, b_mode;
+    int64_t M, N, K;
+    const double* A;
+    int64_t lda;
+    const double* B;
+    int64_t ldb;
+    double* C;
+    int64_t ldc;
+    double alpha, beta;
+    const double* alpha_dev;
+    int32_t flags, group_m, splits, wave_ctas, serpentine, reserved;
+    double* splitk_ws;
+    int64_t splitk_ws_elems;
+    double diag_add;
+    double* ssq_partials;
+    int64_t ssq_partials_elems;
+    int64_t batch, a_batch_rows, b_batch_rows, c_batch_elems;
+} ces_gemm_desc;
+int ces_gemm_ex(void* stream, const ces_gemm_desc* desc);
 
 /* ---- Metropolis-Hastings on the true forward model: MCMC.model_mh (ces/sample.py:121-196) ---------------------------
  * n_chains independent chains of n_mcmc proposals, one warp per chain, the loop entirely on the device (csrc/mcmc.cu).
