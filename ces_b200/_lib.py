@@ -49,7 +49,7 @@ class GemmDesc(ctypes.Structure):
                 ("wave_ctas", ctypes.c_int32), ("serpentine", ctypes.c_int32), ("reserved", ctypes.c_int32),
                 ("splitk_ws", _dp), ("splitk_ws_elems", _i64), ("diag_add", _dbl), ("ssq_partials", _dp),
                 ("ssq_partials_elems", _i64), ("batch", _i64), ("a_batch_rows", _i64), ("b_batch_rows", _i64),
-                ("c_batch_elems", _i64)]
+                ("c_batch_elems", _i64), ("row_vec", _dp)]
 
     def __init__(self, **kw):
         base = dict(struct_size=ctypes.sizeof(GemmDesc), alpha=1.0, serpentine=-1, batch=1)

@@ -33,6 +33,7 @@ struct ces_handle_s {
     double *xi_pad = nullptr, *expU = nullptr;
     double *Cuu = nullptr, *L = nullptr, *Linv = nullptr, *M = nullptr, *Minv = nullptr, *cb = nullptr;
     double *D = nullptr, *ssq_partials = nullptr, *splitk_ws = nullptr, *v_ws = nullptr;
+    double *dvec = nullptr, *uc = nullptr;   // single GPU: c = E^T w0 (J) and U~ c / J (p), the rank-one part of D and V
     int64_t ssq_cap = 0, splitk_cap = 0, ssq_used = 0, v_ws_planes = 4;
     int syrk_splits = 1;
     int* info = nullptr;
@@ -42,6 +43,7 @@ struct ces_handle_s {
     // K11 (time_step 'constant' / 'mix'): D re-solved with Gamma -> h*C^pp + Gamma
     std::vector<double> gamma_host;
     double *GammaD = nullptr, *Cpp = nullptr, *Mk = nullptr, *MkLinv = nullptr, *MkInv = nullptr, *Wr = nullptr, *cpp_ws = nullptr, *eig_ws = nullptr;
+    double* zr = nullptr;               // M^-1 c: the w0 of the re-solve
     int cpp_splits = 1;
     // host staging
     double* hS = nullptr;   // pinned, S_COUNT doubles + 1 int
@@ -238,6 +240,7 @@ int ces_create(int64_t p, int64_t k, int64_t J_local, int64_t J_global, int rank
     A_(Cuu, p * h->ldp); A_(L, p * h->ldp); A_(Linv, round_up(p, CHOL_NB) * kLinvLd);
     A_(D, slots * h->ldJ * h->ldD);
     A_(ssq_partials, h->ssq_cap); A_(splitk_ws, h->splitk_cap);
+    A_(dvec, h->ldJ); A_(uc, p);
 #undef A_
     if (s == CES_OK) {
         void* ip = nullptr;
@@ -449,8 +452,124 @@ struct InteractRange {
     bool finish = true;                  // last call of a step: reduce the partials into S[S_SSQ]
 };
 
-static int interaction_loops(ces_handle_t h, const double* Wsrc, bool accumulate_ssq, int first, int count,
+// V = U~ D as a GEMM over the contraction K; split 2-4 ways when the d/128 x N/128 tiles quantise badly on 148 SMs
+// (e.g. 512 tiles = 3.46 waves) and the partial planes fit the V workspace.
+static int v_gemm(ces_handle_t h, GemmCall& g) {
+    const double tiles = (double)gemm_tiles(g.M, g.N);
+    int best = 1;
+    double best_eff = 0.0;
+    for (int sp = 1; sp <= 4; ++sp) {
+        const double waves = tiles * sp / 148.0;
+        const double eff = waves / ceil(waves);
+        if (eff > best_eff + 0.02) { best_eff = eff; best = sp; }
+        if (best_eff >= 0.97) break;
+    }
+    if (best > 1 && g.K >= 64 * best && (int64_t)best * g.N <= h->v_ws_planes * h->panel) {
+        if (!h->v_ws) CES_TRY(dalloc(h, &h->v_ws, h->v_ws_planes * h->p * h->panel));
+        g.splits = best;
+        g.splitk_ws = h->v_ws;
+    }
+    return gemm(h->st, g);
+}
+
+// Event pair around a D launch (ces_profile_*), credited with the flops of the outputs it forms.
+static int profile_begin(ces_handle_t h) {
+    if (!h->profile) return CES_OK;
+    while (h->ev_pool.size() < h->ev_used + 2) {
+        cudaEvent_t e;
+        CES_CUDA(cudaEventCreate(&e));
+        h->ev_pool.push_back(e);
+    }
+    CES_CUDA(cudaEventRecord(h->ev_pool[h->ev_used], h->st));
+    return CES_OK;
+}
+static int profile_end(ces_handle_t h, double flops) {
+    if (!h->profile) return CES_OK;
+    CES_CUDA(cudaEventRecord(h->ev_pool[h->ev_used + 1], h->st));
+    h->ev_used += 2;
+    h->prof_flops += flops;
+    return CES_OK;
+}
+
+// Single GPU.  With R = E + c_g 1^T (c_g = mean - y) and W = B R for the symmetric B (Gamma^-1, or M^-1 in the re-solve):
+//   J D = E^T W = S + c 1^T,   S = E^T B E  symmetric,   c = E^T w0,   w0 = B c_g.
+// Column panel [a, b) of D forms only the lower trapezoid of S / J: D workspace row r stands for particle a + r, and the
+// launch covers the tiles tn <= tm of E[:, a:J]^T W[:, a:b], storing (acc - c_i) / J (the row term on the last
+// contraction chunk).  The strictly lower tiles of the panel's diagonal block are mirrored into its upper tiles; the rows
+// above the panel (particles < a) are the transposes of earlier panels, whose products have already added them:
+//   V[:, a:b] (+)= U~[:, a:J] Dws[0:J-a, :],    V[:, b:J] (+)= U~[:, a:b] Dws[b-a:J-a, :]^T,
+// and once per step V += (U~ c / J) 1^T.  Every entry of D still comes from the J x J contraction: half the D flops of
+// forming both triangles, the same V flops.  ||D||_F^2 is taken from the stored values plus the row term, a tile below
+// the diagonal counting for its mirror too (GEMM_C_LOWER_TRAP).  `w0` must be ready when the last chunk of panel 0 runs.
+static int symmetric_loops(ces_handle_t h, const double* Wsrc, const double* w0, bool accumulate_ssq, const InteractRange& rg) {
+    const int64_t p = h->p, k = h->k, ld = h->ldJ, J = h->Jl;
+    cudaStream_t st = h->st;
+    if (rg.reset) h->ssq_used = 0;
+    int64_t npart = h->ssq_used;
+    const double invJ = 1.0 / (double)h->Jg;
+    const int64_t c_end = rg.c_end < 0 ? J : rg.c_end;
+    const int64_t k_lo = rg.k_lo, k_hi = rg.k_hi < 0 ? k : rg.k_hi;
+    const bool last_chunk = (k_hi == k);
+    double* E = e_block(h, 0);
+    double* Ut = ut_block(h, 0);
+    if (rg.do_d && last_chunk && rg.c_begin == 0) CES_TRY(col_dot(st, E, ld, k, J, w0, h->qpart, h->dvec));
+    for (int64_t a = rg.c_begin; a < c_end; a += h->panel) {
+        const int64_t nc = (c_end - a) < h->panel ? (c_end - a) : h->panel;
+        const int64_t b = a + nc;
+        if (rg.do_d) {
+            GemmCall g1;
+            g1.a_mode = A_KM; g1.b_mode = B_KN;
+            g1.M = (int)(J - a); g1.N = (int)nc; g1.K = (int)(k_hi - k_lo);
+            g1.A = E + k_lo * ld + a; g1.lda = ld;
+            g1.B = Wsrc + k_lo * ld + a; g1.ldb = ld;
+            g1.C = h->D; g1.ldc = h->ldD;
+            g1.alpha = invJ;
+            g1.beta = k_lo > 0 ? 1.0 : 0.0;
+            g1.flags = GEMM_C_LOWER_TRAP;
+            if (last_chunk) g1.row_vec = h->dvec + a;
+            if (accumulate_ssq && last_chunk) {
+                const int64_t tiles = gemm_trap_tiles(g1.M, g1.N);
+                if (npart + tiles > h->ssq_cap) return fail(CES_ERR_STATE, "phase3: partial-sum buffer too small%s", "");
+                g1.ssq_partials = h->ssq_partials + npart;
+                npart += tiles;
+            }
+            CES_TRY(profile_begin(h));
+            CES_TRY(gemm(st, g1));
+            CES_TRY(profile_end(h, 2.0 * (double)g1.K * (double)gemm_trap_entries(g1.M, g1.N)));
+            if (last_chunk) CES_TRY(mirror_lower_tiles(st, h->D, h->ldD, nc));
+        }
+        if (!rg.do_v) continue;
+        GemmCall g2;
+        g2.a_mode = A_MK; g2.b_mode = B_KN;
+        g2.M = (int)p; g2.N = (int)nc; g2.K = (int)(J - a);
+        g2.A = Ut + a; g2.lda = ld;
+        g2.B = h->D; g2.ldb = h->ldD;
+        g2.C = h->V + a; g2.ldc = ld;
+        g2.beta = a > 0 ? 1.0 : 0.0;
+        CES_TRY(v_gemm(h, g2));
+        if (b < J) {
+            GemmCall g3;
+            g3.a_mode = A_MK; g3.b_mode = B_NK;
+            g3.M = (int)p; g3.N = (int)(J - b); g3.K = (int)nc;
+            g3.A = Ut + a; g3.lda = ld;
+            g3.B = h->D + nc * h->ldD; g3.ldb = h->ldD;
+            g3.C = h->V + b; g3.ldc = ld;
+            g3.beta = a > 0 ? 1.0 : 0.0;
+            CES_TRY(v_gemm(h, g3));
+        }
+    }
+    h->ssq_used = npart;
+    if (rg.do_v && c_end == J) {
+        CES_TRY(row_dot(st, Ut, ld, p, J, h->dvec, invJ, h->uc));
+        CES_TRY(add_col_vector(st, h->V, ld, p, J, h->uc, 1.0, nullptr));
+    }
+    if (accumulate_ssq && rg.finish) CES_TRY(sum_vector(st, h->ssq_partials, npart, h->S + S_SSQ));
+    return CES_OK;
+}
+
+static int interaction_loops(ces_handle_t h, const double* Wsrc, const double* w0, bool accumulate_ssq, int first, int count,
                              const InteractRange& rg = InteractRange()) {
+    if (h->nranks == 1) return symmetric_loops(h, Wsrc, w0, accumulate_ssq, rg);
     const int64_t p = h->p, k = h->k, ld = h->ldJ;
     cudaStream_t st = h->st;
     if (first == 0 && rg.reset) h->ssq_used = 0;
@@ -484,19 +603,10 @@ static int interaction_loops(ces_handle_t h, const double* Wsrc, bool accumulate
                 g1.ssq_partials = h->ssq_partials + npart;
                 npart += tiles;
             }
-            if (rg.do_d && h->profile) {
-                while (h->ev_pool.size() < h->ev_used + 2) {
-                    cudaEvent_t e;
-                    CES_CUDA(cudaEventCreate(&e));
-                    h->ev_pool.push_back(e);
-                }
-                CES_CUDA(cudaEventRecord(h->ev_pool[h->ev_used], st));
-            }
-            if (rg.do_d) CES_TRY(gemm(st, g1));
-            if (rg.do_d && h->profile) {
-                CES_CUDA(cudaEventRecord(h->ev_pool[h->ev_used + 1], st));
-                h->ev_used += 2;
-                h->prof_flops += 2.0 * (double)g1.K * (double)g1.M * (double)g1.N * run;
+            if (rg.do_d) {
+                CES_TRY(profile_begin(h));
+                CES_TRY(gemm(st, g1));
+                CES_TRY(profile_end(h, 2.0 * (double)g1.K * (double)g1.M * (double)g1.N * run));
             }
             if (!rg.do_v) { i += run; continue; }
             GemmCall g2;
@@ -511,25 +621,10 @@ static int interaction_loops(ces_handle_t h, const double* Wsrc, bool accumulate
                 if (!h->v_ws) CES_TRY(dalloc(h, &h->v_ws, h->v_ws_planes * p * h->panel));
                 g2.batch = run; g2.a_batch_rows = p; g2.b_batch_rows = h->Jl;
                 g2.splitk_ws = h->v_ws;
+                CES_TRY(gemm(st, g2));
             } else {
-                // wave quantisation: d/128 x nc/128 tiles of a long contraction rarely fill 148 SMs evenly (e.g. 512
-                // tiles = 3.46 waves); splitting the contraction 2-4 ways makes the tail negligible
-                const double tiles = (double)gemm_tiles(g2.M, g2.N);
-                int best = 1;
-                double best_eff = 0.0;
-                for (int sp = 1; sp <= 4; ++sp) {
-                    const double waves = tiles * sp / 148.0;
-                    const double eff = waves / ceil(waves);
-                    if (eff > best_eff + 0.02) { best_eff = eff; best = sp; }
-                    if (best_eff >= 0.97) break;
-                }
-                if (best > 1 && g2.K >= 64 * best) {
-                    if (!h->v_ws) CES_TRY(dalloc(h, &h->v_ws, h->v_ws_planes * p * h->panel));
-                    g2.splits = best;
-                    g2.splitk_ws = h->v_ws;
-                }
+                CES_TRY(v_gemm(h, g2));
             }
-            CES_TRY(gemm(st, g2));
             i += run;
         }
     }
@@ -546,7 +641,7 @@ int ces_phase3_interact(ces_handle_t h, int rule, int skip_interaction) {
     CES_TRY(start_cholesky(h, rule));
     if (skip_interaction) return CES_OK;       // 'constant' step size: D is formed once, by ces_phase3c_resolve
     mark(h, "phase3:begin");
-    CES_TRY(interaction_loops(h, h->W, true, 0, h->nranks));
+    CES_TRY(interaction_loops(h, h->W, h->zvec, true, 0, h->nranks));
     mark(h, "phase3:end");
     return CES_OK;
 }
@@ -558,7 +653,7 @@ int ces_phase3_blocks(ces_handle_t h, int rule, int first, int count) {
     if (first == 0) CES_TRY(start_cholesky(h, rule));
     if (count == 0) return CES_OK;
     mark(h, first == 0 ? "phase3:own:begin" : "phase3:rest:begin");
-    CES_TRY(interaction_loops(h, h->W, true, first, count));
+    CES_TRY(interaction_loops(h, h->W, h->zvec, true, first, count));
     mark(h, first == 0 ? "phase3:own:end" : "phase3:rest:end");
     return CES_OK;
 }
@@ -617,6 +712,7 @@ int ces_phase3b_cpp(ces_handle_t h) {
         CES_TRY(dalloc(h, &h->MkInv, k * h->ldk));
         CES_TRY(dalloc(h, &h->MkLinv, round_up(k, CHOL_NB) * kLinvLd));
         CES_TRY(dalloc(h, &h->Wr, k * ld));
+        CES_TRY(dalloc(h, &h->zr, k));
         CES_TRY(dalloc(h, &h->GammaD, k * h->ldk));
         if (!h->R) CES_TRY(dalloc(h, &h->R, k * ld));
         CES_TRY(upload_square(h, h->gamma_host.data(), k, h->GammaD, h->ldk));
@@ -652,8 +748,9 @@ int ces_phase3c_resolve(ces_handle_t h, int rule) {
     g.M = (int)k; g.N = (int)h->Jl; g.K = (int)k;
     g.A = h->MkInv; g.lda = h->ldk; g.B = h->R; g.ldb = ld; g.C = h->Wr; g.ldc = ld;
     CES_TRY(gemm(st, g));
+    CES_TRY(matvec(st, h->MkInv, h->ldk, k, h->cvec, h->zr));   // w0 = M^-1 c of the single-GPU schedule
     // the step size stays the one computed from the Gamma-only D (ces/calibrate.py:437 precedes :439-441)
-    return interaction_loops(h, h->Wr, false, 0, h->nranks);
+    return interaction_loops(h, h->Wr, h->zr, false, 0, h->nranks);
 }
 
 // time_step='spectral' (ces/calibrate.py:249-251): radspec = eigvals(D).real.max() = lambda_max(Gamma^-1 C^pp), see eig.cu.
@@ -1183,7 +1280,9 @@ int ces_host_interact_chunk(ces_handle_t h, int chunk) {
         rg.c_begin = 0; rg.c_end = h->panel < h->Jl ? h->panel : h->Jl; rg.k_lo = r0; rg.k_hi = r0 + nr;
         rg.do_v = false; rg.reset = (chunk == 0); rg.finish = false;
         mark(h, ck[chunk]);
-        CES_TRY(interaction_loops(h, h->W, true, 0, 1, rg));
+        // the last chunk applies the rank-one row term, from z = Gamma^-1 c (finish_g recomputes the same z later)
+        if (h->nranks == 1 && chunk == h->hb_nchunk - 1) CES_TRY(scale_vector(h->st, h->ginv_diag, h->cvec, h->zvec, h->k));
+        CES_TRY(interaction_loops(h, h->W, h->zvec, true, 0, 1, rg));
         mark(h, dk[chunk]);
     }
     return CES_OK;
@@ -1219,19 +1318,19 @@ int ces_host_interact_own(ces_handle_t h) {
         const int64_t panel0 = h->panel < h->Jl ? h->panel : h->Jl;
         InteractRange rv;                         // V of the first panel, then the remaining panels as usual
         rv.c_begin = 0; rv.c_end = panel0; rv.do_d = false; rv.reset = false; rv.finish = whole && (panel0 >= h->Jl);
-        CES_TRY(interaction_loops(h, h->W, true, 0, 1, rv));
+        CES_TRY(interaction_loops(h, h->W, h->zvec, true, 0, 1, rv));
         mark(h, "V0");
         if (panel0 < h->Jl) {
             InteractRange rr;
             rr.c_begin = panel0; rr.reset = false; rr.finish = whole;
-            CES_TRY(interaction_loops(h, h->W, true, 0, 1, rr));
+            CES_TRY(interaction_loops(h, h->W, h->zvec, true, 0, 1, rr));
             mark(h, "panels:rest");
         }
         return CES_OK;
     }
     InteractRange all;
     all.finish = whole;
-    return interaction_loops(h, h->W, true, 0, 1, all);
+    return interaction_loops(h, h->W, h->zvec, true, 0, 1, all);
 }
 
 int ces_host_update(ces_handle_t h, int ts_kind, double fixed_h, double* Uout_host, double* hk_host, double* metrics_host) {
@@ -1616,7 +1715,7 @@ int ces_gemm_ex(void* stream, const ces_gemm_desc* d) {
     if (d->a_mode < 0 || d->a_mode > 1 || d->b_mode < 0 || d->b_mode > 1 || d->M < 1 || d->N < 1 || d->K < 1 || d->M > lim ||
         d->N > lim || d->K > lim || d->batch < 1 || d->batch > 65535 || d->a_batch_rows < 0 || d->b_batch_rows < 0 ||
         d->a_batch_rows > lim || d->b_batch_rows > lim || d->c_batch_elems < 0 || d->splits < 0 || d->splits > 65535 || d->group_m < 0 ||
-        (d->flags & ~(GEMM_A_LOWER_TRI | GEMM_C_LOWER_ONLY | GEMM_B_UPPER_TRI)) != 0)
+        (d->flags & ~(GEMM_A_LOWER_TRI | GEMM_C_LOWER_ONLY | GEMM_B_UPPER_TRI | GEMM_C_LOWER_TRAP)) != 0)
         return fail(CES_ERR_INVALID, "ces_gemm_ex: bad mode, size, batch or flags%s", "");
     if (!gemm_ld_ok(d->a_mode, d->b_mode, d->M, d->N, d->K, d->lda, d->ldb, d->ldc))
         return fail(CES_ERR_INVALID, "ces_gemm_ex: leading dimension smaller than the operand's stored row%s", "");
@@ -1625,8 +1724,10 @@ int ces_gemm_ex(void* stream, const ces_gemm_desc* d) {
     const int64_t planes = d->batch > 1 ? d->batch : (d->splits > 1 ? (d->splits < kb ? d->splits : kb) : 1);
     if (d->splitk_ws && planes * d->M * d->N > d->splitk_ws_elems)
         return fail(CES_ERR_INVALID, "ces_gemm_ex: workspace smaller than (splits or batch) * M * N%s", "");
-    if (d->ssq_partials && (int64_t)gemm_tiles((int)d->M, (int)d->N) * d->batch > d->ssq_partials_elems)
-        return fail(CES_ERR_INVALID, "ces_gemm_ex: partials buffer smaller than gemm_tiles(M, N) * batch%s", "");
+    const int64_t tiles = (d->flags & GEMM_C_LOWER_TRAP) && d->M >= d->N ? gemm_trap_tiles((int)d->M, (int)d->N)
+                                                                           : (int64_t)gemm_tiles((int)d->M, (int)d->N);
+    if (d->ssq_partials && tiles * d->batch > d->ssq_partials_elems)
+        return fail(CES_ERR_INVALID, "ces_gemm_ex: partials buffer smaller than the launched tiles * batch%s", "");
     GemmCall g;
     g.a_mode = d->a_mode; g.b_mode = d->b_mode;
     g.M = (int)d->M; g.N = (int)d->N; g.K = (int)d->K;
@@ -1637,6 +1738,7 @@ int ces_gemm_ex(void* stream, const ces_gemm_desc* d) {
     g.splits = d->splits; g.splitk_ws = d->splitk_ws; g.diag_add = d->diag_add;
     g.batch = d->batch; g.a_batch_rows = d->a_batch_rows; g.b_batch_rows = d->b_batch_rows; g.c_batch_elems = d->c_batch_elems;
     g.wave_ctas = d->wave_ctas; g.serpentine = d->serpentine;
+    g.row_vec = d->row_vec;
     return gemm(static_cast<cudaStream_t>(stream), g);
 }
 

@@ -392,6 +392,59 @@ __global__ void __launch_bounds__(256) row_scale_kernel(const double* __restrict
     if (j >= cols) return;
     X[(size_t)blockIdx.y * ld + j] *= diag[blockIdx.y];
 }
+// col_dot: partial sums over this CTA's rows of X[m, j] v[m] -> part[blockIdx.y][ld] (two columns per thread, as
+// data_forms), then one fixed-order sum over the row blocks per column: deterministic.
+__global__ void __launch_bounds__(256) col_dot_kernel(const double* __restrict__ X, long long ld, int rows,
+                                                      const double* __restrict__ v, double* __restrict__ part,
+                                                      int rows_per_cta) {
+    const long long j = 2 * ((long long)blockIdx.x * 256 + threadIdx.x);
+    if (j >= ld) return;
+    const int m0 = blockIdx.y * rows_per_cta;
+    double a0 = 0.0, a1 = 0.0;
+#pragma unroll 4
+    for (int r = 0; r < rows_per_cta; ++r) {
+        const int m = m0 + r;
+        if (m >= rows) break;
+        const double2 x = *reinterpret_cast<const double2*>(X + (size_t)m * ld + j);
+        const double w = v[m];
+        a0 += x.x * w; a1 += x.y * w;
+    }
+    *reinterpret_cast<double2*>(part + (size_t)blockIdx.y * ld + j) = make_double2(a0, a1);
+}
+__global__ void __launch_bounds__(256) col_dot_finish_kernel(const double* __restrict__ part, int ny, long long ld,
+                                                             long long cols, double* __restrict__ out) {
+    const long long j = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (j >= cols) return;
+    double s = 0.0;
+    for (int y = 0; y < ny; ++y) s += part[(size_t)y * ld + j];
+    out[j] = s;
+}
+int col_dot(cudaStream_t st, const double* X, int64_t ld, int64_t rows, int64_t cols, const double* v, double* part,
+            double* out) {
+    const int rpc = form_rows_per_cta(rows, ld);
+    const int ny = (int)ceil_div(rows, rpc);
+    col_dot_kernel<<<dim3((unsigned)ceil_div(ld, 512), (unsigned)ny), 256, 0, st>>>(X, ld, (int)rows, v, part, rpc);
+    col_dot_finish_kernel<<<(unsigned)ceil_div(cols, 256), 256, 0, st>>>(part, ny, ld, cols, out);
+    CES_LAUNCHED(2);
+    return CES_OK;
+}
+
+// row_dot: one CTA per row, fixed-order block sum
+__global__ void __launch_bounds__(256) row_dot_kernel(const double* __restrict__ X, long long ld, long long cols,
+                                                      const double* __restrict__ v, double s, double* __restrict__ out) {
+    __shared__ double scratch[32];
+    const double* row = X + (size_t)blockIdx.x * ld;
+    double a = 0.0;
+    for (long long i = threadIdx.x; i < cols; i += 256) a += row[i] * v[i];
+    const double t = block_sum(a, scratch);
+    if (threadIdx.x == 0) out[blockIdx.x] = s * t;
+}
+int row_dot(cudaStream_t st, const double* X, int64_t ld, int64_t rows, int64_t cols, const double* v, double s, double* out) {
+    row_dot_kernel<<<(unsigned)rows, 256, 0, st>>>(X, ld, cols, v, s, out);
+    CES_LAUNCHED(1);
+    return CES_OK;
+}
+
 int row_scale(cudaStream_t st, const double* diag, double* X, int64_t ld, int64_t rows, int64_t cols) {
     dim3 grid((unsigned)ceil_div(cols, 256), (unsigned)rows);
     row_scale_kernel<<<grid, 256, 0, st>>>(diag, X, ld, cols);

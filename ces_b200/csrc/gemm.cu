@@ -30,6 +30,38 @@ static int launch_modes(cudaStream_t st, const GemmCall& c, const CUtensorMap& m
 
 int gemm_tiles(int M, int N) { return (int)(ceil_div(M, GEMM_BM) * ceil_div(N, GEMM_BN)); }
 
+int64_t gemm_trap_tiles(int M, int N) {
+    const int64_t tm = ceil_div(M, GEMM_BM), tn = ceil_div(N, GEMM_BN);
+    return tm * tn - tn * (tn - 1) / 2;
+}
+
+int64_t gemm_trap_entries(int M, int N) {
+    int64_t e = 0;
+    for (int64_t n0 = 0; n0 < N; n0 += GEMM_BN) e += (N - n0 < GEMM_BN ? N - n0 : GEMM_BN) * (M - n0);
+    return e;
+}
+
+// 32 x 32 blocks through shared memory (coalesced on both sides); a block lies inside one 128 x 128 tile
+__global__ void __launch_bounds__(256) mirror_lower_tiles_kernel(double* __restrict__ C, long long ldc, int n) {
+    __shared__ double blk[32][33];
+    const int r0 = blockIdx.y * 32, c0 = blockIdx.x * 32;          // destination block (upper tile)
+    if (r0 / GEMM_BM >= c0 / GEMM_BN) return;
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    for (int y = ty; y < 32; y += 8)
+        if (c0 + y < n && r0 + tx < n) blk[y][tx] = C[(size_t)(c0 + y) * ldc + r0 + tx];
+    __syncthreads();
+    for (int y = ty; y < 32; y += 8)
+        if (r0 + y < n && c0 + tx < n) C[(size_t)(r0 + y) * ldc + c0 + tx] = blk[tx][y];
+}
+
+int mirror_lower_tiles(cudaStream_t st, double* C, int64_t ldc, int64_t n) {
+    if (n <= GEMM_BN) return CES_OK;
+    const unsigned b = (unsigned)ceil_div(n, 32);
+    mirror_lower_tiles_kernel<<<dim3(b, b), 256, 0, st>>>(C, ldc, (int)n);
+    CES_LAUNCHED(1);
+    return CES_OK;
+}
+
 int gemm_sm_count() {
     static int sms_of[kMaxDevices] = {};
     int& sms = sms_of[device_slot()];
@@ -58,6 +90,12 @@ int gemm(cudaStream_t st, const GemmCall& c) {
     if (splits > 1 && !via_ws) return fail(CES_ERR_INVALID, "gemm: split-K needs a workspace%s", "");
     if (via_ws && c.ssq_partials) return fail(CES_ERR_INVALID, "gemm: workspace path cannot produce sum-of-squares partials%s", "");
     if (!via_ws && c.diag_add != 0.0) return fail(CES_ERR_INVALID, "gemm: diag_add needs the workspace path%s", "");
+    if (c.row_vec && via_ws) return fail(CES_ERR_INVALID, "gemm: row_vec needs the direct epilogue%s", "");
+    if (c.flags & GEMM_C_LOWER_TRAP) {
+        if (c.M < c.N) return fail(CES_ERR_INVALID, "gemm: GEMM_C_LOWER_TRAP needs M >= N%s", "");
+        if (via_ws || nb > 1 || (c.flags & GEMM_C_LOWER_ONLY))
+            return fail(CES_ERR_INVALID, "gemm: GEMM_C_LOWER_TRAP excludes the workspace, batching and GEMM_C_LOWER_ONLY%s", "");
+    }
     if (c.flags & GEMM_C_LOWER_ONLY) {
         if (c.M != c.N) return fail(CES_ERR_INVALID, "gemm: GEMM_C_LOWER_ONLY needs a square C%s", "");
         // the skipped tiles would leave their partial slots unwritten
@@ -102,7 +140,10 @@ int gemm(cudaStream_t st, const GemmCall& c) {
     a.kblocks_per_split = (int)ceil_div(kb_total, splits);
     a.splits = (int)ceil_div(kb_total, a.kblocks_per_split);
     a.splitk_ws = c.splitk_ws;
-    dim3 grid((unsigned)(a.tiles_m * a.tiles_n), (unsigned)nb, (unsigned)a.splits);
+    a.row_vec = c.row_vec;
+    const int64_t ctas = (c.flags & GEMM_C_LOWER_TRAP) ? (int64_t)a.tiles_m * a.tiles_n - (int64_t)a.tiles_n * (a.tiles_n - 1) / 2
+                                                       : (int64_t)a.tiles_m * a.tiles_n;
+    dim3 grid((unsigned)ctas, (unsigned)nb, (unsigned)a.splits);
     CES_TRY(bm == 64 ? launch_modes<64>(st, c, ma, mb, a, grid) : launch_modes<128>(st, c, ma, mb, a, grid));
     if (via_ws) {
         const long long total = (long long)c.M * c.N;

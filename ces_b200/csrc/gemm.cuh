@@ -53,7 +53,31 @@ struct GemmArgs {
     int a_batch_rows, b_batch_rows;
     long long c_batch_elems;
     int wave_ctas;             // CTAs resident at once (SM count); used by GEMM_SERPENTINE_K
+    const double* row_vec;     // optional [M]: stored value alpha * (acc - row_vec[m]) (+ beta * C)
 };
+
+// GEMM_C_LOWER_TRAP: linear CTA index -> tile (tm, tn) of the lower trapezoid tn <= tm (tiles_m >= tiles_n), launched
+// compactly.  Same grouped rasterisation as the full grid with the tiles above the diagonal left out: in a group of gs
+// row tiles starting at f, columns tn < f have all gs rows, columns f <= tn < f + gs the rows tn .. f + gs - 1.
+__device__ __forceinline__ void trap_tile(int L, int tiles_m, int tiles_n, int group_m, int& tm, int& tn) {
+    for (int f = 0; f < tiles_m; f += group_m) {
+        const int gs = min(tiles_m - f, group_m);
+        const int full = min(f, tiles_n);
+        const int nd = max(min(f + gs, tiles_n) - f, 0);      // columns crossing the group's diagonal
+        const int cnt = full * gs + nd * gs - nd * (nd - 1) / 2;
+        if (L < cnt) {
+            if (L < full * gs) { tm = f + L % gs; tn = L / gs; return; }
+            L -= full * gs;
+            for (int c = f;; ++c) {
+                const int rows = f + gs - c;
+                if (L < rows) { tn = c; tm = c + L; return; }
+                L -= rows;
+            }
+        }
+        L -= cnt;
+    }
+    tm = tn = 0;   // not reached for L < the trapezoid's tile count
+}
 
 // Byte offset of element (row r, contraction index kk) in a contraction-contiguous 128x16 tile.
 __device__ __forceinline__ uint32_t off_kc(int r, int kk) {
@@ -92,7 +116,9 @@ gemm_dmma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
 
     // ---- tile coordinates (grouped rasterisation: consecutive CTAs share B panels and a few A panels)
     int tm, tn;
-    {
+    if (args.flags & GEMM_C_LOWER_TRAP) {
+        trap_tile(blockIdx.x, args.tiles_m, args.tiles_n, args.group_m, tm, tn);
+    } else {
         const int L = blockIdx.x;
         const int per_group = args.group_m * args.tiles_n;
         const int gid = L / per_group;
@@ -232,11 +258,23 @@ gemm_dmma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     double* out = to_ws ? args.splitk_ws + (size_t)(blockIdx.z + blockIdx.y) * (size_t)args.M * (size_t)args.N
                         : args.C + (size_t)blockIdx.y * (size_t)args.c_batch_elems;
     const long long ldo = to_ws ? (long long)args.N : args.ldc;
+    // The sum of squares is that of alpha * acc (+ beta * C), before the row term is taken off.  A trapezoid tile below
+    // the diagonal also stands for its mirror (row and column indices swapped), whose row term is row_vec[n].
+    const bool mirror = (args.flags & GEMM_C_LOWER_TRAP) && tm != tn;
+    double shift_n[NJ][2];
+#pragma unroll
+    for (int j = 0; j < NJ; ++j)
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            const int n = n_base + ((B_MODE == 1) ? perm_kc(j, 2 * t + e) : perm_mc(j, 2 * t + e));
+            shift_n[j][e] = (mirror && args.row_vec && n < args.N) ? alpha * args.row_vec[n] : 0.0;
+        }
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
         const int m = m_base + ((A_MODE == 0) ? perm_kc(i, g) : perm_mc(i, g));
         if (m >= args.M) continue;
         double* row = out + (size_t)m * ldo;
+        const double rv = args.row_vec ? args.row_vec[m] : 0.0;
         // beta != 0: all of this row's old values are loaded before the first store (independent loads in flight;
         // interleaved with the stores they would serialise on possible aliasing -- the epilogue is exposed, one CTA per SM)
         double old[NJ][2];
@@ -258,9 +296,15 @@ gemm_dmma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
                 if (to_ws) {
                     row[n] = acc[i][j][e];
                 } else {
-                    double v = alpha * acc[i][j][e];
+                    double v = alpha * (acc[i][j][e] - rv);
                     if (beta != 0.0) v += beta * old[j][e];
-                    ssq += v * v;           // of the value stored: a contraction accumulated in chunks (beta = 1) sums the final D
+                    // of the value stored (plus the row term): a contraction accumulated in chunks (beta = 1) sums the final D
+                    const double d = v + alpha * rv;
+                    ssq += d * d;
+                    if (mirror) {
+                        const double dt = v + shift_n[j][e];
+                        ssq += dt * dt;
+                    }
                     row[n] = v;
                 }
             }

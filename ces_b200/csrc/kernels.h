@@ -13,6 +13,8 @@ enum GemmFlags : int {
     GEMM_C_LOWER_ONLY = 2,   // compute only tiles with tn <= tm (symmetric result)
     GEMM_B_UPPER_TRI = 4,    // B (KN) is upper triangular: columns of tile tn need kk < (tn+1)*BN only
     GEMM_SERPENTINE_K = 8,   // odd waves of CTAs traverse the contraction axis backwards (L2 reuse across waves)
+    GEMM_C_LOWER_TRAP = 32,  // M >= N: launch only the tiles with tn <= tm (lower trapezoid), one CTA each; the
+                             // sum-of-squares partials count every tile below the diagonal twice (itself and its mirror)
 };
 
 enum AMode : int { A_MK = 0, A_KM = 1 };
@@ -37,10 +39,16 @@ struct GemmCall {
     // walk of the contraction axis (ces_gemm_ex): CTAs per wave (0 = SM count), serpentine -1 = CES_GEMM_SERPENTINE / on,
     // 0 = off, 1 = on
     int wave_ctas = 0, serpentine = -1;
+    const double* row_vec = nullptr;  // [M], direct epilogue only: C = alpha (AB - row_vec 1^T) (+ beta C)
 };
 
 int gemm(cudaStream_t st, const GemmCall& c);
 int gemm_tiles(int M, int N);
+int64_t gemm_trap_tiles(int M, int N);   // tiles of the lower trapezoid (GEMM_C_LOWER_TRAP), M >= N
+int64_t gemm_trap_entries(int M, int N); // entries of C inside those tiles: the outputs a GEMM_C_LOWER_TRAP launch forms
+// C[r][c] = C[c][r] for r < c < n in different 128 x 128 tiles: completes the upper tiles of a symmetric n x n block
+// whose lower tiles a GEMM_C_LOWER_TRAP launch formed
+int mirror_lower_tiles(cudaStream_t st, double* C, int64_t ldc, int64_t n);
 int gemm_sm_count();   // SMs of the current device = CTAs of one wave of the GEMM (one CTA per SM)
 
 // Device scalar block of a handle (doubles).
@@ -71,6 +79,11 @@ int data_forms(cudaStream_t st, const double* E, const double* W, int64_t ld, in
 int finish_forms(cudaStream_t st, const double* qpart, int ny, int64_t ld, int64_t cols, bool square, double* part,
                  double* out);
 int sum_vector(cudaStream_t st, const double* v, int64_t n, double* out);
+// out[j] = sum_m X[m, j] v[m] for j < cols (X: rows x cols, ld); part holds form_row_blocks(rows, ld) * ld doubles
+int col_dot(cudaStream_t st, const double* X, int64_t ld, int64_t rows, int64_t cols, const double* v, double* part,
+            double* out);
+// out[r] = s * sum_j X[r, j] v[j] for r < rows
+int row_dot(cudaStream_t st, const double* X, int64_t ld, int64_t rows, int64_t cols, const double* v, double s, double* out);
 int row_sumsq(cudaStream_t st, const double* X, int64_t ld, int64_t rows, int64_t cols, double* out);
 int matvec(cudaStream_t st, const double* M, int64_t ld, int64_t n, const double* x, double* y);
 int scale_vector(cudaStream_t st, const double* d, const double* x, double* y, int64_t n);

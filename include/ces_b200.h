@@ -242,7 +242,11 @@ int ces_forward_map(ces_handle_t h, int map_kind, const double* A_dev, int64_t l
 
 /* Named device buffers of the handle, for the host-side collectives and for tests:
  * "sums" (k+p), "cuu" (p x ldp), "e_all" (nranks x k x ldJ), "ut_all" (nranks x p x ldJ), "scalars" (16),
- * "w" (k x ldJ), "v" (p x ldJ), "chol" (p x ldp), "cpp" (k x ldk, after ces_phase3b_cpp), "d_panel".  rows/cols/ld may be NULL. */
+ * "w" (k x ldJ), "v" (p x ldJ), "chol" (p x ldp), "cpp" (k x ldk, after ces_phase3b_cpp), "d_panel".  rows/cols/ld may be NULL.
+ * "d_panel" is the D workspace of the last column panel [a, b).  With nranks > 1 it holds that panel of D.  On a single
+ * GPU it holds S / J with J D = S + (E^T w0) 1^T (S = E^T Gamma^-1 E symmetric, w0 = Gamma^-1 (mean - y)): row r stands
+ * for particle a + r, rows 0 .. J - a - 1 are filled on and below the diagonal tiles and its top (b - a) x (b - a)
+ * block is complete. */
 int ces_buffer(ces_handle_t h, const char* name, double** ptr_dev, int64_t* rows, int64_t* cols, int64_t* ld);
 
 /* Number of kernels this handle has launched since creation (bench.py's gpu_launches). */
@@ -333,10 +337,13 @@ int ces_potri(void* stream, double* A_dev, int64_t ld, int64_t n, double* Ainv_d
  *   C[M,N] = alpha (* *alpha_dev) * sum_kk op(A)(m,kk) op(B)(kk,n) + beta * C  (+ diag_add on the diagonal)
  * flags: 1 = op(A) lower triangular (row tile tm reads kk < 128 (tm + 1) only, entries above the diagonal inside that
  * range must be zero), 2 = only tiles on or below the diagonal (square C; mirrored when a workspace is given),
- * 4 = op(B) upper triangular (column tile tn reads kk < 128 (tn + 1) only).  splits > 1 splits the contraction into
- * planes of splitk_ws (splits*M*N doubles) that a reduce kernel sums; with a workspace alpha / beta / diag_add are
- * applied there.  ssq_partials (no workspace, flag 2 excluded) receives one sum of squares of the stored values per
- * 128 x 128 tile and problem.  batch > 1: problem z shifts A's and B's stored rows by z*a_batch_rows / z*b_batch_rows
+ * 4 = op(B) upper triangular (column tile tn reads kk < 128 (tn + 1) only), 32 = lower trapezoid (M >= N, no
+ * workspace, batch 1, not with flag 2): only the tiles with tn <= tm are launched, one CTA each, in the order of the full
+ * grid with the others left out.  splits > 1 splits the contraction into planes of splitk_ws (splits*M*N doubles) that
+ * a reduce kernel sums; with a workspace alpha / beta / diag_add are applied there.  row_vec (M doubles, no workspace):
+ * C = alpha * (op(A) op(B) - row_vec 1^T) + beta * C.  ssq_partials (no workspace, flag 2 excluded) receives one
+ * partial per launched tile and problem: the sum of squares of the stored values plus alpha * row_vec[m]; with flag 32 a
+ * tile below the diagonal adds its mirror too, stored value plus alpha * row_vec[n] (rows and columns index one set).  batch > 1: problem z shifts A's and B's stored rows by z*a_batch_rows / z*b_batch_rows
  * (0 = shared) and writes C + z*c_batch_elems, or, with a workspace, all problems are summed into C.  group_m (0 = 16):
  * row tiles per rasterisation group.  wave_ctas (0 = SM count) and serpentine (-1 = environment default, 0 = off,
  * 1 = on): odd waves of wave_ctas CTAs walk the contraction backwards.  struct_size must be sizeof(ces_gemm_desc), the
@@ -360,6 +367,7 @@ typedef struct ces_gemm_desc {
     double* ssq_partials;
     int64_t ssq_partials_elems;
     int64_t batch, a_batch_rows, b_batch_rows, c_batch_elems;
+    const double* row_vec;
 } ces_gemm_desc;
 int ces_gemm_ex(void* stream, const ces_gemm_desc* desc);
 
