@@ -55,8 +55,10 @@ import numpy as np
 from .engine import Engine
 
 _METRIC_KEYS = ("self-bias", "self-bias-data", "bias-data", "bias", "t")
-_RULE_METHOD = {"eks": "eks_update", "aldi": "eks_update_aldi", "aldi_constant": "eks_update_aldi_constant",
-                "eki": "eki_update"}
+# ``update_rule`` the reference records for each rule (its names: not those of the methods)
+_UPDATE_RULE = {"eks": "eks_update", "aldi": "eks_update_linear", "aldi_constant": "eks_update_aldi", "eki": "eki_update"}
+# options of ``run`` / ``eks_update*`` that may also be set as attributes, with their defaults
+_OPTION_DEFAULTS = {"formulation": "interaction", "noise": "cholesky", "rng": "numpy", "seed": 0}
 
 
 _SMALL_BYTES = 1 << 20
@@ -438,6 +440,10 @@ class sampling(enka):
             self.radspec = []
             self.metrics = dict((key, []) for key in _METRIC_KEYS)
 
+    def _option(self, kwargs, name):
+        """An option of the call: the keyword argument, else the attribute of that name, else its default."""
+        return kwargs.get(name, getattr(self, name, _OPTION_DEFAULTS[name]))
+
     def _step_options(self, rule, kwargs):
         """(fixed_h, resolve) for Engine.step from the reference's ``time_step`` kwargs
         (ces/calibrate.py:247-260 for hk; :439-441 / :470-473 for the hk C^pp + Gamma re-solve of D)."""
@@ -463,12 +469,12 @@ class sampling(enka):
     def _noise_options(self, rule, kwargs, J, cols=None):
         """(ensemble?, explicit J x J xi or None) from the ``noise`` kwarg / attribute, checked before any device work.
         ``cols``: this rank's column count when the caller may pass only its own columns of xi (``local_shard``)."""
-        mode = kwargs.get('noise', getattr(self, 'noise', 'cholesky'))
+        mode = self._option(kwargs, 'noise')
         if mode not in ('cholesky', 'ensemble'):
             raise ValueError("noise must be 'cholesky' or 'ensemble', got %r" % (mode,))
         if mode == 'cholesky' or rule == 'eki':                  # eki has no noise term
             return False, None
-        if kwargs.get('formulation', getattr(self, 'formulation', 'interaction')) == 'factored':
+        if self._option(kwargs, 'formulation') == 'factored':
             raise ValueError("noise='ensemble' needs formulation='interaction': the factored formulation never gathers "
                              "U - ubar")
         xi = kwargs.get('xi', None)
@@ -482,6 +488,7 @@ class sampling(enka):
 
     # ------------------------------------------------------------------ single updates on numpy arrays
     def _update_host(self, rule, y_obs, U0, Geval, Gamma, kwargs):
+        self.update_rule = _UPDATE_RULE[rule]
         self._ensure_metrics()
         fixed, resolve = self._step_options(rule, kwargs)
         U0 = np.asarray(U0, dtype=np.float64)
@@ -506,7 +513,7 @@ class sampling(enka):
             # the J x J xi: this rank's columns of the caller's array, or the device's Philox stream keyed by the step
             if xi_ens is not None and xi_ens.shape[1] == eng.J and eng.cols != eng.J:
                 xi_ens = xi_ens[:, eng.col_lo:eng.col_hi]
-            noise = ('ensemble', int(kwargs.get('seed', getattr(self, 'seed', 0))), len(self.metrics['t']), xi_ens)
+            noise = ('ensemble', int(self._option(kwargs, 'seed')), len(self.metrics['t']), xi_ens)
         elif rule != 'eki':
             # the full (p, J) draw on every rank -- the same global stream as the reference -- unless the caller
             # passes its own (possibly sharded) noise
@@ -521,7 +528,7 @@ class sampling(enka):
         elif local and xi is not None and xi.shape[1] == eng.J and eng.J != eng.cols:
             xi = xi[:, eng.col_lo:eng.col_hi]
         opts = dict(fixed_h=fixed, switch=kwargs.get('switch', 1.), resolve=resolve,
-                    formulation=kwargs.get('formulation', getattr(self, 'formulation', 'interaction')), noise=noise)
+                    formulation=self._option(kwargs, 'formulation'), noise=noise)
         Uk, hk, met = eng.step_host(rule, U0, Gk, xi, **opts)
         if stale is not None and stale():
             # a large problem array was edited in place since the previous call: the device copy has just been
@@ -553,23 +560,19 @@ class sampling(enka):
         ``local_shard=True``), or by default the device's Philox stream keyed by ``seed`` and the step count
         ``len(self.metrics['t'])``.  The update then draws nothing from numpy's global generator (``rng`` does not apply);
         a forward model's own draws, such as ``banana``'s, are unaffected."""
-        self.update_rule = 'eks_update'
         return self._update_host('eks', y_obs, U0, Geval, Gamma, kwargs)
 
     def eks_update_aldi(self, y_obs, U0, Geval, Gamma, iter, **kwargs):
         """ALDI step, the default (ces/calibrate.py:451-490)."""
-        self.update_rule = 'eks_update_linear'
         return self._update_host('aldi', y_obs, U0, Geval, Gamma, kwargs)
 
     def eks_update_aldi_constant(self, y_obs, U0, Geval, Gamma, iter, **kwargs):
         """ALDI step with h = 0.1 / max|drift| (ces/calibrate.py:492-529)."""
-        self.update_rule = 'eks_update_aldi'
         return self._update_host('aldi_constant', y_obs, U0, Geval, Gamma, kwargs)
 
     def eki_update(self, y_obs, U0, Geval, Gamma, iter, **kwargs):
         """Deterministic ensemble Kalman inversion step U - h (U - ubar) D: the part every EKS rule shares
         (first two terms of ces/calibrate.py:444 / :484).  The reference ships no EKI class (SURVEY.md F3)."""
-        self.update_rule = 'eki_update'
         return self._update_host('eki', y_obs, U0, Geval, Gamma, kwargs)
 
     # ------------------------------------------------------------------ the run loop
@@ -588,7 +591,7 @@ class sampling(enka):
         kind = getattr(model, 'device_kind', None)
         if not (device_map and eng.nranks == 1 and kind in _lib.MAPS and self.p <= 8 and self.n_obs <= 16
                 and 2 <= eng.J <= 512 and self.T >= 1 and self._step_options(rule, kwargs) == (None, None)
-                and kwargs.get('formulation', getattr(self, 'formulation', 'interaction')) == 'interaction'
+                and self._option(kwargs, 'formulation') == 'interaction'
                 and getattr(self, 'fused_run', True) and kwargs.get('xi', None) is None
                 and not self._noise_options(rule, kwargs, eng.J)[0]):
             return False
@@ -598,7 +601,7 @@ class sampling(enka):
         torch = eng.torch
         A_dev, lda, b_dev, params = model._device_args(torch)
         par = np.ascontiguousarray(params, dtype=np.float64) if params is not None else None
-        device_rng = kwargs.get('rng', getattr(self, 'rng', 'numpy')) == 'device'
+        device_rng = self._option(kwargs, 'rng') == 'device'
         xi_all, state = None, None
         fdraws = int(getattr(model, 'rng_draws_per_call', 0)) * J    # normals the reference's forward loop draws per pass
         host_noise = rule != 'eki' and not device_rng
@@ -622,7 +625,7 @@ class sampling(enka):
                 ctypes.c_void_p(A_dev.data_ptr()) if A_dev is not None else None, int(lda),
                 ctypes.c_void_p(b_dev.data_ptr()) if b_dev is not None else None,
                 _lib.host_ptr(par) if par is not None else None, _lib.host_ptr(U0),
-                _lib.host_ptr(xi_all) if xi_all is not None else None, int(kwargs.get('seed', getattr(self, 'seed', 0))),
+                _lib.host_ptr(xi_all) if xi_all is not None else None, int(self._option(kwargs, 'seed')),
                 len(t_hist), T, float(t_hist[-1]) if len(t_hist) else 0.0, 1 if len(t_hist) else 0,
                 float(kwargs.get('t_tol', 2.)), _lib.host_ptr(Ut), _lib.host_ptr(Gt), _lib.host_ptr(S), _lib.host_ptr(tv),
                 ctypes.byref(n)))
@@ -633,8 +636,7 @@ class sampling(enka):
                 np.random.normal(0, 1, [n, fdraws + (p * J if host_noise else 0)])
             if fdraws:
                 np.random.normal(0, 1, fdraws)                   # the final forward pass
-        self.update_rule = {'eks': 'eks_update', 'aldi': 'eks_update_linear', 'aldi_constant': 'eks_update_aldi',
-                            'eki': 'eki_update'}[rule]
+        self.update_rule = _UPDATE_RULE[rule]
         # step scalars -> metrics (sums over particles / J), cumulative times
         for name, col in (('self-bias', 1), ('bias', 2), ('self-bias-data', 3), ('bias-data', 4)):
             self.metrics[name].extend((S[:n, col] / J).tolist())
@@ -695,7 +697,7 @@ class sampling(enka):
             self.Uall = list(getattr(self, 'Uall', []))
             self.Gall = list(getattr(self, 'Gall', []))
         self._ensure_metrics()
-        known = rule in _RULE_METHOD
+        known = rule in _UPDATE_RULE
 
         device_model = (not is_pde) and self._is_device_model(model)
         if self._fused_small_run(eng, y_obs, U0, model, rule, kwargs, save_online, trace, known and device_model):
@@ -823,23 +825,20 @@ class sampling(enka):
                       else host_trace.push(gather_dev(G_cur, self.n_obs)))
                 tickets.append((tu, tg))
             if known:
-                setattr(self, 'update_rule', {'eks': 'eks_update', 'aldi': 'eks_update_linear',
-                                              'aldi_constant': 'eks_update_aldi', 'eki': 'eki_update'}[rule])
+                self.update_rule = _UPDATE_RULE[rule]
                 xi_dev, noise = None, None
                 if ensemble:
-                    noise = ('ensemble', int(kwargs.get('seed', getattr(self, 'seed', 0))), len(self.metrics['t']), xi_ens)
+                    noise = ('ensemble', int(self._option(kwargs, 'seed')), len(self.metrics['t']), xi_ens)
                 elif rule != 'eki':
-                    if kwargs.get('rng', getattr(self, 'rng', 'numpy')) == 'device':
+                    if self._option(kwargs, 'rng') == 'device':
                         # production mode: Philox noise generated on the device, nothing crosses PCIe
-                        xi_dev = eng.normal_noise(self.p, kwargs.get('seed', getattr(self, 'seed', 0)),
-                                                  len(self.metrics['t']))
+                        xi_dev = eng.normal_noise(self.p, self._option(kwargs, 'seed'), len(self.metrics['t']))
                     else:
                         xi = self._draw_noise((self.p, J), kwargs)      # same stream on every rank
                         xi_dev = torch.from_numpy(np.ascontiguousarray(xi[:, lo:hi])).to(dev)
                 fixed, resolve = self._step_options(rule, kwargs)     # 'mix' depends on the time reached so far
                 U_dev, hk, met = eng.step(rule, U_dev, G_cur, xi_dev, fixed_h=fixed, switch=kwargs.get('switch', 1.),
-                                          resolve=resolve, noise=noise,
-                                          formulation=kwargs.get('formulation', getattr(self, 'formulation', 'interaction')))
+                                          resolve=resolve, noise=noise, formulation=self._option(kwargs, 'formulation'))
                 self._record(met, hk)
                 if resolve == 'spectral':
                     self.radspec.append(1. / hk)

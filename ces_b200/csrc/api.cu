@@ -2,6 +2,7 @@
 #include <cmath>
 #include <cstring>
 #include <cstdlib>
+#include <optional>
 #include <string>
 #include <vector>
 #include "../../include/ces_b200.h"
@@ -177,6 +178,80 @@ int valid(ces_handle_t h, bool need_problem) {
     return CES_OK;
 }
 
+// The noise operand xi a step needs: the Cholesky noise of the noisy rules (EKI has no noise term, ensemble noise its own).
+bool needs_xi(ces_handle_t h, int rule) { return rule != CES_RULE_EKI && !ensemble_noise(h); }
+
+// The arguments of a step, checked by every entry point before any device work.  std::nullopt: the entry point takes no
+// such argument (its rule is phase 2's).  CES_TS_KEEP (`keep_ok`) is for phase 4 only: it keeps ces_peek_step_size's h.
+int check_step(ces_handle_t h, const char* who, std::optional<int> rule, std::optional<int> ts_kind, bool keep_ok,
+               std::optional<int> formulation, bool have_ptrs) {
+    if (rule && (*rule < CES_RULE_EKS || *rule > CES_RULE_EKI)) return fail(CES_ERR_INVALID, "unknown update rule %s%lld", "", *rule);
+    if (ts_kind && *ts_kind != CES_TS_FROBENIUS && *ts_kind != CES_TS_FIXED && !(keep_ok && *ts_kind == CES_TS_KEEP))
+        return fail(CES_ERR_INVALID, "unknown step-size rule%s", "");
+    if (formulation && *formulation != CES_FORM_INTERACTION && *formulation != CES_FORM_FACTORED)
+        return fail(CES_ERR_INVALID, "unknown formulation%s", "");
+    if (formulation == CES_FORM_FACTORED && ensemble_noise(h) && rule.value_or(h->last_rule) != CES_RULE_EKI)
+        return fail(CES_ERR_INVALID, "ensemble noise needs the interaction formulation (the factored one never gathers U~)%s", "");
+    if (!have_ptrs) return fail(CES_ERR_INVALID, "%s: null pointer", who);
+    return CES_OK;
+}
+
+// Split-K count of a GEMM with `tiles` output tiles contracting over `contraction`: fill two waves of 148 SMs, with at
+// most one split per k-block and at most 64.
+int splitk_count(int64_t tiles, int64_t contraction) {
+    int64_t sp = ceil_div(296, tiles);
+    const int64_t kb = ceil_div(contraction, GEMM_BK);
+    if (sp > kb) sp = kb;
+    if (sp > 64) sp = 64;
+    return sp < 1 ? 1 : (int)sp;
+}
+
+// The whole step in one single-CTA kernel (small problems, where launch latency dominates otherwise).  The kernel draws
+// the reference's Cholesky noise only.
+bool small_path(ces_handle_t h, int formulation) {
+    return h->use_small && !ensemble_noise(h) && formulation == CES_FORM_INTERACTION && small_step_eligible(h->p, h->k, h->Jl);
+}
+
+// The fields of a single-CTA call that come from the handle and the step's settings; operands are the caller's.
+SmallStepCall small_call(ces_handle_t h, int rule, int ts_kind, double fixed_h, double switch_) {
+    SmallStepCall c{};
+    c.p = h->p; c.k = h->k; c.J = h->Jl; c.rule = rule; c.ts_kind = ts_kind; c.fixed_h = fixed_h; c.switch_ = switch_;
+    c.y = h->y; c.mu = h->mu; c.ustar = h->ustar; c.bprior = h->bprior;
+    c.ginv_diag = h->gamma_diag ? h->ginv_diag : nullptr; c.Ginv = h->gamma_diag ? nullptr : h->Ginv;
+    c.sinv_diag = h->sinv_diag; c.sig_diag = h->sig_diag;
+    c.Sinv = h->sigma_diag ? nullptr : h->Sinv; c.Sigma0 = h->sigma_diag ? nullptr : h->Sigma0;
+    c.ldk = h->ldk; c.ldp = h->ldp;
+    return c;
+}
+
+// The end of a step: download the step scalars and, when a host destination is pending (one-shot), U_next on the same
+// synchronisation; refuse a factorisation of C^uu that failed; hand out hk and the metrics (sums over particles / J).
+// The pivot is the device int of potrf (`pivot_on_device`) or S[S_INFO] (the single-CTA kernel).
+int finish_step(ces_handle_t h, const double* Uout, int64_t ldo, bool pivot_on_device, double* hk_host, double* metrics_host) {
+    cudaStream_t st = h->st;
+    CES_CUDA(cudaMemcpyAsync(h->hS, h->S, S_COUNT * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (h->pending_out && h->cols > 0) {
+        const size_t wbytes = h->cols * sizeof(double);
+        if (ldo == h->cols) CES_CUDA(cudaMemcpyAsync(h->pending_out, Uout, (size_t)h->pending_rows * wbytes, cudaMemcpyDeviceToHost, st));
+        else CES_CUDA(cudaMemcpy2DAsync(h->pending_out, wbytes, Uout, ldo * sizeof(double), wbytes, h->pending_rows, cudaMemcpyDeviceToHost, st));
+    }
+    h->pending_out = nullptr;
+    if (pivot_on_device) {
+        CES_TRY(check_info(h, "cov(U)"));   // synchronises the stream
+    } else {
+        CES_CUDA(cudaStreamSynchronize(st));
+        if (h->hS[S_INFO] != 0.0)
+            return fail(CES_ERR_NOT_SPD, "%s: matrix is not positive definite (pivot %lld)", "cov(U)", (long long)h->hS[S_INFO]);
+    }
+    if (hk_host) *hk_host = h->hS[S_H];
+    if (metrics_host) {
+        const double J = (double)h->Jg;
+        metrics_host[0] = h->hS[S_SELF_BIAS] / J; metrics_host[1] = h->hS[S_BIAS] / J;
+        metrics_host[2] = h->hS[S_SELF_DATA] / J; metrics_host[3] = h->hS[S_BIAS_DATA] / J;
+    }
+    return CES_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -219,18 +294,8 @@ int ces_create(int64_t p, int64_t k, int64_t J_local, int64_t J_global, int rank
     const int ny = nyk0 > nyp0 ? nyk0 : nyp0;
     const int64_t tiles_per_rank = ceil_div(J_local, GEMM_BM) * ceil_div(J_local, GEMM_BN) + ceil_div(J_local, GEMM_BM) * ceil_div(J_local, panel);
     h->ssq_cap = tiles_per_rank * nranks + 16;
-    // SYRK split-K: fill ~2 waves of 148 SMs with (lower tiles) x splits CTAs.
-    {
-        const int64_t tm = ceil_div(p, GEMM_BM);
-        const int64_t lower = tm * (tm + 1) / 2;
-        int64_t sp = ceil_div(296, lower);
-        const int64_t kb = ceil_div(h->ldJ, GEMM_BK);
-        if (sp > kb) sp = kb;
-        if (sp > 64) sp = 64;
-        if (sp < 1) sp = 1;
-        h->syrk_splits = (int)sp;
-        h->splitk_cap = sp * p * p;
-    }
+    h->syrk_splits = splitk_count(gemm_trap_tiles((int)p, (int)p), h->ldJ);   // C^uu: lower tiles only
+    h->splitk_cap = h->syrk_splits * p * p;
 #define A_(ptr, n) if (s == CES_OK && !h->forward_only) s = dalloc(h, &h->ptr, (n))
     A_(y, k); A_(ginv_diag, k); A_(mu, p); A_(ustar, p); A_(sinv_diag, p); A_(sig_diag, p); A_(bprior, p);
     A_(sums, k + p); A_(cvec, k); A_(zvec, k); A_(S, S_COUNT); A_(cb, p);
@@ -685,7 +750,7 @@ static int start_cholesky(ces_handle_t h, int rule) {
 
 int ces_peek_step_size(ces_handle_t h, int ts_kind, double fixed_h, double* hk_host) {
     CES_TRY(valid(h, true));
-    if (ts_kind != CES_TS_FROBENIUS && ts_kind != CES_TS_FIXED) return fail(CES_ERR_INVALID, "unknown step-size rule%s", "");
+    CES_TRY(check_step(h, "peek", std::nullopt, ts_kind, false, std::nullopt, true));
     const double alphaJ = (double)(h->p + 1) / (double)h->Jg;
     CES_TRY(step_scalars(h->st, h->S, ts_kind == CES_TS_FIXED ? 1 : 0, fixed_h, alphaJ, ens_inv_nc(h, h->last_rule)));
     CES_CUDA(cudaMemcpyAsync(h->hS, h->S, S_COUNT * sizeof(double), cudaMemcpyDeviceToHost, h->st));
@@ -699,15 +764,9 @@ int ces_phase3b_cpp(ces_handle_t h) {
     const int64_t k = h->k, ld = h->ldJ;
     cudaStream_t st = h->st;
     if (!h->Cpp) {
-        const int64_t tm = ceil_div(k, GEMM_BM), lower = tm * (tm + 1) / 2;
-        int64_t sp = ceil_div(296, lower);
-        const int64_t kb = ceil_div(ld, GEMM_BK);
-        if (sp > kb) sp = kb;
-        if (sp > 64) sp = 64;
-        if (sp < 1) sp = 1;
-        h->cpp_splits = (int)sp;
+        h->cpp_splits = splitk_count(gemm_trap_tiles((int)k, (int)k), ld);
         CES_TRY(dalloc(h, &h->Cpp, k * h->ldk));
-        CES_TRY(dalloc(h, &h->cpp_ws, sp * k * k));
+        CES_TRY(dalloc(h, &h->cpp_ws, h->cpp_splits * k * k));
         CES_TRY(dalloc(h, &h->Mk, k * h->ldk));
         CES_TRY(dalloc(h, &h->MkInv, k * h->ldk));
         CES_TRY(dalloc(h, &h->MkLinv, round_up(k, CHOL_NB) * kLinvLd));
@@ -783,25 +842,14 @@ __global__ void __launch_bounds__(256) gram_dot_kernel(const double* __restrict_
 int ces_phase3f_products(ces_handle_t h, int rule) {
     CES_TRY(valid(h, true));
     if (rule != h->last_rule) return fail(CES_ERR_STATE, "phase3f: rule differs from phase2%s", "");
-    if (ensemble_noise(h) && rule != CES_RULE_EKI)
-        return fail(CES_ERR_INVALID, "ensemble noise needs the interaction formulation (the factored one never gathers U~)%s", "");
+    CES_TRY(check_step(h, "phase3f", std::nullopt, std::nullopt, false, CES_FORM_FACTORED, true));
     const int64_t p = h->p, k = h->k, ld = h->ldJ;
     cudaStream_t st = h->st;
     if (!h->P1) {
-        const int64_t tm = ceil_div(k, GEMM_BM), lower = tm * (tm + 1) / 2;
-        int64_t sp = ceil_div(296, lower);
-        const int64_t kb = ceil_div(ld, GEMM_BK);
-        if (sp > kb) sp = kb;
-        if (sp > 64) sp = 64;
-        if (sp < 1) sp = 1;
-        h->gram_splits = (int)sp;
+        h->gram_splits = splitk_count(gemm_trap_tiles((int)k, (int)k), ld);
         // P1 has few (d/128 x k/128) tiles and a long contraction: split it so the tiles fill the machine
-        int64_t sp1 = ceil_div(296, ceil_div(p, GEMM_BM) * ceil_div(k, GEMM_BN));
-        if (sp1 > kb) sp1 = kb;
-        if (sp1 > 64) sp1 = 64;
-        if (sp1 < 1) sp1 = 1;
-        h->p1_splits = (int)sp1;
-        const int64_t ws = sp * k * k > sp1 * p * k ? sp * k * k : sp1 * p * k;
+        h->p1_splits = splitk_count(gemm_tiles((int)p, (int)k), ld);
+        const int64_t ws = h->gram_splits * k * k > h->p1_splits * p * k ? h->gram_splits * k * k : h->p1_splits * p * k;
         CES_TRY(dalloc(h, &h->P1, p * h->ldk));
         CES_TRY(dalloc(h, &h->GE, k * h->ldk));
         CES_TRY(dalloc(h, &h->GW, k * h->ldk));
@@ -909,10 +957,8 @@ int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, con
                       const double* xi, int64_t ldxi, double* Uout, int64_t ldo, double* hk_host, double* metrics_host) {
     CES_TRY(valid(h, true));
     if (rule != h->last_rule) return fail(CES_ERR_STATE, "phase4: rule differs from phase2%s", "");
+    CES_TRY(check_step(h, "phase4", std::nullopt, ts_kind, true, std::nullopt, U && Uout && (xi || !needs_xi(h, rule))));
     const bool ens = ensemble_noise(h);
-    if (!U || !Uout || (rule != CES_RULE_EKI && !ens && !xi)) return fail(CES_ERR_INVALID, "phase4: null pointer%s", "");
-    if (ts_kind != CES_TS_FROBENIUS && ts_kind != CES_TS_FIXED && ts_kind != CES_TS_KEEP)
-        return fail(CES_ERR_INVALID, "unknown step-size rule%s", "");
     const int64_t p = h->p, ld = h->ldJ;
     cudaStream_t st = h->st;
     const double alphaJ = (double)(p + 1) / (double)h->Jg;
@@ -1031,25 +1077,13 @@ int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, con
             CES_TRY(ens ? add_ensemble_noise(h, 0, h->cols, Uout, ldo) : gemm(st, noise));
         }
     }
-    CES_CUDA(cudaMemcpyAsync(h->hS, S, S_COUNT * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (h->pending_out && !downloaded && h->cols > 0) {   // result copy rides on the same final synchronisation
-        const size_t wbytes = h->cols * sizeof(double);
-        if (ldo == h->cols) CES_CUDA(cudaMemcpyAsync(h->pending_out, Uout, (size_t)h->pending_rows * wbytes, cudaMemcpyDeviceToHost, st));
-        else CES_CUDA(cudaMemcpy2DAsync(h->pending_out, wbytes, Uout, ldo * sizeof(double), wbytes, h->pending_rows, cudaMemcpyDeviceToHost, st));
-    }
-    h->pending_out = nullptr;           // one-shot
     mark(h, "phase4:computed");
-    if (downloaded) { mark(h, "phase4:downloaded", h->out_st); CES_CUDA(cudaStreamSynchronize(h->out_st)); }
-    CES_TRY(check_info(h, "cov(U)"));   // synchronises the stream
-    if (hk_host) *hk_host = h->hS[S_H];
-    if (metrics_host) {
-        const double J = (double)h->Jg;
-        metrics_host[0] = h->hS[S_SELF_BIAS] / J;
-        metrics_host[1] = h->hS[S_BIAS] / J;
-        metrics_host[2] = h->hS[S_SELF_DATA] / J;
-        metrics_host[3] = h->hS[S_BIAS_DATA] / J;
-    }
-    return CES_OK;
+    if (!downloaded) return finish_step(h, Uout, ldo, true, hk_host, metrics_host);
+    mark(h, "phase4:downloaded", h->out_st);
+    h->pending_out = nullptr;           // already on its way, chunk by chunk
+    const int s = finish_step(h, Uout, ldo, true, hk_host, metrics_host);
+    CES_CUDA(cudaStreamSynchronize(h->out_st));   // the host copy is complete whatever the status
+    return s;
 }
 
 static int interaction_phase(ces_handle_t h, int rule, int formulation) {
@@ -1057,7 +1091,6 @@ static int interaction_phase(ces_handle_t h, int rule, int formulation) {
         CES_TRY(ces_phase3f_products(h, rule));
         return ces_phase3f_finish(h, rule);
     }
-    if (formulation != CES_FORM_INTERACTION) return fail(CES_ERR_INVALID, "unknown formulation%s", "");
     return ces_phase3_interact(h, rule, 0);
 }
 
@@ -1066,40 +1099,13 @@ int ces_step(ces_handle_t h, int rule, int ts_kind, double fixed_h, double switc
              double* hk_host, double* metrics_host) {
     CES_TRY(valid(h, true));
     if (h->nranks != 1) return fail(CES_ERR_STATE, "ces_step is single-GPU; use the phases with nranks > 1%s", "");
-    if (formulation == CES_FORM_FACTORED && ensemble_noise(h) && rule != CES_RULE_EKI)
-        return fail(CES_ERR_INVALID, "ensemble noise needs the interaction formulation (the factored one never gathers U~)%s", "");
-    // the single-kernel path draws the reference's Cholesky noise only
-    if (h->use_small && !ensemble_noise(h) && formulation == CES_FORM_INTERACTION && small_step_eligible(h->p, h->k, h->Jl)) {
-        // small problems: the whole update in one single-CTA kernel (launch latency dominates otherwise)
-        if (rule < CES_RULE_EKS || rule > CES_RULE_EKI) return fail(CES_ERR_INVALID, "unknown update rule %s%lld", "", rule);
-        if (ts_kind != CES_TS_FROBENIUS && ts_kind != CES_TS_FIXED) return fail(CES_ERR_INVALID, "unknown step-size rule%s", "");
-        if (!U || !G || !Uout || (rule != CES_RULE_EKI && !xi)) return fail(CES_ERR_INVALID, "ces_step: null pointer%s", "");
-        SmallStepCall c;
-        c.p = h->p; c.k = h->k; c.J = h->Jl; c.rule = rule; c.ts_kind = ts_kind; c.fixed_h = fixed_h; c.switch_ = switch_;
-        c.U = U; c.G = G; c.xi = xi; c.ldu = ldu; c.ldg = ldg; c.ldxi = ldxi; c.out = Uout; c.ldo = ldo;
-        c.y = h->y; c.mu = h->mu; c.ustar = h->ustar; c.bprior = h->bprior;
-        c.ginv_diag = h->gamma_diag ? h->ginv_diag : nullptr; c.Ginv = h->gamma_diag ? nullptr : h->Ginv;
-        c.sinv_diag = h->sinv_diag; c.sig_diag = h->sig_diag;
-        c.Sinv = h->sigma_diag ? nullptr : h->Sinv; c.Sigma0 = h->sigma_diag ? nullptr : h->Sigma0;
-        c.ldk = h->ldk; c.ldp = h->ldp; c.S = h->S;
+    CES_TRY(check_step(h, "ces_step", rule, ts_kind, false, formulation, U && G && Uout && (xi || !needs_xi(h, rule))));
+    if (small_path(h, formulation)) {
+        SmallStepCall c = small_call(h, rule, ts_kind, fixed_h, switch_);
+        c.U = U; c.G = G; c.xi = xi; c.ldu = ldu; c.ldg = ldg; c.ldxi = ldxi; c.out = Uout; c.ldo = ldo; c.S = h->S;
         h->last_rule = rule;
         CES_TRY(small_step(h->st, c));
-        CES_CUDA(cudaMemcpyAsync(h->hS, h->S, S_COUNT * sizeof(double), cudaMemcpyDeviceToHost, h->st));
-        if (h->pending_out) {
-            const size_t wbytes = h->Jl * sizeof(double);
-            if (ldo == h->Jl) CES_CUDA(cudaMemcpyAsync(h->pending_out, Uout, (size_t)h->pending_rows * wbytes, cudaMemcpyDeviceToHost, h->st));
-            else CES_CUDA(cudaMemcpy2DAsync(h->pending_out, wbytes, Uout, ldo * sizeof(double), wbytes, h->pending_rows, cudaMemcpyDeviceToHost, h->st));
-        }
-        CES_CUDA(cudaStreamSynchronize(h->st));
-        if (h->hS[S_INFO] != 0.0)
-            return fail(CES_ERR_NOT_SPD, "%s: matrix is not positive definite (pivot %lld)", "cov(U)", (long long)h->hS[S_INFO]);
-        if (hk_host) *hk_host = h->hS[S_H];
-        if (metrics_host) {
-            const double J = (double)h->Jg;
-            metrics_host[0] = h->hS[S_SELF_BIAS] / J; metrics_host[1] = h->hS[S_BIAS] / J;
-            metrics_host[2] = h->hS[S_SELF_DATA] / J; metrics_host[3] = h->hS[S_BIAS_DATA] / J;
-        }
-        return CES_OK;
+        return finish_step(h, Uout, ldo, false, hk_host, metrics_host);
     }
     CES_TRY(ces_phase1_sums(h, U, ldu, G, ldg));
     CES_TRY(ces_phase2_centre(h, rule, U, ldu, G, ldg));
@@ -1191,11 +1197,7 @@ int ces_host_chunk_schedule(int64_t k, int64_t J_local, int64_t panel, int nrank
 int ces_host_begin(ces_handle_t h, int rule, int formulation, const double* U, const double* G, const double* xi,
                    int* nchunks_out, int64_t* bounds_out /* [9] */) {
     CES_TRY(valid(h, true));
-    if (rule < CES_RULE_EKS || rule > CES_RULE_EKI) return fail(CES_ERR_INVALID, "unknown update rule %s%lld", "", rule);
-    if (formulation != CES_FORM_INTERACTION && formulation != CES_FORM_FACTORED) return fail(CES_ERR_INVALID, "unknown formulation%s", "");
-    if (formulation == CES_FORM_FACTORED && ensemble_noise(h) && rule != CES_RULE_EKI)
-        return fail(CES_ERR_INVALID, "ensemble noise needs the interaction formulation (the factored one never gathers U~)%s", "");
-    if ((!U || !G) && h->cols > 0) return fail(CES_ERR_INVALID, "ces_host_begin: null pointer%s", "");
+    CES_TRY(check_step(h, "ces_host_begin", rule, std::nullopt, false, formulation, (U && G) || h->cols == 0));
     CES_TRY(host_staging(h));
     const int64_t p = h->p, k = h->k, ld = h->ldJ, w = h->cols;
     // ---- uploads, all on the copy stream, in the order the main stream needs them: G in row chunks (ces_host_chunk_schedule),
@@ -1350,11 +1352,9 @@ int ces_step_host(ces_handle_t h, int rule, int ts_kind, double fixed_h, double 
                   const double* G, const double* xi, double* Uout, double* hk_host, double* metrics_host) {
     CES_TRY(valid(h, true));
     if (h->nranks != 1) return fail(CES_ERR_STATE, "ces_step_host is single-GPU; use the ces_host_* pieces with nranks > 1%s", "");
-    if (!U || !G || !Uout) return fail(CES_ERR_INVALID, "ces_step_host: null pointer%s", "");
+    CES_TRY(check_step(h, "ces_step_host", rule, ts_kind, false, formulation, U && G && Uout && (xi || !needs_xi(h, rule))));
     const int64_t p = h->p, k = h->k, ld = h->ldJ;
-    const bool small = h->use_small && !ensemble_noise(h) && formulation == CES_FORM_INTERACTION &&
-                       small_step_eligible(h->p, h->k, h->Jl);
-    if (small) {
+    if (small_path(h, formulation)) {
         // tiny problems keep everything on one stream -- extra streams and events would cost more than the copies
         CES_TRY(host_staging(h));
         if (xi) CES_CUDA(host_h2d(h, h->stage_xi, xi, p, h->st));
@@ -1396,8 +1396,7 @@ int ces_small_run(ces_handle_t h, int rule, int ts_kind, double fixed_h, double 
     if (h->nranks != 1) return fail(CES_ERR_STATE, "ces_small_run is single-GPU%s", "");
     const int64_t p = h->p, k = h->k, J = h->Jl;
     if (!small_step_eligible(p, k, J)) return fail(CES_ERR_INVALID, "ces_small_run: the problem is too large for the single-CTA path%s", "");
-    if (rule < CES_RULE_EKS || rule > CES_RULE_EKI) return fail(CES_ERR_INVALID, "unknown update rule %s%lld", "", rule);
-    if (ts_kind != CES_TS_FROBENIUS && ts_kind != CES_TS_FIXED) return fail(CES_ERR_INVALID, "unknown step-size rule%s", "");
+    CES_TRY(check_step(h, "ces_small_run", rule, ts_kind, false, std::nullopt, true));
     if (T < 1 || !U0_host || !Utrace_host || !Gtrace_host || !S_host || !t_host || !nsteps_host)
         return fail(CES_ERR_INVALID, "ces_small_run: bad argument%s", "");
     if (map_kind < CES_MAP_LINEAL || map_kind > CES_MAP_BANANA) return fail(CES_ERR_INVALID, "ces_small_run: unknown map kind%s", "");
@@ -1423,14 +1422,8 @@ int ces_small_run(ces_handle_t h, int rule, int ts_kind, double fixed_h, double 
         if (xi_host) CES_CUDA(cudaMemcpyAsync(Xi, xi_host, (size_t)nx * sizeof(double), cudaMemcpyHostToDevice, st));
         else for (int64_t it = 0; it < T; ++it) CES_TRY(fill_normal(st, Xi + it * p * J, J, p, J, 0, seed, step0 + (uint64_t)it));
     }
-    SmallStepCall c;
-    c.p = p; c.k = k; c.J = J; c.rule = rule; c.ts_kind = ts_kind; c.fixed_h = fixed_h; c.switch_ = switch_;
-    c.U = nullptr; c.G = nullptr; c.xi = nullptr; c.ldu = c.ldg = c.ldxi = c.ldo = J; c.out = nullptr;
-    c.y = h->y; c.mu = h->mu; c.ustar = h->ustar; c.bprior = h->bprior;
-    c.ginv_diag = h->gamma_diag ? h->ginv_diag : nullptr; c.Ginv = h->gamma_diag ? nullptr : h->Ginv;
-    c.sinv_diag = h->sinv_diag; c.sig_diag = h->sig_diag;
-    c.Sinv = h->sigma_diag ? nullptr : h->Sinv; c.Sigma0 = h->sigma_diag ? nullptr : h->Sigma0;
-    c.ldk = h->ldk; c.ldp = h->ldp; c.S = nullptr;
+    SmallStepCall c = small_call(h, rule, ts_kind, fixed_h, switch_);   // operands: the run's own buffers
+    c.ldu = c.ldg = c.ldxi = c.ldo = J;
     SmallRunCall rc;
     rc.T = T; rc.map_kind = map_kind; rc.have_t0 = have_t0; rc.t0 = t0; rc.t_tol = t_tol;
     rc.A = A_dev; rc.lda = lda; rc.b = b_dev;

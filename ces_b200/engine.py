@@ -417,6 +417,19 @@ class Engine(object):
             "device ensembles must be float64 CUDA tensors with the particle axis contiguous"
         return ctypes.c_void_p(t.data_ptr()), int(t.stride(0))
 
+    @staticmethod
+    def _step_args(rule, fixed_h, formulation):
+        """The library's codes for a step's options: (rule, step-size rule, h, formulation).  ``fixed_h`` None: the
+        step size 1 / (||D||_F + 1e-8)."""
+        if formulation not in _lib.FORMULATIONS:
+            raise ValueError("formulation must be 'interaction' or 'factored'")
+        ts, fh = (_lib.TS_FROBENIUS, 0.0) if fixed_h is None else (_lib.TS_FIXED, float(fixed_h))
+        return _lib.RULES[rule], ts, fh, _lib.FORMULATIONS[formulation]
+
+    def _results(self):
+        """(hk, metrics dict) of the step that has just ended."""
+        return float(self._hk.value), {key: float(self._met[i]) for i, key in enumerate(_METRIC_KEYS)}
+
     # ------------------------------------------------------------------ one update
     def step(self, rule, U, G, xi, out=None, fixed_h=None, switch=1.0, resolve=None, formulation="interaction", noise=None):
         with self.on_stream():
@@ -429,10 +442,8 @@ class Engine(object):
         the reference's Cholesky noise, or ("ensemble", seed, step, xi_ens or None) (``set_noise``; xi is then
         ignored and may be None)."""
         torch = self.torch
+        r, ts, fh, form = self._step_args(rule, fixed_h, formulation)
         self._apply_noise(noise)
-        r = _lib.RULES[rule]
-        ts = _lib.TS_FIXED if fixed_h is not None else _lib.TS_FROBENIUS
-        fh = float(fixed_h) if fixed_h is not None else 0.0
         if out is None:
             out = torch.empty_like(U)
         Up, ldu = self._dev(U)
@@ -443,11 +454,9 @@ class Engine(object):
         else:
             Xp, ldx = ctypes.c_void_p(0), 0
         lib, h = self.lib, self.h
-        if formulation not in ("interaction", "factored"):
-            raise ValueError("formulation must be 'interaction' or 'factored'")
         if self.nranks == 1 and resolve is None:
-            _lib.check(lib.ces_step(h, r, ts, fh, float(switch), _lib.FORMULATIONS[formulation], Up, ldu, Gp, ldg, Xp, ldx,
-                                    Op, ldo, ctypes.byref(self._hk), self._met))
+            _lib.check(lib.ces_step(h, r, ts, fh, float(switch), form, Up, ldu, Gp, ldg, Xp, ldx, Op, ldo,
+                                    ctypes.byref(self._hk), self._met))
         else:
             def peek():
                 hk = ctypes.c_double()
@@ -498,8 +507,7 @@ class Engine(object):
                 phases["peer_wait"] = lambda: _lib.check(lib.ces_peer_gather_wait(h))
             comm = (self.dist, self.group, self.rank) if self.nranks > 1 else None
             run_phases(phases, self.buffer, comm, self.p, self.k, rule, resolve, formulation)
-        met = {key: float(self._met[i]) for i, key in enumerate(_METRIC_KEYS)}
-        return out, float(self._hk.value), met
+        return (out,) + self._results()
 
     def step_host(self, rule, U, G, xi, fixed_h=None, switch=1.0, resolve=None, formulation="interaction", noise=None):
         """The same update on host numpy arrays: the copies to and from the device are part of the call.  This is what
@@ -507,8 +515,7 @@ class Engine(object):
         (``nranks > 1``): this rank's (p, cols) / (k, cols) shards in, its (p, cols) shard of U_next out, the phases
         with their collectives in between (``_step_host_sharded``).  ``noise`` as in ``step`` (a host xi_ens is
         uploaded)."""
-        if formulation not in _lib.FORMULATIONS:
-            raise ValueError("formulation must be 'interaction' or 'factored'")
+        r, ts, fh, form = self._step_args(rule, fixed_h, formulation)
         if self.nranks != 1:
             return self._step_host_sharded(rule, U, G, xi, fixed_h, switch, resolve, formulation, noise)
         if resolve is not None:
@@ -519,9 +526,6 @@ class Engine(object):
                                      switch=switch, resolve=resolve, formulation=formulation, noise=noise)
             return out.cpu().numpy(), hk, met
         self._apply_noise(noise)
-        r = _lib.RULES[rule]
-        ts = _lib.TS_FIXED if fixed_h is not None else _lib.TS_FROBENIUS
-        fh = float(fixed_h) if fixed_h is not None else 0.0
         U = np.ascontiguousarray(U, dtype=np.float64)
         G = np.ascontiguousarray(G, dtype=np.float64)
         assert U.shape == (self.p, self.J) and G.shape == (self.k, self.J), (U.shape, G.shape)
@@ -537,11 +541,9 @@ class Engine(object):
             xp = _lib.host_ptr(xi)
         else:
             xp = None
-        _lib.check(self.lib.ces_step_host(self.h, r, ts, fh, float(switch), _lib.FORMULATIONS[formulation],
-                                          _lib.host_ptr(U), _lib.host_ptr(G), xp,
+        _lib.check(self.lib.ces_step_host(self.h, r, ts, fh, float(switch), form, _lib.host_ptr(U), _lib.host_ptr(G), xp,
                                           _lib.host_ptr(out), ctypes.byref(self._hk), self._met))
-        met = {key: float(self._met[i]) for i, key in enumerate(_METRIC_KEYS)}
-        return out, float(self._hk.value), met
+        return (out,) + self._results()
 
     def _pinned(self, name, shape):
         """Reusable page-locked staging array (numpy view of a torch pinned tensor)."""
@@ -570,11 +572,9 @@ class Engine(object):
         with self.on_stream():
             if resolve is None and formulation == "interaction":
                 self._apply_noise(noise)
-                r = _lib.RULES[rule]
-                ts = _lib.TS_FIXED if fixed_h is not None else _lib.TS_FROBENIUS
+                r, ts, fh, form = self._step_args(rule, fixed_h, formulation)
                 nch, bounds = ctypes.c_int(), (ctypes.c_int64 * 9)()
-                _lib.check(lib.ces_host_begin(h, r, 0, ptr(U), ptr(G), ptr(xi), ctypes.byref(nch), bounds))
-                fh = float(fixed_h) if fixed_h is not None else 0.0
+                _lib.check(lib.ces_host_begin(h, r, form, ptr(U), ptr(G), ptr(xi), ctypes.byref(nch), bounds))
                 out_ptr = host.data_ptr() if self.cols else None
                 phases = {
                     "sums_g": lambda c: _lib.check(lib.ces_host_sums_g(h, c)),
@@ -593,8 +593,7 @@ class Engine(object):
                     phases["peer_wait"] = lambda: _lib.check(lib.ces_peer_gather_wait(h))
                 run_host_phases(phases, self.buffer, (dist, group, self.rank), self.p, self.k, rule,
                                 [int(bounds[i]) for i in range(nch.value + 1)])
-                met = {key: float(self._met[i]) for i, key in enumerate(_METRIC_KEYS)}
-                return host.numpy(), float(self._hk.value), met
+                return (host.numpy(),) + self._results()
             # ---- non-default modes: plain uploads (xi on a side stream: only the last phase needs it), device phases
             if "h2d" not in self._views:
                 self._views["h2d"] = torch.cuda.Stream()

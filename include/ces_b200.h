@@ -155,10 +155,12 @@ int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, con
  * CES_ERR_ALIGN), which must stay valid until the step's phase 4 has run.  In ensemble mode the xi argument of phase 4,
  * ces_step and ces_step_host is ignored and may be NULL, and the single-kernel path of small problems is not taken.
  * CES_ERR_INVALID for an unknown kind or a NULL handle; ensemble mode with CES_FORM_FACTORED (which never gathers
- * U - ubar) is refused by ces_step, ces_host_begin and ces_phase3f_products.  No device work. */
+ * U - ubar) is refused by ces_step, ces_step_host, ces_host_begin and ces_phase3f_products.  No device work. */
 int ces_set_noise(ces_handle_t h, int kind, uint64_t seed, uint64_t step, const double* xi_dev, int64_t ldxi);
 
-/* One whole single-GPU step on device buffers (nranks must be 1). */
+/* One whole single-GPU step on device buffers (nranks must be 1).  ts_kind is CES_TS_FROBENIUS or CES_TS_FIXED
+ * (CES_TS_KEEP belongs to phase 4).  An unknown rule, step-size rule or formulation, and a NULL U, G or Uout, or xi
+ * where the rule's Cholesky noise needs it, return CES_ERR_INVALID before any device work; so does ces_step_host. */
 int ces_step(ces_handle_t h, int rule, int ts_kind, double fixed_h, double switch_, int formulation,
              const double* U_dev, int64_t ldu, const double* G_dev, int64_t ldg, const double* xi_dev, int64_t ldxi,
              double* Uout_dev, int64_t ldo, double* hk_host, double* metrics_host);
