@@ -535,7 +535,7 @@ class sampling(enka):
             # refreshed; repeat the step with the current data (the noise already drawn is reused)
             Uk, hk, met = eng.step_host(rule, U0, Gk, xi, **opts)
         if eng.nranks > 1 and not local:
-            Uk = eng.gather_columns_host(Uk)
+            Uk = eng.gather_columns(eng.torch.from_numpy(Uk).cuda(), Uk.shape[0]).cpu().numpy()
         self._record(met, hk)
         if resolve == 'spectral':
             self.radspec.append(1. / hk)            # ces/calibrate.py:250
@@ -778,14 +778,9 @@ class sampling(enka):
         def gather_dev(local, rows, private=True):
             """Full (rows, J) DEVICE tensor from the column shards; single GPU: the tensor itself, or a private copy when
             the caller will overwrite it before an asynchronous reader is done (the forward-output buffer)."""
-            if eng.nranks == 1:
-                big = local.numel() * 8 >= _HostTrace.SMALL
-                return local.clone() if (private and big) else local
-            parts = [torch.empty(rows, eng.Jl, dtype=torch.float64, device=dev) for _ in range(eng.nranks)]
-            padded = torch.zeros(rows, eng.Jl, dtype=torch.float64, device=dev)
-            padded[:, :hi - lo] = local
-            eng.dist.all_gather(parts, padded, group=group)
-            return torch.cat(parts, dim=1)[:, :J].contiguous()
+            if eng.nranks == 1 and private and local.numel() * 8 >= _HostTrace.SMALL:
+                return local.clone()
+            return eng.gather_columns(local, rows)
 
         def gather_host(local, rows):
             """Full (rows, J) host array from the column shards (synchronous)."""

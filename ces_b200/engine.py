@@ -28,105 +28,51 @@ def shard_range(J, rank, nranks):
     return lo, min(J, lo + w)
 
 
-def run_phases(phases, buffer, comm, p, k, rule, resolve=None, formulation="interaction"):
-    """One update as phases with the collectives of a column-sharded ensemble in between
-    (include/ces_b200.h).  ``comm`` is None on a single GPU, else ``(dist, group, rank)``:
+def _allreduce(buffer, comm):
+    """``allreduce(name, lo=None, hi=None, op="sum")``: all-reduce ("sum" or "max") of the named buffer, or in place of
+    columns lo:hi of its first row (a contiguous view, no staging copies); nothing on a single GPU (``comm`` None)."""
+    if comm is None:
+        return lambda name, lo=None, hi=None, op="sum": None
+    dist, group, _ = comm
 
-        sums      -> all-reduce(sum)  "sums"  (k + p doubles)            means of G and U
-        centre    -> all-reduce(sum)  "cuu"   (p x ldp)                  C^uu from the local U~ U~^T
-                     all-gather       "e_all", "ut_all" (rank-major)     every rank needs all of E and U~
-        interact  -> all-reduce(sum)  "scalars"[0:5]                     ||D||_F^2 and the four diagnostics
-        [peek -> cpp -> all-reduce(sum) "cpp" (k x ldk) -> resolve]      non-default time_step only (K11)
-        drift     -> all-reduce(max)  "scalars"[5:6]                     aldi_constant only
-        update
+    def allreduce(name, lo=None, hi=None, op="sum"):
+        t = buffer(name) if lo is None else buffer(name)[0, lo:hi]
+        dist.all_reduce(t, op=dist.ReduceOp.MAX if op == "max" else dist.ReduceOp.SUM, group=group)
+    return allreduce
 
-    ``formulation``: "interaction" forms D = (1/J) E^T W in panels (the reference's formulation, the default);
-    "factored" computes the same V = U~ D as (1/J)(U~ E^T) W and ||D||_F through two k x k Gram matrices, with
-    all-reduces of "p1", "gram_e", "gram_w" instead of the all-gathers (opt-in, see DESIGN.md).
 
-    ``resolve``: None (default step size rule), "always" ('constant': D is formed once, with
-    hk C^pp + Gamma), ``(t_last, threshold)`` ('mix': re-solve when t_last + hk > threshold,
-    ces/calibrate.py:470-473), or "spectral" (hk = 1 / lambda_max(D), :249-251: the "spectral" phase sets the
-    step size from the all-reduced C^pp and the update is called with the marker "spectral").  ``phases`` maps the names to callables, ``buffer(name)`` returns the torch
-    tensor a collective runs on.  The engine passes the ctypes calls; tests/test_multirank_gloo.py passes a
-    numpy stand-in to exercise this orchestration over gloo without a GPU."""
-    if comm is not None:
+def _start_gather(phases, buffer, comm, p, k, mark):
+    """Start moving the other ranks' blocks of E and U~ into "e_all" / "ut_all" (rank-major) and return the wait for
+    them: the peer pulls when the peers are mapped (ces_peer_gather: copy engines over NVLink, CUDA IPC), else two in-place
+    asynchronous all-gathers.  Called right after the all-reduce of C^uu, which is the cross-rank ordering the pulls
+    need.  This rank's own blocks are already in place, so the work on them can run before the wait."""
+    if "peer_gather" in phases:
+        phases["peer_gather"]()
+        waits = [phases["peer_wait"]]
+    else:
         dist, group, rank = comm
+        e_all, ut_all = buffer("e_all"), buffer("ut_all")
+        waits = [dist.all_gather_into_tensor(e_all, e_all[rank * k:(rank + 1) * k], group=group, async_op=True).wait,
+                 dist.all_gather_into_tensor(ut_all, ut_all[rank * p:(rank + 1) * p], group=group, async_op=True).wait]
 
-        def allreduce(t, op=None):
-            dist.all_reduce(t, group=group) if op is None else dist.all_reduce(t, op=op, group=group)
+    def wait():
+        for w in waits:
+            w()
+        mark("gather:e,ut:waited")
+    return wait
 
-        def allreduce_slice(t, lo, hi, op=None):
-            allreduce(t[0, lo:hi], op)        # a contiguous view: reduced in place, no staging copies
-    else:
-        rank = 0
 
-        def allreduce(t, op=None):
-            return None
-
-        def allreduce_slice(t, lo, hi, op=None):
-            return None
-
-    mark = phases.get("mark", lambda name: None)      # per-phase timeline (Engine.timeline), no-op by default
-    phases["sums"]()
-    allreduce(buffer("sums") if comm is not None else None)
-    mark("allreduce:sums:done")
-    phases["centre"]()
-    if formulation == "factored":
-        if resolve is not None:
-            raise NotImplementedError("the factored formulation supports the default step-size rule only")
-        if comm is not None:
-            allreduce(buffer("cuu"))
-        phases["products"]()
-        if comm is not None:
-            for name in ("p1", "gram_e", "gram_w"):
-                allreduce(buffer(name))
-        phases["finish_factored"]()
-    else:
-        overlapped = False
-        if comm is not None:
-            allreduce(buffer("cuu"))
-            mark("allreduce:cuu:done")
-            e_all, ut_all = buffer("e_all"), buffer("ut_all")
-            e_own, ut_own = e_all[rank * k:(rank + 1) * k], ut_all[rank * p:(rank + 1) * p]
-            if "peer_gather" in phases and resolve != "always" and "interact_own" in phases:
-                # the other ranks' blocks are pulled by copy engines over NVLink (ces_peer_gather: peers mapped through
-                # CUDA IPC) while the D / V GEMMs of this rank's own block run with every SM; the all-reduce of C^uu
-                # just queued is the cross-rank ordering the pulls need
-                phases["peer_gather"]()
-                phases["interact_own"]()
-                phases["peer_wait"]()
-                mark("peer_gather:waited")
-                phases["interact_rest"]()
-                overlapped = True
-            elif dist.get_backend(group) == "nccl" and resolve != "always" and "interact_own" in phases:
-                # NCCL: in-place all-gathers started asynchronously; the D / V GEMMs of this rank's own block (already
-                # in place after the centring phase) run while the other ranks' blocks arrive over NVLink
-                works = [dist.all_gather_into_tensor(e_all, e_own, group=group, async_op=True),
-                         dist.all_gather_into_tensor(ut_all, ut_own, group=group, async_op=True)]
-                phases["interact_own"]()
-                for wk in works:
-                    wk.wait()
-                mark("allgather:e,ut:waited")
-                phases["interact_rest"]()
-                overlapped = True
-            elif "peer_gather" in phases:
-                phases["peer_gather"]()
-                phases["peer_wait"]()
-            else:
-                dist.all_gather_into_tensor(e_all, e_own.clone(), group=group)
-                dist.all_gather_into_tensor(ut_all, ut_own.clone(), group=group)
-        if not overlapped:
-            phases["interact"](resolve == "always")
-    if comm is not None:
-        allreduce_slice(buffer("scalars"), 0, 5)
-        mark("allreduce:scalars:done")
+def _end_step(phases, allreduce, mark, rule, resolve):
+    """The end of an update, after the interaction: all-reduce of ||D||_F^2 and the diagnostics, the step size (and the
+    re-solve of D for a non-default ``resolve``, see ``run_phases``), the drift with its MAX all-reduce (aldi_constant),
+    the update."""
+    allreduce("scalars", 0, 5)
+    mark("allreduce:scalars:done")
     keep = False
     if resolve == "spectral":
         # hk = 1 / lambda_max(D) (ces/calibrate.py:249-251); lambda_max(D) = lambda_max(Gamma^-1 C^pp), see csrc/eig.cu
         phases["cpp"]()
-        if comm is not None:
-            allreduce(buffer("cpp"))
+        allreduce("cpp")
         phases["spectral"]()
         phases["update"]("spectral")
         return
@@ -134,15 +80,69 @@ def run_phases(phases, buffer, comm, p, k, rule, resolve=None, formulation="inte
         hk = phases["peek"]()
         if resolve == "always" or resolve[0] + hk > resolve[1]:
             phases["cpp"]()
-            if comm is not None:
-                allreduce(buffer("cpp"))
+            allreduce("cpp")
             phases["resolve"]()
         keep = True
     if rule == "aldi_constant":
         phases["drift"]()
-        if comm is not None:
-            allreduce_slice(buffer("scalars"), 5, 6, dist.ReduceOp.MAX)
+        allreduce("scalars", 5, 6, "max")
     phases["update"](keep)
+
+
+def run_phases(phases, buffer, comm, p, k, rule, resolve=None, formulation="interaction"):
+    """One update as phases with the collectives of a column-sharded ensemble in between
+    (include/ces_b200.h).  ``comm`` is None on a single GPU, else ``(dist, group, rank)``:
+
+        sums      -> all-reduce(sum)  "sums"  (k + p doubles)            means of G and U
+        centre    -> all-reduce(sum)  "cuu"   (p x ldp)                  C^uu from the local U~ U~^T
+                     gathers          "e_all", "ut_all" (rank-major)     every rank needs all of E and U~
+        interact  -> all-reduce(sum)  "scalars"[0:5]                     ||D||_F^2 and the four diagnostics
+        [peek -> cpp -> all-reduce(sum) "cpp" (k x ldk) -> resolve]      non-default time_step only (K11)
+        drift     -> all-reduce(max)  "scalars"[5:6]                     aldi_constant only
+        update
+
+    With several ranks the interaction runs in two parts, this rank's own block of E and U~ (``interact_own``) while the
+    other ranks' blocks arrive, the rest (``interact_rest``) after them; with ``resolve`` "always" D is formed by the
+    re-solve, so the gathers are waited for before ``interact`` (which then only starts the factorisation of C^uu).
+
+    ``formulation``: "interaction" forms D = (1/J) E^T W in panels (the reference's formulation, the default);
+    "factored" computes the same V = U~ D as (1/J)(U~ E^T) W and ||D||_F through two k x k Gram matrices, with
+    all-reduces of "p1", "gram_e", "gram_w" instead of the gathers (opt-in, see DESIGN.md).
+
+    ``resolve``: None (default step size rule), "always" ('constant': D is formed once, with
+    hk C^pp + Gamma), ``(t_last, threshold)`` ('mix': re-solve when t_last + hk > threshold,
+    ces/calibrate.py:470-473), or "spectral" (hk = 1 / lambda_max(D), :249-251: the "spectral" phase sets the
+    step size from the all-reduced C^pp and the update is called with the marker "spectral").  ``phases`` maps the
+    names to callables, ``buffer(name)`` returns the torch tensor a collective runs on.  The engine passes the ctypes
+    calls; tests/test_multirank_gloo.py passes a numpy stand-in to exercise this orchestration over gloo without a GPU."""
+    allreduce = _allreduce(buffer, comm)
+    mark = phases.get("mark", lambda name: None)      # per-phase timeline (Engine.timeline), no-op by default
+    phases["sums"]()
+    allreduce("sums")
+    mark("allreduce:sums:done")
+    phases["centre"]()
+    if formulation == "factored":
+        if resolve is not None:
+            raise NotImplementedError("the factored formulation supports the default step-size rule only")
+        allreduce("cuu")
+        phases["products"]()
+        for name in ("p1", "gram_e", "gram_w"):
+            allreduce(name)
+        phases["finish_factored"]()
+    elif comm is None:
+        phases["interact"](resolve == "always")
+    else:
+        allreduce("cuu")
+        mark("allreduce:cuu:done")
+        wait = _start_gather(phases, buffer, comm, p, k, mark)
+        if resolve == "always":
+            wait()
+            phases["interact"](True)
+        else:
+            phases["interact_own"]()
+            wait()
+            phases["interact_rest"]()
+    _end_step(phases, allreduce, mark, rule, resolve)
 
 
 def run_host_phases(phases, buffer, comm, p, k, rule, bounds):
@@ -154,55 +154,29 @@ def run_host_phases(phases, buffer, comm, p, k, rule, bounds):
         sums_u        -> all-reduce(sum) "sums"[k:k+p]
         centre_u      -> all-reduce(sum) "cuu";  gathers of "e_all" / "ut_all" started (peer pulls, or all-gathers)
         interact_chunk(last), interact_own   (run while the other ranks' blocks arrive)
-        interact_rest -> all-reduce(sum) "scalars"[0:5]
-        [drift        -> all-reduce(max) "scalars"[5:6]]          aldi_constant only
-        update
+        interact_rest, then the end of ``run_phases`` with the default step-size rule
 
     The last chunk's share of the own block's D panel is deferred until the gathers have been started, so they run under
     it.  ``phases`` maps the names to callables (the engine passes the ctypes calls of the library;
     tests/test_multirank_gloo.py passes a numpy stand-in and runs this over gloo without a GPU)."""
-    dist, group, rank = comm
+    allreduce = _allreduce(buffer, comm)
     mark = phases.get("mark", lambda name: None)
-    sums = buffer("sums")
-    nchunks = len(bounds) - 1
-    last = nchunks - 1
-    for c in range(nchunks):
+    last = len(bounds) - 2
+    for c in range(last + 1):
         phases["sums_g"](c)
-        dist.all_reduce(sums[0, bounds[c]:bounds[c + 1]], group=group)
+        allreduce("sums", bounds[c], bounds[c + 1])
         phases["centre_g"](c, c != last)
     phases["sums_u"]()
-    dist.all_reduce(sums[0, k:k + p], group=group)
+    allreduce("sums", k, k + p)
     phases["centre_u"]()
-    dist.all_reduce(buffer("cuu"), group=group)
+    allreduce("cuu")
     mark("allreduce:cuu:done")
-    e_all, ut_all = buffer("e_all"), buffer("ut_all")
-    e_own, ut_own = e_all[rank * k:(rank + 1) * k], ut_all[rank * p:(rank + 1) * p]
-    if "peer_gather" in phases:
-        phases["peer_gather"]()
-        phases["interact_chunk"](last)
-        phases["interact_own"]()
-        phases["peer_wait"]()
-    elif dist.get_backend(group) == "nccl":
-        works = [dist.all_gather_into_tensor(e_all, e_own, group=group, async_op=True),
-                 dist.all_gather_into_tensor(ut_all, ut_own, group=group, async_op=True)]
-        phases["interact_chunk"](last)
-        phases["interact_own"]()
-        for wk in works:
-            wk.wait()
-    else:
-        dist.all_gather_into_tensor(e_all, e_own.clone(), group=group)
-        dist.all_gather_into_tensor(ut_all, ut_own.clone(), group=group)
-        phases["interact_chunk"](last)
-        phases["interact_own"]()
-    mark("gather:e,ut:waited")
+    wait = _start_gather(phases, buffer, comm, p, k, mark)
+    phases["interact_chunk"](last)
+    phases["interact_own"]()
+    wait()
     phases["interact_rest"]()
-    scal = buffer("scalars")
-    dist.all_reduce(scal[0, 0:5], group=group)
-    mark("allreduce:scalars:done")
-    if rule == "aldi_constant":
-        phases["drift"]()
-        dist.all_reduce(scal[0, 5:6], op=dist.ReduceOp.MAX, group=group)
-    phases["update"]()
+    _end_step(phases, allreduce, mark, rule, None)
 
 
 @contextlib.contextmanager
@@ -476,7 +450,7 @@ class Engine(object):
 
             def update(keep):
                 ev = getattr(self, "_xi_ready", None)
-                if ev is not None:                  # sharded host step: the noise was uploaded on a side stream
+                if ev is not None:                  # host-staged step: the noise was uploaded on a side stream
                     torch.cuda.current_stream().wait_event(ev)
                     self._xi_ready = None
                 if keep == "spectral":
@@ -486,45 +460,48 @@ class Engine(object):
                 _lib.check(lib.ces_phase4_update(h, r, kind, val, Up, ldu, Xp, ldx, Op, ldo, ctypes.byref(self._hk),
                                                  self._met))
 
-            phases = {
-                "sums": lambda: _lib.check(lib.ces_phase1_sums(h, Up, ldu, Gp, ldg)),
-                "centre": lambda: _lib.check(lib.ces_phase2_centre(h, r, Up, ldu, Gp, ldg)),
-                "interact": lambda skip: _lib.check(lib.ces_phase3_interact(h, r, 1 if skip else 0)),
-                "interact_own": lambda: _lib.check(lib.ces_phase3_blocks(h, r, 0, 1)),
-                "interact_rest": lambda: _lib.check(lib.ces_phase3_blocks(h, r, 1, self.nranks - 1)),
-                "peek": peek,
-                "cpp": lambda: _lib.check(lib.ces_phase3b_cpp(h)),
-                "resolve": lambda: _lib.check(lib.ces_phase3c_resolve(h, r)),
-                "spectral": spectral,
-                "products": lambda: _lib.check(lib.ces_phase3f_products(h, r)),
-                "finish_factored": lambda: _lib.check(lib.ces_phase3f_finish(h, r)),
-                "drift": lambda: _lib.check(lib.ces_phase4a_drift(h, float(switch))),
-                "update": update,
-                "mark": self.mark,
-            }
-            if self.peer_gather:
-                phases["peer_gather"] = lambda: _lib.check(lib.ces_peer_gather(h))
-                phases["peer_wait"] = lambda: _lib.check(lib.ces_peer_gather_wait(h))
-            comm = (self.dist, self.group, self.rank) if self.nranks > 1 else None
-            run_phases(phases, self.buffer, comm, self.p, self.k, rule, resolve, formulation)
+            phases = self._phases(
+                r, switch,
+                sums=lambda: _lib.check(lib.ces_phase1_sums(h, Up, ldu, Gp, ldg)),
+                centre=lambda: _lib.check(lib.ces_phase2_centre(h, r, Up, ldu, Gp, ldg)),
+                interact=lambda skip: _lib.check(lib.ces_phase3_interact(h, r, 1 if skip else 0)),
+                interact_own=lambda: _lib.check(lib.ces_phase3_blocks(h, r, 0, 1)),
+                peek=peek,
+                cpp=lambda: _lib.check(lib.ces_phase3b_cpp(h)),
+                resolve=lambda: _lib.check(lib.ces_phase3c_resolve(h, r)),
+                spectral=spectral,
+                products=lambda: _lib.check(lib.ces_phase3f_products(h, r)),
+                finish_factored=lambda: _lib.check(lib.ces_phase3f_finish(h, r)),
+                update=update)
+            run_phases(phases, self.buffer, self._comm(), self.p, self.k, rule, resolve, formulation)
         return (out,) + self._results()
+
+    def _phases(self, r, switch, **own):
+        """The phase table of ``run_phases`` / ``run_host_phases``: the library calls both step paths share, plus ``own``."""
+        lib, h = self.lib, self.h
+        phases = {
+            "interact_rest": lambda: _lib.check(lib.ces_phase3_blocks(h, r, 1, self.nranks - 1)),
+            "drift": lambda: _lib.check(lib.ces_phase4a_drift(h, float(switch))),
+            "mark": self.mark,
+        }
+        if self.peer_gather:
+            phases["peer_gather"] = lambda: _lib.check(lib.ces_peer_gather(h))
+            phases["peer_wait"] = lambda: _lib.check(lib.ces_peer_gather_wait(h))
+        phases.update(own)
+        return phases
+
+    def _comm(self):
+        return (self.dist, self.group, self.rank) if self.nranks > 1 else None
 
     def step_host(self, rule, U, G, xi, fixed_h=None, switch=1.0, resolve=None, formulation="interaction", noise=None):
         """The same update on host numpy arrays: the copies to and from the device are part of the call.  This is what
-        ``sampling.eks_update*`` invoke.  Single GPU: (p, J) / (k, J) arrays through ``ces_step_host``.  Column-sharded
-        (``nranks > 1``): this rank's (p, cols) / (k, cols) shards in, its (p, cols) shard of U_next out, the phases
-        with their collectives in between (``_step_host_sharded``).  ``noise`` as in ``step`` (a host xi_ens is
-        uploaded)."""
+        ``sampling.eks_update*`` invoke.  Single GPU with the default step-size rule: (p, J) / (k, J) arrays through
+        ``ces_step_host``.  Otherwise (column-sharded: this rank's (p, cols) / (k, cols) shards in, its (p, cols) shard of
+        U_next out) the phases with their collectives in between (``_step_host_staged``).  ``noise`` as in ``step`` (a host
+        xi_ens is uploaded)."""
         r, ts, fh, form = self._step_args(rule, fixed_h, formulation)
-        if self.nranks != 1:
-            return self._step_host_sharded(rule, U, G, xi, fixed_h, switch, resolve, formulation, noise)
-        if resolve is not None:
-            # non-default time_step: the phase-by-phase device path, with explicit copies around it
-            torch = self.torch
-            dev = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).cuda()
-            out, hk, met = self.step(rule, dev(U), dev(G), dev(xi) if xi is not None else None, fixed_h=fixed_h,
-                                     switch=switch, resolve=resolve, formulation=formulation, noise=noise)
-            return out.cpu().numpy(), hk, met
+        if self.nranks != 1 or resolve is not None:
+            return self._step_host_staged(rule, U, G, xi, fixed_h, switch, resolve, formulation, noise)
         self._apply_noise(noise)
         U = np.ascontiguousarray(U, dtype=np.float64)
         G = np.ascontiguousarray(G, dtype=np.float64)
@@ -552,13 +529,14 @@ class Engine(object):
             self._views[key] = self.torch.empty(tuple(shape), dtype=self.torch.float64, pin_memory=True)
         return self._views[key]
 
-    def _step_host_sharded(self, rule, U, G, xi, fixed_h, switch, resolve, formulation, noise=None):
-        """Column shard on host arrays.  Default rule set (no re-solve of D, interaction formulation): the pipelined
-        pieces of the library's host step (include/ces_b200.h) with this rank's collectives in between -- G uploads in
-        row chunks while the chunks already on the device are summed (all-reduce of that slice of the means), centred and
-        contracted into the own block's first D panel; U and xi follow behind; U_next comes back in overlapped column
-        chunks.  Other modes: plain uploads, then the device-pointer phases."""
-        torch, lib, h, dist, group = self.torch, self.lib, self.h, self.dist, self.group
+    def _step_host_staged(self, rule, U, G, xi, fixed_h, switch, resolve, formulation, noise=None):
+        """This rank's columns on host arrays, through the phases.  Column shard with the default rule set (no re-solve
+        of D, interaction formulation): the pipelined pieces of the library's host step (include/ces_b200.h) with this
+        rank's collectives in between -- G uploads in row chunks while the chunks already on the device are summed
+        (all-reduce of that slice of the means), centred and contracted into the own block's first D panel; U and xi
+        follow behind; U_next comes back in overlapped column chunks.  Other modes (and a single GPU with a non-default
+        step-size rule): uploads into reused device buffers, then the device-pointer phases."""
+        torch, lib, h = self.torch, self.lib, self.h
         U = np.ascontiguousarray(U, dtype=np.float64)
         G = np.ascontiguousarray(G, dtype=np.float64)
         assert U.shape == (self.p, self.cols) and G.shape == (self.k, self.cols), (U.shape, G.shape, self.cols)
@@ -570,28 +548,23 @@ class Engine(object):
         host = torch.empty((self.p, self.cols), dtype=torch.float64, pin_memory=self.p * self.cols * 8 >= (1 << 20))
         ptr = lambda a: (_lib.host_ptr(a) if a is not None and a.size else None)
         with self.on_stream():
-            if resolve is None and formulation == "interaction":
+            if self.nranks > 1 and resolve is None and formulation == "interaction":
                 self._apply_noise(noise)
                 r, ts, fh, form = self._step_args(rule, fixed_h, formulation)
                 nch, bounds = ctypes.c_int(), (ctypes.c_int64 * 9)()
                 _lib.check(lib.ces_host_begin(h, r, form, ptr(U), ptr(G), ptr(xi), ctypes.byref(nch), bounds))
                 out_ptr = host.data_ptr() if self.cols else None
-                phases = {
-                    "sums_g": lambda c: _lib.check(lib.ces_host_sums_g(h, c)),
-                    "centre_g": lambda c, interact: _lib.check(lib.ces_host_centre_g(h, c, 1 if interact else 0)),
-                    "interact_chunk": lambda c: _lib.check(lib.ces_host_interact_chunk(h, c)),
-                    "sums_u": lambda: _lib.check(lib.ces_host_sums_u(h)),
-                    "centre_u": lambda: _lib.check(lib.ces_host_centre_u(h)),
-                    "interact_own": lambda: _lib.check(lib.ces_host_interact_own(h)),
-                    "interact_rest": lambda: _lib.check(lib.ces_phase3_blocks(h, r, 1, self.nranks - 1)),
-                    "drift": lambda: _lib.check(lib.ces_phase4a_drift(h, float(switch))),
-                    "update": lambda: _lib.check(lib.ces_host_update(h, ts, fh, out_ptr, ctypes.byref(self._hk), self._met)),
-                    "mark": self.mark,
-                }
-                if self.peer_gather:
-                    phases["peer_gather"] = lambda: _lib.check(lib.ces_peer_gather(h))
-                    phases["peer_wait"] = lambda: _lib.check(lib.ces_peer_gather_wait(h))
-                run_host_phases(phases, self.buffer, (dist, group, self.rank), self.p, self.k, rule,
+                phases = self._phases(
+                    r, switch,
+                    sums_g=lambda c: _lib.check(lib.ces_host_sums_g(h, c)),
+                    centre_g=lambda c, interact: _lib.check(lib.ces_host_centre_g(h, c, 1 if interact else 0)),
+                    interact_chunk=lambda c: _lib.check(lib.ces_host_interact_chunk(h, c)),
+                    sums_u=lambda: _lib.check(lib.ces_host_sums_u(h)),
+                    centre_u=lambda: _lib.check(lib.ces_host_centre_u(h)),
+                    interact_own=lambda: _lib.check(lib.ces_host_interact_own(h)),
+                    update=lambda keep: _lib.check(lib.ces_host_update(h, ts, fh, out_ptr, ctypes.byref(self._hk),
+                                                                       self._met)))
+                run_host_phases(phases, self.buffer, self._comm(), self.p, self.k, rule,
                                 [int(bounds[i]) for i in range(nch.value + 1)])
                 return (host.numpy(),) + self._results()
             # ---- non-default modes: plain uploads (xi on a side stream: only the last phase needs it), device phases
@@ -622,16 +595,16 @@ class Engine(object):
             main.synchronize()
             return host.numpy(), hk, met
 
-    def gather_columns_host(self, local):
-        """Full (rows, J) host array from every rank's (rows, cols) host shard (all ranks receive it)."""
+    def gather_columns(self, local, rows):
+        """(rows, J) device tensor of every rank's (rows, cols) device shard, on every rank; ``local`` itself on a single
+        GPU.  The shards are gathered in place into one zero-padded (nranks, rows, Jl) buffer."""
+        if self.nranks == 1:
+            return local
         torch = self.torch
-        local = np.ascontiguousarray(local, dtype=np.float64)
-        rows = local.shape[0]
-        pad = torch.zeros(rows, self.Jl, dtype=torch.float64, device="cuda")
-        pad[:, :self.cols] = torch.from_numpy(local).cuda()
-        full = torch.empty(self.nranks, rows, self.Jl, dtype=torch.float64, device="cuda")
-        self.dist.all_gather_into_tensor(full.view(-1), pad.view(-1), group=self.group)
-        return full.permute(1, 0, 2).reshape(rows, self.nranks * self.Jl)[:, :self.J].cpu().numpy()
+        full = torch.zeros(self.nranks, rows, self.Jl, dtype=torch.float64, device="cuda")
+        full[self.rank, :, :self.cols] = local
+        self.dist.all_gather_into_tensor(full.view(-1), full[self.rank].view(-1), group=self.group)
+        return full.permute(1, 0, 2).reshape(rows, self.nranks * self.Jl)[:, :self.J]
 
     # ------------------------------------------------------------------ forward maps
     def forward_map(self, kind, U, G, A=None, lda=0, b=None, params=None):

@@ -2,8 +2,8 @@
 
 Implements, on CPU torch tensors, exactly the buffer contract of include/ces_b200.h ("sums", "cuu",
 "e_all", "ut_all", "scalars"; rank-major blocks, zero-padded shard columns) so that
-ces_b200.engine.run_sharded_phases -- the host orchestration of the collectives -- can be exercised
-with gloo and world_size 2 on a machine without a GPU.  It is never imported by the product.
+ces_b200.engine.run_phases / run_host_phases -- the host orchestration of the collectives -- can be
+exercised with gloo and world_size 2 on a machine without a GPU.  It is never imported by the product.
 """
 import numpy as np
 import torch
@@ -30,28 +30,43 @@ class NumpyPhases(object):
     def buffer(self, name):
         return self.buf[name]
 
-    def bind(self, rule, U, G, xi, switch=1.0, fixed_h=None):
+    def bind(self, rule, U, G, xi, switch=1.0, fixed_h=None, peer=False):
+        """The phases of ces_b200.engine.run_phases.  ``peer``: add stand-ins for the peer pulls (ces_peer_gather: an
+        in-place all-gather of "e_all" / "ut_all" over the default group; ces_peer_gather_wait: nothing to wait for)."""
         self.rule, self.U, self.G, self.xi, self.switch, self.fixed_h = rule, U, G, xi, switch, fixed_h
         ldk = (self.k + 15) // 16 * 16
         self.buf["cpp"] = torch.zeros(self.k, ldk, dtype=torch.float64)
         self.buf["p1"] = torch.zeros(self.p, ldk, dtype=torch.float64)
         self.buf["gram_e"] = torch.zeros(self.k, ldk, dtype=torch.float64)
         self.buf["gram_w"] = torch.zeros(self.k, ldk, dtype=torch.float64)
-        return {"sums": self.sums, "centre": self.centre, "interact": self.interact, "drift": self.drift,
-                "update": self.update, "peek": self.peek, "cpp": self.cpp, "resolve": self.resolve,
-                "products": self.products, "finish_factored": self.finish_factored, "spectral": self.spectral}
+        return dict({"sums": self.sums, "centre": self.centre, "interact": self.interact, "interact_own": self.interact_own,
+                     "interact_rest": self.interact_rest, "drift": self.drift, "update": self.update, "peek": self.peek,
+                     "cpp": self.cpp, "resolve": self.resolve, "products": self.products,
+                     "finish_factored": self.finish_factored, "spectral": self.spectral}, **self._peer(peer))
+
+    def _peer(self, peer):
+        if not peer:
+            return {}
+
+        def gather():
+            import torch.distributed as dist
+
+            for name, rows in (("e_all", self.k), ("ut_all", self.p)):
+                b = self.buf[name]
+                dist.all_gather_into_tensor(b, b[self.rank * rows:(self.rank + 1) * rows])
+        return {"peer_gather": gather, "peer_wait": lambda: None}
 
     # ---- the pipelined host step in pieces (ces_host_*; ces_b200.engine.run_host_phases).  Needs a diagonal Gamma: a row
     # chunk of W = Gamma^-1 (G - y) is then a function of the same rows of G only.
-    def bind_host(self, rule, U, G, xi, bounds, switch=1.0):
+    def bind_host(self, rule, U, G, xi, bounds, switch=1.0, peer=False):
         self.rule, self.U, self.G, self.xi, self.switch, self.fixed_h = rule, U, G, xi, switch, None
         self.bounds = list(bounds)
         self.W = np.zeros((self.k, self.cols))
         self.D_own = np.zeros((self.Jl, self.cols))
         self.calls = []
-        return {"sums_g": self.h_sums_g, "centre_g": self.h_centre_g, "interact_chunk": self.h_interact_chunk,
-                "sums_u": self.h_sums_u, "centre_u": self.h_centre_u, "interact_own": self.h_interact_own,
-                "interact_rest": self.h_interact_rest, "drift": self.drift, "update": self.update}
+        return dict({"sums_g": self.h_sums_g, "centre_g": self.h_centre_g, "interact_chunk": self.h_interact_chunk,
+                     "sums_u": self.h_sums_u, "centre_u": self.h_centre_u, "interact_own": self.h_interact_own,
+                     "interact_rest": self.interact_rest, "drift": self.drift, "update": self.update}, **self._peer(peer))
 
     def _rows(self, c):
         return slice(self.bounds[c], self.bounds[c + 1])
@@ -116,16 +131,6 @@ class NumpyPhases(object):
         self.V = Ut @ self.D_own
         self._ssq = (self.D_own ** 2).sum()
 
-    def h_interact_rest(self):
-        p, k = self.p, self.k
-        e_all, ut_all = self.buf["e_all"].numpy(), self.buf["ut_all"].numpy()
-        for i in range(1, self.nranks):
-            s = (self.rank + i) % self.nranks
-            D = (e_all[s * k:(s + 1) * k, :self.Jl].T @ self.W) / self.J
-            self._ssq += (D ** 2).sum()
-            self.V += ut_all[s * p:(s + 1) * p, :self.Jl] @ D
-        self.buf["scalars"][0, 0] = self._ssq
-
     def sums(self):
         s = np.concatenate([self.G.sum(axis=1), self.U.sum(axis=1)])
         self.buf["sums"][0] = torch.from_numpy(s)
@@ -156,24 +161,34 @@ class NumpyPhases(object):
         cuu[:] = 0.0
         cuu[:, :p] = C
 
-    def _loops(self, W):
-        p, k, c = self.p, self.k, self.cols
+    def _block(self, s, W):
+        """Rank s's block of D = (1/J) E^T W: its ||.||_F^2 into _ssq, its share of V = U~ D into V."""
+        p, k = self.p, self.k
         e_all, ut_all = self.buf["e_all"].numpy(), self.buf["ut_all"].numpy()
-        ssq = 0.0
-        V = np.zeros((p, c))
+        D = (e_all[s * k:(s + 1) * k, :self.Jl].T @ W) / self.J
+        self._ssq += (D ** 2).sum()
+        self.V += ut_all[s * p:(s + 1) * p, :self.Jl] @ D
+
+    def _loops(self, W):
+        self.V, self._ssq = np.zeros((self.p, self.cols)), 0.0
         for s in range(self.nranks):
-            Es = e_all[s * k:(s + 1) * k, :self.Jl]
-            Uts = ut_all[s * p:(s + 1) * p, :self.Jl]
-            D = (Es.T @ W) / self.J
-            ssq += (D ** 2).sum()
-            V += Uts @ D
-        self.V = V
-        return ssq
+            self._block(s, W)
+        return self._ssq
 
     def interact(self, skip=False):
         self.C = self.buf["cuu"].numpy()[:, :self.p].copy()
         if not skip:
             self.buf["scalars"][0, 0] = self._loops(self.W)
+
+    def interact_own(self):
+        self.C = self.buf["cuu"].numpy()[:, :self.p].copy()
+        self.V, self._ssq = np.zeros((self.p, self.cols)), 0.0
+        self._block(self.rank, self.W)
+
+    def interact_rest(self):
+        for i in range(1, self.nranks):
+            self._block((self.rank + i) % self.nranks, self.W)
+        self.buf["scalars"][0, 0] = self._ssq
 
     def products(self):
         p, k, c = self.p, self.k, self.cols
