@@ -87,6 +87,12 @@ def _identity(a):
     return (id(a), a.__array_interface__['data'][0], a.shape, a.strides, a.dtype.str)
 
 
+# Largest J of the one-launch run with noise='ensemble': the kernel draws J^2 / 2 Box-Muller pairs per iteration on one SM.
+# Measured per iteration (p = 8, k = 16, B200): 0.61x the per-iteration loop on the phases at J = 256, 1.01x at 384
+# (DESIGN.md section 4g, profiles/r08_bench_small_ensemble_noise.json).
+_FUSED_ENSEMBLE_J_MAX = 256
+
+
 def _consume_model_rng(model, n_particles):
     """Advance numpy's global generator by what the reference's per-particle loop over ``model`` would have drawn
     (``rng_draws_per_call`` normals per evaluation; only ``banana`` has any, ces/utils.py:122)."""
@@ -582,21 +588,24 @@ class sampling(enka):
         cumulative time and the ``t_tol`` stopping rule run back to back on the device, the trace is the chain of
         ensembles the kernel leaves in HBM, and the host downloads everything once.  Same results as the iteration-by-
         iteration loop below (same arithmetic per step; the noise is the numpy stream the reference would consume: all T
-        draws are taken in one call and the generator is rewound to where an early stop leaves it).  Returns False when
-        the configuration needs the general loop."""
+        draws are taken in one call and the generator is rewound to where an early stop leaves it).  ``noise='ensemble'``
+        runs here too up to J = _FUSED_ENSEMBLE_J_MAX: the kernel draws the device stream keyed by ``seed`` at step
+        ``len(self.metrics['t']) + i``, or reads the one (J, J) ``xi``, as the general loop does.  Returns False when the
+        configuration needs the general loop."""
         import ctypes
 
         from . import _lib
 
         kind = getattr(model, 'device_kind', None)
+        ensemble, xi_ens = self._noise_options(rule, kwargs, eng.J)
         if not (device_map and eng.nranks == 1 and kind in _lib.MAPS and self.p <= 8 and self.n_obs <= 16
-                and 2 <= eng.J <= 512 and self.T >= 1 and self._step_options(rule, kwargs) == (None, None)
+                and 2 <= eng.J <= (_FUSED_ENSEMBLE_J_MAX if ensemble else 512) and self.T >= 1
+                and self._step_options(rule, kwargs) == (None, None)
                 and self._option(kwargs, 'formulation') == 'interaction'
-                and getattr(self, 'fused_run', True) and kwargs.get('xi', None) is None
-                and not self._noise_options(rule, kwargs, eng.J)[0]):
+                and getattr(self, 'fused_run', True) and (ensemble or kwargs.get('xi', None) is None)):
             return False
         p, k, J, T = self.p, self.n_obs, eng.J, int(self.T)
-        if (T + 1) * (2 * p + k) * J * 8 > (1 << 28):
+        if (T + 1) * ((p if ensemble else 2 * p) + k) * J * 8 > (1 << 28):     # traces (+ the T x p x J Cholesky xi)
             return False
         torch = eng.torch
         A_dev, lda, b_dev, params = model._device_args(torch)
@@ -604,7 +613,7 @@ class sampling(enka):
         device_rng = self._option(kwargs, 'rng') == 'device'
         xi_all, state = None, None
         fdraws = int(getattr(model, 'rng_draws_per_call', 0)) * J    # normals the reference's forward loop draws per pass
-        host_noise = rule != 'eki' and not device_rng
+        host_noise = rule != 'eki' and not device_rng and not ensemble
         if host_noise or fdraws:
             # per iteration the reference draws [forward pass: fdraws][update: p * J] (:351-352 then :447,488,527), and
             # fdraws once more for the final forward pass; all T iterations are drawn in one call (the same stream)
@@ -620,6 +629,7 @@ class sampling(enka):
         tv = np.empty(T)
         n = ctypes.c_int64()
         with eng.on_stream():
+            eng._apply_noise(('ensemble', int(self._option(kwargs, 'seed')), len(t_hist), xi_ens) if ensemble else None)
             _lib.check(eng.lib.ces_small_run(
                 eng.h, _lib.RULES[rule], _lib.TS_FROBENIUS, 0.0, float(kwargs.get('switch', 1.)), _lib.MAPS[kind],
                 ctypes.c_void_p(A_dev.data_ptr()) if A_dev is not None else None, int(lda),

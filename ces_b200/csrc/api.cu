@@ -184,7 +184,7 @@ bool needs_xi(ces_handle_t h, int rule) { return rule != CES_RULE_EKI && !ensemb
 // The arguments of a step, checked by every entry point before any device work.  std::nullopt: the entry point takes no
 // such argument (its rule is phase 2's).  CES_TS_KEEP (`keep_ok`) is for phase 4 only: it keeps ces_peek_step_size's h.
 int check_step(ces_handle_t h, const char* who, std::optional<int> rule, std::optional<int> ts_kind, bool keep_ok,
-               std::optional<int> formulation, bool have_ptrs) {
+               std::optional<int> formulation, bool have_ptrs, bool no_host_xi = true) {
     if (rule && (*rule < CES_RULE_EKS || *rule > CES_RULE_EKI)) return fail(CES_ERR_INVALID, "unknown update rule %s%lld", "", *rule);
     if (ts_kind && *ts_kind != CES_TS_FROBENIUS && *ts_kind != CES_TS_FIXED && !(keep_ok && *ts_kind == CES_TS_KEEP))
         return fail(CES_ERR_INVALID, "unknown step-size rule%s", "");
@@ -193,6 +193,7 @@ int check_step(ces_handle_t h, const char* who, std::optional<int> rule, std::op
     if (formulation == CES_FORM_FACTORED && ensemble_noise(h) && rule.value_or(h->last_rule) != CES_RULE_EKI)
         return fail(CES_ERR_INVALID, "ensemble noise needs the interaction formulation (the factored one never gathers U~)%s", "");
     if (!have_ptrs) return fail(CES_ERR_INVALID, "%s: null pointer", who);
+    if (!no_host_xi) return fail(CES_ERR_INVALID, "%s: ensemble noise takes its xi from ces_set_noise, not xi_host", who);
     return CES_OK;
 }
 
@@ -206,10 +207,15 @@ int splitk_count(int64_t tiles, int64_t contraction) {
     return sp < 1 ? 1 : (int)sp;
 }
 
-// The whole step in one single-CTA kernel (small problems, where launch latency dominates otherwise).  The kernel draws
-// the reference's Cholesky noise only.
+// Largest J of the single-CTA step with ensemble noise: its J^2 / 2 Box-Muller pairs per step run on one SM, the phases'
+// noise pass on all of them.  Measured per iteration of sampling.run (p = 8, k = 16, B200): 0.88x the phases' time at
+// J = 128, 1.04x at 192 (DESIGN.md section 4g, profiles/r08_bench_small_ensemble_noise.json).
+constexpr int64_t kSmallEnsembleJMax = 128;
+
+// The whole step in one single-CTA kernel (small problems, where launch latency dominates otherwise).
 bool small_path(ces_handle_t h, int formulation) {
-    return h->use_small && !ensemble_noise(h) && formulation == CES_FORM_INTERACTION && small_step_eligible(h->p, h->k, h->Jl);
+    return h->use_small && formulation == CES_FORM_INTERACTION && small_step_eligible(h->p, h->k, h->Jl) &&
+           (!ensemble_noise(h) || h->Jl <= kSmallEnsembleJMax);
 }
 
 // The fields of a single-CTA call that come from the handle and the step's settings; operands are the caller's.
@@ -221,6 +227,8 @@ SmallStepCall small_call(ces_handle_t h, int rule, int ts_kind, double fixed_h, 
     c.sinv_diag = h->sinv_diag; c.sig_diag = h->sig_diag;
     c.Sinv = h->sigma_diag ? nullptr : h->Sinv; c.Sigma0 = h->sigma_diag ? nullptr : h->Sigma0;
     c.ldk = h->ldk; c.ldp = h->ldp;
+    c.ensemble = ensemble_noise(h) && rule != CES_RULE_EKI;      // eki has no noise term: the same kernel either way
+    if (c.ensemble) { c.xi = h->noise_xi; c.ldxi = h->noise_ldxi; c.seed = h->noise_seed; c.step = h->noise_step; }
     return c;
 }
 
@@ -1102,7 +1110,8 @@ int ces_step(ces_handle_t h, int rule, int ts_kind, double fixed_h, double switc
     CES_TRY(check_step(h, "ces_step", rule, ts_kind, false, formulation, U && G && Uout && (xi || !needs_xi(h, rule))));
     if (small_path(h, formulation)) {
         SmallStepCall c = small_call(h, rule, ts_kind, fixed_h, switch_);
-        c.U = U; c.G = G; c.xi = xi; c.ldu = ldu; c.ldg = ldg; c.ldxi = ldxi; c.out = Uout; c.ldo = ldo; c.S = h->S;
+        c.U = U; c.G = G; c.ldu = ldu; c.ldg = ldg; c.out = Uout; c.ldo = ldo; c.S = h->S;
+        if (!c.ensemble) { c.xi = xi; c.ldxi = ldxi; }
         h->last_rule = rule;
         CES_TRY(small_step(h->st, c));
         return finish_step(h, Uout, ldo, false, hk_host, metrics_host);
@@ -1357,7 +1366,7 @@ int ces_step_host(ces_handle_t h, int rule, int ts_kind, double fixed_h, double 
     if (small_path(h, formulation)) {
         // tiny problems keep everything on one stream -- extra streams and events would cost more than the copies
         CES_TRY(host_staging(h));
-        if (xi) CES_CUDA(host_h2d(h, h->stage_xi, xi, p, h->st));
+        if (xi && !ensemble_noise(h)) CES_CUDA(host_h2d(h, h->stage_xi, xi, p, h->st));
         CES_CUDA(host_h2d(h, h->stage_U, U, p, h->st));
         CES_CUDA(host_h2d(h, h->stage_G, G, k, h->st));
         h->pending_out = Uout;
@@ -1396,14 +1405,14 @@ int ces_small_run(ces_handle_t h, int rule, int ts_kind, double fixed_h, double 
     if (h->nranks != 1) return fail(CES_ERR_STATE, "ces_small_run is single-GPU%s", "");
     const int64_t p = h->p, k = h->k, J = h->Jl;
     if (!small_step_eligible(p, k, J)) return fail(CES_ERR_INVALID, "ces_small_run: the problem is too large for the single-CTA path%s", "");
-    CES_TRY(check_step(h, "ces_small_run", rule, ts_kind, false, std::nullopt, true));
+    CES_TRY(check_step(h, "ces_small_run", rule, ts_kind, false, std::nullopt, true, !(xi_host && ensemble_noise(h))));
     if (T < 1 || !U0_host || !Utrace_host || !Gtrace_host || !S_host || !t_host || !nsteps_host)
         return fail(CES_ERR_INVALID, "ces_small_run: bad argument%s", "");
     if (map_kind < CES_MAP_LINEAL || map_kind > CES_MAP_BANANA) return fail(CES_ERR_INVALID, "ces_small_run: unknown map kind%s", "");
     if ((map_kind == CES_MAP_LINEAL || map_kind == CES_MAP_LINEAL_LOG) ? !A_dev : (!params_host || p != 2 || k != 2))
         return fail(CES_ERR_INVALID, "ces_small_run: the map needs A (lineal) or two parameters with p = k = 2%s", "");
     cudaStream_t st = h->st;
-    const int64_t nu = (T + 1) * p * J, ng = (T + 1) * k * J, nx = (rule == CES_RULE_EKI) ? 0 : T * p * J;
+    const int64_t nu = (T + 1) * p * J, ng = (T + 1) * k * J, nx = needs_xi(h, rule) ? T * p * J : 0;
     const int64_t total = nu + ng + nx + T * S_COUNT + T + 2;
     if (h->run_ws_len < total) {
         if (h->run_ws) cudaFree(h->run_ws);
@@ -1423,7 +1432,8 @@ int ces_small_run(ces_handle_t h, int rule, int ts_kind, double fixed_h, double 
         else for (int64_t it = 0; it < T; ++it) CES_TRY(fill_normal(st, Xi + it * p * J, J, p, J, 0, seed, step0 + (uint64_t)it));
     }
     SmallStepCall c = small_call(h, rule, ts_kind, fixed_h, switch_);   // operands: the run's own buffers
-    c.ldu = c.ldg = c.ldxi = c.ldo = J;
+    c.ldu = c.ldg = c.ldo = J;
+    if (!c.ensemble) c.ldxi = J;
     SmallRunCall rc;
     rc.T = T; rc.map_kind = map_kind; rc.have_t0 = have_t0; rc.t0 = t0; rc.t_tol = t_tol;
     rc.A = A_dev; rc.lda = lda; rc.b = b_dev;

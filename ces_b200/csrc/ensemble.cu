@@ -517,13 +517,9 @@ int fill_normal(cudaStream_t st, double* X, int64_t ld, int64_t rows, int64_t co
     return CES_OK;
 }
 
-// xi (J x J) of the ensemble noise sqrt(2h / n_C) (U - ubar) xi: element (s, j) -- source particle s, target particle j --
-// from Philox4x32-10 keyed by the seed at the counter (j >> 1, TAG_ENS, s, step), the cosine of the Box-Muller pair for
-// even j and the sine for odd j.  Word 1 carries the tag where fill_normal has the high half of its pair index, so the two
-// streams never share a counter at the same (seed, step).  An element depends only on (seed, step, global s, global j):
-// any block of rows and columns, odd offsets included, reproduces what one GPU draws.  Rows go on blockIdx.y with a
-// grid-stride loop (gridDim.y <= 65535 < J).
-constexpr uint32_t TAG_ENS = 0x454E;
+// A block of xi (J x J) of the ensemble noise sqrt(2h / n_C) (U - ubar) xi, elements as rng.cuh ensemble_noise_pair draws
+// them.  An element depends only on (seed, step, global s, global j): any block of rows and columns, odd offsets included,
+// reproduces what one GPU draws.  Rows go on blockIdx.y with a grid-stride loop (gridDim.y <= 65535 < J).
 __global__ void __launch_bounds__(256) fill_ensemble_noise_kernel(double* __restrict__ X, long long ld, long long rows,
                                                                   long long cols, long long row_offset, long long col_offset,
                                                                   unsigned long long seed, unsigned long long step) {
@@ -531,14 +527,10 @@ __global__ void __launch_bounds__(256) fill_ensemble_noise_kernel(double* __rest
     const long long j = (long long)(2 * gpair) - col_offset;               // local index of the pair's first column (may be -1)
     if (j >= cols) return;
     for (long long r = blockIdx.y; r < rows; r += gridDim.y) {
-        uint32_t c[4] = {(uint32_t)gpair, TAG_ENS, (uint32_t)(row_offset + r), (uint32_t)step};
-        philox4(c, (uint32_t)seed, (uint32_t)(seed >> 32));
-        const double rad = sqrt(-2.0 * log(u53(c[0], c[1])));
-        double sn, cs;
-        sincospi(2.0 * u53(c[2], c[3]), &sn, &cs);
+        const double2 z = ensemble_noise_pair(seed, step, (unsigned long long)(row_offset + r), gpair);
         double* row = X + (size_t)r * ld;
-        if (j >= 0) row[j] = rad * cs;
-        if (j + 1 < cols) row[j + 1] = rad * sn;
+        if (j >= 0) row[j] = z.x;
+        if (j + 1 < cols) row[j + 1] = z.y;
     }
 }
 int fill_ensemble_noise(cudaStream_t st, double* X, int64_t ld, int64_t rows, int64_t cols, int64_t row_offset,

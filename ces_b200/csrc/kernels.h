@@ -135,6 +135,10 @@ struct SmallStepCall {
     const double *y, *mu, *ustar, *bprior, *ginv_diag, *Ginv, *sinv_diag, *sig_diag, *Sinv, *Sigma0;
     int64_t ldk, ldp;
     double* S;
+    // CES_NOISE_ENSEMBLE (not for eki): xi / ldxi are the J x J xi or NULL, which draws the stream at (seed, step); a run
+    // keys iteration i at step + i
+    bool ensemble;
+    uint64_t seed, step;
 };
 bool small_step_eligible(int64_t p, int64_t k, int64_t J);
 int small_step(cudaStream_t st, const SmallStepCall& c);

@@ -95,6 +95,22 @@ __device__ __forceinline__ void philox_normal_pair(unsigned long long seed, int 
     *z0 = rad * cs;
     if (z1) *z1 = rad * sn;
 }
+// xi of the ensemble noise sqrt(2h / n_C) (U - ubar) xi (J x J; row s: source particle, column j: target particle), the one
+// definition of its elements: Philox4x32-10 keyed by the seed at the counter (j >> 1, TAG_ENS, s, step), whose Box-Muller
+// pair is (xi[s, 2 m], xi[s, 2 m + 1]) for m = j >> 1 -- the cosine for even j, the sine for odd j.  Word 1 carries the
+// tag where fill_normal has the high half of its pair index, so the two streams never share a counter at the same
+// (seed, step).  Drawn by fill_ensemble_noise_kernel (ensemble.cu) and inside the single-CTA kernels (small.cu).
+constexpr uint32_t TAG_ENS = 0x454E;
+__device__ __forceinline__ double2 ensemble_noise_pair(unsigned long long seed, unsigned long long step,
+                                                       unsigned long long s, unsigned long long m) {
+    uint32_t c[4] = {(uint32_t)m, TAG_ENS, (uint32_t)s, (uint32_t)step};
+    philox4(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+    const double rad = sqrt(-2.0 * log(u53(c[0], c[1])));
+    double sn, cs;
+    sincospi(2.0 * u53(c[2], c[3]), &sn, &cs);
+    return make_double2(rad * cs, rad * sn);
+}
+
 // the accept test's uniform of chain c at step it: its own counter (it, c, 0xffffffff, tag)
 __device__ __forceinline__ double philox_accept_uniform(unsigned long long seed, int it, int c, uint32_t tag) {
     uint32_t ctr[4] = {(uint32_t)it, (uint32_t)c, 0xffffffffu, tag};

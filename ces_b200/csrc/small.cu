@@ -5,7 +5,12 @@
 // memory, D never stored -- thread j accumulates its column of V = U~ D while streaming over the particles i
 // (d_ij = e_i . w_j / J), together with the Frobenius sum.  Step size, chol(C^uu) (and the implicit-prior factor for
 // the semi-implicit rule) are computed by thread 0 between two barriers.
+//
+// The noise form is a template parameter ENS of the kernels.  false: the reference's sqrt(2h) chol(C^uu) xi with a p x J
+// xi.  true (CES_NOISE_ENSEMBLE): sqrt(2h / n_C) U~ xi with a J x J xi, read from the caller's matrix or drawn in the
+// kernel from the stream of ces_fill_ensemble_noise; chol(C^uu) is then not formed.
 #include "kernels.h"
+#include "rng.cuh"
 
 namespace ces {
 
@@ -69,6 +74,40 @@ __device__ __forceinline__ void interaction_column_p(const double* Es, const dou
     else interaction_column<KK, 8>(Es, Uts, J, p, w, invJ, v, ssq);
 }
 
+// Column j of the ensemble noise before its scale: n = sum_s U~[:, s] xi[s, j], s in order, P a compile-time trip count as
+// in interaction_column.  xi != nullptr: the caller's J x J matrix (ld ldxi).  Otherwise the Box-Muller pair of (s, j >> 1)
+// (rng.cuh ensemble_noise_pair) is drawn once per step: of threads 2m and 2m + 1, the even one draws the pairs of the even
+// rows s and the odd one those of the odd rows, and each hands its partner the partner's half of the pair by a shuffle.
+// Four rows per trip put two independent draws in flight per thread (a CTA of J threads has few warps to hide the latency
+// of log / sincospi).  Both forms read xi[s, j] in the same order into the same FMAs, so the stream and its fill give
+// bit-identical columns.  Every lane of the CTA must call it (the shuffles); a lane past J gets values nobody reads.
+template <int PP>
+__device__ __forceinline__ void ensemble_noise_column(const double* __restrict__ Uts, int J, int p, int j, const double* xi,
+                                                      long long ldxi, unsigned long long seed, unsigned long long step,
+                                                      double (&n)[SMALL_P_MAX]) {
+    const bool on = j < J, odd = j & 1;
+    for (int s0 = 0; s0 < J; s0 += 4) {
+        double x[4];
+        if (xi) {
+#pragma unroll
+            for (int r = 0; r < 4; ++r) x[r] = (on && s0 + r < J) ? xi[(size_t)(s0 + r) * ldxi + j] : 0.0;
+        } else {
+            const double2 za = ensemble_noise_pair(seed, step, (unsigned long long)(s0 + odd), (unsigned long long)(j >> 1));
+            const double2 zb = ensemble_noise_pair(seed, step, (unsigned long long)(s0 + 2 + odd), (unsigned long long)(j >> 1));
+            const double oa = __shfl_xor_sync(0xffffffffu, odd ? za.x : za.y, 1);
+            const double ob = __shfl_xor_sync(0xffffffffu, odd ? zb.x : zb.y, 1);
+            x[0] = odd ? oa : za.x; x[1] = odd ? za.y : oa;
+            x[2] = odd ? ob : zb.x; x[3] = odd ? zb.y : ob;
+        }
+#pragma unroll
+        for (int r = 0; r < 4; ++r)
+            if (s0 + r < J)
+#pragma unroll
+                for (int q = 0; q < PP; ++q)
+                    if (q < p) n[q] = fma(Uts[q * J + s0 + r], x[r], n[q]);
+    }
+}
+
 __device__ __forceinline__ void block_reduce5(double (&v)[5], double (*scratch)[32], bool take_max4) {
     // sums of v[0..3] (+ v[4]: sum, or max when take_max4); every thread returns the totals
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
@@ -89,7 +128,10 @@ __device__ __forceinline__ void block_reduce5(double (&v)[5], double (*scratch)[
 
 // One update by the whole CTA (one thread per particle).  Every thread of the CTA must call it (barriers inside); it
 // returns with the new column written to a.out and the step scalars in a.S (thread 0), without a trailing barrier.
-__device__ __forceinline__ void small_step_body(const SmallArgs& a, double* sm, double (*scratch)[32]) {
+// ENS: the ensemble noise, xi = a.xi (J x J, ld a.ldxi) or the stream at (seed, step); eki takes ENS = false.
+template <bool ENS>
+__device__ __forceinline__ void small_step_body(const SmallArgs& a, double* sm, double (*scratch)[32], unsigned long long seed,
+                                                unsigned long long step) {
     const int p = a.p, k = a.k, J = a.J;
     double* Es = sm;                    // k x J   E = G - mean
     double* Uts = Es + (size_t)k * J;   // p x J   U~ = U - mean
@@ -98,7 +140,7 @@ __device__ __forceinline__ void small_step_body(const SmallArgs& a, double* sm, 
     double* Ls = Cs + SP * SP;          // p x p   chol(C^uu)
     double* Ms = Ls + SP * SP;          // p x p   chol(Sigma0 + h C)   (eks)
     double* cb = Ms + SP * SP;          // p       C Sigma0^-1 mu       (eks)
-    double* sc = cb + SP;               // scalars: h, sqrt2h
+    double* sc = cb + SP;               // scalars: h, sqrt2h (ENS: sqrt(2h / n_C) in place of sqrt2h)
     const int j = threadIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
     const bool on = j < J;
 
@@ -241,8 +283,14 @@ __device__ __forceinline__ void small_step_body(const SmallArgs& a, double* sm, 
         a.S[S_INFO] = 0.0;
         a.S[S_SSQ] = red[0]; a.S[S_SELF_BIAS] = red[1]; a.S[S_BIAS] = red[2]; a.S[S_SELF_DATA] = red[3]; a.S[S_BIAS_DATA] = red[4];
         a.S[S_MAXDRIFT] = maxdrift; a.S[S_H] = h; a.S[S_SQRT2H] = sc[1]; a.S[S_NEG_H] = -h; a.S[S_H_ALPHA] = h * alphaJ;
-        // chol(C^uu) (:446, :487, :526), and chol(Sigma0 + h C) for the implicit prior step (:443, SURVEY.md F6)
-        for (int pass = 0; pass < ((a.rule == CES_RULE_EKS) ? 2 : 1); ++pass) {
+        if constexpr (ENS) {
+            // sqrt(2h / n_C), n_C of the rule's own C^uu (api.cu ens_inv_nc)
+            const double inv_nc = (a.rule == CES_RULE_EKS) ? 1.0 / (double)J : 1.0 / (double)(J - 1);
+            sc[1] = sqrt(2.0 * h * inv_nc);
+            a.S[S_ENS_ALPHA] = sc[1];
+        }
+        // chol(C^uu) (:446, :487, :526; not with ENS), and chol(Sigma0 + h C) for the implicit prior step (:443, SURVEY.md F6)
+        for (int pass = ENS ? 1 : 0; pass < ((a.rule == CES_RULE_EKS) ? 2 : 1); ++pass) {
             double* Lm = pass == 0 ? Ls : Ms;
             for (int r = 0; r < p; ++r)
                 for (int c = 0; c <= r; ++c) {
@@ -268,18 +316,27 @@ __device__ __forceinline__ void small_step_body(const SmallArgs& a, double* sm, 
             }
     }
     __syncthreads();
+    double noise[SP];
+    if constexpr (ENS) {
+#pragma unroll
+        for (int q = 0; q < SP; ++q) noise[q] = 0.0;
+        if (p <= 2) ensemble_noise_column<2>(Uts, J, p, j, a.xi, a.ldxi, seed, step, noise);
+        else if (p <= 4) ensemble_noise_column<4>(Uts, J, p, j, a.xi, a.ldxi, seed, step, noise);
+        else ensemble_noise_column<8>(Uts, J, p, j, a.xi, a.ldxi, seed, step, noise);
+    }
     if (!on) return;                    // (no barrier follows inside this function)
 
     // ---- assemble U_{n+1}[:, j]
     const double h = sc[0], s2h = sc[1];
-    double noise[SP];
+    if constexpr (!ENS) {
 #pragma unroll
-    for (int q = 0; q < SP; ++q) {
-        double s = 0.0;
-        if (q < p && a.rule != CES_RULE_EKI)
+        for (int q = 0; q < SP; ++q) {
+            double s = 0.0;
+            if (q < p && a.rule != CES_RULE_EKI)
 #pragma unroll
-            for (int n = 0; n < SP; ++n) if (n <= q) s += Ls[q * SP + n] * a.xi[(size_t)n * a.ldxi + j];
-        noise[q] = s;
+                for (int n = 0; n < SP; ++n) if (n <= q) s += Ls[q * SP + n] * a.xi[(size_t)n * a.ldxi + j];
+            noise[q] = s;
+        }
     }
     double o[SP];
     if (a.rule == CES_RULE_ALDI) {
@@ -329,10 +386,11 @@ __device__ __forceinline__ void small_step_body(const SmallArgs& a, double* sm, 
     for (int q = 0; q < SP; ++q) if (q < p) a.out[(size_t)q * a.ldo + j] = o[q];
 }
 
-__global__ void __launch_bounds__(512, 1) small_step_kernel(const SmallArgs a) {
+template <bool ENS>
+__global__ void __launch_bounds__(512, 1) small_step_kernel(const SmallArgs a, unsigned long long seed, unsigned long long step) {
     extern __shared__ double sm[];
     __shared__ double scratch[5][32];
-    small_step_body(a, sm, scratch);
+    small_step_body<ENS>(a, sm, scratch, seed, step);
 }
 
 // ---- the whole sampling.run loop of a small problem in ONE launch (BASELINE config 1: d = 2, k = 10, J = 100, T = 1000).
@@ -354,6 +412,7 @@ struct SmallRunArgs {
     double* Sall;                       // T x S_COUNT
     double* tvec;                       // T cumulative times
     int* nsteps;                        // [0]: updates performed
+    unsigned long long seed, step0;     // ENS without an explicit xi: iteration i draws the stream at (seed, step0 + i)
 };
 
 __device__ __forceinline__ void small_forward(const SmallRunArgs& r, const double* U, double* G, int j) {
@@ -382,6 +441,7 @@ __device__ __forceinline__ void small_forward(const SmallRunArgs& r, const doubl
     }
 }
 
+template <bool ENS>
 __global__ void __launch_bounds__(512, 1) small_run_kernel(const SmallRunArgs r) {
     extern __shared__ double sm[];
     __shared__ double scratch[5][32];
@@ -398,10 +458,10 @@ __global__ void __launch_bounds__(512, 1) small_run_kernel(const SmallRunArgs r)
         if (on) small_forward(r, Ucur, Gcur, j);            // own column: read back by the same thread below
         SmallArgs a = r.base;
         a.U = Ucur; a.ldu = J; a.G = Gcur; a.ldg = J;
-        a.xi = r.Xi ? r.Xi + (size_t)it * p * J : nullptr; a.ldxi = J;
+        if constexpr (!ENS) { a.xi = r.Xi ? r.Xi + (size_t)it * p * J : nullptr; a.ldxi = J; }   // ENS: one J x J xi or NULL
         a.out = r.Utrace + (size_t)(it + 1) * p * J; a.ldo = J;
         a.S = r.Sall + (size_t)it * S_COUNT;
-        small_step_body(a, sm, scratch);
+        small_step_body<ENS>(a, sm, scratch, r.seed, r.step0 + (unsigned long long)it);
         __syncthreads();                                    // every column of slot it + 1 is written, a.S is complete
         if (j == 0) {
             const double h = a.S[S_H];
@@ -421,6 +481,22 @@ bool small_step_eligible(int64_t p, int64_t k, int64_t J) {
     return p <= SMALL_P_MAX && k <= SMALL_K_MAX && J <= 512 && J >= 2;
 }
 
+static size_t small_smem(const SmallStepCall& c) {
+    return ((size_t)(c.k + c.p) * c.J + (SK + SP) + 3 * SP * SP + SP + 8) * sizeof(double);
+}
+
+// Dynamic shared memory above 48 KB for one kernel (each kernel keeps its own setting per device).
+template <auto Kernel>
+static int allow_smem(size_t smem) {
+    static size_t configured_of[kMaxDevices] = {};
+    size_t& configured = configured_of[device_slot()];
+    if (smem > 48 * 1024 && smem > configured) {
+        CES_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        configured = smem;
+    }
+    return CES_OK;
+}
+
 int small_step(cudaStream_t st, const SmallStepCall& c) {
     SmallArgs a;
     a.p = (int)c.p; a.k = (int)c.k; a.J = (int)c.J; a.rule = c.rule; a.ts_kind = c.ts_kind;
@@ -432,14 +508,14 @@ int small_step(cudaStream_t st, const SmallStepCall& c) {
     a.Sinv = c.Sinv; a.Sigma0 = c.Sigma0; a.ldk = c.ldk; a.ldp = c.ldp;
     a.S = c.S;
     const int threads = (int)round_up(c.J, 32);
-    const size_t smem = ((size_t)(c.k + c.p) * c.J + (SK + SP) + 3 * SP * SP + SP + 8) * sizeof(double);
-    static size_t configured_of[kMaxDevices] = {};
-    size_t& configured = configured_of[device_slot()];
-    if (smem > 48 * 1024 && smem > configured) {
-        CES_CUDA(cudaFuncSetAttribute(small_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = smem;
+    const size_t smem = small_smem(c);
+    if (c.ensemble) {
+        CES_TRY(allow_smem<small_step_kernel<true>>(smem));
+        small_step_kernel<true><<<1, threads, smem, st>>>(a, c.seed, c.step);
+    } else {
+        CES_TRY(allow_smem<small_step_kernel<false>>(smem));
+        small_step_kernel<false><<<1, threads, smem, st>>>(a, 0, 0);
     }
-    small_step_kernel<<<1, threads, smem, st>>>(a);
     CES_LAUNCHED(1);
     return CES_OK;
 }
@@ -457,15 +533,17 @@ int small_run(cudaStream_t st, const SmallStepCall& c, const SmallRunCall& rc) {
     r.T = (int)rc.T; r.map_kind = rc.map_kind; r.have_t0 = rc.have_t0; r.t0 = rc.t0; r.t_tol = rc.t_tol;
     r.A = rc.A; r.lda = rc.lda; r.b = rc.b; r.par0 = rc.par0; r.par1 = rc.par1;
     r.Utrace = rc.Utrace; r.Gtrace = rc.Gtrace; r.Xi = rc.Xi; r.Sall = rc.Sall; r.tvec = rc.tvec; r.nsteps = rc.nsteps;
+    r.seed = c.seed; r.step0 = c.step;
     const int threads = (int)round_up(c.J, 32);
-    const size_t smem = ((size_t)(c.k + c.p) * c.J + (SK + SP) + 3 * SP * SP + SP + 8) * sizeof(double);
-    static size_t configured_of[kMaxDevices] = {};
-    size_t& configured = configured_of[device_slot()];
-    if (smem > 48 * 1024 && smem > configured) {
-        CES_CUDA(cudaFuncSetAttribute(small_run_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = smem;
+    const size_t smem = small_smem(c);
+    if (c.ensemble) {
+        a.xi = c.xi; a.ldxi = c.ldxi;   // one J x J xi for every iteration, or NULL (the stream)
+        CES_TRY(allow_smem<small_run_kernel<true>>(smem));
+        small_run_kernel<true><<<1, threads, smem, st>>>(r);
+    } else {
+        CES_TRY(allow_smem<small_run_kernel<false>>(smem));
+        small_run_kernel<false><<<1, threads, smem, st>>>(r);
     }
-    small_run_kernel<<<1, threads, smem, st>>>(r);
     CES_LAUNCHED(1);
     return CES_OK;
 }

@@ -153,7 +153,9 @@ int ces_phase4_update(ces_handle_t h, int rule, int ts_kind, double fixed_h, con
  * (seed, step), exactly as ces_fill_ensemble_noise draws it; otherwise a J_global x cols_local device matrix of this
  * rank's columns (row s = global particle s) with a 16-byte aligned base and an even ldxi >= cols_local (else
  * CES_ERR_ALIGN), which must stay valid until the step's phase 4 has run.  In ensemble mode the xi argument of phase 4,
- * ces_step and ces_step_host is ignored and may be NULL, and the single-kernel path of small problems is not taken.
+ * ces_step and ces_step_host is ignored and may be NULL.  Small problems keep the single-kernel path of ces_step /
+ * ces_step_host up to J = 128 here (p <= 8, k <= 16; the phases are faster above it) and ces_small_run up to J = 512: the
+ * kernel draws the same stream itself, or reads xi_dev, with the same result to the last bit either way.
  * CES_ERR_INVALID for an unknown kind or a NULL handle; ensemble mode with CES_FORM_FACTORED (which never gathers
  * U - ubar) is refused by ces_step, ces_step_host, ces_host_begin and ces_phase3f_products.  No device work. */
 int ces_set_noise(ces_handle_t h, int kind, uint64_t seed, uint64_t step, const double* xi_dev, int64_t ldxi);
@@ -227,7 +229,9 @@ int ces_set_pending_output(ces_handle_t h, double* host_out);
  * e.g. BASELINE config 1: d = 2, k = 10, J = 100, 1000 iterations) with one of the ces.utils maps as forward model, in ONE
  * kernel launch: per iteration the forward map, the update, the cumulative pseudo-time and the stopping rule t > t_tol.
  * U0_host: p x J.  xi_host: T x p x J pre-drawn N(0,1) noise (the caller's numpy stream), or NULL: device noise from
- * (seed, step0 + iteration).  t0 / have_t0: time reached by earlier runs of the same sampler (resume).  Outputs (host):
+ * (seed, step0 + iteration).  With CES_NOISE_ENSEMBLE (ces_set_noise) the noisy rules take the ensemble noise instead:
+ * xi_dev of ces_set_noise at every iteration, or the stream at (its seed, its step + iteration); seed and step0 are then
+ * unused, and a non-NULL xi_host returns CES_ERR_INVALID before any device work.  t0 / have_t0: time reached by earlier runs of the same sampler (resume).  Outputs (host):
  * Utrace (n + 1) x p x J and Gtrace (n + 1) x k x J -- slot i is the ensemble before update i, slot n the final one --,
  * S_host n x 16 step scalars (layout of ces_buffer "scalars"; the four diagnostics are sums over particles), t_host n
  * cumulative times, *nsteps = n <= T updates performed.  A/b as in ces_forward_map (device), params_host its two scalars. */

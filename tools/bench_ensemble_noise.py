@@ -9,6 +9,17 @@ sizes on the full 16 x 16 model (p = 256), the forward solve included.  The card
 in the same process and written with the numbers.
 
     python tools/bench_ensemble_noise.py [--repeats 3] [--steps 3] [--out profiles/r06_bench_ensemble_noise.json]
+
+``--small`` times the single-CTA regime instead: sampling.run(T) of the aldi rule with the lineal map at BASELINE config 1
+(p = 2, k = 10, J = 100) and at p = 8, k = 16, J = 128 ... 512, four arms alternated per repeat -- the Cholesky noise
+in one launch (config 1's path), the ensemble noise in one launch, the ensemble noise through the per-iteration loop
+(``fused_run = False``) on the phases (``CES_NO_SMALL_PATH=1``) and on the one-kernel step.  ms per iteration (wall clock
+around the call, which ends in a synchronisation), launches per run, and the deviation of the one-launch ensemble run from
+the phase loop.  The arms set the J limits of the ensemble noise on the single-CTA path: the one-launch run against the
+phase loop (calibrate.py _FUSED_ENSEMBLE_J_MAX, lifted here), the one-kernel step against the phases (csrc/api.cu
+kSmallEnsembleJMax; above it the last arm takes the phases, as its launch count shows).
+
+    python tools/bench_ensemble_noise.py --small [--repeats 3] [--out profiles/r08_bench_small_ensemble_noise.json]
 """
 import argparse
 import ctypes
@@ -186,14 +197,90 @@ def darcy_rows(repeats, T):
     return rows
 
 
+SMALL_SHAPES = [("cfg1", 2, 10, 100)] + [("p8k16", 8, 16, J) for J in (128, 192, 256, 384, 512)]
+SMALL_ARMS = {"cholesky_fused": dict(fused=True, small=True, kw={}),
+              "ensemble_fused": dict(fused=True, small=True, kw=dict(noise="ensemble", seed=3)),
+              "ensemble_loop_phases": dict(fused=False, small=False, kw=dict(noise="ensemble", seed=3)),
+              "ensemble_loop_small_step": dict(fused=False, small=True, kw=dict(noise="ensemble", seed=3))}
+
+
+def small_problem(name, p, k, J):
+    if name == "cfg1":
+        sys.path.insert(0, ROOT)
+        from bench import cfg1_problem
+
+        pr = cfg1_problem()
+        return pr["A"], pr["ustar"], pr["y"], pr["Gamma"], pr["U0"]
+    rs = np.random.RandomState(1000 * p + J)
+    A = rs.normal(size=(k, p)) / np.sqrt(p)
+    ustar = rs.normal(size=(p, 1))
+    return A, ustar, A @ ustar[:, 0] + 0.1 * rs.normal(size=k), 0.01 * np.eye(k), 3.0 * rs.normal(size=(p, J))
+
+
+def small_rows(repeats, T):
+    from ces_b200 import calibrate, utils
+
+    calibrate._FUSED_ENSEMBLE_J_MAX = 512       # time the one-launch arm at every J, past the limit that it sets too
+    rows = []
+    for name, p, k, J in SMALL_SHAPES:
+        A, ustar, y, Gamma, U0 = small_problem(name, p, k, J)
+        model = utils.lineal(A)
+        samplers = {}
+        for arm, cfg in SMALL_ARMS.items():
+            s = calibrate.sampling(p, k, J)
+            s.ustar, s.mu, s.sigma, s.T, s.fused_run = ustar, np.zeros((p, 1)), 100.0 * np.eye(p), T, cfg["fused"]
+            if not cfg["small"]:
+                os.environ["CES_NO_SMALL_PATH"] = "1"          # read when the handle is created
+            s._get_engine(J)
+            os.environ.pop("CES_NO_SMALL_PATH", None)
+            samplers[arm] = s
+
+        def run(arm):
+            s = samplers[arm]
+            s.metrics = dict((key, []) for key in ("self-bias", "self-bias-data", "bias-data", "bias", "t"))
+            s.Uall, s.Gall = [], []
+            np.random.seed(3)
+            n0 = s._engine.launch_count()
+            t0 = time.perf_counter()
+            s.run(y, U0.copy(), model, Gamma, None, t_tol=1e30, **SMALL_ARMS[arm]["kw"])
+            ms = 1e3 * (time.perf_counter() - t0) / len(s.metrics["t"])
+            return ms, s._engine.launch_count() - n0
+
+        for arm in SMALL_ARMS:
+            run(arm)
+        times, launches = {a: [] for a in SMALL_ARMS}, {}
+        for _ in range(repeats):
+            for arm in SMALL_ARMS:
+                ms, launches[arm] = run(arm)
+                times[arm].append(ms)
+        ref = samplers["ensemble_loop_phases"].Ustar
+        dev = float(np.abs(samplers["ensemble_fused"].Ustar - ref).max() / np.abs(ref).max())
+        mean = {a: float(np.mean(v)) for a, v in times.items()}
+        rec = {"workload": name, "p": p, "k": k, "J": J, "rule": "aldi", "map": "lineal", "iterations_per_run": T,
+               "ms_per_iteration": {a: stats(v) for a, v in times.items()}, "launches_per_run": launches,
+               "ensemble_fused_over_cholesky_fused": mean["ensemble_fused"] / mean["cholesky_fused"],
+               "ensemble_fused_over_loop_phases": mean["ensemble_fused"] / mean["ensemble_loop_phases"],
+               "small_step_over_phases_per_iteration": mean["ensemble_loop_small_step"] / mean["ensemble_loop_phases"],
+               "ensemble_fused_vs_loop_phases_max_rel_dev": dev}
+        print(json.dumps(rec), flush=True)
+        rows.append(rec)
+        for s in samplers.values():
+            s._engine.close()
+            s._engine = None
+    return rows
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--repeats", type=int, default=3)
     ap.add_argument("--steps", type=int, default=3)
     ap.add_argument("--darcy-iterations", type=int, default=20)
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r06_bench_ensemble_noise.json"))
+    ap.add_argument("--out", default=None, help="default: profiles/r06_bench_ensemble_noise.json, "
+                                                "profiles/r08_bench_small_ensemble_noise.json with --small")
     ap.add_argument("--only", default="", help="comma-separated J values of the update workloads (default: all)")
     ap.add_argument("--no-darcy", action="store_true")
+    ap.add_argument("--small", action="store_true", help="the single-CTA regime only (sampling.run of small problems)")
+    ap.add_argument("--small-iterations", type=int, default=1000)
     args = ap.parse_args()
     if args.repeats < 3:
         ap.error("--repeats must be >= 3")
@@ -201,6 +288,15 @@ def main():
 
     if not torch.cuda.is_available():
         raise SystemExit("bench_ensemble_noise needs a CUDA device (sm_100a)")
+    if args.small:
+        out = args.out or os.path.join(ROOT, "profiles", "r08_bench_small_ensemble_noise.json")
+        result = {"card": card(), "repeats": args.repeats, "small": small_rows(args.repeats, args.small_iterations)}
+        result["card_after"] = card()
+        os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
+        with open(out, "w") as fh:
+            json.dump(result, fh, indent=1)
+        print("wrote", out)
+        return
     result = {"card": card(), "repeats": args.repeats, "update": [], "darcy": []}
     only = {int(x) for x in args.only.split(",") if x}
     for name, p, k, J in UPDATE_WORKLOADS:
@@ -209,10 +305,11 @@ def main():
     if not args.no_darcy:
         result["darcy"] = darcy_rows(args.repeats, args.darcy_iterations)
     result["card_after"] = card()
-    os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-    with open(args.out, "w") as fh:
+    out = args.out or os.path.join(ROOT, "profiles", "r06_bench_ensemble_noise.json")
+    os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
+    with open(out, "w") as fh:
         json.dump(result, fh, indent=1)
-    print("wrote", args.out)
+    print("wrote", out)
 
 
 if __name__ == "__main__":
