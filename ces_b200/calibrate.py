@@ -101,6 +101,12 @@ def _consume_model_rng(model, n_particles):
         np.random.normal(0, 1, [int(n_particles), draws])
 
 
+def _save_iteration(where, it, U, G):
+    """The online files of iteration ``it``: ``ensemble_NNNN.npy`` / ``Gensemble_NNNN.npy`` in the directory ``where``."""
+    np.save(where + 'ensemble_' + str(it).zfill(4), U)
+    np.save(where + 'Gensemble_' + str(it).zfill(4), G)
+
+
 class _HostTrace(object):
     """Device -> host copies of the per-iteration ensembles that do not stall the loop (``trace`` / ``save_online`` of
     ``sampling.run``; SURVEY.md section 8f-1).  ``push`` queues an asynchronous copy into fresh page-locked memory on a side
@@ -115,28 +121,35 @@ class _HostTrace(object):
         self.stream = None
         self.items = []
 
-    def push(self, dev_tensor):
+    def push(self, a, reused=False):
+        """``a``: a device tensor, or a host array that is kept as it is.  ``reused``: the caller overwrites the tensor
+        before an asynchronous copy may have completed, so that copy reads a private clone."""
         torch = self.torch
-        if dev_tensor.numel() * dev_tensor.element_size() < self.SMALL:
-            self.items.append((dev_tensor.cpu(), None, None))
-            return len(self.items) - 1
-        if self.stream is None:
-            self.stream = torch.cuda.Stream()
-        host = torch.empty(dev_tensor.shape, dtype=dev_tensor.dtype, pin_memory=True)
-        self.stream.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(self.stream):
-            host.copy_(dev_tensor, non_blocking=True)
-            done = torch.cuda.Event()
-            done.record(self.stream)
-        self.items.append((host, done, dev_tensor))
+        if isinstance(a, np.ndarray):
+            self.items.append((a, None, None))
+        elif a.numel() * a.element_size() < self.SMALL:
+            self.items.append((a.cpu().numpy(), None, None))
+        else:
+            if reused:
+                a = a.clone()
+            if self.stream is None:
+                self.stream = torch.cuda.Stream()
+            host = torch.empty(a.shape, dtype=a.dtype, pin_memory=True)
+            self.stream.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(self.stream):
+                host.copy_(a, non_blocking=True)
+                done = torch.cuda.Event()
+                done.record(self.stream)
+            self.items.append((host, done, a))
         return len(self.items) - 1
 
     def get(self, ticket):
         host, done, _ = self.items[ticket]
         if done is not None:
             done.synchronize()
+            host = host.numpy()
             self.items[ticket] = (host, None, None)
-        return host.numpy()
+        return host
 
 
 class enka(object):
@@ -281,15 +294,17 @@ class enka(object):
             print('There is nothing to save')
             return
         if online:
-            np.save(path + file + 'ensemble_' + str(counter).zfill(4), self.Uall[-1])
-            np.save(path + file + 'Gensemble_' + str(counter).zfill(4), self.Gall[-1])
+            _save_iteration(path + file, counter, self.Uall[-1], self.Gall[-1])
         else:
             np.save(path + file + 'ensemble', self.Ustar)
             np.save(path + file + 'Gensemble', self.Gstar)
             if all:
                 np.save(path + file + 'ensemble_path', self.Uall)
                 np.save(path + file + 'Gensemble_path', self.Gall)
-        with open(path + file + 'metrics.pkl', "wb") as fh:
+        self._save_metrics(path + file)
+
+    def _save_metrics(self, where):
+        with open(where + 'metrics.pkl', "wb") as fh:
             pickle.dump(self.metrics, fh)
 
     def load(self, path='./', eks_dir='ces/', ix_ensemble=False, flag_metrics=False):
@@ -493,10 +508,28 @@ class sampling(enka):
         return True, xi
 
     # ------------------------------------------------------------------ single updates on numpy arrays
-    def _update_host(self, rule, y_obs, U0, Geval, Gamma, kwargs):
+    def _start_step(self, rule, kwargs, noise):
+        """Begin a step of ``rule``: set ``update_rule`` to the reference's name of it and return the keywords of
+        ``Engine.step`` / ``step_host``.  ``noise``: (ensemble?, J x J xi or None) from ``_noise_options``; the ensemble
+        noise is keyed by the step count ``len(self.metrics['t'])``."""
         self.update_rule = _UPDATE_RULE[rule]
+        fixed, resolve = self._step_options(rule, kwargs)     # 'mix' depends on the time reached so far
+        ensemble, xi = noise
+        return dict(fixed_h=fixed, switch=kwargs.get('switch', 1.), resolve=resolve,
+                    formulation=self._option(kwargs, 'formulation'),
+                    noise=('ensemble', int(self._option(kwargs, 'seed')), len(self.metrics['t']), xi) if ensemble else None)
+
+    def _record(self, met, hk, resolve):
+        """A step's metrics and cumulative time; with time_step='spectral' also lambda_max = 1 / hk (ces/calibrate.py:250)."""
+        for key in ('self-bias', 'bias', 'self-bias-data', 'bias-data'):
+            self.metrics[key].append(met[key])
+        self._advance_time(hk)
+        if resolve == 'spectral':
+            self.radspec.append(1. / hk)
+
+    def _update_host(self, rule, y_obs, U0, Geval, Gamma, kwargs):
         self._ensure_metrics()
-        fixed, resolve = self._step_options(rule, kwargs)
+        self._step_options(rule, kwargs)            # validates time_step before any work
         U0 = np.asarray(U0, dtype=np.float64)
         group = getattr(self, 'group', None)
         local = bool(kwargs.get('local_shard', False)) and group is not None
@@ -514,12 +547,10 @@ class sampling(enka):
         stale = self._sync_problem(eng, y_obs, Gamma, defer_large=True)
         Gk = np.asarray(Geval, dtype=np.float64)[:self.n_obs]
         xi = None
-        noise = None
         if ensemble:
             # the J x J xi: this rank's columns of the caller's array, or the device's Philox stream keyed by the step
             if xi_ens is not None and xi_ens.shape[1] == eng.J and eng.cols != eng.J:
                 xi_ens = xi_ens[:, eng.col_lo:eng.col_hi]
-            noise = ('ensemble', int(self._option(kwargs, 'seed')), len(self.metrics['t']), xi_ens)
         elif rule != 'eki':
             # the full (p, J) draw on every rank -- the same global stream as the reference -- unless the caller
             # passes its own (possibly sharded) noise
@@ -533,8 +564,7 @@ class sampling(enka):
                 xi = xi[:, lo:hi]
         elif local and xi is not None and xi.shape[1] == eng.J and eng.J != eng.cols:
             xi = xi[:, eng.col_lo:eng.col_hi]
-        opts = dict(fixed_h=fixed, switch=kwargs.get('switch', 1.), resolve=resolve,
-                    formulation=self._option(kwargs, 'formulation'), noise=noise)
+        opts = self._start_step(rule, kwargs, (ensemble, xi_ens))
         Uk, hk, met = eng.step_host(rule, U0, Gk, xi, **opts)
         if stale is not None and stale():
             # a large problem array was edited in place since the previous call: the device copy has just been
@@ -542,9 +572,7 @@ class sampling(enka):
             Uk, hk, met = eng.step_host(rule, U0, Gk, xi, **opts)
         if eng.nranks > 1 and not local:
             Uk = eng.gather_columns(eng.torch.from_numpy(Uk).cuda(), Uk.shape[0]).cpu().numpy()
-        self._record(met, hk)
-        if resolve == 'spectral':
-            self.radspec.append(1. / hk)            # ces/calibrate.py:250
+        self._record(met, hk, opts['resolve'])
         return Uk
 
     def _draw_noise(self, shape, kwargs):
@@ -552,11 +580,6 @@ class sampling(enka):
         if xi is not None:
             return np.asarray(xi, dtype=np.float64)
         return np.random.normal(0, 1, [shape[0], shape[1]])
-
-    def _record(self, met, hk):
-        for key in ('self-bias', 'bias', 'self-bias-data', 'bias-data'):
-            self.metrics[key].append(met[key])
-        self._advance_time(hk)
 
     def eks_update(self, y_obs, U0, Geval, Gamma, iter, **kwargs):
         """Semi-implicit EKS step (ces/calibrate.py:418-449).
@@ -582,7 +605,48 @@ class sampling(enka):
         return self._update_host('eki', y_obs, U0, Geval, Gamma, kwargs)
 
     # ------------------------------------------------------------------ the run loop
-    def _fused_small_run(self, eng, y_obs, U0, model, rule, kwargs, save_online, trace, device_map):
+    def _ensembles_dir(self, model, tag=''):
+        """``directory/ensembles/<model_name><tag>-JJJJ[-NN]/`` (NN: ``nexp``): ``online_path`` without a tag, and the
+        directory of the online save with the tag ``-eks-LLL`` (LLL: ``model.l_window``)."""
+        return (self.directory + '/ensembles/' + model.model_name + tag + '-' + str(self.J).zfill(4)
+                + ('-' + str(self.nexp).zfill(2) if hasattr(self, 'nexp') else '') + '/')
+
+    def _online_dir(self, model):
+        """The directory of ``run``'s online save, created: the files of ``enka.save(online=True)`` (ces/calibrate.py:371-385;
+        the reference reads ``model.l_window`` there, which its own Darcy model lacks: defaulted to 0)."""
+        where = self._ensembles_dir(model, '-eks-' + str(getattr(model, 'l_window', 0)).zfill(3))
+        try:
+            os.makedirs(where)
+        except OSError:
+            pass
+        return where
+
+    def _end_run(self, model, Us, Gs, U, G):
+        """The results of ``run`` (ces/calibrate.py:404-416) from the final ensemble ``U`` and forward output ``G`` ('pde':
+        the statistics stacked on the final states).  With a trace (``Us`` / ``Gs``: each iteration's ensemble and output
+        before its update; None without), ``Uall`` / ``Gall`` continue those of an earlier run and end with U / G."""
+        if Us is not None:
+            self.Uall = np.asarray(list(getattr(self, 'Uall', [])) + list(Us) + [U])
+            self.Gall = np.asarray(list(getattr(self, 'Gall', [])) + list(Gs) + [G])
+        self.Ustar = U
+        self.Gstar = G[:self.n_obs, :]
+        self.online_path = self._ensembles_dir(model)
+
+    def _carry_state(self, ws_pool, W_end, final):
+        """The next initial states ``W0`` of a 'pde' model (ces/calibrate.py:317-327, 390-396): a draw from the ``ws`` pool,
+        appended to ``Wall`` except after the final pass; without a pool, the final states ``W_end`` of the pass (a host
+        array, or None while they are kept on the device only).  Returns True when the final states carry over."""
+        if ws_pool is not None:
+            widx = np.random.randint(ws_pool.shape[0], size=self.J)
+            if not final:
+                self.Wall.append(widx)
+            self.W0 = ws_pool[widx].T
+            return False
+        if W_end is not None:
+            self.W0 = np.copy(W_end)
+        return True
+
+    def _fused_small_run(self, eng, U0, model, rule, kwargs, first, noise, save_online, trace):
         """The whole loop in ONE kernel launch (``ces_small_run``) when the problem fits a single CTA (p <= 8, k <= 16,
         J <= 512 -- BASELINE config 1) and the forward model is one of the ``ces_b200.utils`` maps: forward, update,
         cumulative time and the ``t_tol`` stopping rule run back to back on the device, the trace is the chain of
@@ -590,18 +654,18 @@ class sampling(enka):
         iteration loop below (same arithmetic per step; the noise is the numpy stream the reference would consume: all T
         draws are taken in one call and the generator is rewound to where an early stop leaves it).  ``noise='ensemble'``
         runs here too up to J = _FUSED_ENSEMBLE_J_MAX: the kernel draws the device stream keyed by ``seed`` at step
-        ``len(self.metrics['t']) + i``, or reads the one (J, J) ``xi``, as the general loop does.  Returns False when the
-        configuration needs the general loop."""
+        ``len(self.metrics['t']) + i``, or reads the one (J, J) ``xi``, as the general loop does.  ``first``: the
+        ``_step_options`` of the first step, ``noise``: the ``_noise_options``.  Returns False when the configuration
+        needs the general loop."""
         import ctypes
 
         from . import _lib
 
         kind = getattr(model, 'device_kind', None)
-        ensemble, xi_ens = self._noise_options(rule, kwargs, eng.J)
-        if not (device_map and eng.nranks == 1 and kind in _lib.MAPS and self.p <= 8 and self.n_obs <= 16
+        ensemble = noise[0]
+        if not (eng.nranks == 1 and kind in _lib.MAPS and self.p <= 8 and self.n_obs <= 16
                 and 2 <= eng.J <= (_FUSED_ENSEMBLE_J_MAX if ensemble else 512) and self.T >= 1
-                and self._step_options(rule, kwargs) == (None, None)
-                and self._option(kwargs, 'formulation') == 'interaction'
+                and first == (None, None) and self._option(kwargs, 'formulation') == 'interaction'
                 and getattr(self, 'fused_run', True) and (ensemble or kwargs.get('xi', None) is None)):
             return False
         p, k, J, T = self.p, self.n_obs, eng.J, int(self.T)
@@ -628,10 +692,11 @@ class sampling(enka):
         S = np.empty((T, 16))
         tv = np.empty(T)
         n = ctypes.c_int64()
+        opts = self._start_step(rule, kwargs, noise)
         with eng.on_stream():
-            eng._apply_noise(('ensemble', int(self._option(kwargs, 'seed')), len(t_hist), xi_ens) if ensemble else None)
+            eng._apply_noise(opts['noise'])
             _lib.check(eng.lib.ces_small_run(
-                eng.h, _lib.RULES[rule], _lib.TS_FROBENIUS, 0.0, float(kwargs.get('switch', 1.)), _lib.MAPS[kind],
+                eng.h, _lib.RULES[rule], _lib.TS_FROBENIUS, 0.0, float(opts['switch']), _lib.MAPS[kind],
                 ctypes.c_void_p(A_dev.data_ptr()) if A_dev is not None else None, int(lda),
                 ctypes.c_void_p(b_dev.data_ptr()) if b_dev is not None else None,
                 _lib.host_ptr(par) if par is not None else None, _lib.host_ptr(U0),
@@ -646,32 +711,16 @@ class sampling(enka):
                 np.random.normal(0, 1, [n, fdraws + (p * J if host_noise else 0)])
             if fdraws:
                 np.random.normal(0, 1, fdraws)                   # the final forward pass
-        self.update_rule = _UPDATE_RULE[rule]
         # step scalars -> metrics (sums over particles / J), cumulative times
         for name, col in (('self-bias', 1), ('bias', 2), ('self-bias-data', 3), ('bias-data', 4)):
             self.metrics[name].extend((S[:n, col] / J).tolist())
         self.metrics['t'].extend(tv[:n].tolist())
         if save_online:
-            tag = model.model_name + '-eks-' + str(getattr(model, 'l_window', 0)).zfill(3) + '-' + str(self.J).zfill(4)
-            if hasattr(self, 'nexp'):
-                tag += '-' + str(self.nexp).zfill(2)
-            where = self.directory + '/ensembles/' + tag + '/'
-            try:
-                os.makedirs(where)
-            except OSError:
-                pass
+            where = self._online_dir(model)
             for it in range(n):
-                np.save(where + 'ensemble_' + str(it).zfill(4), Ut[it])
-                np.save(where + 'Gensemble_' + str(it).zfill(4), Gt[it])
-            with open(where + 'metrics.pkl', "wb") as fh:
-                pickle.dump(self.metrics, fh)
-        if trace:
-            self.Uall = np.asarray(list(getattr(self, 'Uall', [])) + list(Ut[:n + 1]))
-            self.Gall = np.array(list(getattr(self, 'Gall', [])) + list(Gt[:n + 1]))
-        self.Ustar = Ut[n].copy()
-        self.Gstar = Gt[n].copy()
-        tail = '-' + str(self.J).zfill(4) + ('-' + str(self.nexp).zfill(2) if hasattr(self, 'nexp') else '') + '/'
-        self.online_path = self.directory + '/ensembles/' + model.model_name + tail
+                _save_iteration(where, it, Ut[it], Gt[it])
+            self._save_metrics(where)
+        self._end_run(model, Ut[:n] if trace else None, Gt[:n] if trace else None, Ut[n].copy(), Gt[n].copy())
         return True
 
     def run(self, y_obs, U0, model, Gamma, Jnoise, save_online=False, trace=True, **kwargs):
@@ -692,7 +741,7 @@ class sampling(enka):
             raise ValueError("model.type must be 'map' or 'pde'")
         is_pde = (mtype == 'pde')
         self._ensure_metrics()
-        self._step_options(rule, kwargs)            # validates time_step before any work
+        first = self._step_options(rule, kwargs)            # validates time_step before any work
         group = getattr(self, 'group', None)
 
         U0 = np.ascontiguousarray(U0, dtype=np.float64)
@@ -702,185 +751,106 @@ class sampling(enka):
         self._sync_problem(eng, y_obs, Gamma)
         lo, hi = eng.col_lo, eng.col_hi
         dev = torch.device("cuda", torch.cuda.current_device())
-
-        if trace:
-            self.Uall = list(getattr(self, 'Uall', []))
-            self.Gall = list(getattr(self, 'Gall', []))
-        self._ensure_metrics()
         known = rule in _UPDATE_RULE
-
         device_model = (not is_pde) and self._is_device_model(model)
-        if self._fused_small_run(eng, y_obs, U0, model, rule, kwargs, save_online, trace, known and device_model):
+        if known and device_model and self._fused_small_run(eng, U0, model, rule, kwargs, first, (ensemble, xi_ens),
+                                                            save_online, trace):
             return
+
         U_dev = torch.from_numpy(U0[:, lo:hi].copy()).to(dev)
         if xi_ens is not None:
             xi_ens = torch.from_numpy(np.ascontiguousarray(xi_ens[:, lo:hi])).to(dev)     # the same xi every iteration
+        G_dev = torch.empty(self.n_obs, hi - lo, dtype=torch.float64, device=dev)
         if is_pde:
             # initial conditions of the integrator, one per particle (ces/calibrate.py:317-327)
-            t_ode, ws_pool = kwargs.get('t', None), kwargs.get('ws', None)
+            t_ode, ws_pool, update_wt = kwargs.get('t', None), kwargs.get('ws', None), kwargs.get('update_wt', True)
             if ws_pool is not None:
-                widx = np.random.randint(ws_pool.shape[0], size=self.J)
-                self.W0 = ws_pool[widx].T
-                self.Wall = [widx]
+                self.Wall = []
+                self._carry_state(ws_pool, None, final=False)
             else:
                 self.W0 = np.tile(kwargs.get('wt', None), self.J).reshape(self.J, model.n_state).T
-        G_dev = torch.empty(self.n_obs, hi - lo, dtype=torch.float64, device=dev)
-
         device_pde = is_pde and getattr(model, 'device_kind', None) is not None and hasattr(model, 'evaluate_ensemble_pde')
-        pde_state = {}
-
-        def forward_pde_device(U_dev, final):
-            """The same protocol with the ensemble integrated on the device (ces_b200.utils Lorenz models): statistics
-            into G_dev, final states into a device buffer that becomes the next W0 (:390-396) without touching the host;
-            the (n_obs + n_state, J) host array of the reference is assembled only when the trace or the result needs it."""
-            if 'W0' not in pde_state or ws_pool is not None:
-                pde_state['W0'] = torch.from_numpy(np.ascontiguousarray(self.W0[:, lo:hi])).to(dev)
-                pde_state['Wend'] = torch.empty_like(pde_state['W0'])
-            model.evaluate_ensemble_pde(eng, U_dev, pde_state['W0'], t_ode, G_dev, pde_state['Wend'])
-            G_full = None
-            if trace or final:
-                G_full = np.vstack([gather_host(G_dev, self.n_obs), gather_host(pde_state['Wend'], model.n_state)])
-            if kwargs.get('update_wt', True):
-                if ws_pool is not None:
-                    widx = np.random.randint(ws_pool.shape[0], size=self.J)
-                    if not final:
-                        self.Wall.append(widx)
-                    self.W0 = ws_pool[widx].T
-                else:
-                    pde_state['W0'], pde_state['Wend'] = pde_state['Wend'], pde_state['W0']
-                    if G_full is not None:
-                        self.W0 = np.copy(G_full[self.n_obs:, :])
-            return G_dev, G_full
-
-        def forward_pde(U_dev, final):
-            """Statistics + carried-over state (ces/calibrate.py:342-350, 390-396): the user's integrator on the host for
-            this rank's particles; the full (n_obs + n_state, J) array is needed on every rank for the next W0."""
-            if device_pde:
-                return forward_pde_device(U_dev, final)
-            U_loc = U_dev.cpu().numpy()
-            G_loc = self.G_pde_ens(np.vstack([U_loc, self.W0[:, lo:hi]]), model, t_ode)
-            if eng.nranks > 1:
-                G_full = gather_host(torch.from_numpy(np.ascontiguousarray(G_loc)).to(dev), G_loc.shape[0])
-            else:
-                G_full = G_loc
-            if kwargs.get('update_wt', True):
-                if ws_pool is not None:
-                    widx = np.random.randint(ws_pool.shape[0], size=self.J)
-                    if not final:
-                        self.Wall.append(widx)
-                    self.W0 = ws_pool[widx].T
-                else:
-                    self.W0 = np.copy(G_full[self.n_obs:, :])
-            G_dev.copy_(torch.from_numpy(np.ascontiguousarray(G_full[:self.n_obs, lo:hi])))
-            return G_dev, G_full
-
-        def forward(U_dev, final=False):
-            if is_pde:
-                return forward_pde(U_dev, final)
-            if device_model:
-                model.evaluate_ensemble(eng, U_dev, G_dev)
-                _consume_model_rng(model, J)                # (every rank: the stream is global)
-                return G_dev, None
-            G_host = self._host_G_ens(U_dev.cpu().numpy(), model)
-            G_dev.copy_(torch.from_numpy(np.ascontiguousarray(G_host[:self.n_obs])))
-            return G_dev, G_host
-
-        def gather_dev(local, rows, private=True):
-            """Full (rows, J) DEVICE tensor from the column shards; single GPU: the tensor itself, or a private copy when
-            the caller will overwrite it before an asynchronous reader is done (the forward-output buffer)."""
-            if eng.nranks == 1 and private and local.numel() * 8 >= _HostTrace.SMALL:
-                return local.clone()
-            return eng.gather_columns(local, rows)
+        W_dev = []                      # device 'pde' models: this rank's [W0, final states] in HBM
 
         def gather_host(local, rows):
             """Full (rows, J) host array from the column shards (synchronous)."""
-            return gather_dev(local, rows, private=False).cpu().numpy()
+            return eng.gather_columns(local, rows).cpu().numpy()
+
+        def forward(U_dev, final=False):
+            """G(U_dev) into G_dev (ces/calibrate.py:342-352, 390-396).  Returns the full host array of the outputs when
+            the pass has one, else None: a host map's on a single GPU; a 'pde' model's statistics stacked on the final
+            states, which the device integrators assemble on the host only for the trace or the final pass."""
+            if not is_pde:
+                if device_model:
+                    model.evaluate_ensemble(eng, U_dev, G_dev)
+                    _consume_model_rng(model, J)                # (every rank: the stream is global)
+                    return None
+                G_host = self._host_G_ens(U_dev.cpu().numpy(), model)
+                G_dev.copy_(torch.from_numpy(np.ascontiguousarray(G_host[:self.n_obs])))
+                return G_host if eng.nranks == 1 else None      # several ranks: this rank's columns only
+            if device_pde:
+                # the ces_b200.utils Lorenz models: the ensemble integrated on the device
+                if not W_dev or ws_pool is not None:
+                    W0 = torch.from_numpy(np.ascontiguousarray(self.W0[:, lo:hi])).to(dev)
+                    W_dev[:] = [W0, torch.empty_like(W0)]
+                model.evaluate_ensemble_pde(eng, U_dev, W_dev[0], t_ode, G_dev, W_dev[1])
+                G_full = None
+                if trace or final:
+                    G_full = np.vstack([gather_host(G_dev, self.n_obs), gather_host(W_dev[1], model.n_state)])
+            else:
+                # the user's integrator on the host for this rank's particles; every rank needs the full array (next W0)
+                G_full = self.G_pde_ens(np.vstack([U_dev.cpu().numpy(), self.W0[:, lo:hi]]), model, t_ode)
+                if eng.nranks > 1:
+                    G_full = gather_host(torch.from_numpy(np.ascontiguousarray(G_full)).to(dev), G_full.shape[0])
+                G_dev.copy_(torch.from_numpy(np.ascontiguousarray(G_full[:self.n_obs, lo:hi])))
+            if update_wt:
+                carried = self._carry_state(ws_pool, None if G_full is None else G_full[self.n_obs:], final)
+                if carried and device_pde:
+                    W_dev.reverse()                     # the final states become the next W0 without leaving HBM
+            return G_full
 
         # trace / save_online: asynchronous device->host copies into page-locked memory (no stall of the loop); the
         # arrays of iteration i are materialised when iteration i + 1 has been queued (online save) or after the loop
         host_trace = _HostTrace(torch) if (trace or save_online) else None
-        tickets = []                    # per iteration: (U ticket | array, G ticket | array)
-        saved_upto = [0]
-
-        def flush_online(upto):
-            """np.save the iterations [saved_upto, upto) whose copies were queued earlier (ces/calibrate.py:371-385)."""
-            if not (save_online and eng.rank == 0):
-                return
-            tag = model.model_name + '-eks-' + str(getattr(model, 'l_window', 0)).zfill(3) + '-' + str(self.J).zfill(4)
-            if hasattr(self, 'nexp'):
-                tag += '-' + str(self.nexp).zfill(2)
-            where = self.directory + '/ensembles/' + tag + '/'
-            try:
-                os.makedirs(where)
-            except OSError:
-                pass
-            for it in range(saved_upto[0], upto):
-                tu, tg = tickets[it]
-                Uh = host_trace.get(tu) if isinstance(tu, int) else tu
-                Gh = host_trace.get(tg) if isinstance(tg, int) else tg
-                np.save(where + 'ensemble_' + str(it).zfill(4), Uh)
-                np.save(where + 'Gensemble_' + str(it).zfill(4), Gh)
-            saved_upto[0] = max(saved_upto[0], upto)
-
+        tickets = []                    # per iteration: (U ticket, G ticket)
+        online = save_online and eng.rank == 0
+        device_rng = self._option(kwargs, 'rng') == 'device'
         for i in range(self.T):
-            G_cur, G_host = forward(U_dev)
+            G_host = forward(U_dev)
             if host_trace is not None:
-                tu = host_trace.push(gather_dev(U_dev, self.p, private=False))     # every update returns a new tensor
-                tg = (G_host if (G_host is not None and (eng.nranks == 1 or is_pde))
-                      else host_trace.push(gather_dev(G_cur, self.n_obs)))
-                tickets.append((tu, tg))
+                tu = host_trace.push(eng.gather_columns(U_dev, self.p))        # every update returns a new tensor
+                G_i = G_host if G_host is not None else eng.gather_columns(G_dev, self.n_obs)
+                tickets.append((tu, host_trace.push(G_i, reused=G_i is G_dev)))
             if known:
-                self.update_rule = _UPDATE_RULE[rule]
-                xi_dev, noise = None, None
-                if ensemble:
-                    noise = ('ensemble', int(self._option(kwargs, 'seed')), len(self.metrics['t']), xi_ens)
-                elif rule != 'eki':
-                    if self._option(kwargs, 'rng') == 'device':
+                opts = self._start_step(rule, kwargs, (ensemble, xi_ens))
+                xi_dev = None
+                if not ensemble and rule != 'eki':
+                    if device_rng:
                         # production mode: Philox noise generated on the device, nothing crosses PCIe
                         xi_dev = eng.normal_noise(self.p, self._option(kwargs, 'seed'), len(self.metrics['t']))
                     else:
                         xi = self._draw_noise((self.p, J), kwargs)      # same stream on every rank
                         xi_dev = torch.from_numpy(np.ascontiguousarray(xi[:, lo:hi])).to(dev)
-                fixed, resolve = self._step_options(rule, kwargs)     # 'mix' depends on the time reached so far
-                U_dev, hk, met = eng.step(rule, U_dev, G_cur, xi_dev, fixed_h=fixed, switch=kwargs.get('switch', 1.),
-                                          resolve=resolve, noise=noise, formulation=self._option(kwargs, 'formulation'))
-                self._record(met, hk)
-                if resolve == 'spectral':
-                    self.radspec.append(1. / hk)
+                U_dev, hk, met = eng.step(rule, U_dev, G_dev, xi_dev, **opts)
+                self._record(met, hk, opts['resolve'])
             # an unknown ``update`` leaves the ensemble unchanged and records nothing, like :364-369 --
             # the reference then fails on the empty ``metrics['t']``; so do we
-            if save_online:
-                # same files as enka.save(online=True, counter=i) (:371-385; the reference reads model.l_window there,
-                # which its own Darcy model lacks: defaulted to 0).  Iteration i - 1 is written now, while iteration i's
-                # copies are still in flight; metrics.pkl follows the latest completed update like the reference's
-                flush_online(i)
-                if eng.rank == 0:
-                    tag = model.model_name + '-eks-' + str(getattr(model, 'l_window', 0)).zfill(3) + '-' + str(self.J).zfill(4)
-                    if hasattr(self, 'nexp'):
-                        tag += '-' + str(self.nexp).zfill(2)
-                    try:
-                        os.makedirs(self.directory + '/ensembles/' + tag + '/')
-                    except OSError:
-                        pass
-                    with open(self.directory + '/ensembles/' + tag + '/metrics.pkl', "wb") as fh:
-                        pickle.dump(self.metrics, fh)
+            if online:
+                # iteration i - 1's files are written now, while iteration i's copies are still in flight; metrics.pkl
+                # follows the latest completed update like the reference's
+                where = self._online_dir(model)
+                if i:
+                    _save_iteration(where, i - 1, *map(host_trace.get, tickets[i - 1]))
+                self._save_metrics(where)
             if self.metrics['t'][-1] > kwargs.get('t_tol', 2.):
                 break
-        flush_online(len(tickets))
-        if trace:
-            for tu, tg in tickets:
-                self.Uall.append(host_trace.get(tu) if isinstance(tu, int) else tu)
-                self.Gall.append(host_trace.get(tg) if isinstance(tg, int) else tg)
+        if online:
+            where = self._online_dir(model)
+            if tickets:
+                _save_iteration(where, len(tickets) - 1, *map(host_trace.get, tickets[-1]))
+        Us = [host_trace.get(tu) for tu, _ in tickets] if trace else None
+        Gs = [host_trace.get(tg) for _, tg in tickets] if trace else None
 
-        G_cur, G_host = forward(U_dev, final=True)
-        U_fin = gather_host(U_dev, self.p)
-        G_fin = G_host if (G_host is not None and (eng.nranks == 1 or is_pde)) else gather_host(G_cur, self.n_obs)
-        if trace:
-            self.Uall.append(U_fin)
-            self.Gall.append(G_fin)
-            self.Uall = np.asarray(self.Uall)
-            self.Gall = np.array(self.Gall)
-        self.Ustar = U_fin
-        self.Gstar = G_fin[:self.n_obs, :]
-        tail = '-' + str(self.J).zfill(4) + ('-' + str(self.nexp).zfill(2) if hasattr(self, 'nexp') else '') + '/'
-        self.online_path = self.directory + '/ensembles/' + model.model_name + tail
+        G_host = forward(U_dev, final=True)
+        self._end_run(model, Us, Gs, gather_host(U_dev, self.p),
+                      G_host if G_host is not None else gather_host(G_dev, self.n_obs))
